@@ -65,7 +65,34 @@ def parse():
     ap.add_argument("--no-path", action="store_true", help="N > 1: skip the frame-parallel camera-path sub-record")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-ref-cuda", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the frame of the last timed step to DIR/frame.npy (see dump_frame), "
+                         "so that two builds can be compared output for output on the same inputs")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.warmup < 0:
+        ap.error("--warmup must not be negative")
+    if args.dump_outputs and (args.impl, args.workload) != ("ours", "frame"):
+        ap.error("--dump-outputs needs --impl ours --workload frame")
+    return args
+
+
+DUMP_MAX_PIXELS = 1 << 21      # 2 Mi pixels x 4 channels x float32 = 32 MiB
+
+
+def dump_frame(directory: str, frame) -> None:
+    """DIR/frame.npy: the RGBA8 bytes of `frame` ([h, w, 4] uint8) as float32 -- the whole frame, shape [h, w, 4], or for
+    a frame of more than DUMP_MAX_PIXELS pixels (the 4K frame has 8.3 M) that many pixels drawn with a fixed seed, shape
+    [n, 4], with their row-major indices y * w + x in DIR/frame_pixel_index.npy (float64, exact), the same on every run."""
+    import numpy as np
+    px = frame.cpu().numpy()
+    os.makedirs(directory, exist_ok=True)
+    if px.shape[0] * px.shape[1] > DUMP_MAX_PIXELS:
+        idx = np.sort(np.random.Generator(np.random.PCG64(0)).choice(px.shape[0] * px.shape[1], DUMP_MAX_PIXELS, replace=False))
+        px = px.reshape(-1, 4)[idx]
+        np.save(os.path.join(directory, "frame_pixel_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(directory, "frame.npy"), px.astype(np.float32))
 
 
 # ------------------------------------------------------------------------------------------------------
@@ -519,6 +546,8 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_frame(args.dump_outputs, pipe_dev.last_frame())     # the headline's device-resident frames; pipe_host has its own
 
     # ---- roofline of the dominant kernel (render_kernel): FP32 FMA pipe -------------------------------
     traffic = {"bytes": None, "source": "no ncu capture for this workload (see profiles/)"}

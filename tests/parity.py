@@ -5,6 +5,10 @@
   pixels whose class agrees and is not captured; tolerance 1e-5 rad (north_star)
 * linear RGB: |dc| / max(|c_ref|, 1e-3) per channel on final_hdr with effects off; tolerance 1e-3 (north_star)
 """
+import hashlib
+import json
+import os
+
 import numpy as np
 
 DIR_TOL_RAD = 1e-5
@@ -57,3 +61,24 @@ def census(ref, new):
         "rgb_p999_rel": float(np.quantile(pix, 0.999)),
         "rgb_frac_over_tol": float(np.mean(pix > RGB_TOL_REL)),
     }
+
+
+# Where the reference's own CUDA builds (oracle/_ref) are absent, the GPU tests that compare with them check the exact
+# part of that comparison: the arrays those tests require to be bit-identical to the reference's, against sha256 digests
+# of the reference's arrays committed in tests/golden/reference_exact_digests.json (tests/tools/make_reference_digests.py
+# writes them from the reference builds, after running the tests' own checks against those builds).  The parts compared
+# within a tolerance (touched pixels, probe quantiles) are checked only where the reference builds are present.
+REFERENCE_DIGESTS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_exact_digests.json")
+
+
+def digests(arrays):
+    """sha256 of the bytes (C order) of each array of a dict."""
+    return {k: hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest() for k, a in arrays.items()}
+
+
+def assert_reference_digests(key, parts):
+    with open(REFERENCE_DIGESTS) as f:
+        want = json.load(f)[key]
+    got = digests(parts)
+    assert sorted(got) == sorted(want), key
+    assert got == want, f"{key}: {sorted(k for k in want if got[k] != want[k])} differ from the reference's"

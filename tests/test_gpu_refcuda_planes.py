@@ -16,7 +16,7 @@ import numpy as np
 import pytest
 
 from inputs import disk_points, phase_space
-from parity import CAMERAS, DIR_TOL_RAD, RGB_TOL_REL, census
+from parity import CAMERAS, DIR_TOL_RAD, RGB_TOL_REL, assert_reference_digests, census
 
 pytestmark = pytest.mark.gpu
 
@@ -40,6 +40,22 @@ def refcuda():
 
 
 @pytest.fixture(scope="module")
+def refcuda_pair():
+    """(instrumented, plain) builds of the reference's CUDA kernel, or None where they are not built: the tests then check
+    the exact part of their comparison against committed digests of the reference's arrays (tests/parity.py)."""
+    from oracle import RefCuda, RefCudaPlanes
+    return (RefCudaPlanes(), RefCuda()) if RefCudaPlanes.available() and RefCuda.available() else None
+
+
+@pytest.fixture(scope="module")
+def host_headers(ora):
+    """The reference headers compiled for a host (oracle/_ref/libref_host.so) where built, else the oracle port, which
+    tests/test_oracle_golden.py holds bit for bit to golden vectors generated from those headers."""
+    from oracle import Oracle, available
+    return Oracle("reference", auto_build=False) if available("reference") else ora
+
+
+@pytest.fixture(scope="module")
 def sky_big():
     import relativisticraytracer_b200 as rrt
     return rrt.procedural_sky(4096, 2048)
@@ -56,6 +72,61 @@ def _ours(gpu, sky_np, cam, spin, flags, w, h, fx):
     g["rgba"] = out.cpu().numpy()
     sky.close()
     return g
+
+
+def fmad_planes_case(gpu, sky_np, cam, spin, w=480, h=270):
+    import relativisticraytracer_b200 as rrt
+    return f"fmad_planes/{cam}/{spin}/{w}x{h}", _ours(gpu, sky_np, cam, spin, 3 | FMAD, w, h, rrt.effects_off())
+
+
+def full_size_case(gpu, sky_np, w, h, cam):
+    """effects off (planes) and reference default effects (the frame as the viewer shows it), a = 0.99"""
+    import relativisticraytracer_b200 as rrt
+    g = _ours(gpu, sky_np, cam, 0.99, 3 | FMAD, w, h, rrt.effects_off())
+    gd = _ours(gpu, sky_np, cam, 0.99, 3 | FMAD, w, h, rrt.default_effects())
+    return f"fmad_full_size/{cam}/{w}x{h}", dict(g, fxd_rgba=gd["rgba"], fxd_cls=gd["cls"])
+
+
+def media_probes_case(gpu, spin):
+    import relativisticraytracer_b200 as rrt
+    prm = rrt.default_params(spin_a=spin, flags=3 | FMAD)
+    pts = disk_points(seed=31, n=1 << 15)
+    q, v = phase_space(seed=32, n=1 << 15)
+    r = np.linalg.norm(q, axis=1).astype(np.float32)
+    return f"fmad_media_probes/{spin}", {
+        "disk_density": gpu.disk_density(prm, pts, 1.0), "dust_density": gpu.dust_density(prm, pts, 1.0),
+        "redshift": gpu.redshift(prm, q, v), "disk_temperature": gpu.disk_temperature(prm, r)}
+
+
+# The exact parts of each comparison below: arrays that must be bit-identical between our build and the reference's,
+# formed the same way from either side (ours, or the reference's planes + plain frame), with OUR touched mask where the
+# check is restricted to untouched pixels.  tests/tools/make_reference_digests.py digests them from the reference side.
+def planes_exact(src, rgba, touched):
+    """class, step count, exit velocity and position on every pixel; final_hdr and the 8-bit frame (rows flipped to
+    [y][x]) on every pixel whose ray touched no medium"""
+    import relativisticraytracer_b200 as rrt
+    return {"cls": np.ascontiguousarray(src["cls"] & rrt.CLS_MASK, dtype=np.uint8),
+            "steps": np.ascontiguousarray(src["steps"], dtype=np.int32),
+            "vel": _bits(src["vel"][..., :3]), "pos": _bits(src["pos"][..., :3]),
+            "hdr_untouched": _bits(src["hdr"][..., :3])[~touched],
+            "rgba_untouched": np.ascontiguousarray(rgba[::-1][~touched], dtype=np.uint8)}
+
+
+def touched_of(cls):
+    import relativisticraytracer_b200 as rrt
+    return (cls & rrt.CLSF_TOUCHED) != 0
+
+
+def full_size_exact(src, rgba, rgba_default_fx, touched, touched_default_fx):
+    return dict(planes_exact(src, rgba, touched),
+                fxd_rgba_untouched=np.ascontiguousarray(rgba_default_fx[::-1][~touched_default_fx], dtype=np.uint8))
+
+
+def probes_exact(disk, dust, temperature):
+    """zero / non-zero pattern of the densities away from the radius gates, disk temperature bit for bit"""
+    ok = _away_from_gates(disk_points(seed=31, n=1 << 15))
+    return {"disk_density_zero": np.asarray(disk)[ok] == 0.0, "dust_density_zero": np.asarray(dust)[ok] == 0.0,
+            "disk_temperature": _bits(temperature)}
 
 
 def _bits(a):
@@ -106,40 +177,49 @@ def test_instrumentation_does_not_change_the_reference_kernel(gpu, refp, refcuda
 
 @pytest.mark.parametrize("cam", ["C0", "C1", "C2", "C3"])
 @pytest.mark.parametrize("spin", [0.0, 0.99])
-def test_fmad_planes_equal_reference_cuda_arithmetic(gpu, refp, refcuda, sky_small, cam, spin):
+def test_fmad_planes_equal_reference_cuda_arithmetic(gpu, refcuda_pair, sky_small, cam, spin):
     import relativisticraytracer_b200 as rrt
     w, h = 480, 270
+    key, g = fmad_planes_case(gpu, sky_small, cam, spin, w, h)
+    if refcuda_pair is None:
+        assert_reference_digests(key, planes_exact(g, g["rgba"], touched_of(g["cls"])))
+        return
+    refp, refcuda = refcuda_pair
     cg, fx = rrt.camera_state_from(*CAMERAS[cam]), rrt.effects_off()
     plain, _, _ = refcuda.render(spin, cg, fx, sky_small, 1.0, w, h)
     P = refp.render(spin, cg, fx, sky_small, 1.0, w, h)
-    g = _ours(gpu, sky_small, cam, spin, 3 | FMAD, w, h, fx)
     _check_fmad_against_reference_cuda(g, P, plain, f"{cam} a={spin} {w}x{h}")
 
 
 @pytest.mark.parametrize("w,h,cam", [(1920, 1080, "C0"), (1920, 1080, "C1"), (3840, 2160, "C0")])
-def test_fmad_full_size_frames_equal_reference_cuda(gpu, refp, refcuda, sky_big, w, h, cam):
+def test_fmad_full_size_frames_equal_reference_cuda(gpu, refcuda_pair, sky_big, w, h, cam):
     """BASELINE configs 3 (1080p disk + dust) and 4 (the 4K bench frame), a = 0.99, against the reference's own kernel on
     the same GPU: planes at float precision and the 8-bit frame with the reference's default effects."""
     import relativisticraytracer_b200 as rrt
+    key, g = full_size_case(gpu, sky_big, w, h, cam)
+    if refcuda_pair is None:
+        assert_reference_digests(key, full_size_exact(g, g["rgba"], g["fxd_rgba"], touched_of(g["cls"]), touched_of(g["fxd_cls"])))
+        return
+    refp, refcuda = refcuda_pair
     cg = rrt.camera_state_from(*CAMERAS[cam])
     fx = rrt.effects_off()
     plain, _, _ = refcuda.render(0.99, cg, fx, sky_big, 1.0, w, h)
     P = refp.render(0.99, cg, fx, sky_big, 1.0, w, h)
-    g = _ours(gpu, sky_big, cam, 0.99, 3 | FMAD, w, h, fx)
     _check_fmad_against_reference_cuda(g, P, plain, f"{cam} {w}x{h}")
     # and the frame as the viewer shows it (bloom, vignette, lens distortion on: reference defaults)
     fxd = rrt.default_effects()
     plain_d, _, _ = refcuda.render(0.99, cg, fxd, sky_big, 1.0, w, h)
-    gd = _ours(gpu, sky_big, cam, 0.99, 3 | FMAD, w, h, fxd)
-    touched = (gd["cls"] & rrt.CLSF_TOUCHED) != 0
-    d = np.abs(gd["rgba"].astype(int) - plain_d.astype(int)).max(axis=-1)[::-1]
+    touched = (g["fxd_cls"] & rrt.CLSF_TOUCHED) != 0
+    d = np.abs(g["fxd_rgba"].astype(int) - plain_d.astype(int)).max(axis=-1)[::-1]
     assert d[~touched].max() == 0
     assert d.max() <= 1 and (d > 0).sum() <= max(3, w * h // 200000)
 
 
-def test_strict_1080p_frame_against_reference_headers_on_host(gpu, ref, sky_smooth):
+def test_strict_1080p_frame_against_reference_headers_on_host(gpu, host_headers, sky_smooth):
     """The strict contract at BASELINE's 1080p size against oracle/_ref/libref_host.so (the reference's unmodified
-    headers, -ffp-contract=off): trajectory bit-identical on every pixel, linear RGB within north_star's 1e-3."""
+    headers, -ffp-contract=off; the oracle port where that is not built): trajectory bit-identical on every pixel,
+    linear RGB within north_star's 1e-3."""
+    ref = host_headers
     import relativisticraytracer_b200 as rrt
     w, h = 1920, 1080
     fx = rrt.effects_off()
@@ -181,18 +261,22 @@ def _away_from_gates(pts, eps=2e-3):
 
 
 @pytest.mark.parametrize("spin", [0.0, 0.99])
-def test_fmad_media_probes_against_nvcc_compiled_reference_functions(gpu, refp, spin):
+def test_fmad_media_probes_against_nvcc_compiled_reference_functions(gpu, refcuda_pair, spin):
     """getAccretionDensity / getDustCloudDensity / calculateRedshiftFactor / getDiskTemperature of the FMAD unit vs the
     reference's functions compiled by nvcc with its default -fmad=true (a probe kernel in libref_cuda_planes.so).
     nvcc fuses a function differently standalone than inlined into raymarch_kernel, so this pair is close, not
     bit-identical (the bit-level pin of the media path is the whole-frame test above): the noise hash extracts the
     fraction of numbers ~1e4, so one ulp in its argument moves a lattice value by ~1e-3 and the contrast shaping
     (pow 1.6 / pow 4, smoothstep) amplifies that on a small share of samples."""
-    import relativisticraytracer_b200 as rrt
-    prm = rrt.default_params(spin_a=spin, flags=3 | FMAD)
+    key, ours_all = media_probes_case(gpu, spin)
+    if refcuda_pair is None:
+        assert_reference_digests(key, probes_exact(ours_all["disk_density"], ours_all["dust_density"], ours_all["disk_temperature"]))
+        return
+    refp = refcuda_pair[0]
     pts = disk_points(seed=31, n=1 << 15)
     ok = _away_from_gates(pts)
-    for what, ours in (("disk_density", gpu.disk_density(prm, pts, 1.0)), ("dust_density", gpu.dust_density(prm, pts, 1.0))):
+    for what in ("disk_density", "dust_density"):
+        ours = ours_all[what]
         want = refp.probe(what, spin, pts, None, 1.0)
         assert np.array_equal(ours[ok] == 0.0, want[ok] == 0.0), f"{what}: zero / non-zero pattern differs away from the gates"
         err = np.abs(ours.astype(np.float64) - want)[ok]
@@ -202,10 +286,10 @@ def test_fmad_media_probes_against_nvcc_compiled_reference_functions(gpu, refp, 
         assert np.quantile(rel, 0.999) < 5e-3, (what, float(np.quantile(rel, 0.999)))
         assert np.mean(ours[ok].view(np.uint32) == want[ok].view(np.uint32)) > 0.9, what
     q, v = phase_space(seed=32, n=1 << 15)
-    g_ours, g_want = gpu.redshift(prm, q, v), refp.probe("redshift", spin, q, v, 0.0)
+    g_ours, g_want = ours_all["redshift"], refp.probe("redshift", spin, q, v, 0.0)
     fin = np.isfinite(g_want)
     assert np.array_equal(fin, np.isfinite(g_ours))
     assert np.abs(g_ours[fin] - g_want[fin]).max() <= 2e-5 * np.maximum(np.abs(g_want[fin]), 1.0).max()
     np.testing.assert_allclose(g_ours[fin], g_want[fin], rtol=2e-5, atol=1e-6)
     r = np.linalg.norm(q, axis=1).astype(np.float32)
-    assert np.array_equal(gpu.disk_temperature(prm, r).view(np.uint32), refp.probe("disk_temperature", spin, r).view(np.uint32))
+    assert np.array_equal(ours_all["disk_temperature"].view(np.uint32), refp.probe("disk_temperature", spin, r).view(np.uint32))

@@ -5,16 +5,19 @@ the reference tree).  Checker: oracle/_ref/libref_stb.so = that header compiled 
 product's bytes must equal stb_image's byte for byte -- on the two assets the reference ships, and on files generated
 here with PIL that walk the decoder's subset: JPEG 4:4:4 / 4:2:2 / 4:2:0 / 4:4:0 / 4:1:1, grey, odd sizes, restart
 intervals, high and low quality; PNG grey / grey+alpha / RGB / RGBA / palette (1, 2, 4, 8 bit, with tRNS), all five
-row filters.  Files outside the subset must be refused, not decoded differently.  CPU only."""
+row filters.  Files outside the subset must be refused, not decoded differently.  Where stb_image is not built, the PNG
+files are checked against PIL's decoder instead (see png_ref).  CPU only."""
 import ctypes as C
 import hashlib
 import io
+import json
 import os
 
 import numpy as np
 import pytest
 
-REF_ASSETS = os.path.join(os.environ.get("RRT_REFERENCE_TREE", "/root/reference"), "assets", "skyboxes")
+# the reference's skybox assets, where a copy of its tree is named by RRT_REFERENCE_TREE
+REF_ASSETS = os.path.join(os.environ["RRT_REFERENCE_TREE"], "assets", "skyboxes") if "RRT_REFERENCE_TREE" in os.environ else None
 # sha256 of the RGBA8 bytes stb_image v2.30 returns for the reference's assets (the pin when the tree is absent is
 # the synthetic-file test below; these two make sure the shipped files themselves keep decoding to the same bytes)
 GOLDEN_SHA256 = {
@@ -23,11 +26,36 @@ GOLDEN_SHA256 = {
 }
 
 
+STB_LIB = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "libref_stb.so")
+# The JPEG files the JPEG tests decode, as PIL wrote them from _gradient (write_jpeg), and the sha256 of the RGBA8 bytes
+# stb_image returns for each (tests/tools/make_golden_jpeg.py): the check where libref_stb.so is not built.
+JPEG_GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "jpeg")
+
+
 @pytest.fixture(scope="module")
 def stb(built):
-    path = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "libref_stb.so")
-    if not os.path.exists(path):
+    if not os.path.exists(STB_LIB):
         pytest.skip("oracle/_ref/libref_stb.so not built (reference tree absent at build time)")
+    return _stb_loader(STB_LIB)
+
+
+@pytest.fixture(scope="module")
+def stb_if_built(built):
+    return _stb_loader(STB_LIB) if os.path.exists(STB_LIB) else None
+
+
+@pytest.fixture(scope="module")
+def png_ref(built):
+    """Checker for PNG files: stb_image where oracle/_ref/libref_stb.so is built, else PIL.  PNG is lossless, so its RGBA8
+    bytes are fixed by the file and every conforming decoder returns the same ones (not so for JPEG, whose IDCT and chroma
+    upsampling differ from decoder to decoder: the JPEG tests check stb_image's own bytes, see JPEG_GOLD)."""
+    if os.path.exists(STB_LIB):
+        return _stb_loader(STB_LIB)
+    from PIL import Image
+    return lambda path: np.asarray(Image.open(path).convert("RGBA"))
+
+
+def _stb_loader(path):
     lib = C.CDLL(path)
     lib.refstb_load.restype = C.POINTER(C.c_uint8)
     lib.refstb_load.argtypes = [C.c_char_p, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]
@@ -56,7 +84,7 @@ def _gradient(w, h, seed):
 
 def test_reference_assets_decode_to_stb_bytes(built, stb):
     import relativisticraytracer_b200 as rrt
-    if not os.path.isdir(REF_ASSETS):
+    if REF_ASSETS is None or not os.path.isdir(REF_ASSETS):
         pytest.skip("reference assets not present")
     for name, (w, h, sha) in GOLDEN_SHA256.items():
         path = os.path.join(REF_ASSETS, name)
@@ -88,35 +116,45 @@ JPEG_CASES = [
 ]
 
 
-@pytest.mark.parametrize("case", JPEG_CASES, ids=lambda c: f"{c[0]}x{c[1]}-{c[2]}-{c[3]}-q{c[4]}" + ("-rst" if c[5] else ""))
-def test_generated_jpeg_equals_stb(built, stb, tmp_path, case):
-    from PIL import Image
-    import relativisticraytracer_b200 as rrt
+JPEG_411 = (150, 100, "RGB", "4:1:1", 85, {})   # seed 7
+
+
+def jpeg_name(case):
     w, h, mode, sub, q, extra = case
-    img = _gradient(w, h, seed=w * 1000 + h)
-    im = Image.fromarray(img if mode == "RGB" else img[..., 0])
-    path = str(tmp_path / "t.jpg")
+    return f"{w}x{h}-{mode.lower()}-{(sub or 'grey').replace(':', '')}-q{q}" + "".join(f"-{k}" for k in extra) + ".jpg"
+
+
+def write_jpeg(case, path):
+    from PIL import Image
+    w, h, mode, sub, q, extra = case
+    img = _gradient(w, h, seed=7 if case == JPEG_411 else w * 1000 + h)
     kw = dict(quality=q, **extra)
     if sub is not None:
         kw["subsampling"] = sub
-    im.save(path, "JPEG", **kw)
-    want = stb(path)
-    assert want is not None
-    got = rrt.decode_image(path)
-    assert got.shape == want.shape == (h, w, 4)
-    assert np.array_equal(got, want), f"{int((got != want).sum())} bytes differ, max {int(np.abs(got.astype(int) - want).max())}"
+    Image.fromarray(img if mode == "RGB" else img[..., 0]).save(path, "JPEG", **kw)
 
 
-def test_jpeg_4_1_1_sampling_equals_stb(built, stb, tmp_path):
-    """4:1:1 (chroma 4x1): stb_image has no filter for that ratio and falls back to nearest neighbour -- so must we."""
-    from PIL import Image
+def _check_jpeg_against_stb(case, stb_if_built):
     import relativisticraytracer_b200 as rrt
-    path = str(tmp_path / "t411.jpg")
-    try:
-        Image.fromarray(_gradient(150, 100, seed=7)).save(path, "JPEG", quality=85, subsampling="4:1:1")
-    except (ValueError, TypeError, KeyError):
-        pytest.skip("this PIL build cannot write 4:1:1")
-    assert np.array_equal(rrt.decode_image(path), stb(path))
+    w, h = case[:2]
+    path = os.path.join(JPEG_GOLD, jpeg_name(case))
+    got = rrt.decode_image(path)
+    assert got.shape == (h, w, 4)
+    if stb_if_built is not None:
+        want = stb_if_built(path)
+        assert np.array_equal(got, want), f"{int((got != want).sum())} bytes differ, max {int(np.abs(got.astype(int) - want).max())}"
+    with open(os.path.join(JPEG_GOLD, "stb_rgba_sha256.json")) as f:
+        assert hashlib.sha256(got.tobytes()).hexdigest() == json.load(f)[jpeg_name(case)], "bytes differ from stb_image's"
+
+
+@pytest.mark.parametrize("case", JPEG_CASES, ids=lambda c: f"{c[0]}x{c[1]}-{c[2]}-{c[3]}-q{c[4]}" + ("-rst" if c[5] else ""))
+def test_generated_jpeg_equals_stb(built, stb_if_built, case):
+    _check_jpeg_against_stb(case, stb_if_built)
+
+
+def test_jpeg_4_1_1_sampling_equals_stb(built, stb_if_built):
+    """4:1:1 (chroma 4x1): stb_image has no filter for that ratio and falls back to nearest neighbour -- so must we."""
+    _check_jpeg_against_stb(JPEG_411, stb_if_built)
 
 
 def test_progressive_and_cmyk_jpeg_are_refused(built, tmp_path):
@@ -150,7 +188,7 @@ PNG_CASES = ["L", "LA", "RGB", "RGBA", "P", "P-trns", "1", "P2", "P4", "L-trns",
 
 @pytest.mark.parametrize("kind", PNG_CASES)
 @pytest.mark.parametrize("size", [(61, 37), (128, 64), (1, 1), (7, 300)])
-def test_generated_png_equals_stb(built, stb, tmp_path, kind, size):
+def test_generated_png_equals_stb(built, png_ref, tmp_path, kind, size):
     from PIL import Image
     import relativisticraytracer_b200 as rrt
     w, h = size
@@ -183,7 +221,7 @@ def test_generated_png_equals_stb(built, stb, tmp_path, kind, size):
         kw["transparency"] = tuple(int(x) for x in img[0, 0])
     path = str(tmp_path / "t.png")
     im.save(path, "PNG", **kw)
-    want = stb(path)
+    want = png_ref(path)
     assert want is not None
     got = rrt.decode_image(path)
     assert got.shape == want.shape == (h, w, 4)
@@ -213,7 +251,7 @@ def test_png_16bit_and_interlaced_are_refused(built, tmp_path):
     assert e.value.code == _capi.ERR_UNSUPPORTED
 
 
-def test_decode_from_memory_and_stored_deflate_blocks(built, stb, tmp_path):
+def test_decode_from_memory_and_stored_deflate_blocks(built, png_ref, tmp_path):
     """rrt_image_decode on a buffer, and a PNG whose zlib stream uses stored (uncompressed) blocks."""
     import struct
     import zlib
@@ -238,5 +276,5 @@ def test_decode_from_memory_and_stored_deflate_blocks(built, stb, tmp_path):
     got = np.ctypeslib.as_array(px, shape=(hh.value, ww.value, 4)).copy()
     lib.rrt_image_free(px)
     assert np.array_equal(got[..., :3], img) and (got[..., 3] == 255).all()
-    assert np.array_equal(got, stb(path))
+    assert np.array_equal(got, png_ref(path))
     assert lib.rrt_image_decode(buf, 4, C.byref(px), C.byref(ww), C.byref(hh)) == _capi.ERR_UNSUPPORTED   # not an image
