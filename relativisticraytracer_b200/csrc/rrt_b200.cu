@@ -6,8 +6,8 @@
 // Where things are:
 //   include/rrt_device.cuh   device math: the two rounding contracts, geodesic RHS, RK4, noise, densities
 //   csrc/rrt_kernel.cuh      render_kernel (one 8x4 tile per persistent warp), per-ray helpers, probe kernels
-//   csrc/rrt_variants.cuh    two measured-and-rejected alternatives to render_kernel; only in builds made with
-//                            EXTRA=-DRRT_WITH_VARIANTS (then selectable with RRT_KERNEL_VARIANT=2, 3, strict contract)
+//   csrc/rrt_packed.cuh      render_kernel_p (two rays per thread, no medium), FMAD contract only
+//   csrc/rrt_split.cuh       the split pipeline of launches with a medium: trace / media / fold kernels
 //   this file                band assembly, self-test / roofline probes, rrt_context, every extern "C" entry point
 //
 // Launch organisation (B200: 148 SMs, no tensor-core work on this path -- it is FP32 FMA-pipe bound):
@@ -35,9 +35,6 @@ using rrt::V3;
 using rrt::mk;
 
 #include "rrt_kernel.cuh"
-#ifdef RRT_WITH_VARIANTS
-#include "rrt_variants.cuh"   // measured alternatives to render_kernel (RRT_KERNEL_VARIANT=2, 3), strict contract only
-#endif
 
 namespace {
 
@@ -129,10 +126,9 @@ struct rrt_context {
     unsigned long long* d_counters = nullptr;
     unsigned int* d_tickets = nullptr;
     unsigned ticket_next = 0;
-    // which FMAD render kernel: 0 auto (packed f32x2, two rays per thread, for launches without a medium; the scalar kernel
-    // otherwise -- measured, profiles/r2_history.md), 1 always scalar, 2 always packed.  RRT_KERNEL=auto|scalar|packed.
-    int kernel_choice = 0;
-    int kernel_variant = 1;  // 1 tile-per-warp (the product); 2 / 3 only in -DRRT_WITH_VARIANTS builds (RRT_KERNEL_VARIANT)
+    // fused FMAD launches without a medium use the packed f32x2 kernel (two rays per thread; measured,
+    // profiles/r2_history.md) unless RRT_KERNEL=scalar pins the scalar one.  RRT_KERNEL=auto|scalar.
+    bool scalar_kernel = false;
     // launch configuration of every render kernel seen so far (resident CTAs per SM, carve-out applied): queried once
     struct LaunchCfg { const void* kern; int per_sm; };
     LaunchCfg launch_cfg[16] = {};
@@ -301,17 +297,11 @@ int rrt_context_create(int device, rrt_context** out) {
     if (!ctx) return fail(nullptr, RRT_ERR_NOMEM, "out of host memory");
     ctx->device = device;
     ctx->sm_count = prop.multiProcessorCount;
-    if (const char* k = std::getenv("RRT_KERNEL")) ctx->kernel_choice = !std::strcmp(k, "packed") ? 2 : (!std::strcmp(k, "scalar") ? 1 : 0);
+    if (const char* k = std::getenv("RRT_KERNEL")) ctx->scalar_kernel = !std::strcmp(k, "scalar");
     if (const char* k = std::getenv("RRT_PIPELINE")) ctx->pipeline = !std::strcmp(k, "split") ? RRT_PIPELINE_SPLIT : (!std::strcmp(k, "fused") ? RRT_PIPELINE_FUSED : RRT_PIPELINE_AUTO);
     if (const char* k = std::getenv("RRT_TRACE")) ctx->trace_choice = !std::strcmp(k, "packed") ? 2 : (!std::strcmp(k, "scalar") ? 1 : 0);
     if (const char* k = std::getenv("RRT_POOL_MB")) { const long long mb = std::atoll(k); if (mb > 0) ctx->pool_bytes_max = (size_t)mb << 20; }
     if (const char* k = std::getenv("RRT_MAX_PASSES")) { const int n = std::atoi(k); if (n >= 1 && n <= kMaxPasses) ctx->max_passes = n; }
-#ifdef RRT_WITH_VARIANTS
-    if (const char* kv = std::getenv("RRT_KERNEL_VARIANT")) {
-        const int k = std::atoi(kv);
-        if (k >= 1 && k <= 3) ctx->kernel_variant = k;
-    }
-#endif
     DevGuard g(device);
     if ((e = cudaMalloc(&ctx->d_counters, sizeof(rrt_counters))) != cudaSuccess ||
         (e = cudaMemset(ctx->d_counters, 0, sizeof(rrt_counters))) != cudaSuccess ||
@@ -619,22 +609,12 @@ int rrt_render(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, c
     const bool fmad = (prm->flags & RRT_FLAG_FMAD) != 0;
     const rrtk::KernelSet* ks = fmad ? rrtk::rrt_kernels_fmad() : rrtk::rrt_kernels_strict();
     void (*kern)(const FrameArgs) = ks->render[spin ? 1 : 0][media ? 1 : 0];
-    int variant = 1;
     long long rays_per_block = kRenderBlock;
-    if (ks->render_packed[0][0] && (ctx->kernel_choice == 2 || (ctx->kernel_choice == 0 && !media))) {
-        kern = ks->render_packed[spin ? 1 : 0][media ? 1 : 0];
+    if (fmad && !media && !ctx->scalar_kernel) {
+        kern = ks->render_packed[spin ? 1 : 0];
         rays_per_block = 64;
     }
-#ifdef RRT_WITH_VARIANTS
-    // measured alternatives (strict arithmetic only): 2 two rays per thread (f32x2), 3 wavefront in a warp
-    variant = fmad ? 1 : ctx->kernel_variant;
-    if (variant == 2) kern = spin ? (media ? render_kernel2<true, true> : render_kernel2<true, false>)
-                                  : (media ? render_kernel2<false, true> : render_kernel2<false, false>);
-    else if (variant == 3) kern = spin ? (media ? render_kernel3<true, true> : render_kernel3<true, false>)
-                                       : (media ? render_kernel3<false, true> : render_kernel3<false, false>);
-#endif
     if ((long long)w * local_rows > (1ll << 30)) return fail(ctx, RRT_ERR_BAD_ARG, "rrt_render: band larger than 2^30 pixels");
-    const int block = variant == 1 ? kRenderBlock : kBlock;
     // Resident CTAs per SM and the shared-memory carve-out are properties of (kernel, device): asked for once per
     // context, not per frame.  The carve-out stays at the shared-memory end although render_kernel declares no shared
     // memory: every resident CTA still reserves 1 KB of it, and with one-warp CTAs (24-32 per SM) a small carve-out
@@ -644,11 +624,10 @@ int rrt_render(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, c
         if (ctx->launch_cfg[i].kern == (const void*)kern) per_sm = ctx->launch_cfg[i].per_sm;
     if (per_sm == 0) {
         RRT_CU(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        RRT_CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, block, 0));
+        RRT_CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kRenderBlock, 0));
         if (per_sm < 1) per_sm = 1;
         if (ctx->n_launch_cfg < 16) ctx->launch_cfg[ctx->n_launch_cfg++] = {(const void*)kern, per_sm};
     }
-    if (variant != 1) rays_per_block = (variant == 2 ? 2 : 1) * (long long)block;
     // A persistent launch normally fills every resident-CTA slot.  When the caller keeps n frames in flight, each
     // launch takes 1/n of the slots so that the n kernels run side by side from the start: a launch then lasts
     // n times longer than its critical path (one tile of disk-plane rays, ~17 ms at 4K) needs, instead of ending
@@ -657,8 +636,8 @@ int rrt_render(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, c
     const long long need = ((long long)w * local_rows + rays_per_block - 1) / rays_per_block;
     if (grid > need) grid = need;
     // A launch with a medium goes through the split pipeline (csrc/rrt_split.cuh) unless the caller pinned the fused
-    // kernel, a measured variant or the tile log is selected, or the pool cannot be allocated.
-    if (media && variant == 1 && ctx->pipeline != RRT_PIPELINE_FUSED && (!ctx->tile_log || ctx->pipeline == RRT_PIPELINE_SPLIT) && prm->max_steps + 2 <= 128 * (rrtk::kDescChunks - 2)) {
+    // kernel, the tile log is selected, or the pool cannot be allocated.
+    if (media && ctx->pipeline != RRT_PIPELINE_FUSED && (!ctx->tile_log || ctx->pipeline == RRT_PIPELINE_SPLIT) && prm->max_steps + 2 <= 128 * (rrtk::kDescChunks - 2)) {
         const rrtk::SplitKernels* sk = fmad ? rrtk::rrt_split_kernels_fmad() : rrtk::rrt_split_kernels_strict();
         // the tracer: two rays per thread in packed f32x2 registers where that kernel exists (FMAD contract), else one per thread
         const bool packed_trace = sk->trace_packed[0] != nullptr && ctx->trace_choice != 1 &&
@@ -676,7 +655,7 @@ int rrt_render(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, c
             return render_split(ctx, A, spin, fmad, packed_trace, grid_trace, st, pl);
         if (ctx->pipeline == RRT_PIPELINE_SPLIT) return fail(ctx, RRT_ERR_NOMEM, "rrt_render: no memory for the sample pool of the split pipeline");
     }
-    kern<<<(unsigned)grid, block, 0, st>>>(A);
+    kern<<<(unsigned)grid, kRenderBlock, 0, st>>>(A);
     RRT_CU(ctx, cudaGetLastError());
     ctx->launches += 1;
     return RRT_OK;

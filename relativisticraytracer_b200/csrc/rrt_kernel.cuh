@@ -34,7 +34,7 @@ struct FrameArgs {
 // kernels of one rounding contract
 struct KernelSet {
     void (*render[2][2])(const FrameArgs);  // [spin != 0][media]
-    void (*render_packed[2][2])(const FrameArgs);  // two rays per thread in f32x2 registers (rrt_packed.cuh); FMAD contract only
+    void (*render_packed[2])(const FrameArgs);  // [spin != 0]; two rays per thread in f32x2 registers, no medium (rrt_packed.cuh); FMAD contract only
     void (*acc)(Consts, int, const float*, const float*, float*);
     void (*rk4)(Consts, int, float*, float*, const float*);
     void (*euler)(Consts, int, float*, float*, const float*);
@@ -57,53 +57,19 @@ using rrtk::FrameArgs;
 
 namespace {
 
-
-
-constexpr int kTileW = 8, kTileH = 4;  // one warp = 8x4 pixels (measured variants)
-// render_kernel's own tile shape (a build-time experiment knob; 8x4 measured best or equal, profiles/r1_history.md)
-#ifndef RRT_TILE_W
-#define RRT_TILE_W 8
-#endif
-constexpr int kRTileW = RRT_TILE_W, kRTileH = 32 / RRT_TILE_W;
-static_assert(kRTileW * kRTileH == 32 && (kRTileW & (kRTileW - 1)) == 0, "a tile is one warp");
-constexpr int kBlock = 128;          // CTA size of the measured variants (rrt_variants.cuh)
+// render_kernel's tile: 8x4 pixels, one warp (8x4 measured best or equal, profiles/r1_history.md)
+constexpr int kRTileW = 8, kRTileH = 4;
 // render_kernel's warps share nothing (no shared memory, no barrier), so its CTA is ONE warp: a CTA's slot is
 // handed to the next launch the moment that warp runs out of tickets, instead of waiting for the slowest of four --
 // which is what lets the frames of a sequence overlap cleanly (rrt_set_frames_in_flight, FramePipeline).
-#ifndef RRT_RENDER_BLOCK
-#define RRT_RENDER_BLOCK 32
-#endif
-constexpr int kRenderBlock = RRT_RENDER_BLOCK;
-// steps per unchecked vacuum burst of the render loop (0 = no burst code)
-#ifndef RRT_BURST_K
-#define RRT_BURST_K 8
-#endif
-// how many of those steps one trip of the burst loop holds, for the geodesic-only and for the media kernels
-#ifndef RRT_BURST_UNROLL
-#define RRT_BURST_UNROLL 4
-#endif
-#ifndef RRT_BURST_UNROLL_MEDIA
-#define RRT_BURST_UNROLL_MEDIA 1
-#endif
-#ifndef RRT_MIN_BLOCKS
-#define RRT_MIN_BLOCKS 1
-#endif
+constexpr int kRenderBlock = 32;
+// steps per unchecked vacuum burst of the render loop
+constexpr int kBurst = 8;
 // The media variant of the render kernel is asked to fit 24 warps per SM, i.e. <= 80 registers: the
 // out-of-line media code stalls on libdevice call chains and MUFU latency, and six warps per scheduler hide
 // that better than the four the unconstrained 109-register build gets (4K C0 78.5 -> 76.2 ms, C3 147.6 -> 135.4;
 // 7 and 8 CTAs are no better).  The geodesic-only variant needs ~72 registers anyway.
-#ifndef RRT_MIN_BLOCKS_MEDIA
-#define RRT_MIN_BLOCKS_MEDIA (6 * 128 / RRT_RENDER_BLOCK)
-#endif
-
-#ifdef RRT_WITH_GROUP_STEPS
-// profiling build (-DRRT_WITH_TILE_LOG -DRRT_WITH_GROUP_STEPS): how many times a warp EXECUTED the checked step for a tile (one count per group of lanes that run it
-// together): equals the longest ray's checked steps while the tile's lanes stay converged
-__shared__ unsigned g_dbg_group_steps[8];
-__device__ __forceinline__ unsigned dbg_group_steps(int warp) { return min(g_dbg_group_steps[warp], 0xfffffu); }
-#else
-__device__ __forceinline__ unsigned dbg_group_steps(int) { return 0u; }
-#endif
+constexpr int kMinBlocks = 1, kMinBlocksMedia = 24;
 
 struct RayResult {
     float hdr[3], T, I[3];
@@ -301,8 +267,7 @@ __device__ __forceinline__ void trace_ray(const FrameArgs& A, int x, int y, RayR
     // one compare per step for "redo with the general code": smallest stage radius below acc_rmin (or NaN), or
     // the whole ray outside the fast domain (+inf: every step is redone)
     const float redo_below = fast_ok ? C.acc_rmin : __int_as_float(0x7f800000);
-#if RRT_BURST_K > 0
-        constexpr int kBurst = RRT_BURST_K, kBurstUnroll = MEDIA == kMediaInline ? RRT_BURST_UNROLL_MEDIA : RRT_BURST_UNROLL;
+    constexpr int kBurstUnroll = MEDIA == kMediaInline ? 1 : 4;   // steps per trip of the burst loop
     static_assert(kBurst % kBurstUnroll == 0, "burst length must be a multiple of its unroll factor");
     // every threshold a checked vacuum step compares a radius against from above: zones (:56-58), horizon (:47),
     // geodesics.h:33 through the redo guard
@@ -310,7 +275,6 @@ __device__ __forceinline__ void trace_ray(const FrameArgs& A, int x, int y, RayR
     // entry window: kBurst steps of |v| ~ 1 (1.25 allowed) must fit between the zone sphere and the escape sphere
     const float burst_margin = 1.25f * (float)kBurst * C.h[0];
     const float burst_lo = burst_min + burst_margin, burst_hi = 250.0f - burst_margin;
-#endif
     // Two-level loop.  The inner loop holds what (nearly) every step needs -- the branch-free RK4 step and, in
     // lock-step for the lanes that are inside a medium, the out-of-line media sample -- and nothing else; the
     // general-domain redo of a step (practically never taken) is done by the outer loop, which then re-enters,
@@ -338,7 +302,6 @@ __device__ __forceinline__ void trace_ray(const FrameArgs& A, int x, int y, RayR
         // standing alone at the top of every iteration (it was ~20 % of the stall samples there).
         float r2 = rrt::norm2_loop(p);
         r = rrt::sqrt_rn_fast(r2);                                                            // :44
-#if RRT_BURST_K > 0
         // ---- phase 1: vacuum bursts ------------------------------------------------------------------------------
         // Most steps (94 % of the headline frame's) happen outside every step-size zone, with the whole-warp step h[0]
         // and no medium; there the horizon test (:47), the zone logic (:54-62), the media branch (:67) and the escape test
@@ -384,14 +347,10 @@ __device__ __forceinline__ void trace_ray(const FrameArgs& A, int x, int y, RayR
                 break;
             }
         }
-#endif
         // ---- phase 2: checked steps, until the ray ends or the whole warp is back in the burst window ------------------
         bool rewind = false;
 #pragma unroll 1
         while (it < max_steps) {                                                              // :41
-#ifdef RRT_WITH_GROUP_STEPS
-            if ((threadIdx.x & 31) == __ffs(__activemask()) - 1) atomicAdd(&g_dbg_group_steps[threadIdx.x >> 5], 1u);
-#endif
             if (r < C.horizon_r) { ev = kCaptured; break; }                                   // :47-51
             unsigned z = 0;
             float rmin;
@@ -400,11 +359,7 @@ __device__ __forceinline__ void trace_ray(const FrameArgs& A, int x, int y, RayR
             // Which lanes take the general step below (step size from the zone table) and which the constant-step copy:
             // see the `else` branch.  With bursts in a media kernel the checked vacuum step is 1 in kBurst + 1, and the
             // instruction cache has no room for a third copy of the step next to the media code, so it uses this one.
-#ifdef RRT_TWO_CHECKED   // A/B knob: keep the constant-step copy of the checked vacuum step in the media kernels too
-            constexpr bool kOneCheckedStep = !RRT_FMAD;
-#else
-                        constexpr bool kOneCheckedStep = !RRT_FMAD || (MEDIA == kMediaInline && RRT_BURST_K > 0);
-#endif
+            constexpr bool kOneCheckedStep = !RRT_FMAD || MEDIA == kMediaInline;
             if (kOneCheckedStep || r < zone_rmax) {
                 float h = C.h[0], h6 = C.h6[0];
                 int zsel = 0;
@@ -443,12 +398,10 @@ __device__ __forceinline__ void trace_ray(const FrameArgs& A, int x, int y, RayR
             if (r > 250.0f && rrt::dot3(q, v) > 0.0f) { ev = kEscaped; break; }               // :120
             r2 = r2_next;
             r = r_next;
-#if RRT_BURST_K > 0
             {   // one VOTE per checked step: the lanes in the loop here, the qualifying ones inside the branch
                 const unsigned in_loop = __activemask();
                 if (r >= burst_lo && r <= burst_hi && it >= burst_after && it + kBurst < max_steps && __activemask() == in_loop) { rewind = true; break; }
             }
-#endif
         }
         if (rewind) continue;   // back to phase 1 (p, v, it carry over; r2 / r are recomputed from p, bit for bit the same)
         if (ev == kRedo) {
@@ -481,7 +434,7 @@ __device__ __forceinline__ void trace_ray(const FrameArgs& A, int x, int y, RayR
 }
 
 template <bool SPIN, bool MEDIA>
-__global__ void __launch_bounds__(kRenderBlock, MEDIA ? RRT_MIN_BLOCKS_MEDIA : RRT_MIN_BLOCKS) render_kernel(const __grid_constant__ FrameArgs A) {
+__global__ void __launch_bounds__(kRenderBlock, MEDIA ? kMinBlocksMedia : kMinBlocks) render_kernel(const __grid_constant__ FrameArgs A) {
     const int lane = threadIdx.x & 31;
     const int ntx = (A.w + kRTileW - 1) / kRTileW;
     const int nty = (A.local_rows + kRTileH - 1) / kRTileH;
@@ -511,11 +464,6 @@ __global__ void __launch_bounds__(kRenderBlock, MEDIA ? RRT_MIN_BLOCKS_MEDIA : R
 #ifdef RRT_WITH_TILE_LOG
         unsigned long long t_begin = 0;
         if (A.tile_log) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_begin));
-#ifdef RRT_WITH_GROUP_STEPS
-        __syncwarp();
-        if (lane == 0) g_dbg_group_steps[threadIdx.x >> 5] = 0u;
-        __syncwarp();
-#endif
 #endif
         RayResult R;
         NoEmit no_emit;
@@ -536,7 +484,7 @@ __global__ void __launch_bounds__(kRenderBlock, MEDIA ? RRT_MIN_BLOCKS_MEDIA : R
                 asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
                 unsigned long long* e = A.tile_log + 4ull * tile;
                 e[0] = t_begin; e[1] = t_end; e[2] = ((unsigned long long)ty << 32) | (unsigned)tx;
-                e[3] = ((unsigned long long)smid << 32) | (unsigned)most | (dbg_group_steps(threadIdx.x >> 5) << 12);
+                e[3] = ((unsigned long long)smid << 32) | (unsigned)most;
             }
         }
 #endif
@@ -636,9 +584,9 @@ namespace {
 const rrtk::KernelSet kKernelSet = {
     {{render_kernel<false, false>, render_kernel<false, true>}, {render_kernel<true, false>, render_kernel<true, true>}},
 #if RRT_FMAD
-    {{render_kernel_p<false, false>, render_kernel_p<false, true>}, {render_kernel_p<true, false>, render_kernel_p<true, true>}},
+    {render_kernel_p<false>, render_kernel_p<true>},
 #else
-    {{nullptr, nullptr}, {nullptr, nullptr}},
+    {nullptr, nullptr},
 #endif
     k_acc, k_rk4, k_euler, k_redshift, k_hash31, k_noise3d, k_fbm, k_disk_temp, k_disk_density, k_dust_density,
 };

@@ -183,18 +183,11 @@ __device__ __forceinline__ unsigned next_tile(const FrameArgs& A, const SplitArg
 // ---- emitter: the sample rows of one tracing warp -----------------------------------------------------------------
 // Shared memory per warp: tab[j] = slot index of the j-th chunk the CURRENT tile's rows can touch; tab[0] is the chunk the
 // warp was in when the tile began.  Chunks a tile did not reach stay in the table for the next tile.
-#ifndef RRT_STORE256
-#define RRT_STORE256 1   // a slot is one 32-byte sector: write it with ONE 256-bit store (sm_100: STG.256) instead of two halves
-#endif
+// A slot is one 32-byte sector: it is written with ONE 256-bit store (sm_100: STG.256) instead of two halves.
 __device__ __forceinline__ void pool_put(uint4* slots, unsigned slot, uint4 a, uint4 b) {
-#if RRT_STORE256
     asm volatile("st.global.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(slots + 2ull * slot), "r"(a.x), "r"(a.y), "r"(a.z),
                  "r"(a.w), "r"(b.x), "r"(b.y), "r"(b.z), "r"(b.w)
                  : "memory");
-#else
-    slots[2ull * slot] = a;
-    slots[2ull * slot + 1] = b;
-#endif
 }
 // A chunk for the calling lane's table entry (kNone: the pool is exhausted).  Only called between tiles.
 __device__ __forceinline__ unsigned claim_chunk(const SplitArgs& S) {
@@ -330,7 +323,7 @@ __device__ __forceinline__ void redo_later(const SplitArgs& S, unsigned tile, in
 
 // ---- pass kernel 1: trajectories ------------------------------------------------------------------------------------
 template <bool SPIN>
-__global__ void __launch_bounds__(kRenderBlock, RRT_MIN_BLOCKS) trace_kernel(const __grid_constant__ FrameArgs A,
+__global__ void __launch_bounds__(kRenderBlock, kMinBlocks) trace_kernel(const __grid_constant__ FrameArgs A,
                                                                               const __grid_constant__ SplitArgs S) {
     __shared__ unsigned chunk_tab[kRenderBlock / 32][kDescChunks];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -365,11 +358,6 @@ __global__ void __launch_bounds__(kRenderBlock, RRT_MIN_BLOCKS) trace_kernel(con
 #ifdef RRT_WITH_TILE_LOG
         unsigned long long t_begin = 0;
         if (A.tile_log) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_begin));
-#ifdef RRT_WITH_GROUP_STEPS
-        __syncwarp();
-        if (lane == 0) g_dbg_group_steps[warp] = 0u;
-        __syncwarp();
-#endif
 #endif
         if (px.valid) trace_ray<SPIN, kMediaEmit>(A, px.x, px.y, R, em);
         __syncwarp();
@@ -384,7 +372,7 @@ __global__ void __launch_bounds__(kRenderBlock, RRT_MIN_BLOCKS) trace_kernel(con
                 unsigned long long* e = A.tile_log + 4ull * tile;
                 const int ntx = (A.w + kRTileW - 1) / kRTileW;
                 e[0] = t_begin; e[1] = t_end; e[2] = ((unsigned long long)(px.ly / kRTileH) << 32) | (unsigned)(tile % (unsigned)ntx);
-                e[3] = ((unsigned long long)smid << 32) | (unsigned)most | (dbg_group_steps(warp) << 12);
+                e[3] = ((unsigned long long)smid << 32) | (unsigned)most;
             }
         }
 #endif
@@ -445,7 +433,7 @@ struct Emitter2 {
 };
 
 template <bool SPIN>
-__global__ void __launch_bounds__(32, RRT_PACKED_MIN_BLOCKS) trace_kernel_p(const __grid_constant__ FrameArgs A, const __grid_constant__ SplitArgs S) {
+__global__ void __launch_bounds__(32, kPackedMinBlocks) trace_kernel_p(const __grid_constant__ FrameArgs A, const __grid_constant__ SplitArgs S) {
     using rrtp::F2;
     using rrtp::V3x2;
     __shared__ unsigned chunk_tab[kDescChunks];
@@ -462,8 +450,6 @@ __global__ void __launch_bounds__(32, RRT_PACKED_MIN_BLOCKS) trace_kernel_p(cons
     const bool fast_ok = rrt::dot3(cam_p, cam_p) < 1.0e8f && C.acc_rmin < C.horizon_r && C.horizon_r >= 1e-3f;
     const float redo_below = fast_ok ? C.acc_rmin : __int_as_float(0x7f800000);
     const V3 park_p = mk(0.0f, 100.0f, 0.0f), park_v = mk(0.0f, 0.0f, 0.0f);   // inert state of a finished half, see render_kernel_p
-#if RRT_BURST_K > 0
-    constexpr int kBurst = RRT_BURST_K;
     const float burst_min = fmaxf(zone_rmax, fmaxf(C.horizon_r, redo_below));
     const float burst_margin = 1.25f * (float)kBurst * C.h[0];
     const float burst_lo = burst_min + burst_margin, burst_hi = 250.0f - burst_margin;
@@ -490,7 +476,6 @@ __global__ void __launch_bounds__(32, RRT_PACKED_MIN_BLOCKS) trace_kernel_p(cons
         if (m == 1) return mn >= zb_floor && mx < 18.0f;                         // :56
         return mn >= 18.0f && mx < C.disk_zone_r && my < C.disk_zone_y;          // :57 and not :56
     };
-#endif
     TileCounters cnt;
     Emitter2 em(S, tab, C);
     unsigned taken = 0, row_next = 0;
@@ -541,7 +526,6 @@ __global__ void __launch_bounds__(32, RRT_PACKED_MIN_BLOCKS) trace_kernel_p(cons
             F2 R2 = rrtp::norm2_loop_2(P);
             F2 R = rrtp::sqrt2(R2);                                                              // :44
             for (;;) {
-#if RRT_BURST_K > 0
                 // ---- phase 1: unchecked vacuum bursts, warp-uniform (see render_kernel_p / trace_ray) ------------------
                 {
                     const unsigned in_loop = __activemask();
@@ -570,7 +554,6 @@ __global__ void __launch_bounds__(32, RRT_PACKED_MIN_BLOCKS) trace_kernel_p(cons
                         burst_after = it + kBurst;
                         break;
                     }
-#ifndef RRT_NO_ZONE_BURSTS
                     // ---- phase 1b: zone bursts, one zone per ray --------------------------------------------------------------
 #pragma unroll 1
                     for (;;) {
@@ -619,9 +602,7 @@ __global__ void __launch_bounds__(32, RRT_PACKED_MIN_BLOCKS) trace_kernel_p(cons
                         zburst_after = it + kBurst;
                         break;
                     }
-#endif
                 }
-#endif
                 // ---- phase 2: checked iterations ----------------------------------------------------------------------
                 bool rewind = false;
 #pragma unroll 1
@@ -699,21 +680,17 @@ __global__ void __launch_bounds__(32, RRT_PACKED_MIN_BLOCKS) trace_kernel_p(cons
                         R2 = R2n;
                         R = Rn;
                     }
-#if RRT_BURST_K > 0
                     {
                         const unsigned in_loop = __activemask();
                         float r0, r1;
                         rrtp::upk(R, r0, r1);
                         if (fminf(r0, r1) >= burst_lo && fmaxf(r0, r1) <= burst_hi && it >= burst_after && it + kBurst < max_steps &&
                             __activemask() == in_loop) { rewind = true; break; }
-#ifndef RRT_NO_ZONE_BURSTS
                         float y0, y1;
                         rrtp::upk(P.y, y0, y1);
                         if (it >= zburst_after && it + kBurst < max_steps && (!alive[0] || zone_for_burst(r0, fabsf(y0)) >= 0) &&
                             (!alive[1] || zone_for_burst(r1, fabsf(y1)) >= 0) && __activemask() == in_loop) { rewind = true; break; }
-#endif
                     }
-#endif
                 }
                 if (!rewind) break;
             }
@@ -834,11 +811,7 @@ __global__ void __launch_bounds__(kMediaBlock, 4) media_kernel(const __grid_cons
             const unsigned tag = b_w[i].w;   // 0 for the lanes behind the group's last sample
             float dd = 0.0f, base_d = 0.0f;
             const V3 q = mk(__uint_as_float(a.x), __uint_as_float(a.y), __uint_as_float(a.z));
-#ifdef RRT_MEDIA_UNGATED
-            if (tag & 1u) dd = rrt::disk_density(C, q, A.time);                               // :68
-#else
             if (tag & 1u) dd = rrt::disk_density_gated(C, q, A.time);                         // :68 (0 where the gate of :71 cannot pass)
-#endif
             if (tag & 2u) base_d = rrt::dust_base(C, q);                                      // :69, densities.h:70-84
             dd_w[i] = dd;
             dc_w[i] = 0.0f;
@@ -945,7 +918,7 @@ __global__ void __launch_bounds__(128) fold_kernel(const __grid_constant__ Frame
 
 // ---- after the last pass: whatever the split passes left, with the fused code ------------------------------------------
 template <bool SPIN>
-__global__ void __launch_bounds__(kRenderBlock, RRT_MIN_BLOCKS_MEDIA) sweep_kernel(const __grid_constant__ FrameArgs A,
+__global__ void __launch_bounds__(kRenderBlock, kMinBlocksMedia) sweep_kernel(const __grid_constant__ FrameArgs A,
                                                                                     const __grid_constant__ SplitArgs S) {
     const int lane = threadIdx.x & 31;
     const unsigned ntiles = num_tiles(A);

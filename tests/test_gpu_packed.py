@@ -1,8 +1,9 @@
-"""render_kernel_p (csrc/rrt_packed.cuh: two rays per thread in packed f32x2 registers, FMAD contract) against render_kernel.
-Each half of a packed instruction is rounded like the scalar instruction it replaces, so frames, parity planes and counters
-must be bit-identical whichever kernel traced them -- for every camera, with and without media, for ragged sizes (odd
-widths leave a thread with one ray), bands, and the step budget's edge.  RRT_KERNEL=scalar|packed|auto is read when a
-context is created; auto (the default) uses the packed kernel for launches without a medium."""
+"""render_kernel_p (csrc/rrt_packed.cuh: two rays per thread in packed f32x2 registers, FMAD contract, no medium) against
+render_kernel.  Each half of a packed instruction is rounded like the scalar instruction it replaces, so frames, parity
+planes and counters must be bit-identical whichever kernel traced them -- for every camera, for ragged sizes (odd widths
+leave a thread with one ray), bands, and the step budget's edge.  RRT_KERNEL=auto|scalar is read when a context is
+created; auto (the default) uses the packed kernel for launches without a medium, scalar always uses render_kernel.
+Launches with a medium go through the split pipeline, which tests/test_gpu_split.py checks against render_kernel."""
 import os
 
 import numpy as np
@@ -22,9 +23,10 @@ def pair(built):
     old = os.environ.get("RRT_KERNEL")
     made = {}
     try:
-        for k in ("scalar", "packed"):
-            os.environ["RRT_KERNEL"] = k
-            made[k] = rrt.Renderer(0)
+        os.environ["RRT_KERNEL"] = "scalar"
+        made["scalar"] = rrt.Renderer(0)
+        os.environ.pop("RRT_KERNEL")
+        made["packed"] = rrt.Renderer(0)   # auto: the packed kernel for these launches
     finally:
         if old is None:
             os.environ.pop("RRT_KERNEL", None)
@@ -60,7 +62,7 @@ def _same(a, b, tag):
 
 
 @pytest.mark.parametrize("cam", ["C0", "C1", "C2", "C3"])
-@pytest.mark.parametrize("spin,flags", [(0.99, 7), (0.0, 7), (0.99, 4), (0.0, 4), (0.99, 5)])
+@pytest.mark.parametrize("spin,flags", [(0.99, 4), (0.0, 4)])
 def test_packed_equals_scalar(pair, sky_small, cam, spin, flags):
     scalar, packed = pair
     w, h = 203, 117      # odd width: the last thread of a row owns a single ray
@@ -71,10 +73,10 @@ def test_packed_equals_scalar_bands_budget_and_one_pixel(pair, sky_small):
     import relativisticraytracer_b200 as rrt
     scalar, packed = pair
     for band in (rrt.Band(0, 3, 8), rrt.Band(2, 3, 8), rrt.Band(1, 2, 1)):
-        _same(_frame(scalar, sky_small, "C1", 0.99, 7, 160, 90, band=band), _frame(packed, sky_small, "C1", 0.99, 7, 160, 90, band=band), "band")
+        _same(_frame(scalar, sky_small, "C1", 0.99, 4, 160, 90, band=band), _frame(packed, sky_small, "C1", 0.99, 4, 160, 90, band=band), "band")
     for steps in (0, 1, 7, 8, 9, 17, 333):    # around the burst length
-        _same(_frame(scalar, sky_small, "C0", 0.99, 7, 64, 36, max_steps=steps), _frame(packed, sky_small, "C0", 0.99, 7, 64, 36, max_steps=steps), f"max_steps={steps}")
-    _same(_frame(scalar, sky_small, "C0", 0.99, 7, 1, 1), _frame(packed, sky_small, "C0", 0.99, 7, 1, 1), "1x1")
+        _same(_frame(scalar, sky_small, "C0", 0.99, 4, 64, 36, max_steps=steps), _frame(packed, sky_small, "C0", 0.99, 4, 64, 36, max_steps=steps), f"max_steps={steps}")
+    _same(_frame(scalar, sky_small, "C0", 0.99, 4, 1, 1), _frame(packed, sky_small, "C0", 0.99, 4, 1, 1), "1x1")
     _same(_frame(scalar, sky_small, "C2", 0.99, 4, 2, 5, fx="off"), _frame(packed, sky_small, "C2", 0.99, 4, 2, 5, fx="off"), "2x5")
 
 

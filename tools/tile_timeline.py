@@ -55,14 +55,10 @@ for frac in (0.5, 0.8, 0.9, 0.95, 0.98, 0.99, 1.0):
 last_start = beg.max()
 print(f"last tile handed out at {last_start:.2f} ms ({last_start / span * 100:.1f} % of the span): after that the launch only drains")
 order = np.argsort(-end)[:12]
-print("tiles finishing last:  end ms   start ms  duration ms   row  col   sm  longest ray (steps)  checked-step executions by the warp")
+print("tiles finishing last:  end ms   start ms  duration ms   row  col   sm  longest ray (steps)")
 for i in order:
-    print(f"                     {end[i]:8.2f} {beg[i]:9.2f} {dur[i]:11.2f} {L[i, 2] >> 32:5d} {L[i, 2] & 0xffffffff:4d} {L[i, 3] >> 32:4d} {L[i, 3] & 0xfff:8d} {(L[i, 3] >> 12) & 0xfffff:8d}")
+    print(f"                     {end[i]:8.2f} {beg[i]:9.2f} {dur[i]:11.2f} {L[i, 2] >> 32:5d} {L[i, 2] & 0xffffffff:4d} {L[i, 3] >> 32:4d} {L[i, 3] & 0xffffffff:8d}")
 slow = np.argsort(-dur)[:8]
 print("longest tiles:         end ms   start ms  duration ms   row  col   sm  longest ray (steps)")
 for i in slow:
-    print(f"                     {end[i]:8.2f} {beg[i]:9.2f} {dur[i]:11.2f} {L[i, 2] >> 32:5d} {L[i, 2] & 0xffffffff:4d} {L[i, 3] >> 32:4d} {L[i, 3] & 0xfff:8d} {(L[i, 3] >> 12) & 0xfffff:8d}")
-ex = (L[:, 3] >> 12) & 0xfffff
-mx = L[:, 3] & 0xfff
-print(f"checked-step executions per tile / longest ray's steps: median {np.median(ex / np.maximum(mx, 1)):.2f}, p99 {np.quantile(ex / np.maximum(mx, 1), .99):.2f}, max {(ex / np.maximum(mx, 1)).max():.2f}; "
-      f"sum of executions {int(ex.sum())} vs sum of longest-ray steps {int(mx.sum())}")
+    print(f"                     {end[i]:8.2f} {beg[i]:9.2f} {dur[i]:11.2f} {L[i, 2] >> 32:5d} {L[i, 2] & 0xffffffff:4d} {L[i, 3] >> 32:4d} {L[i, 3] & 0xffffffff:8d}")
