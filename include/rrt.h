@@ -163,6 +163,21 @@ int rrt_render(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, c
                uint64_t sky_texture, float time, int w, int h, const rrt_band* band, void* d_out, int out_layout,
                const rrt_planes* planes, void* stream);
 
+/* Re-runs only the step after the ray loop (sky, final_hdr = I + bg*T, bloom, vignette, CA, tonemap, row-flipped store)
+ * from the planes a previous rrt_render wrote: a new sky, exposure or bloom / vignette / CA setting without a new trace.
+ * `traced` must carry vel, emis, hdr (only .w = T is read) and cls of that render, full-frame indexed [y*w + x] as
+ * rrt_render writes them; other members are ignored.  Writes d_out (layout as in rrt_render, only the band's rows) and/or
+ * hdr_out (float4 per pixel, full-frame indexed, the band's pixels only; may be traced->hdr itself).  Uses prm->exposure
+ * and the contract bit prm->flags & RRT_FLAG_FMAD, and every rrt_effects field.  Asynchronous on `stream`; adds nothing
+ * to the counters.
+ * Contract: if the planes were written by rrt_render(P, cam, F, S, time, w, h, band, ...), then
+ * rrt_shade(P', F', S', w, h, band, ...) writes exactly the bytes and hdr values of rrt_render(P*, cam, F*, S', time, w,
+ * h, band, ...), where P* is P with P'.exposure and F* is F with the bloom, vignette and CA fields of F'.  This needs P'
+ * to have the RRT_FLAG_FMAD bit of P and F' the use_lens / distortion_amount of F: those decide the rays and the
+ * vignette's image-plane coordinate, and changing them needs a new trace. */
+int rrt_shade(rrt_context* ctx, const rrt_params* prm, const rrt_effects* fx, uint64_t sky_texture, int w, int h,
+              const rrt_band* band, const rrt_planes* traced, void* d_out, int out_layout, float* hdr_out, void* stream);
+
 /* Same call with a HOST destination: renders into a context-owned device frame, copies it to
  * host_rgba (w*h*4 bytes, reference layout) and synchronises.  This is the end-to-end entry point. */
 int rrt_render_host(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, const rrt_effects* fx,
@@ -205,8 +220,8 @@ int rrt_set_sample_pool(rrt_context* ctx, size_t max_bytes_per_stream, int max_p
  * tiles, [1] tiles left to the closing fused sweep, [2] tiles traced by the passes, [3] passes enqueued, [4] tiles of
  * the launch, [5] pool size in Ki slots of 32 bytes; all 0 when no frame went through the split pipeline. */
 int rrt_split_stats(rrt_context* ctx, uint32_t out[8]);
-/* Kernels this context has launched so far for rrt_render* and rrt_assemble_bands (1 per fused frame; 3 per pass + 1
- * per split frame): what a benchmark reports as its launch count. */
+/* Kernels this context has launched so far for rrt_render*, rrt_shade and rrt_assemble_bands (1 per fused frame; 3 per
+ * pass + 1 per split frame; 1 per rrt_shade): what a benchmark reports as its launch count. */
 uint64_t rrt_kernel_launches(rrt_context* ctx);
 
 /* Number of rows a band owns in an h-row image (packed buffer height). */

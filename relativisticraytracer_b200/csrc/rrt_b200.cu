@@ -5,7 +5,7 @@
 //
 // Where things are:
 //   include/rrt_device.cuh   device math: the two rounding contracts, geodesic RHS, RK4, noise, densities
-//   csrc/rrt_kernel.cuh      render_kernel (one 8x4 tile per persistent warp), per-ray helpers, probe kernels
+//   csrc/rrt_kernel.cuh      render_kernel (one 8x4 tile per persistent warp), per-ray helpers, shade_kernel, probe kernels
 //   csrc/rrt_packed.cuh      render_kernel_p (two rays per thread, no medium), FMAD contract only
 //   csrc/rrt_split.cuh       the split pipeline of launches with a medium: trace / media / fold kernels
 //   this file                band assembly, self-test / roofline probes, rrt_context, every extern "C" entry point
@@ -656,6 +656,42 @@ int rrt_render(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, c
         if (ctx->pipeline == RRT_PIPELINE_SPLIT) return fail(ctx, RRT_ERR_NOMEM, "rrt_render: no memory for the sample pool of the split pipeline");
     }
     kern<<<(unsigned)grid, kRenderBlock, 0, st>>>(A);
+    RRT_CU(ctx, cudaGetLastError());
+    ctx->launches += 1;
+    return RRT_OK;
+}
+
+int rrt_shade(rrt_context* ctx, const rrt_params* prm, const rrt_effects* fx, uint64_t sky_texture, int w, int h,
+              const rrt_band* band, const rrt_planes* traced, void* d_out, int out_layout, float* hdr_out, void* stream) {
+    if (!ctx) return RRT_ERR_BAD_ARG;
+    if (!prm || !fx || w <= 0 || h <= 0 || sky_texture == 0 || (out_layout != RRT_OUT_FRAME && out_layout != RRT_OUT_PACKED) ||
+        !traced || !traced->vel || !traced->emis || !traced->hdr || !traced->cls || (!d_out && !hdr_out))
+        return fail(ctx, RRT_ERR_BAD_ARG, "rrt_shade: bad argument");
+    rrt_band b = {0, 1, 1};
+    if (band) b = *band;
+    const int local_rows = rrt_band_rows(&b, h);
+    if (local_rows < 0) return fail(ctx, RRT_ERR_BAD_ARG, "rrt_shade: bad band");
+    if (local_rows == 0) return RRT_OK;
+    if ((long long)w * local_rows > (1ll << 30)) return fail(ctx, RRT_ERR_BAD_ARG, "rrt_shade: band larger than 2^30 pixels");
+
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DevGuard g(ctx->device);
+    FrameArgs A;
+    std::memset(&A, 0, sizeof(A));   // no camera, counters, ticket or tile log: nothing is traced
+    A.C = make_consts(*prm);         // finish_ray_inl reads exposure only
+    A.fx = *fx;
+    A.w = w;
+    A.h = h;
+    A.band_rank = b.rank;
+    A.band_nranks = b.nranks;
+    A.band_group = b.group;
+    A.local_rows = local_rows;
+    A.out_layout = out_layout;
+    A.out = (uchar4*)d_out;
+    A.planes.hdr = hdr_out;
+    A.sky = (cudaTextureObject_t)sky_texture;
+    const long long n = (long long)w * local_rows;
+    kset(prm)->shade<<<(unsigned)((n + kShadeBlock - 1) / kShadeBlock), kShadeBlock, 0, (cudaStream_t)stream>>>(A, *traced);
     RRT_CU(ctx, cudaGetLastError());
     ctx->launches += 1;
     return RRT_OK;

@@ -1,5 +1,5 @@
-// rrt_kernel.cuh -- the render kernel (one 8x4-pixel tile per persistent warp), its per-ray helpers and the
-// function-level probe kernels.  Compiled TWICE, once per rounding contract (include/rrt_device.cuh):
+// rrt_kernel.cuh -- the render kernel (one 8x4-pixel tile per persistent warp), its per-ray helpers, the re-shading
+// kernel (rrt_shade) and the function-level probe kernels.  Compiled TWICE, once per rounding contract (include/rrt_device.cuh):
 //   rrt_b200.cu   RRT_FMAD = 0, nvcc -fmad=false   -> rrt_kernels_strict()
 //   rrt_fmad.cu   RRT_FMAD = 1, nvcc -fmad=true    -> rrt_kernels_fmad()
 // Everything with device code sits in an anonymous namespace (internal linkage per translation unit); the
@@ -45,6 +45,7 @@ struct KernelSet {
     void (*disk_temp)(Consts, int, const float*, float*);
     void (*disk_density)(Consts, int, const float*, float, float*);
     void (*dust_density)(Consts, int, const float*, float, float*);
+    void (*shade)(const FrameArgs, const rrt_planes);  // rrt_shade: the step after the ray loop, from traced planes
 };
 const KernelSet* rrt_kernels_strict();
 const KernelSet* rrt_kernels_fmad();
@@ -514,6 +515,32 @@ __global__ void __launch_bounds__(kRenderBlock, MEDIA ? kMinBlocksMedia : kMinBl
     }
 }
 
+// ---- re-shading (rrt_shade) -------------------------------------------------------------------------
+// Everything after the ray loop again -- finish_ray_inl itself, so every byte is the one the render wrote for the same
+// inputs -- from the planes a render left behind: I from `emis`, T from `hdr.w`, the exit velocity from `vel` (not
+// `dir`: unit3 of an already normalised vector need not return the same bits) and the end bits from `cls`.  A.planes
+// holds only the optional hdr output, which may be `traced.hdr` itself (each thread reads its pixel before it writes
+// it).  One thread per pixel of the band, rows mapped like render_kernel's.
+constexpr int kShadeBlock = 256;
+__global__ void __launch_bounds__(kShadeBlock) shade_kernel(const __grid_constant__ FrameArgs A, const __grid_constant__ rrt_planes traced) {
+    const int i = blockIdx.x * kShadeBlock + threadIdx.x;   // w * local_rows <= 2^30 (rrt_shade)
+    if (i >= A.w * A.local_rows) return;
+    const int ly = i / A.w, x = i - ly * A.w;
+    const int grp = ly / A.band_group;
+    const int y = (grp * A.band_nranks + A.band_rank) * A.band_group + (ly - grp * A.band_group);
+    if (y >= A.h) return;
+    const size_t pix = (size_t)y * A.w + x;
+    const float4 v = reinterpret_cast<const float4*>(traced.vel)[pix];
+    const float4 I = reinterpret_cast<const float4*>(traced.emis)[pix];
+    const float4 hdr = reinterpret_cast<const float4*>(traced.hdr)[pix];
+    const unsigned cls = traced.cls[pix];
+    const unsigned end = ((cls & RRT_CLS_MASK) == RRT_CLS_CAPTURED ? kEndCaptured : 0u) |
+                         ((cls & RRT_CLSF_TOUCHED) ? kEndTouched : 0u) | ((cls & RRT_CLSF_EXHAUSTED) ? kEndExhausted : 0u);
+    float uvx, uvy;
+    pixel_uv(A, x, y, uvx, uvy);
+    finish_ray_inl(A, x, y, ly, uvx, uvy, I.x, I.y, I.z, hdr.w, mk(0.f, 0.f, 0.f), mk(v.x, v.y, v.z), 0, end);
+}
+
 // ---- probe kernels ---------------------------------------------------------------------------------
 __device__ __forceinline__ V3 ld3(const float* a, int i) { return mk(a[3 * i], a[3 * i + 1], a[3 * i + 2]); }
 __device__ __forceinline__ void st3(float* a, int i, V3 v) { a[3 * i] = v.x; a[3 * i + 1] = v.y; a[3 * i + 2] = v.z; }
@@ -589,6 +616,7 @@ const rrtk::KernelSet kKernelSet = {
     {nullptr, nullptr},
 #endif
     k_acc, k_rk4, k_euler, k_redshift, k_hash31, k_noise3d, k_fbm, k_disk_temp, k_disk_density, k_dust_density,
+    shade_kernel,
 };
 }  // namespace
 

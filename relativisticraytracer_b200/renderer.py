@@ -82,6 +82,8 @@ class Sky:
 
 PLANE_SPECS = {"hdr": (4, torch.float32), "dir": (4, torch.float32), "emis": (4, torch.float32),
                "pos": (4, torch.float32), "vel": (4, torch.float32), "cls": (0, torch.uint8), "steps": (0, torch.int32)}
+# the planes Renderer.shade / rrt_shade re-shade a traced frame from (16 + 16 + 16 + 1 bytes per pixel)
+TRACE_PLANES = ("hdr", "emis", "vel", "cls")
 
 
 class PeerFrame:
@@ -168,28 +170,56 @@ class Renderer:
                planes: Optional[dict] = None, stream: Optional[torch.cuda.Stream] = None) -> torch.Tensor:
         """rrt_render: one frame (or one band of it) into a device uchar4 tensor; asynchronous."""
         tex = sky.texture if isinstance(sky, Sky) else int(sky)
-        rows = h if layout == OUT_FRAME else self.band_rows(band, h)
-        if isinstance(out, PeerFrame):      # a frame that lives on the encoding GPU (possibly another process's)
-            assert layout == OUT_FRAME and out.nbytes >= h * w * 4
-            out_ptr = out.ptr
-        else:
-            if out is None:
-                out = torch.empty((rows, w, 4), dtype=torch.uint8, device=self.device)
-            assert out.is_cuda and out.dtype == torch.uint8 and out.is_contiguous() and out.numel() >= rows * w * 4
-            out_ptr = out.data_ptr()
-        pl = None
-        if planes:
-            pl = Planes()
-            for n, t in planes.items():
-                ch, dt = PLANE_SPECS[n]
-                assert t.is_cuda and t.dtype == dt and t.is_contiguous() and t.numel() == h * w * max(ch, 1), n
-                setattr(pl, n, t.data_ptr())
+        out, out_ptr = self._frame_out(out, layout, band, w, h)
+        pl = self._planes(planes, w, h) if planes else None
         st = stream if stream is not None else torch.cuda.current_stream(self.device)
         self._check(self._lib.rrt_render(self._ctx, C.byref(prm), C.byref(cam), C.byref(fx), C.c_uint64(tex),
                                          float(time), int(w), int(h), C.byref(band) if band is not None else None,
                                          C.c_void_p(out_ptr), int(layout),
                                          C.byref(pl) if pl is not None else None, C.c_void_p(st.cuda_stream)))
         return out
+
+    def shade(self, prm: Params, fx: Effects, sky: Sky | int, traced: dict, w: int, h: int, *, band: Optional[Band] = None,
+              out: Optional[torch.Tensor] = None, layout: int = OUT_FRAME, hdr_out: Optional[torch.Tensor] = None,
+              stream: Optional[torch.cuda.Stream] = None) -> torch.Tensor:
+        """rrt_shade: the step after the ray loop (sky, bloom, vignette, chromatic aberration, exposure tonemap, store)
+        again from the planes of an earlier ``render(..., planes=traced)`` with at least TRACE_PLANES, without tracing;
+        asynchronous.  Gives the bytes (and ``hdr_out`` values) of a fresh render with this sky, exposure and bloom /
+        vignette / CA settings; ``prm`` must keep the trace's FLAG_FMAD bit and ``fx`` its lens fields.  ``band``,
+        ``out`` (a tensor or a PeerFrame) and ``layout`` as in ``render``; returns the frame."""
+        tex = sky.texture if isinstance(sky, Sky) else int(sky)
+        out, out_ptr = self._frame_out(out, layout, band, w, h)
+        pl = self._planes(traced, w, h)
+        hdr_ptr = self._plane_ptr("hdr", hdr_out, w, h) if hdr_out is not None else None
+        st = stream if stream is not None else torch.cuda.current_stream(self.device)
+        self._check(self._lib.rrt_shade(self._ctx, C.byref(prm), C.byref(fx), C.c_uint64(tex), int(w), int(h),
+                                        C.byref(band) if band is not None else None, C.byref(pl), C.c_void_p(out_ptr),
+                                        int(layout), C.c_void_p(hdr_ptr), C.c_void_p(st.cuda_stream)))
+        return out
+
+    def _frame_out(self, out, layout: int, band: Optional[Band], w: int, h: int):
+        """(out, device pointer) of a uchar4 destination: a PeerFrame, a device tensor, or None (allocated here)."""
+        if isinstance(out, PeerFrame):      # a frame that lives on the encoding GPU (possibly another process's)
+            assert layout == OUT_FRAME and out.nbytes >= h * w * 4
+            return out, out.ptr
+        rows = h if layout == OUT_FRAME else self.band_rows(band, h)
+        if out is None:
+            out = torch.empty((rows, w, 4), dtype=torch.uint8, device=self.device)
+        assert out.is_cuda and out.dtype == torch.uint8 and out.is_contiguous() and out.numel() >= rows * w * 4
+        return out, out.data_ptr()
+
+    @staticmethod
+    def _plane_ptr(name: str, t: torch.Tensor, w: int, h: int) -> int:
+        ch, dt = PLANE_SPECS[name]
+        assert t.is_cuda and t.dtype == dt and t.is_contiguous() and t.numel() == h * w * max(ch, 1), name
+        return t.data_ptr()
+
+    @classmethod
+    def _planes(cls, planes: dict, w: int, h: int) -> Planes:
+        pl = Planes()
+        for n, t in planes.items():
+            setattr(pl, n, cls._plane_ptr(n, t, w, h))
+        return pl
 
     def render_host(self, prm: Params, cam: Camera, fx: Effects, sky: Sky | int, time: float, w: int, h: int,
                     host_out) -> None:
