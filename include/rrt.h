@@ -178,6 +178,43 @@ int rrt_render(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, c
 int rrt_shade(rrt_context* ctx, const rrt_params* prm, const rrt_effects* fx, uint64_t sky_texture, int w, int h,
               const rrt_band* band, const rrt_planes* traced, void* d_out, int out_layout, float* hdr_out, void* stream);
 
+/* ---- supersampled (anti-aliased) frames: ss x ss rays per pixel, ss = 1 .. 8 --------------------------------------
+ * Sub-sample (i, j) of output pixel (x, y) is pixel (ss*x + i, ss*y + j) of the ss*w x ss*h render with the same
+ * parameters, camera, effects, sky and time, so its ray is that render's ray bit for bit (lens distortion and chromatic
+ * aberration included: they act per sub-sample).  The pixel's linear final_hdr (and T, in .w) is the mean of its ss*ss
+ * sub-samples, summed from (0,0) in row-major order (j outer, i inner) in round-to-nearest float32 and divided by
+ * (float)(ss*ss); bloom, vignette (at the output pixel's own image-plane coordinate), exposure tonemap and the store
+ * then run exactly as in rrt_render.  ss = 1 is rrt_render: same bytes, same hdr values.
+ * Known shift: the sub-samples cover the pixel's footprint [x/w, (x+1)/w) while a 1-sample ray sits on its corner x/w,
+ * so for ss > 1 the image moves by (ss-1)/(2*ss) of a pixel against a 1-sample render.  That is the price of being the
+ * larger render exactly, which is what makes the result checkable bit for bit. */
+
+/* Box-filters an ss*w x ss*h hdr plane (float4, [Y*ss*w + X], as rrt_render / rrt_shade write it) into a w x h frame:
+ * mean of each ss x ss block in a fixed order, then bloom / vignette / tonemap / store exactly as rrt_render.
+ * Writes d_out (layout as in rrt_render, only the band's rows) and/or hdr_out (float4 per pixel, w x h full-frame
+ * indexed, the band's pixels only, the mean before bloom, like rrt_render's hdr plane); hdr_out must not overlap hdr_hi.
+ * Reads only the sub-rows of the band's rows.  Uses prm->exposure and the contract bit prm->flags & RRT_FLAG_FMAD.
+ * Asynchronous on `stream`; adds nothing to the counters and one launch.
+ * Re-shading a supersampled frame: rrt_shade at ss*w x ss*h from the planes of rrt_render(ss*w, ss*h), with hdr_out
+ * set to an ss*w x ss*h plane, followed by rrt_resolve of that plane, gives rrt_render_ss with the new sky, exposure and
+ * effects. */
+int rrt_resolve(rrt_context* ctx, const rrt_params* prm, const rrt_effects* fx, int ss, int w, int h,
+                const rrt_band* band, const float* hdr_hi, void* d_out, int out_layout, float* hdr_out, void* stream);
+
+/* rrt_render with ss x ss rays per pixel: traces the ss*w x ss*h frame into context-owned scratch (hdr plane only,
+ * d_out = NULL, band {rank, nranks, ss*group}) and resolves it with rrt_resolve.  Same arguments as rrt_render plus ss;
+ * planes other than the averaged hdr_out are not offered.
+ * Band {r, N, g} traces band {r, N, ss*g} of the large frame: trace group (ss*y + j) / (ss*g) is y / g, so a rank traces
+ * exactly the sub-rows of its own rows, and band-parallel frames (packed buffers or a peer frame) work as with rrt_render.
+ * Scratch: one 16*ss*ss*w*h-byte plane per call (full-frame even for a band: 133 MB for 1920x1080 at ss = 2, 2.1 GB
+ * for 3840x2160 at ss = 4), taken stream-ordered from a context-owned memory pool that keeps it for the next call, so
+ * calls on different streams can be in flight together.  RRT_ERR_NOMEM, before anything is enqueued, when it cannot be
+ * allocated.  Adds to the counters exactly what rrt_render(ss*w, ss*h) adds (they count sub-rays), and that render's
+ * launches + 1 to rrt_kernel_launches. */
+int rrt_render_ss(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, const rrt_effects* fx,
+                  uint64_t sky_texture, float time, int w, int h, int ss, const rrt_band* band,
+                  void* d_out, int out_layout, float* hdr_out, void* stream);
+
 /* Same call with a HOST destination: renders into a context-owned device frame, copies it to
  * host_rgba (w*h*4 bytes, reference layout) and synchronises.  This is the end-to-end entry point. */
 int rrt_render_host(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, const rrt_effects* fx,
@@ -220,8 +257,9 @@ int rrt_set_sample_pool(rrt_context* ctx, size_t max_bytes_per_stream, int max_p
  * tiles, [1] tiles left to the closing fused sweep, [2] tiles traced by the passes, [3] passes enqueued, [4] tiles of
  * the launch, [5] pool size in Ki slots of 32 bytes; all 0 when no frame went through the split pipeline. */
 int rrt_split_stats(rrt_context* ctx, uint32_t out[8]);
-/* Kernels this context has launched so far for rrt_render*, rrt_shade and rrt_assemble_bands (1 per fused frame; 3 per
- * pass + 1 per split frame; 1 per rrt_shade): what a benchmark reports as its launch count. */
+/* Kernels this context has launched so far for rrt_render*, rrt_shade, rrt_resolve and rrt_assemble_bands (1 per fused
+ * frame; 3 per pass + 1 per split frame; 1 per rrt_shade or rrt_resolve; rrt_render_ss: its ss*w x ss*h render's + 1):
+ * what a benchmark reports as its launch count. */
 uint64_t rrt_kernel_launches(rrt_context* ctx);
 
 /* Number of rows a band owns in an h-row image (packed buffer height). */

@@ -5,7 +5,8 @@
 //
 // Where things are:
 //   include/rrt_device.cuh   device math: the two rounding contracts, geodesic RHS, RK4, noise, densities
-//   csrc/rrt_kernel.cuh      render_kernel (one 8x4 tile per persistent warp), per-ray helpers, shade_kernel, probe kernels
+//   csrc/rrt_kernel.cuh      render_kernel (one 8x4 tile per persistent warp), per-ray helpers, shade_kernel,
+//                            resolve_kernel, probe kernels
 //   csrc/rrt_packed.cuh      render_kernel_p (two rays per thread, no medium), FMAD contract only
 //   csrc/rrt_split.cuh       the split pipeline of launches with a medium: trace / media / fold kernels
 //   this file                band assembly, self-test / roofline probes, rrt_context, every extern "C" entry point
@@ -20,6 +21,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <climits>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -161,7 +163,10 @@ struct rrt_context {
     SamplePool pools[RRT_HOST_SLOTS];
     unsigned long long pool_clock = 0;
     int passes_hint = 2;                  // passes the last frame with history needed: the first guess of a pool without one
-    unsigned long long launches = 0;      // kernels this context has launched for rrt_render* / rrt_assemble_bands
+    // rrt_render_ss's supersampled hdr planes: stream-ordered allocations from this pool (created on first use), which
+    // keeps freed blocks for the next frame instead of returning them to the device
+    cudaMemPool_t ss_pool = nullptr;
+    unsigned long long launches = 0;      // kernels this context has launched for rrt_render* / rrt_shade / rrt_resolve / rrt_assemble_bands
     std::string err;
     std::mutex mu;
 };
@@ -331,6 +336,7 @@ void rrt_context_destroy(rrt_context* ctx) {
         if (pl.h_stats) cudaFreeHost(pl.h_stats);
         if (pl.done) cudaEventDestroy(pl.done);
     }
+    if (ctx->ss_pool) cudaMemPoolDestroy(ctx->ss_pool);
     delete ctx;
 }
 
@@ -695,6 +701,106 @@ int rrt_shade(rrt_context* ctx, const rrt_params* prm, const rrt_effects* fx, ui
     RRT_CU(ctx, cudaGetLastError());
     ctx->launches += 1;
     return RRT_OK;
+}
+
+// What rrt_resolve and rrt_render_ss both check: ss, the ss*w x ss*h frame and the band, whose traced form {rank, nranks,
+// ss*group} must stay within rrt_render's 2^30 rays.  Sets *local_rows, the band's rows of the w x h frame.
+static int check_ss(rrt_context* ctx, const char* what, int ss, int w, int h, const rrt_band* band, int* local_rows) {
+    std::string m = what;
+    if (ss < 1 || ss > 8 || w <= 0 || h <= 0 || (long long)ss * w > INT_MAX || (long long)ss * h > INT_MAX)
+        return fail(ctx, RRT_ERR_BAD_ARG, (m + ": bad argument").c_str());
+    const int rows = rrt_band_rows(band, h);
+    if (rows < 0 || (band && (long long)ss * band->group > INT_MAX)) return fail(ctx, RRT_ERR_BAD_ARG, (m + ": bad band").c_str());
+    if ((long long)ss * ss * w * rows > (1ll << 30)) return fail(ctx, RRT_ERR_BAD_ARG, (m + ": band larger than 2^30 sub-samples").c_str());
+    *local_rows = rows;
+    return RRT_OK;
+}
+
+int rrt_resolve(rrt_context* ctx, const rrt_params* prm, const rrt_effects* fx, int ss, int w, int h, const rrt_band* band,
+                const float* hdr_hi, void* d_out, int out_layout, float* hdr_out, void* stream) {
+    if (!ctx) return RRT_ERR_BAD_ARG;
+    if (!prm || !fx || !hdr_hi || (out_layout != RRT_OUT_FRAME && out_layout != RRT_OUT_PACKED) || (!d_out && !hdr_out))
+        return fail(ctx, RRT_ERR_BAD_ARG, "rrt_resolve: bad argument");
+    int local_rows = 0;
+    if (int rc = check_ss(ctx, "rrt_resolve", ss, w, h, band, &local_rows)) return rc;
+    if (hdr_out) {   // the kernel reads hdr_hi while it writes hdr_out: the two must not share a byte (counted in float4s)
+        const uintptr_t a = (uintptr_t)hdr_hi, b = (uintptr_t)hdr_out;
+        if (b >= a ? (b - a) / 16 < (unsigned long long)ss * ss * w * h : (a - b) / 16 < (unsigned long long)w * h)
+            return fail(ctx, RRT_ERR_BAD_ARG, "rrt_resolve: hdr_out overlaps hdr_hi");
+    }
+    if (local_rows == 0) return RRT_OK;
+
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DevGuard g(ctx->device);
+    FrameArgs A;
+    std::memset(&A, 0, sizeof(A));   // no camera, sky, counters, ticket or tile log: nothing is traced or sampled
+    A.C = make_consts(*prm);         // the post step reads exposure only
+    A.fx = *fx;
+    A.w = w;
+    A.h = h;
+    if (band) {
+        A.band_rank = band->rank;
+        A.band_nranks = band->nranks;
+        A.band_group = band->group;
+    } else {
+        A.band_nranks = A.band_group = 1;
+    }
+    A.local_rows = local_rows;
+    A.out_layout = out_layout;
+    A.out = (uchar4*)d_out;
+    A.planes.hdr = hdr_out;
+    const long long n = (long long)w * local_rows;
+    kset(prm)->resolve<<<(unsigned)((n + kResolveBlock - 1) / kResolveBlock), kResolveBlock, 0, (cudaStream_t)stream>>>(
+        A, (const float4*)hdr_hi, ss);
+    RRT_CU(ctx, cudaGetLastError());
+    ctx->launches += 1;
+    return RRT_OK;
+}
+
+int rrt_render_ss(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, const rrt_effects* fx, uint64_t sky_texture,
+                  float time, int w, int h, int ss, const rrt_band* band, void* d_out, int out_layout, float* hdr_out,
+                  void* stream) {
+    if (!ctx) return RRT_ERR_BAD_ARG;
+    if (!prm || !cam || !fx || sky_texture == 0 || prm->max_steps < 0 || (out_layout != RRT_OUT_FRAME && out_layout != RRT_OUT_PACKED) ||
+        (!d_out && !hdr_out))
+        return fail(ctx, RRT_ERR_BAD_ARG, "rrt_render_ss: bad argument");
+    int local_rows = 0;
+    if (int rc = check_ss(ctx, "rrt_render_ss", ss, w, h, band, &local_rows)) return rc;
+    if (local_rows == 0) return RRT_OK;
+    // output group y / g is trace group (ss*y + j) / (ss*g): the band traces exactly the sub-rows of its own rows
+    rrt_band tb = {0, 1, ss};
+    if (band) tb = {band->rank, band->nranks, ss * band->group};
+    cudaStream_t st = (cudaStream_t)stream;
+    float* hi = nullptr;   // full-frame indexed like every plane of this ABI, so full-frame sized even for a band
+    const unsigned long long n_hi = (unsigned long long)ss * ss * w * h;
+    if (n_hi > SIZE_MAX / 16) return fail(ctx, RRT_ERR_NOMEM, "rrt_render_ss: supersampled hdr plane larger than the address space");
+    {
+        std::lock_guard<std::mutex> lk(ctx->mu);
+        DevGuard g(ctx->device);
+        if (!ctx->ss_pool) {
+            cudaMemPoolProps props;
+            std::memset(&props, 0, sizeof(props));
+            props.allocType = cudaMemAllocationTypePinned;
+            props.location.type = cudaMemLocationTypeDevice;
+            props.location.id = ctx->device;
+            RRT_CU(ctx, cudaMemPoolCreate(&ctx->ss_pool, &props));
+            uint64_t keep = UINT64_MAX;   // hold freed blocks: the next frame of a sequence reuses them without a new allocation
+            RRT_CU(ctx, cudaMemPoolSetAttribute(ctx->ss_pool, cudaMemPoolAttrReleaseThreshold, &keep));
+        }
+        if (cudaMallocFromPoolAsync((void**)&hi, (size_t)16 * n_hi, ctx->ss_pool, st) != cudaSuccess) {
+            cudaGetLastError();
+            return fail(ctx, RRT_ERR_NOMEM, "rrt_render_ss: no memory for the supersampled hdr plane");
+        }
+    }
+    rrt_planes pl;
+    std::memset(&pl, 0, sizeof(pl));
+    pl.hdr = hi;
+    int rc = rrt_render(ctx, prm, cam, fx, sky_texture, time, ss * w, ss * h, &tb, nullptr, RRT_OUT_FRAME, &pl, stream);
+    if (rc == RRT_OK) rc = rrt_resolve(ctx, prm, fx, ss, w, h, band, hi, d_out, out_layout, hdr_out, stream);
+    DevGuard g(ctx->device);
+    const cudaError_t e = cudaFreeAsync(hi, st);   // stream-ordered: the block goes back to the pool once the resolve has read it
+    if (rc == RRT_OK && e != cudaSuccess) return fail(ctx, RRT_ERR_CUDA, "rrt_render_ss: cudaFreeAsync", e);
+    return rc;
 }
 
 int rrt_render_host_async(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, const rrt_effects* fx,

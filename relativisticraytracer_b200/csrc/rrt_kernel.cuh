@@ -1,5 +1,6 @@
 // rrt_kernel.cuh -- the render kernel (one 8x4-pixel tile per persistent warp), its per-ray helpers, the re-shading
-// kernel (rrt_shade) and the function-level probe kernels.  Compiled TWICE, once per rounding contract (include/rrt_device.cuh):
+// kernel (rrt_shade), the supersample resolve kernel (rrt_resolve) and the function-level probe kernels.  Compiled
+// TWICE, once per rounding contract (include/rrt_device.cuh):
 //   rrt_b200.cu   RRT_FMAD = 0, nvcc -fmad=false   -> rrt_kernels_strict()
 //   rrt_fmad.cu   RRT_FMAD = 1, nvcc -fmad=true    -> rrt_kernels_fmad()
 // Everything with device code sits in an anonymous namespace (internal linkage per translation unit); the
@@ -46,6 +47,7 @@ struct KernelSet {
     void (*disk_density)(Consts, int, const float*, float, float*);
     void (*dust_density)(Consts, int, const float*, float, float*);
     void (*shade)(const FrameArgs, const rrt_planes);  // rrt_shade: the step after the ray loop, from traced planes
+    void (*resolve)(const FrameArgs, const float4*, int);  // rrt_resolve: box filter of an ss x ss hdr plane + post step
 };
 const KernelSet* rrt_kernels_strict();
 const KernelSet* rrt_kernels_fmad();
@@ -172,10 +174,10 @@ __device__ __forceinline__ V3 ray_dir(const FrameArgs& A, int x, int y) {
 
 constexpr unsigned kEndCaptured = 1u, kEndTouched = 2u, kEndExhausted = 4u;
 
-// Everything after the loop for one ray: background, final assembly, planes, effects, tonemap, store
-// (reference :123-173).  (uvx, uvy) is the distorted image-plane coordinate of the pixel.
-__device__ __forceinline__ void finish_ray_inl(const FrameArgs& A, int x, int y, int ly, float uvx, float uvy, float Ir, float Ig,
-                                               float Ib, float T, V3 p, V3 v, int steps, unsigned end) {
+// The first half of finish_ray_inl: background, final assembly (reference :123-150) and the planes.  Returns final_hdr
+// in (hr, hg, hb).
+__device__ __forceinline__ void compose_ray_inl(const FrameArgs& A, int x, int y, float Ir, float Ig, float Ib, float T, V3 p,
+                                                V3 v, int steps, unsigned end, float& hr, float& hg, float& hb) {
     using namespace rrt;
     float bg[3] = {0.f, 0.f, 0.f};
     V3 d = mk(0.f, 0.f, 0.f);
@@ -191,7 +193,7 @@ __device__ __forceinline__ void finish_ray_inl(const FrameArgs& A, int x, int y,
         float4 sB = tex2D<float4>(A.sky, 0.5f + (phi0 + -off) / (2.0f * kPi), ty_);
         bg[0] = sR.x; bg[1] = sG.y; bg[2] = sB.z;
     }
-    float hr = mad(bg[0], T, Ir), hg = mad(bg[1], T, Ig), hb = mad(bg[2], T, Ib);  // :148-150
+    hr = mad(bg[0], T, Ir); hg = mad(bg[1], T, Ig); hb = mad(bg[2], T, Ib);  // :148-150
     const bool touched = (end & kEndTouched) != 0, exhausted = (end & kEndExhausted) != 0;
     const size_t pix = (size_t)y * A.w + x;
     const uint8_t cls = (uint8_t)((captured ? RRT_CLS_CAPTURED : (touched ? RRT_CLS_DISK_HIT : RRT_CLS_ESCAPED)) |
@@ -203,7 +205,13 @@ __device__ __forceinline__ void finish_ray_inl(const FrameArgs& A, int x, int y,
     if (A.planes.vel) reinterpret_cast<float4*>(A.planes.vel)[pix] = make_float4(v.x, v.y, v.z, 0.f);
     if (A.planes.cls) A.planes.cls[pix] = cls;
     if (A.planes.steps) A.planes.steps[pix] = steps;
-    if (!A.out) return;
+}
+// The second half: bloom, vignette, exposure tonemap and the store of the pixel's final_hdr (reference :154-168).
+// (uvx, uvy) is the distorted image-plane coordinate of the pixel.  Shared by every render kernel (through
+// finish_ray_inl), shade_kernel and resolve_kernel.
+__device__ __forceinline__ void post_ray_inl(const FrameArgs& A, int x, int y, int ly, float uvx, float uvy, float hr, float hg,
+                                             float hb) {
+    using namespace rrt;
     if (A.fx.use_bloom) {  // :154-157, post_processing.h:27-31
         const float lum = dot3(mk(hr, hg, hb), mk(0.2126f, 0.7152f, 0.0722f));
         float b0 = 0.f, b1 = 0.f, b2 = 0.f;
@@ -225,6 +233,15 @@ __device__ __forceinline__ void finish_ray_inl(const FrameArgs& A, int x, int y,
     const uchar4 px = make_uchar4((unsigned char)(o_r * 255), (unsigned char)(o_g * 255), (unsigned char)(o_b * 255), 255);
     if (A.out_layout == RRT_OUT_FRAME) A.out[(size_t)(A.h - 1 - y) * A.w + x] = px;  // :168
     else A.out[(size_t)ly * A.w + x] = px;
+}
+// Everything after the loop for one ray: background, final assembly, planes, effects, tonemap, store
+// (reference :123-173).  (uvx, uvy) is the distorted image-plane coordinate of the pixel.
+__device__ __forceinline__ void finish_ray_inl(const FrameArgs& A, int x, int y, int ly, float uvx, float uvy, float Ir, float Ig,
+                                               float Ib, float T, V3 p, V3 v, int steps, unsigned end) {
+    float hr, hg, hb;
+    compose_ray_inl(A, x, y, Ir, Ig, Ib, T, p, v, steps, end, hr, hg, hb);
+    if (!A.out) return;
+    post_ray_inl(A, x, y, ly, uvx, uvy, hr, hg, hb);
 }
 // out-of-line copy for the kernels that finalise rays one at a time from several places
 __device__ __noinline__ void finish_ray(const FrameArgs& A, int x, int y, int ly, float Ir, float Ig, float Ib, float T, V3 p,
@@ -541,6 +558,38 @@ __global__ void __launch_bounds__(kShadeBlock) shade_kernel(const __grid_constan
     finish_ray_inl(A, x, y, ly, uvx, uvy, I.x, I.y, I.z, hdr.w, mk(0.f, 0.f, 0.f), mk(v.x, v.y, v.z), 0, end);
 }
 
+// ---- supersample resolve (rrt_resolve, rrt_render_ss) -----------------------------------------------
+// Box filter of an ss*w x ss*h hdr plane `hi` ([Y * ss*w + X]) into the w x h frame of A: output pixel (x, y) is the mean
+// of sub-samples (ss*x + i, ss*y + j), summed from (0, 0) in row-major order (j outer, i inner) and divided by ss*ss, with
+// the explicit round-to-nearest intrinsics so that both contracts give the same bits (and numpy reproduces them).  The
+// mean (.w = mean T) goes to A.planes.hdr, then the render's own post step (bloom, vignette at the output pixel's
+// pixel_uv, tonemap, store) runs on it.  One thread per output pixel of the band, rows mapped like shade_kernel's;
+// neighbouring threads read neighbouring ss*16-byte runs of each sub-row.
+constexpr int kResolveBlock = 256;
+__global__ void __launch_bounds__(kResolveBlock) resolve_kernel(const __grid_constant__ FrameArgs A, const float4* __restrict__ hi, int ss) {
+    const int i = blockIdx.x * kResolveBlock + threadIdx.x;   // w * local_rows <= 2^30 (rrt_resolve)
+    if (i >= A.w * A.local_rows) return;
+    const int ly = i / A.w, x = i - ly * A.w;
+    const int grp = ly / A.band_group;
+    const int y = (grp * A.band_nranks + A.band_rank) * A.band_group + (ly - grp * A.band_group);
+    if (y >= A.h) return;
+    const size_t W = (size_t)ss * A.w;
+    const float4* p = hi + (size_t)ss * y * W + (size_t)ss * x;
+    float4 s = p[0];
+    for (int j = 0; j < ss; ++j)
+        for (int k = j == 0 ? 1 : 0; k < ss; ++k) {
+            const float4 v = p[j * W + k];
+            s.x = __fadd_rn(s.x, v.x); s.y = __fadd_rn(s.y, v.y); s.z = __fadd_rn(s.z, v.z); s.w = __fadd_rn(s.w, v.w);
+        }
+    const float n = (float)(ss * ss);
+    s = make_float4(__fdiv_rn(s.x, n), __fdiv_rn(s.y, n), __fdiv_rn(s.z, n), __fdiv_rn(s.w, n));
+    if (A.planes.hdr) reinterpret_cast<float4*>(A.planes.hdr)[(size_t)y * A.w + x] = s;
+    if (!A.out) return;
+    float uvx, uvy;
+    pixel_uv(A, x, y, uvx, uvy);
+    post_ray_inl(A, x, y, ly, uvx, uvy, s.x, s.y, s.z);
+}
+
 // ---- probe kernels ---------------------------------------------------------------------------------
 __device__ __forceinline__ V3 ld3(const float* a, int i) { return mk(a[3 * i], a[3 * i + 1], a[3 * i + 2]); }
 __device__ __forceinline__ void st3(float* a, int i, V3 v) { a[3 * i] = v.x; a[3 * i + 1] = v.y; a[3 * i + 2] = v.z; }
@@ -616,7 +665,7 @@ const rrtk::KernelSet kKernelSet = {
     {nullptr, nullptr},
 #endif
     k_acc, k_rk4, k_euler, k_redshift, k_hash31, k_noise3d, k_fbm, k_disk_temp, k_disk_density, k_dust_density,
-    shade_kernel,
+    shade_kernel, resolve_kernel,
 };
 }  // namespace
 

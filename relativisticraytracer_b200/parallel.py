@@ -301,19 +301,24 @@ class PathSequence:
     rank 0 (the encoding GPU), which copies them to pinned host memory and hands them to the sink in frame order.  Rounds
     are pipelined ``depth`` deep on separate streams like ``FramePipeline``.  Camera and clock come from the
     C-ABI host functions (``rrt_path_state`` / ``rrt_path_clock``), so frame k is the same pure function of k
-    on every rank count."""
+    on every rank count.  ``ss`` > 1 renders every frame anti-aliased with ss x ss rays per pixel (``Renderer.render_ss``
+    into the slot's device frame, then the same pinned copy), which keeps the photon ring, the disk's inner edge and the
+    stars from crawling between frames."""
 
-    def __init__(self, renderer, w: int, h: int, depth: int = 2):
+    def __init__(self, renderer, w: int, h: int, depth: int = 2, ss: int = 1):
         if not 1 <= depth <= HOST_SLOTS:
             raise ValueError(f"depth must be 1..{HOST_SLOTS}")
-        self.r, self.w, self.h, self.depth = renderer, w, h, depth
+        if not 1 <= ss <= 8:
+            raise ValueError("ss must be 1..8")
+        self.r, self.w, self.h, self.depth, self.ss = renderer, w, h, depth, ss
         self.world = dist.get_world_size() if dist.is_initialized() else 1
         self.rank = dist.get_rank() if dist.is_initialized() else 0
         dev = renderer.device
         self.streams = [torch.cuda.Stream(device=dev) for _ in range(depth)]
         self.events = [torch.cuda.Event() for _ in range(depth)]
         root = self.rank == 0
-        self.local = [torch.zeros((h, w, 4), dtype=torch.uint8, device=dev) for _ in range(depth)] if self.world > 1 else None
+        self.local = ([torch.zeros((h, w, 4), dtype=torch.uint8, device=dev) for _ in range(depth)]
+                      if self.world > 1 or ss > 1 else None)
         self.gathered = ([torch.zeros((self.world, h, w, 4), dtype=torch.uint8, device=dev) for _ in range(depth)]
                          if root and self.world > 1 else None)
         self.host = [torch.zeros((self.world, h, w, 4), dtype=torch.uint8).pin_memory() for _ in range(depth)] if root else None
@@ -349,7 +354,7 @@ class PathSequence:
             mine = frames[self.rank]
             s = self.streams[k]
             with torch.cuda.stream(s):
-                if self.world == 1:
+                if self.world == 1 and self.ss == 1:
                     t = path_clock(mine, fps)
                     cam, _ = path_state(path_index, t)
                     self.r.render_host_async(prm, cam, fx, sky, t, self.w, self.h, self.host[k][0], slot=k, stream=s)
@@ -357,8 +362,13 @@ class PathSequence:
                     if mine is not None:
                         t = path_clock(mine, fps)
                         cam, _ = path_state(path_index, t)
-                        self.r.render(prm, cam, fx, sky, t, self.w, self.h, out=self.local[k], stream=s)
-                    if self.rank == 0:
+                        if self.ss == 1:
+                            self.r.render(prm, cam, fx, sky, t, self.w, self.h, out=self.local[k], stream=s)
+                        else:
+                            self.r.render_ss(prm, cam, fx, sky, t, self.w, self.h, self.ss, out=self.local[k], stream=s)
+                    if self.world == 1:
+                        self.host[k][0].copy_(self.local[k], non_blocking=True)
+                    elif self.rank == 0:
                         dist.gather(self.local[k], list(self.gathered[k].unbind(0)), dst=0)
                         self.host[k].copy_(self.gathered[k], non_blocking=True)
                     else:

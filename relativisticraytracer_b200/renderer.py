@@ -197,6 +197,39 @@ class Renderer:
                                         int(layout), C.c_void_p(hdr_ptr), C.c_void_p(st.cuda_stream)))
         return out
 
+    def render_ss(self, prm: Params, cam: Camera, fx: Effects, sky: Sky | int, time: float, w: int, h: int, ss: int, *,
+                  band: Optional[Band] = None, out=None, layout: int = OUT_FRAME, hdr_out: Optional[torch.Tensor] = None,
+                  stream: Optional[torch.cuda.Stream] = None) -> torch.Tensor:
+        """rrt_render_ss: one anti-aliased frame (or band) with ss x ss rays per pixel, 1 <= ss <= 8; asynchronous.
+        Pixel (x, y) is the box-filtered mean of pixels (ss*x + i, ss*y + j) of the ss*w x ss*h render, then the render's
+        own bloom / vignette / tonemap; ss = 1 is ``render``.  ``hdr_out`` (h, w, 4) float32 receives the averaged linear
+        value (.w = mean T).  ``band``, ``out`` (a tensor or a PeerFrame) and ``layout`` as in ``render``."""
+        tex = sky.texture if isinstance(sky, Sky) else int(sky)
+        out, out_ptr = self._frame_out(out, layout, band, w, h)
+        hdr_ptr = self._plane_ptr("hdr", hdr_out, w, h) if hdr_out is not None else None
+        st = stream if stream is not None else torch.cuda.current_stream(self.device)
+        self._check(self._lib.rrt_render_ss(self._ctx, C.byref(prm), C.byref(cam), C.byref(fx), C.c_uint64(tex), float(time),
+                                            int(w), int(h), int(ss), C.byref(band) if band is not None else None,
+                                            C.c_void_p(out_ptr), int(layout), C.c_void_p(hdr_ptr), C.c_void_p(st.cuda_stream)))
+        return out
+
+    def resolve(self, prm: Params, fx: Effects, hdr_hi: torch.Tensor, ss: int, w: int, h: int, *, band: Optional[Band] = None,
+                out=None, layout: int = OUT_FRAME, hdr_out: Optional[torch.Tensor] = None,
+                stream: Optional[torch.cuda.Stream] = None) -> torch.Tensor:
+        """rrt_resolve: box-filters ``hdr_hi``, the (ss*h, ss*w, 4) float32 hdr plane of a ``render`` or ``shade`` at
+        ss*w x ss*h, into a w x h frame and runs the post step (bloom, vignette, exposure tonemap, store) on it;
+        asynchronous.  ``hdr_out`` ((h, w, 4) float32, not overlapping ``hdr_hi``) receives the mean.  ``band``, ``out``
+        and ``layout`` as in ``render``; returns the frame."""
+        out, out_ptr = self._frame_out(out, layout, band, w, h)
+        assert tuple(hdr_hi.shape) == (ss * h, ss * w, 4), "hdr_hi must be (ss*h, ss*w, 4)"
+        hi_ptr = self._plane_ptr("hdr", hdr_hi, ss * w, ss * h)
+        hdr_ptr = self._plane_ptr("hdr", hdr_out, w, h) if hdr_out is not None else None
+        st = stream if stream is not None else torch.cuda.current_stream(self.device)
+        self._check(self._lib.rrt_resolve(self._ctx, C.byref(prm), C.byref(fx), int(ss), int(w), int(h),
+                                          C.byref(band) if band is not None else None, C.c_void_p(hi_ptr),
+                                          C.c_void_p(out_ptr), int(layout), C.c_void_p(hdr_ptr), C.c_void_p(st.cuda_stream)))
+        return out
+
     def _frame_out(self, out, layout: int, band: Optional[Band], w: int, h: int):
         """(out, device pointer) of a uchar4 destination: a PeerFrame, a device tensor, or None (allocated here)."""
         if isinstance(out, PeerFrame):      # a frame that lives on the encoding GPU (possibly another process's)
