@@ -215,6 +215,44 @@ int rrt_render_ss(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam
                   uint64_t sky_texture, float time, int w, int h, int ss, const rrt_band* band,
                   void* d_out, int out_layout, float* hdr_out, void* stream);
 
+/* ---- captures: one trace, renders at many times -------------------------------------------------------------------
+ * With the camera fixed only the time moves, and the time enters only the disk and dust densities: trajectories, step
+ * counts, classes and the positions of the media samples are the same at every time (a ray ends only at the horizon, on
+ * escape or at max_steps).  A capture traces the frame once, keeps the media samples and the state of the rays the trace
+ * finished, and renders it at any time by evaluating the media and folding them again, without a new trace.
+ * Contract: let the capture be made from (P, cam, F, w, h, band).  rrt_capture_render(P', F', S', t, d_out, layout,
+ * hdr_out) writes exactly the bytes and hdr values of rrt_render(P*, cam, F*, S', t, w, h, band, d_out, layout,
+ * {hdr = hdr_out}), where P* is P with P'.exposure and F* is F with the bloom, vignette and CA fields of F' (the rules of
+ * rrt_shade).  P' must carry P's RRT_FLAG_FMAD bit and F' F's use_lens / distortion_amount, else RRT_ERR_BAD_ARG; every
+ * other field of P' is ignored (the capture keeps P).
+ * Counters: rrt_capture_create adds the trace's (rk4 steps, disk / dust evaluations, classes); each render adds what
+ * depends on the time (dense samples and touched rays of the folded rays) plus everything of the tiles the capture could
+ * not hold, so the capture's counters plus one render's are those of one rrt_render.  Launches (rrt_kernel_launches):
+ * 1 per capture; 3 per render (shade, media, fold), 4 when tiles were left to the fused sweep. */
+typedef struct rrt_capture rrt_capture;
+/* Traces the frame once (no time argument: the trace does not read it) and keeps what a later render needs.  The sky is
+ * sampled by the trace but no render uses it.  Needs a medium (RRT_FLAG_DISK / RRT_FLAG_DUST; without one nothing depends
+ * on the time: re-shade with rrt_shade) and a max_steps the split pipeline can describe; else RRT_ERR_BAD_ARG, as for the
+ * arguments rrt_render refuses.  max_bytes: size of the sample pool the trace runs in (0: the context's sizing rule, as
+ * rrt_render's pool, at most rrt_set_sample_pool's limit).  Tiles whose samples do not fit it are rendered by the fused
+ * sweep at every render: correct for any max_bytes, fast when the frame fits.  Device memory held afterwards: the used
+ * part of the pool (32 B per slot) plus 16 B of media results per slot, the queued ray groups, and four full-frame planes
+ * of 49 B per pixel (vel, emis, hdr, cls; full-frame even for a band).  Synchronises `stream` (a cudaStream_t).
+ * Destroy captures before their context. */
+int rrt_capture_create(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, const rrt_effects* fx,
+                       uint64_t sky_texture, int w, int h, const rrt_band* band, size_t max_bytes, void* stream,
+                       rrt_capture** out);
+/* Evaluates the media at `time`, then folds, shades and stores: d_out (layout as in rrt_render, only the band's rows)
+ * and/or hdr_out (float4 per pixel, full-frame indexed, the band's pixels only).  Asynchronous on `stream`.  One capture
+ * serves one render at a time: each render waits for the capture's previous render, on whatever stream it was enqueued. */
+int rrt_capture_render(rrt_capture* cap, const rrt_params* prm, const rrt_effects* fx, uint64_t sky_texture,
+                       float time, void* d_out, int out_layout, float* hdr_out, void* stream);
+/* [0] media samples kept, [1] pool slots held (32 B each), [2] device bytes held in all, [3] ray groups of 32 queued
+ * for media + fold, [4] tiles left to the fused sweep (16x4 tiles for the packed tracer, else 8x4), [5] 1 if the
+ * packed tracer traced it, [6] tiles of the frame (same unit as [4]), [7] bytes of the pool the trace ran in. */
+int rrt_capture_info(const rrt_capture* cap, uint64_t out[8]);
+void rrt_capture_destroy(rrt_capture* cap);
+
 /* Same call with a HOST destination: renders into a context-owned device frame, copies it to
  * host_rgba (w*h*4 bytes, reference layout) and synchronises.  This is the end-to-end entry point. */
 int rrt_render_host(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, const rrt_effects* fx,
@@ -257,8 +295,9 @@ int rrt_set_sample_pool(rrt_context* ctx, size_t max_bytes_per_stream, int max_p
  * tiles, [1] tiles left to the closing fused sweep, [2] tiles traced by the passes, [3] passes enqueued, [4] tiles of
  * the launch, [5] pool size in Ki slots of 32 bytes; all 0 when no frame went through the split pipeline. */
 int rrt_split_stats(rrt_context* ctx, uint32_t out[8]);
-/* Kernels this context has launched so far for rrt_render*, rrt_shade, rrt_resolve and rrt_assemble_bands (1 per fused
- * frame; 3 per pass + 1 per split frame; 1 per rrt_shade or rrt_resolve; rrt_render_ss: its ss*w x ss*h render's + 1):
+/* Kernels this context has launched so far for rrt_render*, rrt_shade, rrt_resolve, rrt_capture_* and rrt_assemble_bands
+ * (1 per fused frame; 3 per pass + 1 per split frame; 1 per rrt_shade or rrt_resolve; rrt_render_ss: its ss*w x ss*h
+ * render's + 1; 1 per rrt_capture_create, 3 or 4 per rrt_capture_render):
  * what a benchmark reports as its launch count. */
 uint64_t rrt_kernel_launches(rrt_context* ctx);
 

@@ -21,7 +21,9 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <algorithm>
 #include <climits>
+#include <cstddef>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -441,6 +443,19 @@ static int resident_per_sm(rrt_context* ctx, const void* kern, int block, bool m
     return per_sm;
 }
 
+// Slots of a sample pool for one frame, at most max_bytes: ~128 samples per pixel before a frame is cut into passes, plus
+// what the tracing warps hold in reserve: each takes the rows its tile could need in the worst case (max_steps + 1 rows of
+// 1 KiB per ray of a thread) before it traces it.
+static size_t pool_slots(size_t max_bytes, long long local_pixels, long long grid_trace, int rows_per_tile) {
+    size_t want_bytes = (size_t)local_pixels * 4096 + (size_t)grid_trace * ((size_t)rows_per_tile + 256) * 1024;
+    if (want_bytes < (64ull << 20)) want_bytes = 64ull << 20;
+    if (want_bytes > max_bytes) want_bytes = max_bytes;
+    size_t want_slots = want_bytes / kSlotBytes;
+    if (want_slots > 0xfff00000ull) want_slots = 0xfff00000ull;   // slot indices are 32-bit
+    if (want_slots < 1024) want_slots = 1024;
+    return want_slots;
+}
+
 // The pool this stream renders through: its own if it has one, else a free one, else the least recently used one
 // (stream-ordered behind that pool's last frame).  (Re)allocated when the frame needs more than it holds.  Returns null,
 // with no error set, when the memory is not there: the caller renders fused.
@@ -456,14 +471,7 @@ static rrt_context::SamplePool* acquire_pool(rrt_context* ctx, cudaStream_t st, 
             if (!pl || c.last_use < pl->last_use) pl = &c;
         if (pl->done && cudaStreamWaitEvent(st, pl->done, 0) != cudaSuccess) return nullptr;
     }
-    // ~128 samples per pixel before a frame is cut into passes, plus what the tracing warps hold in reserve: each takes
-    // the rows its tile could need in the worst case (max_steps + 1 rows of 1 KiB per ray of a thread) before it traces it
-    size_t want_bytes = (size_t)local_pixels * 4096 + (size_t)grid_trace * ((size_t)rows_per_tile + 256) * 1024;
-    if (want_bytes < (64ull << 20)) want_bytes = 64ull << 20;
-    if (want_bytes > ctx->pool_bytes_max) want_bytes = ctx->pool_bytes_max;
-    size_t want_slots = want_bytes / kSlotBytes;
-    if (want_slots > 0xfff00000ull) want_slots = 0xfff00000ull;   // slot indices are 32-bit
-    if (want_slots < 1024) want_slots = 1024;
+    const size_t want_slots = pool_slots(ctx->pool_bytes_max, local_pixels, grid_trace, rows_per_tile);
     const bool fresh = !pl->in_use;
     const size_t max_slots = ctx->pool_bytes_max / kSlotBytes;
     const bool resize = pl->cap_slots < want_slots || pl->cap_slots > (max_slots > want_slots ? max_slots : want_slots);   // grows; shrinks only below a lowered limit
@@ -501,6 +509,80 @@ static rrt_context::SamplePool* acquire_pool(rrt_context* ctx, cudaStream_t st, 
     return pl;
 }
 
+// The pass arguments every split pass over a pool of cap_slots slots shares (pass, control block and redo lists are the caller's).
+static rrtk::SplitArgs split_args(uint4* slots, size_t cap_slots, rrtk::TileDesc* desc, rrtk::WorkItem* work, size_t work_cap, bool packed_trace,
+                                  int max_steps, long long grid_trace) {
+    rrtk::SplitArgs S;
+    std::memset(&S, 0, sizeof(S));
+    S.slots = slots;
+    S.capacity = (unsigned)cap_slots;
+    // rows per chunk: as many as leave every tracing warp a few chunks, and few enough chunks per tile for a TileDesc
+    unsigned rows = 128;
+    const unsigned rows_min = (unsigned)(((packed_trace ? 2 : 1) * (max_steps + 1) + 1 + rrtk::kDescChunks - 3) / (rrtk::kDescChunks - 2));
+    while (rows > 8 && rows / 2 >= rows_min && (unsigned long long)rows * 32ull * 8ull * (unsigned long long)grid_trace > cap_slots) rows >>= 1;
+    S.chunk_rows = rows;
+    S.chunk_shift = 0;
+    while ((1u << S.chunk_shift) < rows) ++S.chunk_shift;
+    S.high_water = 0xffffffffu;   // a warp takes its tile's worst-case rows before tracing it: a pass simply ends when the pool is used up
+    S.desc = desc;
+    S.work = work;
+    S.work_cap = (unsigned)(work_cap > 0xffffffffull ? 0xffffffffull : work_cap);
+    S.redo_cap = kRedoCap;
+    S.tile16 = packed_trace ? 1u : 0u;
+    return S;
+}
+
+// The split pipeline's tracer for a launch, as rrt_render picks it, and its persistent grid.
+struct TracePlan {
+    bool packed;                                          // two rays per thread in packed f32x2 registers (FMAD contract)
+    void (*kernel)(const FrameArgs, const rrtk::SplitArgs);
+    long long grid;                                       // already divided by the frames in flight
+    unsigned ntiles;                                      // tickets of the launch: 16x4 tiles (packed) or 8x4 tiles
+    unsigned ngroups;                                     // groups of 32 rays a pass can queue
+    int rows_per_tile;                                    // worst-case sample rows of one tile, exit states included
+};
+// Whether a launch with these parameters can go through the split pipeline: a tile's rows must fit a TileDesc.
+static bool split_fits(const rrt_params* prm) { return prm->max_steps + 2 <= 128 * (rrtk::kDescChunks - 2); }
+static TracePlan plan_trace(rrt_context* ctx, const rrt_params* prm, int w, int local_rows) {
+    const bool spin = prm->spin_a != 0.0f, fmad = (prm->flags & RRT_FLAG_FMAD) != 0;
+    const rrtk::SplitKernels* sk = fmad ? rrtk::rrt_split_kernels_fmad() : rrtk::rrt_split_kernels_strict();
+    TracePlan t;
+    // the tracer: two rays per thread in packed f32x2 registers where that kernel exists (FMAD contract), else one per thread
+    t.packed = sk->trace_packed[0] != nullptr && ctx->trace_choice != 1 && 2ll * (prm->max_steps + 1) + 2 <= 128ll * (rrtk::kDescChunks - 2);
+    t.kernel = t.packed ? sk->trace_packed[spin ? 1 : 0] : sk->trace[spin ? 1 : 0];
+    const int per_sm_trace = resident_per_sm(ctx, (const void*)t.kernel, kRenderBlock, true);
+    const unsigned ntiles8 = (unsigned)(((w + kRTileW - 1) / kRTileW) * ((local_rows + kRTileH - 1) / kRTileH));
+    const unsigned ntiles16 = (unsigned)(((w + kTile16W - 1) / kTile16W) * ((local_rows + kTile16H - 1) / kTile16H));
+    t.ntiles = t.packed ? ntiles16 : ntiles8;
+    t.ngroups = t.packed ? 2 * ntiles16 : ntiles8;
+    t.grid = ((long long)ctx->sm_count * per_sm_trace + ctx->frames_in_flight - 1) / ctx->frames_in_flight;
+    if (t.grid > (long long)t.ntiles) t.grid = t.ntiles;
+    if (t.grid > (long long)kRedoCap) t.grid = kRedoCap;
+    t.rows_per_tile = (t.packed ? 2 : 1) * (prm->max_steps + 1) + 1;
+    return t;
+}
+
+// Everything a render kernel reads about the frame except the planes, counters, ticket and tile log.
+static FrameArgs frame_args(const rrt_params& prm, const rrt_camera& cam, const rrt_effects& fx, uint64_t sky_texture, float time, int w,
+                            int h, const rrt_band& b, int local_rows, int out_layout, void* d_out) {
+    FrameArgs A;
+    std::memset(&A, 0, sizeof(A));
+    A.C = make_consts(prm);
+    A.cam = cam;
+    A.fx = fx;
+    A.time = time;
+    A.w = w;
+    A.h = h;
+    A.band_rank = b.rank;
+    A.band_nranks = b.nranks;
+    A.band_group = b.group;
+    A.local_rows = local_rows;
+    A.out_layout = out_layout;
+    A.out = (uchar4*)d_out;
+    A.sky = (cudaTextureObject_t)sky_texture;
+    return A;
+}
+
 // One frame through trace / media / fold passes and the closing sweep.  `grid_trace` = the persistent grid of the
 // tracing kernels for this launch (already divided by the frames in flight).
 static int render_split(rrt_context* ctx, const FrameArgs& A, bool spin, bool fmad, bool packed_trace, long long grid_trace, cudaStream_t st,
@@ -522,23 +604,7 @@ static int render_split(rrt_context* ctx, const FrameArgs& A, bool spin, bool fm
     if (passes < 1) passes = 1;
     if (passes > ctx->max_passes) passes = ctx->max_passes;
 
-    rrtk::SplitArgs S;
-    std::memset(&S, 0, sizeof(S));
-    S.slots = pl->d_slots;
-    S.capacity = (unsigned)pl->cap_slots;
-    // rows per chunk: as many as leave every tracing warp a few chunks, and few enough chunks per tile for a TileDesc
-    unsigned rows = 128;
-    const unsigned rows_min = (unsigned)(((packed_trace ? 2 : 1) * (A.C.max_steps + 1) + 1 + rrtk::kDescChunks - 3) / (rrtk::kDescChunks - 2));
-    while (rows > 8 && rows / 2 >= rows_min && (unsigned long long)rows * 32ull * 8ull * (unsigned long long)grid_trace > pl->cap_slots) rows >>= 1;
-    S.chunk_rows = rows;
-    S.chunk_shift = 0;
-    while ((1u << S.chunk_shift) < rows) ++S.chunk_shift;
-    S.high_water = 0xffffffffu;   // a warp takes its tile's worst-case rows before tracing it: a pass simply ends when the pool is used up
-    S.desc = pl->d_desc;
-    S.work = pl->d_work;
-    S.work_cap = (unsigned)(pl->work_cap > 0xffffffffull ? 0xffffffffull : pl->work_cap);
-    S.redo_cap = kRedoCap;
-    S.tile16 = packed_trace ? 1u : 0u;
+    rrtk::SplitArgs S = split_args(pl->d_slots, pl->cap_slots, pl->d_desc, pl->d_work, pl->work_cap, packed_trace, A.C.max_steps, grid_trace);
     rrtk::PassCtrl* pcs = (rrtk::PassCtrl*)pl->d_ctrl;
     S.stats = (unsigned*)(pl->d_ctrl + sizeof(rrtk::PassCtrl) * (kMaxPasses + 1));
     unsigned* redo = (unsigned*)(pl->d_ctrl + kCtrlHead);
@@ -588,22 +654,8 @@ int rrt_render(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, c
     std::lock_guard<std::mutex> lk(ctx->mu);
     DevGuard g(ctx->device);
     cudaStream_t st = (cudaStream_t)stream;
-    FrameArgs A;
-    std::memset(&A, 0, sizeof(A));
-    A.C = make_consts(*prm);
-    A.cam = *cam;
-    A.fx = *fx;
-    A.time = time;
-    A.w = w;
-    A.h = h;
-    A.band_rank = b.rank;
-    A.band_nranks = b.nranks;
-    A.band_group = b.group;
-    A.local_rows = local_rows;
-    A.out_layout = out_layout;
-    A.out = (uchar4*)d_out;
+    FrameArgs A = frame_args(*prm, *cam, *fx, sky_texture, time, w, h, b, local_rows, out_layout, d_out);
     if (planes) A.planes = *planes;
-    A.sky = (cudaTextureObject_t)sky_texture;
     A.counters = ctx->d_counters;
     A.tile_log = ctx->tile_log;
     A.tile_log_cap = ctx->tile_log_cap;
@@ -643,22 +695,10 @@ int rrt_render(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, c
     if (grid > need) grid = need;
     // A launch with a medium goes through the split pipeline (csrc/rrt_split.cuh) unless the caller pinned the fused
     // kernel, the tile log is selected, or the pool cannot be allocated.
-    if (media && ctx->pipeline != RRT_PIPELINE_FUSED && (!ctx->tile_log || ctx->pipeline == RRT_PIPELINE_SPLIT) && prm->max_steps + 2 <= 128 * (rrtk::kDescChunks - 2)) {
-        const rrtk::SplitKernels* sk = fmad ? rrtk::rrt_split_kernels_fmad() : rrtk::rrt_split_kernels_strict();
-        // the tracer: two rays per thread in packed f32x2 registers where that kernel exists (FMAD contract), else one per thread
-        const bool packed_trace = sk->trace_packed[0] != nullptr && ctx->trace_choice != 1 &&
-                                  2ll * (prm->max_steps + 1) + 2 <= 128ll * (rrtk::kDescChunks - 2);
-        auto k_trace = packed_trace ? sk->trace_packed[spin ? 1 : 0] : sk->trace[spin ? 1 : 0];
-        const int per_sm_trace = resident_per_sm(ctx, (const void*)k_trace, kRenderBlock, true);
-        const unsigned ntiles8 = (unsigned)(((w + kRTileW - 1) / kRTileW) * ((local_rows + kRTileH - 1) / kRTileH));
-        const unsigned ntiles16 = (unsigned)(((w + kTile16W - 1) / kTile16W) * ((local_rows + kTile16H - 1) / kTile16H));
-        const unsigned ntiles = packed_trace ? ntiles16 : ntiles8;
-        long long grid_trace = ((long long)ctx->sm_count * per_sm_trace + ctx->frames_in_flight - 1) / ctx->frames_in_flight;
-        if (grid_trace > (long long)ntiles) grid_trace = ntiles;
-        if (grid_trace > (long long)kRedoCap) grid_trace = kRedoCap;
-        const int rows_per_tile = (packed_trace ? 2 : 1) * (prm->max_steps + 1) + 1;
-        if (rrt_context::SamplePool* pl = acquire_pool(ctx, st, (long long)w * local_rows, packed_trace ? 2 * ntiles16 : ntiles8, grid_trace, rows_per_tile))
-            return render_split(ctx, A, spin, fmad, packed_trace, grid_trace, st, pl);
+    if (media && ctx->pipeline != RRT_PIPELINE_FUSED && (!ctx->tile_log || ctx->pipeline == RRT_PIPELINE_SPLIT) && split_fits(prm)) {
+        const TracePlan tp = plan_trace(ctx, prm, w, local_rows);
+        if (rrt_context::SamplePool* pl = acquire_pool(ctx, st, (long long)w * local_rows, tp.ngroups, tp.grid, tp.rows_per_tile))
+            return render_split(ctx, A, spin, fmad, tp.packed, tp.grid, st, pl);
         if (ctx->pipeline == RRT_PIPELINE_SPLIT) return fail(ctx, RRT_ERR_NOMEM, "rrt_render: no memory for the sample pool of the split pipeline");
     }
     kern<<<(unsigned)grid, kRenderBlock, 0, st>>>(A);
@@ -801,6 +841,260 @@ int rrt_render_ss(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam
     const cudaError_t e = cudaFreeAsync(hi, st);   // stream-ordered: the block goes back to the pool once the resolve has read it
     if (rc == RRT_OK && e != cudaSuccess) return fail(ctx, RRT_ERR_CUDA, "rrt_render_ss: cudaFreeAsync", e);
     return rc;
+}
+
+}  // extern "C"
+
+// ---- captures (rrt_capture_*): one trace kept for renders at other times -----------------------------------------------
+// The trace of a frame with a medium does not read the time: only the densities do, in media_kernel (and in sweep_kernel for
+// tiles the pass could not hold).  A capture runs the split pipeline's trace pass once into a pool it owns and keeps what
+// media + fold need afterwards; each render then evaluates the kept samples at its own time into a separate results array
+// (media_kernel<true>), so the samples survive for the next render.
+struct rrt_capture {
+    rrt_context* ctx = nullptr;
+    rrt_params prm;                   // what the trace used: a render takes prm with its own exposure
+    rrt_camera cam;
+    rrt_effects fx;
+    rrt_band band = {0, 1, 1};
+    int w = 0, h = 0, local_rows = 0;
+    unsigned ntiles = 0;              // tickets of the frame: 16x4 tiles (packed tracer) or 8x4 tiles
+    unsigned tiles_left = 0;          // tickets the pass did not trace: its redo list + the tickets it never took
+    rrtk::SplitArgs S;                // media / fold over what the capture holds; the sweep's pass derives from it
+    char* d_ctrl = nullptr;           // PassCtrl[2] (the pass, the sweep) | stats[8] | ticket | ticket after the pass | redo list
+    uint4* d_slots = nullptr;         // the used prefix of the pool (samples and exit states)
+    uint4* d_results = nullptr;       // {e.rgb, s} per slot of the prefix
+    rrtk::TileDesc* d_desc = nullptr;
+    rrtk::WorkItem* d_work = nullptr;
+    char* d_planes = nullptr;         // vel | emis | hdr (float4) | cls (u8), full frame: the rays the trace finished on the spot
+    rrt_planes planes;
+    uint64_t info[8] = {};
+    cudaEvent_t done = nullptr;       // the last render enqueued
+};
+
+namespace {
+constexpr size_t kCapStats = 2 * sizeof(rrtk::PassCtrl), kCapTicket = kCapStats + 8 * sizeof(unsigned), kCapRedo = 128;
+constexpr size_t kCapCtrlBytes = kCapRedo + sizeof(unsigned) * kRedoCap;
+static_assert(kCapTicket + 2 * sizeof(unsigned) <= kCapRedo, "capture control block layout");
+
+void free_capture(rrt_capture* c) {
+    DevGuard g(c->ctx->device);
+    if (c->done) cudaEventSynchronize(c->done);
+    for (void* p : {(void*)c->d_ctrl, (void*)c->d_slots, (void*)c->d_results, (void*)c->d_desc, (void*)c->d_work, (void*)c->d_planes})
+        if (p) cudaFree(p);
+    if (c->done) cudaEventDestroy(c->done);
+    delete c;
+}
+// The device allocations of a capture under construction, released unless handed over.
+struct DevAlloc {
+    void* p = nullptr;
+    bool get(size_t n) { if (cudaMalloc(&p, n ? n : 1) == cudaSuccess) return true; cudaGetLastError(); p = nullptr; return false; }
+    void* take() { void* q = p; p = nullptr; return q; }
+    ~DevAlloc() { if (p) cudaFree(p); }
+};
+}  // namespace
+
+extern "C" {
+
+// a failed CUDA call inside rrt_capture_create releases the partial capture
+#define CAP_CU(call)                                                                    \
+    do {                                                                                \
+        if (cudaError_t e__ = (call)) return bail(RRT_ERR_CUDA, "rrt_capture_create: " #call, e__); \
+    } while (0)
+int rrt_capture_create(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, const rrt_effects* fx, uint64_t sky_texture, int w,
+                       int h, const rrt_band* band, size_t max_bytes, void* stream, rrt_capture** out) {
+    if (!ctx) return RRT_ERR_BAD_ARG;
+    if (!out || !prm || !cam || !fx || w <= 0 || h <= 0 || sky_texture == 0 || prm->max_steps < 0)
+        return fail(ctx, RRT_ERR_BAD_ARG, "rrt_capture_create: bad argument");
+    *out = nullptr;
+    if (!(prm->flags & (RRT_FLAG_DISK | RRT_FLAG_DUST)))
+        return fail(ctx, RRT_ERR_BAD_ARG, "rrt_capture_create: no medium (RRT_FLAG_DISK / RRT_FLAG_DUST): nothing depends on the time, re-shade with rrt_shade");
+    if (!split_fits(prm)) return fail(ctx, RRT_ERR_BAD_ARG, "rrt_capture_create: max_steps too large for the split pipeline");
+    rrt_band b = {0, 1, 1};
+    if (band) b = *band;
+    const int local_rows = rrt_band_rows(&b, h);
+    if (local_rows < 0) return fail(ctx, RRT_ERR_BAD_ARG, "rrt_capture_create: bad band");
+    if ((long long)w * local_rows > (1ll << 30)) return fail(ctx, RRT_ERR_BAD_ARG, "rrt_capture_create: band larger than 2^30 pixels");
+
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DevGuard g(ctx->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    rrt_capture* c = new (std::nothrow) rrt_capture();
+    if (!c) return fail(ctx, RRT_ERR_NOMEM, "out of host memory");
+    c->ctx = ctx;
+    c->prm = *prm;
+    c->cam = *cam;
+    c->fx = *fx;
+    c->band = b;
+    c->w = w;
+    c->h = h;
+    c->local_rows = local_rows;
+    auto bail = [&](int code, const char* what, cudaError_t e = cudaSuccess) { free_capture(c); return fail(ctx, code, what, e); };
+    const size_t npix = (size_t)w * h;
+    const size_t plane_bytes = npix * (3 * sizeof(float4) + 1);
+    if (cudaEventCreateWithFlags(&c->done, cudaEventDisableTiming) != cudaSuccess) { cudaGetLastError(); return bail(RRT_ERR_CUDA, "rrt_capture_create: event"); }
+    DevAlloc ctrl, planes;
+    if (!ctrl.get(kCapCtrlBytes) || !planes.get(plane_bytes)) return bail(RRT_ERR_NOMEM, "rrt_capture_create: no memory for the capture's planes");
+    c->d_ctrl = (char*)ctrl.take();
+    c->d_planes = (char*)planes.take();
+    std::memset(&c->planes, 0, sizeof(c->planes));
+    c->planes.vel = (float*)c->d_planes;
+    c->planes.emis = (float*)(c->d_planes + npix * sizeof(float4));
+    c->planes.hdr = (float*)(c->d_planes + 2 * npix * sizeof(float4));
+    c->planes.cls = (uint8_t*)(c->d_planes + 3 * npix * sizeof(float4));
+    CAP_CU(cudaMemsetAsync(c->d_ctrl, 0, kCapRedo, st));
+    CAP_CU(cudaMemsetAsync(c->d_planes, 0, plane_bytes, st));   // pixels no kernel of the trace writes read as zeros
+    if (local_rows == 0) {
+        *out = c;
+        return RRT_OK;
+    }
+
+    // the pass: rrt_render's tracer and grid, into a pool of this capture's own
+    const TracePlan tp = plan_trace(ctx, prm, w, local_rows);
+    c->ntiles = tp.ntiles;
+    size_t cap_slots = pool_slots(ctx->pool_bytes_max, (long long)npix, tp.grid, tp.rows_per_tile);
+    if (max_bytes) cap_slots = std::min<size_t>(std::max<size_t>(max_bytes / kSlotBytes, 1024), 0xfff00000ull);
+    const size_t work_cap = cap_slots / kMediaBatch + tp.ngroups + 64;   // as acquire_pool sizes it
+    DevAlloc pool, desc, work;
+    if (!pool.get((cap_slots + kPoolPadSlots) * kSlotBytes) || !desc.get((size_t)tp.ngroups * sizeof(rrtk::TileDesc)) ||
+        !work.get(work_cap * sizeof(rrtk::WorkItem)))
+        return bail(RRT_ERR_NOMEM, "rrt_capture_create: no memory for the sample pool");
+    FrameArgs A = frame_args(*prm, *cam, *fx, sky_texture, 0.0f, w, h, b, local_rows, RRT_OUT_FRAME, nullptr);
+    A.planes = c->planes;
+    A.counters = ctx->d_counters;
+    A.ticket = (unsigned*)(c->d_ctrl + kCapTicket);
+    rrtk::SplitArgs S = split_args((uint4*)pool.p, cap_slots, (rrtk::TileDesc*)desc.p, (rrtk::WorkItem*)work.p, work_cap, tp.packed,
+                                   prm->max_steps, tp.grid);
+    rrtk::PassCtrl* pcs = (rrtk::PassCtrl*)c->d_ctrl;
+    S.pc = pcs;
+    S.redo_out = (unsigned*)(c->d_ctrl + kCapRedo);
+    S.stats = (unsigned*)(c->d_ctrl + kCapStats);
+    tp.kernel<<<(unsigned)tp.grid, kRenderBlock, 0, st>>>(A, S);
+    CAP_CU(cudaGetLastError());
+    ctx->launches += 1;
+    CAP_CU(cudaMemcpyAsync(c->d_ctrl + kCapTicket + sizeof(unsigned), c->d_ctrl + kCapTicket, sizeof(unsigned), cudaMemcpyDeviceToDevice, st));
+    unsigned char head[kCapRedo];
+    CAP_CU(cudaMemcpyAsync(head, c->d_ctrl, kCapRedo, cudaMemcpyDeviceToHost, st));
+    if (cudaError_t e = cudaStreamSynchronize(st)) return bail(RRT_ERR_CUDA, "rrt_capture_create: trace pass", e);
+    rrtk::PassCtrl pc;
+    std::memcpy(&pc, head, sizeof(pc));
+    unsigned ticket;
+    std::memcpy(&ticket, head + kCapTicket, sizeof(ticket));
+
+    // keep the used prefix of the pool, the queued groups and their work items; free the rest (before the results array
+    // is allocated: the peak is the pool plus its used prefix)
+    const size_t used = std::min<size_t>(pc.cursor, cap_slots), held = used + kPoolPadSlots;
+    const size_t n_desc = pc.pend_count, n_work = std::min<size_t>(pc.work_count, work_cap);
+    DevAlloc slots, results, desc_held, work_held;
+    if (!slots.get(held * kSlotBytes) || !desc_held.get(n_desc * sizeof(rrtk::TileDesc)) || !work_held.get(n_work * sizeof(rrtk::WorkItem)))
+        return bail(RRT_ERR_NOMEM, "rrt_capture_create: no memory for the samples");
+    CAP_CU(cudaMemcpyAsync(slots.p, pool.p, held * kSlotBytes, cudaMemcpyDeviceToDevice, st));
+    if (n_desc) CAP_CU(cudaMemcpyAsync(desc_held.p, desc.p, n_desc * sizeof(rrtk::TileDesc), cudaMemcpyDeviceToDevice, st));
+    if (n_work) CAP_CU(cudaMemcpyAsync(work_held.p, work.p, n_work * sizeof(rrtk::WorkItem), cudaMemcpyDeviceToDevice, st));
+    uint64_t samples = 0;
+    if (n_desc) {   // the `total` field of every queued group: a strided copy
+        unsigned* tot = new (std::nothrow) unsigned[n_desc];
+        if (!tot) return bail(RRT_ERR_NOMEM, "out of host memory");
+        cudaError_t e = cudaMemcpy2DAsync(tot, sizeof(unsigned), (const char*)desc.p + offsetof(rrtk::TileDesc, total), sizeof(rrtk::TileDesc),
+                                          sizeof(unsigned), n_desc, cudaMemcpyDeviceToHost, st);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+        for (size_t i = 0; e == cudaSuccess && i < n_desc; ++i) samples += tot[i];
+        delete[] tot;
+        if (e != cudaSuccess) return bail(RRT_ERR_CUDA, "rrt_capture_create: copy of the queued groups", e);
+    }
+    if (cudaError_t e = cudaStreamSynchronize(st)) return bail(RRT_ERR_CUDA, "rrt_capture_create: copy of the samples", e);
+    cudaFree(pool.take());
+    if (!results.get(held * sizeof(uint4))) return bail(RRT_ERR_NOMEM, "rrt_capture_create: no memory for the media results");
+    c->d_slots = (uint4*)slots.take();
+    c->d_results = (uint4*)results.take();
+    c->d_desc = (rrtk::TileDesc*)desc_held.take();
+    c->d_work = (rrtk::WorkItem*)work_held.take();
+    S.slots = c->d_slots;
+    S.results = c->d_results;
+    S.capacity = (unsigned)used;
+    S.desc = c->d_desc;
+    S.work = c->d_work;
+    S.work_cap = (unsigned)n_work;
+    S.redo_in = S.redo_out;
+    S.redo_out = nullptr;
+    c->S = S;
+    const unsigned n_redo = std::min(pc.redo_out_count, kRedoCap);
+    c->tiles_left = n_redo + (ticket < tp.ntiles ? tp.ntiles - ticket : 0u);
+    const uint64_t bytes = held * (kSlotBytes + sizeof(uint4)) + n_desc * sizeof(rrtk::TileDesc) + n_work * sizeof(rrtk::WorkItem) + kCapCtrlBytes + plane_bytes;
+    const uint64_t info[8] = {samples, used, bytes, n_desc, c->tiles_left, tp.packed ? 1u : 0u, tp.ntiles, (uint64_t)cap_slots * kSlotBytes};
+    std::memcpy(c->info, info, sizeof(info));
+    CAP_CU(cudaEventRecord(c->done, st));
+    *out = c;
+    return RRT_OK;
+}
+
+#undef CAP_CU
+
+int rrt_capture_render(rrt_capture* cap, const rrt_params* prm, const rrt_effects* fx, uint64_t sky_texture, float time, void* d_out,
+                       int out_layout, float* hdr_out, void* stream) {
+    if (!cap) return fail(nullptr, RRT_ERR_BAD_ARG, "rrt_capture_render: capture is NULL");
+    rrt_context* ctx = cap->ctx;
+    if (!prm || !fx || sky_texture == 0 || (out_layout != RRT_OUT_FRAME && out_layout != RRT_OUT_PACKED) || (!d_out && !hdr_out))
+        return fail(ctx, RRT_ERR_BAD_ARG, "rrt_capture_render: bad argument");
+    if (((prm->flags ^ cap->prm.flags) & RRT_FLAG_FMAD) || fx->use_lens != cap->fx.use_lens ||
+        std::memcmp(&fx->distortion_amount, &cap->fx.distortion_amount, sizeof(float)) != 0)
+        return fail(ctx, RRT_ERR_BAD_ARG, "rrt_capture_render: the RRT_FLAG_FMAD bit, use_lens and distortion_amount must be the capture's");
+    if (cap->local_rows == 0) return RRT_OK;
+
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DevGuard g(ctx->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    rrt_params P = cap->prm;
+    P.exposure = prm->exposure;
+    const bool fmad = (P.flags & RRT_FLAG_FMAD) != 0;
+    const rrtk::SplitKernels* sk = fmad ? rrtk::rrt_split_kernels_fmad() : rrtk::rrt_split_kernels_strict();
+    FrameArgs A = frame_args(P, cap->cam, *fx, sky_texture, time, cap->w, cap->h, cap->band, cap->local_rows, out_layout, d_out);
+    A.planes.hdr = hdr_out;
+    A.counters = ctx->d_counters;
+    A.ticket = (unsigned*)(cap->d_ctrl + kCapTicket);
+    rrtk::PassCtrl* pcs = (rrtk::PassCtrl*)cap->d_ctrl;
+    const int per_sm_media = resident_per_sm(ctx, (const void*)sk->media_results, kMediaBlock, true);
+    const int per_sm_fold = resident_per_sm(ctx, (const void*)sk->fold_results, 128, false);
+    RRT_CU(ctx, cudaStreamWaitEvent(st, cap->done, 0));   // one render at a time per capture, whatever the streams
+    // 1. every pixel from the planes; right for the rays the trace finished, overwritten below for the others
+    const long long n = (long long)cap->w * cap->local_rows;
+    kset(&P)->shade<<<(unsigned)((n + kShadeBlock - 1) / kShadeBlock), kShadeBlock, 0, st>>>(A, cap->planes);
+    // 2.-4. the kept samples at this time, then fold + finish of the queued rays
+    static_assert(offsetof(rrtk::PassCtrl, fold_ticket) == offsetof(rrtk::PassCtrl, media_ticket) + sizeof(unsigned), "PassCtrl layout");
+    RRT_CU(ctx, cudaMemsetAsync(&pcs[0].media_ticket, 0, 2 * sizeof(unsigned), st));
+    sk->media_results<<<(unsigned)(ctx->sm_count * per_sm_media), kMediaBlock, 0, st>>>(A, cap->S);
+    sk->fold_results<<<(unsigned)(ctx->sm_count * per_sm_fold), 128, 0, st>>>(A, cap->S);
+    int launches = 3;
+    // 5. the tiles the pass could not hold, with the fused code: its redo list first, then the tickets it never took
+    if (cap->tiles_left) {
+        const bool spin = P.spin_a != 0.0f;
+        auto k_sweep = sk->sweep[spin ? 1 : 0];
+        const int per_sm_sweep = resident_per_sm(ctx, (const void*)k_sweep, kRenderBlock, true);
+        RRT_CU(ctx, cudaMemcpyAsync(A.ticket, A.ticket + 1, sizeof(unsigned), cudaMemcpyDeviceToDevice, st));
+        RRT_CU(ctx, cudaMemsetAsync(&pcs[1], 0, sizeof(rrtk::PassCtrl), st));
+        rrtk::SplitArgs S = cap->S;
+        S.pass = 1;
+        S.pc = pcs + 1;
+        S.pc_prev = pcs;
+        long long grid_sweep = ((long long)ctx->sm_count * per_sm_sweep + ctx->frames_in_flight - 1) / ctx->frames_in_flight;
+        if (grid_sweep > (long long)cap->ntiles) grid_sweep = cap->ntiles;
+        k_sweep<<<(unsigned)grid_sweep, kRenderBlock, 0, st>>>(A, S);
+        ++launches;
+    }
+    RRT_CU(ctx, cudaGetLastError());
+    ctx->launches += launches;
+    RRT_CU(ctx, cudaEventRecord(cap->done, st));
+    return RRT_OK;
+}
+
+int rrt_capture_info(const rrt_capture* cap, uint64_t out[8]) {
+    if (!cap) return RRT_ERR_BAD_ARG;
+    if (!out) return fail(cap->ctx, RRT_ERR_BAD_ARG, "rrt_capture_info: out is NULL");
+    std::memcpy(out, cap->info, sizeof(cap->info));
+    return RRT_OK;
+}
+
+void rrt_capture_destroy(rrt_capture* cap) {
+    if (cap) free_capture(cap);
 }
 
 int rrt_render_host_async(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, const rrt_effects* fx,

@@ -34,7 +34,8 @@
 //   fewer samples stay unused (never written, never read).  A lane that stored samples puts its ray's exit state behind
 //   its last one; a lane that stored none finishes its ray on the spot.
 //   sample = {q.xyz, v.xyz, r, tag}, tag = zones | zone_index << 2;  after media_kernel the first 16 bytes are
-//            {e.r, e.g, e.b, s}, s = -1 for a sample that did not pass the 0.001 density gate (:71);
+//            {e.r, e.g, e.b, s}, s = -1 for a sample that did not pass the 0.001 density gate (:71) -- or, for a capture
+//            (rrt_capture_render), the same 16 bytes are written to a separate array `results[slot]` and the sample stays;
 //   state  = {p.xyz, v.xyz, steps | end << 28, 0}, stored by each lane behind its own last sample.
 //   A queued group of 32 rays is described by a TileDesc (chunk bases, first row, row stride, samples per lane);
 //   media_kernel takes its work as (group, first sample) items of kMediaBatch samples, so a disk-plane tile (64 000 samples)
@@ -84,6 +85,7 @@ struct SplitArgs {
     unsigned* stats;          // [0] split passes that took tiles, [1] tiles rendered by sweep_kernel, [2] tiles taken by the split passes
     unsigned pass;
     unsigned tile16;          // tickets and redo lists count 16x4 tiles (the packed tracer) instead of 8x4 tiles
+    uint4* results;           // media_kernel<true> / fold_kernel<true>: {e.rgb, s} per slot, indexed like `slots` (rrt_capture)
 };
 struct SplitKernels {
     void (*trace[2])(const FrameArgs, const SplitArgs);   // [spin != 0]
@@ -91,6 +93,8 @@ struct SplitKernels {
     void (*media)(const FrameArgs, const SplitArgs);
     void (*fold)(const FrameArgs, const SplitArgs);
     void (*sweep[2])(const FrameArgs, const SplitArgs);
+    void (*media_results)(const FrameArgs, const SplitArgs);   // media_kernel<true>: the samples stay, results go to S.results
+    void (*fold_results)(const FrameArgs, const SplitArgs);    // fold_kernel<true>: reads them from there
 };
 const SplitKernels* rrt_split_kernels_strict();
 const SplitKernels* rrt_split_kernels_fmad();
@@ -729,11 +733,14 @@ __device__ __forceinline__ unsigned desc_slot(const SplitArgs& S, const unsigned
 // Stage 1 evaluates, lane per sample, the disk density and the dust envelope.  The dust strands -- 19 value-noise
 // evaluations, needed only where the envelope survived its 0.001 cut (densities.h:84) -- are collected over the whole
 // batch and evaluated 32 at a time.  Stage 3 is media_final for every sample.
+// RESULTS = false overwrites the first 16 bytes of each sample with {e.rgb, s}; RESULTS = true (rrt_capture_render) writes
+// them to S.results[slot] instead and leaves the sample as it is, so the same samples can be evaluated again at another time.
 __device__ __forceinline__ void pool_get(const uint4* slots, unsigned slot, uint4& a, uint4& b) {   // one 256-bit load
     asm volatile("ld.global.v8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
                  : "=r"(a.x), "=r"(a.y), "=r"(a.z), "=r"(a.w), "=r"(b.x), "=r"(b.y), "=r"(b.z), "=r"(b.w)
                  : "l"(slots + 2ull * slot));
 }
+template <bool RESULTS>
 __global__ void __launch_bounds__(kMediaBlock, 4) media_kernel(const __grid_constant__ FrameArgs A, const __grid_constant__ SplitArgs S) {
     __shared__ float s_dd[kMediaBlock / 32][kMediaBatch];
     __shared__ float s_dc[kMediaBlock / 32][kMediaBatch];      // dust envelope, then dust density
@@ -845,8 +852,10 @@ __global__ void __launch_bounds__(kMediaBlock, 4) media_kernel(const __grid_cons
                 const V3 q = mk(__uint_as_float(a.x), __uint_as_float(a.y), __uint_as_float(a.z));
                 const V3 v = mk(__uint_as_float(a.w), __uint_as_float(b.x), __uint_as_float(b.y));
                 const MediaOut m = media_final(C, q, v, __uint_as_float(b.z), C.h[(b.w >> 2) & 3u], dd_w[i], dc_w[i]);
-                S.slots[2ull * slot] = make_uint4(__float_as_uint(m.er), __float_as_uint(m.eg), __float_as_uint(m.eb),
-                                                  __float_as_uint(m.dense ? m.s : -1.0f));
+                const uint4 e = make_uint4(__float_as_uint(m.er), __float_as_uint(m.eg), __float_as_uint(m.eb),
+                                           __float_as_uint(m.dense ? m.s : -1.0f));
+                if (RESULTS) S.results[slot] = e;
+                else S.slots[2ull * slot] = e;
             }
         }
         __syncwarp();
@@ -854,6 +863,8 @@ __global__ void __launch_bounds__(kMediaBlock, 4) media_kernel(const __grid_cons
 }
 
 // ---- pass kernel 3: fold + finish, one warp per queued tile ----------------------------------------------------------
+// RESULTS: read each sample's {e.rgb, s} from S.results (media_kernel<true>) instead of from the sample's slot.
+template <bool RESULTS>
 __global__ void __launch_bounds__(128) fold_kernel(const __grid_constant__ FrameArgs A, const __grid_constant__ SplitArgs S) {
     __shared__ unsigned s_chunk[4][kDescChunks];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -889,7 +900,9 @@ __global__ void __launch_bounds__(128) fold_kernel(const __grid_constant__ Frame
             uint4 e[4];
 #pragma unroll
             for (int u = 0; u < 4; ++u)
-                e[u] = k0 + u < n ? S.slots[2ull * desc_slot(S, chunk, row0, stride, k0 + u, (unsigned)lane)] : make_uint4(0u, 0u, 0u, 0xbf800000u);
+                e[u] = k0 + u < n ? (RESULTS ? S.results[desc_slot(S, chunk, row0, stride, k0 + u, (unsigned)lane)]
+                                             : S.slots[2ull * desc_slot(S, chunk, row0, stride, k0 + u, (unsigned)lane)])
+                                  : make_uint4(0u, 0u, 0u, 0xbf800000u);
 #pragma unroll
             for (int u = 0; u < 4; ++u) {
                 const float s = __uint_as_float(e[u].w);
@@ -960,7 +973,8 @@ const rrtk::SplitKernels kSplitKernels = {
 #else
     {nullptr, nullptr},
 #endif
-    media_kernel, fold_kernel, {sweep_kernel<false>, sweep_kernel<true>},
+    media_kernel<false>, fold_kernel<false>, {sweep_kernel<false>, sweep_kernel<true>},
+    media_kernel<true>, fold_kernel<true>,
 };
 }  // namespace
 

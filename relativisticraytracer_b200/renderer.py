@@ -80,6 +80,55 @@ class Sky:
             pass
 
 
+class Capture:
+    """One traced frame kept for renders at other times (rrt_capture): ``Renderer.capture`` traces once, ``render`` evaluates
+    the disk and dust at a new time and folds, shades and stores without tracing again.  ``render(prm, fx, sky, t)`` gives
+    the bytes of ``Renderer.render`` with the capture's parameters, camera, size and band, ``prm``'s exposure, ``fx``'s
+    bloom / vignette / CA settings, ``sky`` and time ``t``; ``prm`` must keep the capture's FLAG_FMAD bit and ``fx`` its lens
+    fields."""
+
+    def __init__(self, renderer: "Renderer", prm: Params, cam: Camera, fx: Effects, sky: "Sky | int", w: int, h: int, *,
+                 band: Optional[Band] = None, max_bytes: int = 0, stream: Optional[torch.cuda.Stream] = None):
+        tex = sky.texture if isinstance(sky, Sky) else int(sky)
+        self._r, self.w, self.h, self.band = renderer, int(w), int(h), band
+        self._h = C.c_void_p()
+        st = stream if stream is not None else torch.cuda.current_stream(renderer.device)
+        renderer._check(renderer._lib.rrt_capture_create(renderer._ctx, C.byref(prm), C.byref(cam), C.byref(fx), C.c_uint64(tex),
+                                                         self.w, self.h, C.byref(band) if band is not None else None,
+                                                         C.c_size_t(int(max_bytes)), C.c_void_p(st.cuda_stream), C.byref(self._h)))
+
+    def render(self, prm: Params, fx: Effects, sky: "Sky | int", time: float, *, out=None, layout: int = OUT_FRAME,
+               hdr_out: Optional[torch.Tensor] = None, stream: Optional[torch.cuda.Stream] = None) -> torch.Tensor:
+        """rrt_capture_render: the captured frame (or band) at ``time``; asynchronous.  ``out`` (a tensor or a PeerFrame),
+        ``layout`` and ``hdr_out`` ((h, w, 4) float32) as in ``Renderer.render`` / ``Renderer.shade``; returns the frame."""
+        r = self._r
+        tex = sky.texture if isinstance(sky, Sky) else int(sky)
+        out, out_ptr = r._frame_out(out, layout, self.band, self.w, self.h)
+        hdr_ptr = r._plane_ptr("hdr", hdr_out, self.w, self.h) if hdr_out is not None else None
+        st = stream if stream is not None else torch.cuda.current_stream(r.device)
+        r._check(r._lib.rrt_capture_render(self._h, C.byref(prm), C.byref(fx), C.c_uint64(tex), float(time), C.c_void_p(out_ptr),
+                                           int(layout), C.c_void_p(hdr_ptr), C.c_void_p(st.cuda_stream)))
+        return out
+
+    def info(self) -> dict:
+        """rrt_capture_info: what the capture holds."""
+        out = (C.c_uint64 * 8)()
+        self._r._check(self._r._lib.rrt_capture_info(self._h, out))
+        return {"samples": int(out[0]), "slots": int(out[1]), "bytes": int(out[2]), "groups_queued": int(out[3]),
+                "tiles_left": int(out[4]), "packed": bool(out[5]), "tiles": int(out[6]), "pool_bytes": int(out[7])}
+
+    def close(self):
+        if self._h:
+            self._r._lib.rrt_capture_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 PLANE_SPECS = {"hdr": (4, torch.float32), "dir": (4, torch.float32), "emis": (4, torch.float32),
                "pos": (4, torch.float32), "vel": (4, torch.float32), "cls": (0, torch.uint8), "steps": (0, torch.int32)}
 # the planes Renderer.shade / rrt_shade re-shade a traced frame from (16 + 16 + 16 + 1 bytes per pixel)
@@ -229,6 +278,13 @@ class Renderer:
                                           C.byref(band) if band is not None else None, C.c_void_p(hi_ptr),
                                           C.c_void_p(out_ptr), int(layout), C.c_void_p(hdr_ptr), C.c_void_p(st.cuda_stream)))
         return out
+
+    def capture(self, prm: Params, cam: Camera, fx: Effects, sky: Sky | int, w: int, h: int, *, band: Optional[Band] = None,
+                max_bytes: int = 0, stream: Optional[torch.cuda.Stream] = None) -> Capture:
+        """rrt_capture_create: trace the frame (or band) once and keep it for ``Capture.render`` at any time; synchronises.
+        Needs a medium (FLAG_DISK / FLAG_DUST).  ``max_bytes``: the sample pool the trace runs in (0: the context's sizing
+        rule); tiles that do not fit it are rendered by the fused code at every ``Capture.render``."""
+        return Capture(self, prm, cam, fx, sky, w, h, band=band, max_bytes=max_bytes, stream=stream)
 
     def _frame_out(self, out, layout: int, band: Optional[Band], w: int, h: int):
         """(out, device pointer) of a uchar4 destination: a PeerFrame, a device tensor, or None (allocated here)."""
