@@ -253,6 +253,43 @@ int rrt_capture_render(rrt_capture* cap, const rrt_params* prm, const rrt_effect
 int rrt_capture_info(const rrt_capture* cap, uint64_t out[8]);
 void rrt_capture_destroy(rrt_capture* cap);
 
+/* ---- motion-blurred frames: n sub-frames across the shutter interval, n = 1 .. 64 ---------------------------------
+ * Sub-frame i has its own camera cams[i] and time times[i] (caller-supplied HOST arrays) and is exactly
+ * rrt_render(P, cams[i], F, S, times[i], w, h, band, NULL, RRT_OUT_FRAME, {hdr = plane_i}): its ray, step count, media
+ * and sky (chromatic aberration included) are that render's bit for bit.  The pixel's linear final_hdr (and T, in .w) is
+ * the mean of the n planes, summed from plane 0 to plane n-1 in round-to-nearest float32 and divided by (float)n; bloom,
+ * vignette (at the pixel's own image-plane coordinate: use_lens and distortion_amount are common to all sub-frames),
+ * exposure tonemap and the store then run on the mean exactly as in rrt_render.  n = 1 is rrt_render: same bytes, same
+ * hdr values.  rrt_shutter_times gives the times of a centred shutter.
+ * Supersampled and motion-blurred: rrt_resolve_time at ss*w x ss*h with only hdr_out (an ss*w x ss*h plane), then
+ * rrt_resolve(ss) of that plane, averages over time first and then over each pixel's ss x ss block. */
+
+/* The time analogue of rrt_resolve: hdr_stack is n full-frame float4 planes back to back (plane i at i*w*h float4, each
+ * [y*w + x] as rrt_render writes it).  Writes d_out (layout as in rrt_render, only the band's rows) and/or hdr_out (float4
+ * per pixel, full-frame indexed, the band's pixels only, the mean before bloom); hdr_out must not overlap the stack.
+ * Reads only the band's rows.  Uses prm->exposure and the contract bit prm->flags & RRT_FLAG_FMAD.  Asynchronous on
+ * `stream`; adds nothing to the counters and one launch.  RRT_ERR_BAD_ARG for n outside 1..64, no output, a bad band or
+ * layout, or a band of more than 2^30 pixels. */
+int rrt_resolve_time(rrt_context* ctx, const rrt_params* prm, const rrt_effects* fx, int n, int w, int h, const rrt_band* band,
+                     const float* hdr_stack, void* d_out, int out_layout, float* hdr_out, void* stream);
+
+/* Renders the n sub-frames into a stack taken stream-ordered from the context's scratch pool (the one rrt_render_ss uses),
+ * then rrt_resolve_time.  Same arguments as rrt_render with cams / times / n for cam / time, and hdr_out (the mean) for
+ * the planes; bands, RRT_OUT_PACKED and a peer-frame d_out work as in rrt_render.  Scratch: 16*n*w*h bytes per call
+ * (full-frame even for a band: 1.06 GB for 3840x2160 at n = 8); RRT_ERR_NOMEM, before anything is enqueued, when it
+ * cannot be allocated.  Adds to the counters exactly what its n renders add, and their launches + 1. */
+int rrt_render_mb(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cams, const rrt_effects* fx, uint64_t sky_texture,
+                  const float* times, int n, int w, int h, const rrt_band* band, void* d_out, int out_layout, float* hdr_out,
+                  void* stream);
+
+/* rrt_render_mb of a still camera through a capture: n rrt_capture_render calls into the stack (hdr only), then
+ * rrt_resolve_time.  Writes exactly what rrt_render_mb writes with cams[i] = the capture's camera for every i, under
+ * rrt_capture_render's rules: prm must carry the capture's RRT_FLAG_FMAD bit and fx its use_lens / distortion_amount, else
+ * RRT_ERR_BAD_ARG; prm contributes only its exposure.  Waits for the capture's previous render once and is ordered before
+ * its next one.  Scratch as rrt_render_mb.  Adds what n capture renders add to the counters; launches n * (3 or 4) + 1. */
+int rrt_capture_render_mb(rrt_capture* cap, const rrt_params* prm, const rrt_effects* fx, uint64_t sky_texture, const float* times,
+                          int n, void* d_out, int out_layout, float* hdr_out, void* stream);
+
 /* Same call with a HOST destination: renders into a context-owned device frame, copies it to
  * host_rgba (w*h*4 bytes, reference layout) and synchronises.  This is the end-to-end entry point. */
 int rrt_render_host(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, const rrt_effects* fx,
@@ -295,9 +332,10 @@ int rrt_set_sample_pool(rrt_context* ctx, size_t max_bytes_per_stream, int max_p
  * tiles, [1] tiles left to the closing fused sweep, [2] tiles traced by the passes, [3] passes enqueued, [4] tiles of
  * the launch, [5] pool size in Ki slots of 32 bytes; all 0 when no frame went through the split pipeline. */
 int rrt_split_stats(rrt_context* ctx, uint32_t out[8]);
-/* Kernels this context has launched so far for rrt_render*, rrt_shade, rrt_resolve, rrt_capture_* and rrt_assemble_bands
- * (1 per fused frame; 3 per pass + 1 per split frame; 1 per rrt_shade or rrt_resolve; rrt_render_ss: its ss*w x ss*h
- * render's + 1; 1 per rrt_capture_create, 3 or 4 per rrt_capture_render):
+/* Kernels this context has launched so far for rrt_render*, rrt_shade, rrt_resolve*, rrt_capture_* and rrt_assemble_bands
+ * (1 per fused frame; 3 per pass + 1 per split frame; 1 per rrt_shade, rrt_resolve or rrt_resolve_time; rrt_render_ss: its
+ * ss*w x ss*h render's + 1; rrt_render_mb: its n renders' + 1; 1 per rrt_capture_create, 3 or 4 per rrt_capture_render,
+ * n * (3 or 4) + 1 per rrt_capture_render_mb):
  * what a benchmark reports as its launch count. */
 uint64_t rrt_kernel_launches(rrt_context* ctx);
 
@@ -364,6 +402,11 @@ int rrt_path_num_keys(int path_index);
 float rrt_path_duration(int path_index);
 int rrt_path_state(int path_index, float t, rrt_camera* out, float pos_yaw_pitch[5]);
 float rrt_path_clock(int frame, float fps);
+/* The n sub-frame times of a shutter open for `shutter` (0 .. 1) of the frame interval 1/fps, centred on t:
+ * d = shutter / fps, out[i] = t + d * ((i + 0.5f) / n - 0.5f), every operation rounded to float32 on its own (no
+ * contraction).  n = 1 gives t and shutter = 0 gives t n times (a t of -0 may come back as +0).  RRT_ERR_BAD_ARG for shutter outside
+ * [0, 1], fps <= 0, n outside 1..64 or out NULL. */
+int rrt_shutter_times(float t, float shutter, float fps, int n, float* out);
 
 /* ---- frame sink: the step after the hot path ----------------------------------------------------------
  * Pure host code.  Replaces, for headless use, the reference's ScreenRecorder (src/main.cpp:29-124): frames

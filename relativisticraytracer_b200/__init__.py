@@ -9,7 +9,7 @@ from ._capi import (Band, Camera, Counters, Effects, Params, Planes, RrtError, F
                     CLS_DISK_HIT, CLS_ESCAPED, CLS_MASK, CLSF_EXHAUSTED, CLSF_TOUCHED, OUT_FRAME, OUT_PACKED, LIB_PATH,
                     default_effects, default_params, effects_off)
 from .renderer import (TRACE_PLANES, CameraEffects, Capture, CameraState, PeerFrame, Renderer, Sky, camera_state_from, launch_raymarch,
-                       path_clock, path_duration, path_names, path_state, set_launch_params)
+                       path_clock, path_duration, path_names, path_state, set_launch_params, shutter_times)
 from .skybox import decode_image, load_skybox, procedural_sky
 from .sink import FrameSink, ffmpeg_command
 from ._capi import SINK_RGBA, SINK_Y4M, HOST_SLOTS

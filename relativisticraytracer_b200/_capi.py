@@ -71,7 +71,7 @@ SYMBOLS = [
     "rrt_abi_version", "rrt_build_info", "rrt_context_create", "rrt_context_destroy", "rrt_last_error",
     "rrt_default_params", "rrt_default_effects", "rrt_sky_create", "rrt_sky_texture", "rrt_sky_destroy",
     "rrt_render", "rrt_shade", "rrt_resolve", "rrt_render_ss", "rrt_capture_create", "rrt_capture_render", "rrt_capture_info",
-    "rrt_capture_destroy", "rrt_render_host", "rrt_render_host_async", "rrt_band_rows", "rrt_assemble_bands", "rrt_read_counters",
+    "rrt_capture_destroy", "rrt_resolve_time", "rrt_render_mb", "rrt_capture_render_mb", "rrt_shutter_times", "rrt_render_host", "rrt_render_host_async", "rrt_band_rows", "rrt_assemble_bands", "rrt_read_counters",
     "rrt_geodesic_acc_batch", "rrt_rk4_step_batch", "rrt_euler_step_batch", "rrt_redshift_batch",
     "rrt_hash31_batch", "rrt_noise3d_batch", "rrt_fbm_batch", "rrt_disk_temperature_batch",
     "rrt_disk_density_batch", "rrt_dust_density_batch", "rrt_sky_sample_batch", "rrt_fp32_peak_probe",
@@ -123,6 +123,10 @@ def load() -> C.CDLL:
     lib.rrt_capture_info.argtypes = [vp, P(C.c_uint64)]
     lib.rrt_capture_destroy.argtypes = [vp]
     lib.rrt_capture_destroy.restype = None
+    lib.rrt_resolve_time.argtypes = [vp, P(Params), P(Effects), ci, ci, ci, P(Band), vp, vp, ci, vp, vp]
+    lib.rrt_render_mb.argtypes = [vp, P(Params), P(Camera), P(Effects), C.c_uint64, P(cf), ci, ci, ci, P(Band), vp, ci, vp, vp]
+    lib.rrt_capture_render_mb.argtypes = [vp, P(Params), P(Effects), C.c_uint64, P(cf), ci, vp, ci, vp, vp]
+    lib.rrt_shutter_times.argtypes = [cf, cf, cf, ci, P(cf)]
     lib.rrt_render_host.argtypes = [vp, P(Params), P(Camera), P(Effects), C.c_uint64, cf, ci, ci, vp]
     lib.rrt_render_host_async.argtypes = [vp, P(Params), P(Camera), P(Effects), C.c_uint64, cf, ci, ci, vp, ci, vp]
     lib.rrt_band_rows.argtypes = [P(Band), ci]

@@ -756,21 +756,17 @@ static int check_ss(rrt_context* ctx, const char* what, int ss, int w, int h, co
     return RRT_OK;
 }
 
-int rrt_resolve(rrt_context* ctx, const rrt_params* prm, const rrt_effects* fx, int ss, int w, int h, const rrt_band* band,
-                const float* hdr_hi, void* d_out, int out_layout, float* hdr_out, void* stream) {
-    if (!ctx) return RRT_ERR_BAD_ARG;
-    if (!prm || !fx || !hdr_hi || (out_layout != RRT_OUT_FRAME && out_layout != RRT_OUT_PACKED) || (!d_out && !hdr_out))
-        return fail(ctx, RRT_ERR_BAD_ARG, "rrt_resolve: bad argument");
-    int local_rows = 0;
-    if (int rc = check_ss(ctx, "rrt_resolve", ss, w, h, band, &local_rows)) return rc;
-    if (hdr_out) {   // the kernel reads hdr_hi while it writes hdr_out: the two must not share a byte (counted in float4s)
-        const uintptr_t a = (uintptr_t)hdr_hi, b = (uintptr_t)hdr_out;
-        if (b >= a ? (b - a) / 16 < (unsigned long long)ss * ss * w * h : (a - b) / 16 < (unsigned long long)w * h)
-            return fail(ctx, RRT_ERR_BAD_ARG, "rrt_resolve: hdr_out overlaps hdr_hi");
-    }
-    if (local_rows == 0) return RRT_OK;
+// Whether float4 ranges [src, src + src_n) and [dst, dst + dst_n) share a byte.
+static bool f4_overlap(const void* src, unsigned long long src_n, const void* dst, unsigned long long dst_n) {
+    const uintptr_t a = (uintptr_t)src, b = (uintptr_t)dst;
+    return b >= a ? (b - a) / 16 < src_n : (a - b) / 16 < dst_n;
+}
 
-    std::lock_guard<std::mutex> lk(ctx->mu);
+// The launch of rrt_resolve and rrt_resolve_time: resolve_kernel over the band's rows of the w x h frame, n planes of
+// ss*w x ss*h from `src`, one plane_stride (float4) apart.  Arguments checked; ctx->mu held.
+static int launch_resolve(rrt_context* ctx, const rrt_params* prm, const rrt_effects* fx, int ss, int n, int w, int h,
+                          const rrt_band* band, int local_rows, const float* src, size_t plane_stride, void* d_out,
+                          int out_layout, float* hdr_out, cudaStream_t st) {
     DevGuard g(ctx->device);
     FrameArgs A;
     std::memset(&A, 0, sizeof(A));   // no camera, sky, counters, ticket or tile log: nothing is traced or sampled
@@ -789,11 +785,48 @@ int rrt_resolve(rrt_context* ctx, const rrt_params* prm, const rrt_effects* fx, 
     A.out_layout = out_layout;
     A.out = (uchar4*)d_out;
     A.planes.hdr = hdr_out;
-    const long long n = (long long)w * local_rows;
-    kset(prm)->resolve<<<(unsigned)((n + kResolveBlock - 1) / kResolveBlock), kResolveBlock, 0, (cudaStream_t)stream>>>(
-        A, (const float4*)hdr_hi, ss);
+    const long long npix = (long long)w * local_rows;
+    kset(prm)->resolve<<<(unsigned)((npix + kResolveBlock - 1) / kResolveBlock), kResolveBlock, 0, st>>>(
+        A, (const float4*)src, ss, n, plane_stride);
     RRT_CU(ctx, cudaGetLastError());
     ctx->launches += 1;
+    return RRT_OK;
+}
+
+int rrt_resolve(rrt_context* ctx, const rrt_params* prm, const rrt_effects* fx, int ss, int w, int h, const rrt_band* band,
+                const float* hdr_hi, void* d_out, int out_layout, float* hdr_out, void* stream) {
+    if (!ctx) return RRT_ERR_BAD_ARG;
+    if (!prm || !fx || !hdr_hi || (out_layout != RRT_OUT_FRAME && out_layout != RRT_OUT_PACKED) || (!d_out && !hdr_out))
+        return fail(ctx, RRT_ERR_BAD_ARG, "rrt_resolve: bad argument");
+    int local_rows = 0;
+    if (int rc = check_ss(ctx, "rrt_resolve", ss, w, h, band, &local_rows)) return rc;
+    // the kernel reads hdr_hi while it writes hdr_out: the two must not share a byte
+    if (hdr_out && f4_overlap(hdr_hi, (unsigned long long)ss * ss * w * h, hdr_out, (unsigned long long)w * h))
+        return fail(ctx, RRT_ERR_BAD_ARG, "rrt_resolve: hdr_out overlaps hdr_hi");
+    if (local_rows == 0) return RRT_OK;
+
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    return launch_resolve(ctx, prm, fx, ss, 1, w, h, band, local_rows, hdr_hi, 0, d_out, out_layout, hdr_out, (cudaStream_t)stream);
+}
+
+// A stream-ordered block of `bytes` from the context's scratch pool (created on first use), for rrt_render_ss's
+// supersampled plane and the sub-frame stacks of rrt_render_mb / rrt_capture_render_mb.  ctx->mu held.
+static int scratch_alloc(rrt_context* ctx, const char* nomem_msg, size_t bytes, cudaStream_t st, float** out) {
+    DevGuard g(ctx->device);
+    if (!ctx->ss_pool) {
+        cudaMemPoolProps props;
+        std::memset(&props, 0, sizeof(props));
+        props.allocType = cudaMemAllocationTypePinned;
+        props.location.type = cudaMemLocationTypeDevice;
+        props.location.id = ctx->device;
+        RRT_CU(ctx, cudaMemPoolCreate(&ctx->ss_pool, &props));
+        uint64_t keep = UINT64_MAX;   // hold freed blocks: the next frame of a sequence reuses them without a new allocation
+        RRT_CU(ctx, cudaMemPoolSetAttribute(ctx->ss_pool, cudaMemPoolAttrReleaseThreshold, &keep));
+    }
+    if (cudaMallocFromPoolAsync((void**)out, bytes, ctx->ss_pool, st) != cudaSuccess) {
+        cudaGetLastError();
+        return fail(ctx, RRT_ERR_NOMEM, nomem_msg);
+    }
     return RRT_OK;
 }
 
@@ -816,21 +849,8 @@ int rrt_render_ss(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam
     if (n_hi > SIZE_MAX / 16) return fail(ctx, RRT_ERR_NOMEM, "rrt_render_ss: supersampled hdr plane larger than the address space");
     {
         std::lock_guard<std::mutex> lk(ctx->mu);
-        DevGuard g(ctx->device);
-        if (!ctx->ss_pool) {
-            cudaMemPoolProps props;
-            std::memset(&props, 0, sizeof(props));
-            props.allocType = cudaMemAllocationTypePinned;
-            props.location.type = cudaMemLocationTypeDevice;
-            props.location.id = ctx->device;
-            RRT_CU(ctx, cudaMemPoolCreate(&ctx->ss_pool, &props));
-            uint64_t keep = UINT64_MAX;   // hold freed blocks: the next frame of a sequence reuses them without a new allocation
-            RRT_CU(ctx, cudaMemPoolSetAttribute(ctx->ss_pool, cudaMemPoolAttrReleaseThreshold, &keep));
-        }
-        if (cudaMallocFromPoolAsync((void**)&hi, (size_t)16 * n_hi, ctx->ss_pool, st) != cudaSuccess) {
-            cudaGetLastError();
-            return fail(ctx, RRT_ERR_NOMEM, "rrt_render_ss: no memory for the supersampled hdr plane");
-        }
+        if (int rc = scratch_alloc(ctx, "rrt_render_ss: no memory for the supersampled hdr plane", (size_t)16 * n_hi, st, &hi))
+            return rc;
     }
     rrt_planes pl;
     std::memset(&pl, 0, sizeof(pl));
@@ -840,6 +860,68 @@ int rrt_render_ss(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam
     DevGuard g(ctx->device);
     const cudaError_t e = cudaFreeAsync(hi, st);   // stream-ordered: the block goes back to the pool once the resolve has read it
     if (rc == RRT_OK && e != cudaSuccess) return fail(ctx, RRT_ERR_CUDA, "rrt_render_ss: cudaFreeAsync", e);
+    return rc;
+}
+
+// What rrt_resolve_time, rrt_render_mb and rrt_capture_render_mb check: n, the frame, the band (at most 2^30 pixels, like
+// rrt_render) and a stack of n full-frame planes that fits the address space.  Sets *local_rows, the band's rows.
+static int check_mb(rrt_context* ctx, const char* what, int n, int w, int h, const rrt_band* band, int* local_rows) {
+    std::string m = what;
+    if (n < 1 || n > 64 || w <= 0 || h <= 0) return fail(ctx, RRT_ERR_BAD_ARG, (m + ": bad argument").c_str());
+    const int rows = rrt_band_rows(band, h);
+    if (rows < 0) return fail(ctx, RRT_ERR_BAD_ARG, (m + ": bad band").c_str());
+    if ((long long)w * rows > (1ll << 30)) return fail(ctx, RRT_ERR_BAD_ARG, (m + ": band larger than 2^30 pixels").c_str());
+    if ((unsigned long long)w * h > SIZE_MAX / 16 / (unsigned)n)
+        return fail(ctx, RRT_ERR_BAD_ARG, (m + ": sub-frame stack larger than the address space").c_str());
+    *local_rows = rows;
+    return RRT_OK;
+}
+
+int rrt_resolve_time(rrt_context* ctx, const rrt_params* prm, const rrt_effects* fx, int n, int w, int h, const rrt_band* band,
+                     const float* hdr_stack, void* d_out, int out_layout, float* hdr_out, void* stream) {
+    if (!ctx) return RRT_ERR_BAD_ARG;
+    if (!prm || !fx || !hdr_stack || (out_layout != RRT_OUT_FRAME && out_layout != RRT_OUT_PACKED) || (!d_out && !hdr_out))
+        return fail(ctx, RRT_ERR_BAD_ARG, "rrt_resolve_time: bad argument");
+    int local_rows = 0;
+    if (int rc = check_mb(ctx, "rrt_resolve_time", n, w, h, band, &local_rows)) return rc;
+    const unsigned long long plane = (unsigned long long)w * h;
+    if (hdr_out && f4_overlap(hdr_stack, (unsigned long long)n * plane, hdr_out, plane))
+        return fail(ctx, RRT_ERR_BAD_ARG, "rrt_resolve_time: hdr_out overlaps hdr_stack");
+    if (local_rows == 0) return RRT_OK;
+
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    return launch_resolve(ctx, prm, fx, 1, n, w, h, band, local_rows, hdr_stack, (size_t)plane, d_out, out_layout, hdr_out,
+                          (cudaStream_t)stream);
+}
+
+int rrt_render_mb(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cams, const rrt_effects* fx, uint64_t sky_texture,
+                  const float* times, int n, int w, int h, const rrt_band* band, void* d_out, int out_layout, float* hdr_out,
+                  void* stream) {
+    if (!ctx) return RRT_ERR_BAD_ARG;
+    if (!prm || !cams || !fx || !times || sky_texture == 0 || prm->max_steps < 0 ||
+        (out_layout != RRT_OUT_FRAME && out_layout != RRT_OUT_PACKED) || (!d_out && !hdr_out))
+        return fail(ctx, RRT_ERR_BAD_ARG, "rrt_render_mb: bad argument");
+    int local_rows = 0;
+    if (int rc = check_mb(ctx, "rrt_render_mb", n, w, h, band, &local_rows)) return rc;
+    if (local_rows == 0) return RRT_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t plane = (size_t)w * h;   // full-frame indexed like every plane of this ABI, so full-frame sized even for a band
+    float* stack = nullptr;
+    {
+        std::lock_guard<std::mutex> lk(ctx->mu);
+        if (int rc = scratch_alloc(ctx, "rrt_render_mb: no memory for the sub-frame stack", 16 * n * plane, st, &stack)) return rc;
+    }
+    rrt_planes pl;
+    std::memset(&pl, 0, sizeof(pl));
+    int rc = RRT_OK;
+    for (int i = 0; i < n && rc == RRT_OK; ++i) {
+        pl.hdr = stack + 4 * plane * i;
+        rc = rrt_render(ctx, prm, &cams[i], fx, sky_texture, times[i], w, h, band, nullptr, RRT_OUT_FRAME, &pl, stream);
+    }
+    if (rc == RRT_OK) rc = rrt_resolve_time(ctx, prm, fx, n, w, h, band, stack, d_out, out_layout, hdr_out, stream);
+    DevGuard g(ctx->device);
+    const cudaError_t e = cudaFreeAsync(stack, st);   // stream-ordered: the block goes back to the pool once the resolve has read it
+    if (rc == RRT_OK && e != cudaSuccess) return fail(ctx, RRT_ERR_CUDA, "rrt_render_mb: cudaFreeAsync", e);
     return rc;
 }
 
@@ -1029,22 +1111,27 @@ int rrt_capture_create(rrt_context* ctx, const rrt_params* prm, const rrt_camera
 
 #undef CAP_CU
 
-int rrt_capture_render(rrt_capture* cap, const rrt_params* prm, const rrt_effects* fx, uint64_t sky_texture, float time, void* d_out,
-                       int out_layout, float* hdr_out, void* stream) {
-    if (!cap) return fail(nullptr, RRT_ERR_BAD_ARG, "rrt_capture_render: capture is NULL");
-    rrt_context* ctx = cap->ctx;
+}  // extern "C"
+
+// What rrt_capture_render and rrt_capture_render_mb check besides their own arguments: rrt_capture_render's rules.
+static int check_capture_render(rrt_capture* cap, const char* what, const rrt_params* prm, const rrt_effects* fx, uint64_t sky_texture,
+                                void* d_out, int out_layout, float* hdr_out) {
+    const std::string m = what;
     if (!prm || !fx || sky_texture == 0 || (out_layout != RRT_OUT_FRAME && out_layout != RRT_OUT_PACKED) || (!d_out && !hdr_out))
-        return fail(ctx, RRT_ERR_BAD_ARG, "rrt_capture_render: bad argument");
+        return fail(cap->ctx, RRT_ERR_BAD_ARG, (m + ": bad argument").c_str());
     if (((prm->flags ^ cap->prm.flags) & RRT_FLAG_FMAD) || fx->use_lens != cap->fx.use_lens ||
         std::memcmp(&fx->distortion_amount, &cap->fx.distortion_amount, sizeof(float)) != 0)
-        return fail(ctx, RRT_ERR_BAD_ARG, "rrt_capture_render: the RRT_FLAG_FMAD bit, use_lens and distortion_amount must be the capture's");
-    if (cap->local_rows == 0) return RRT_OK;
+        return fail(cap->ctx, RRT_ERR_BAD_ARG, (m + ": the RRT_FLAG_FMAD bit, use_lens and distortion_amount must be the capture's").c_str());
+    return RRT_OK;
+}
 
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    DevGuard g(ctx->device);
-    cudaStream_t st = (cudaStream_t)stream;
+// The kernels of one render of a capture at `time`, enqueued on `st`: shade, media, fold and, when the pass left tiles,
+// the sweep.  Arguments checked, ctx->mu held, `st` ordered after the capture's previous render.
+static int capture_enqueue(rrt_capture* cap, float exposure, const rrt_effects* fx, uint64_t sky_texture, float time, void* d_out,
+                           int out_layout, float* hdr_out, cudaStream_t st) {
+    rrt_context* ctx = cap->ctx;
     rrt_params P = cap->prm;
-    P.exposure = prm->exposure;
+    P.exposure = exposure;
     const bool fmad = (P.flags & RRT_FLAG_FMAD) != 0;
     const rrtk::SplitKernels* sk = fmad ? rrtk::rrt_split_kernels_fmad() : rrtk::rrt_split_kernels_strict();
     FrameArgs A = frame_args(P, cap->cam, *fx, sky_texture, time, cap->w, cap->h, cap->band, cap->local_rows, out_layout, d_out);
@@ -1054,7 +1141,6 @@ int rrt_capture_render(rrt_capture* cap, const rrt_params* prm, const rrt_effect
     rrtk::PassCtrl* pcs = (rrtk::PassCtrl*)cap->d_ctrl;
     const int per_sm_media = resident_per_sm(ctx, (const void*)sk->media_results, kMediaBlock, true);
     const int per_sm_fold = resident_per_sm(ctx, (const void*)sk->fold_results, 128, false);
-    RRT_CU(ctx, cudaStreamWaitEvent(st, cap->done, 0));   // one render at a time per capture, whatever the streams
     // 1. every pixel from the planes; right for the rays the trace finished, overwritten below for the others
     const long long n = (long long)cap->w * cap->local_rows;
     kset(&P)->shade<<<(unsigned)((n + kShadeBlock - 1) / kShadeBlock), kShadeBlock, 0, st>>>(A, cap->planes);
@@ -1082,8 +1168,62 @@ int rrt_capture_render(rrt_capture* cap, const rrt_params* prm, const rrt_effect
     }
     RRT_CU(ctx, cudaGetLastError());
     ctx->launches += launches;
-    RRT_CU(ctx, cudaEventRecord(cap->done, st));
     return RRT_OK;
+}
+
+extern "C" {
+
+int rrt_capture_render(rrt_capture* cap, const rrt_params* prm, const rrt_effects* fx, uint64_t sky_texture, float time, void* d_out,
+                       int out_layout, float* hdr_out, void* stream) {
+    if (!cap) return fail(nullptr, RRT_ERR_BAD_ARG, "rrt_capture_render: capture is NULL");
+    if (int rc = check_capture_render(cap, "rrt_capture_render", prm, fx, sky_texture, d_out, out_layout, hdr_out)) return rc;
+    if (cap->local_rows == 0) return RRT_OK;
+
+    rrt_context* ctx = cap->ctx;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DevGuard g(ctx->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    RRT_CU(ctx, cudaStreamWaitEvent(st, cap->done, 0));   // one render at a time per capture, whatever the streams
+    const int rc = capture_enqueue(cap, prm->exposure, fx, sky_texture, time, d_out, out_layout, hdr_out, st);
+    // recorded even when the enqueue failed part-way: whatever it did enqueue stays ordered before the next render
+    const cudaError_t e = cudaEventRecord(cap->done, st);
+    if (rc != RRT_OK) return rc;
+    if (e != cudaSuccess) return fail(ctx, RRT_ERR_CUDA, "rrt_capture_render: cudaEventRecord", e);
+    return RRT_OK;
+}
+
+int rrt_capture_render_mb(rrt_capture* cap, const rrt_params* prm, const rrt_effects* fx, uint64_t sky_texture, const float* times,
+                          int n, void* d_out, int out_layout, float* hdr_out, void* stream) {
+    if (!cap) return fail(nullptr, RRT_ERR_BAD_ARG, "rrt_capture_render_mb: capture is NULL");
+    rrt_context* ctx = cap->ctx;
+    if (!times) return fail(ctx, RRT_ERR_BAD_ARG, "rrt_capture_render_mb: bad argument");
+    if (int rc = check_capture_render(cap, "rrt_capture_render_mb", prm, fx, sky_texture, d_out, out_layout, hdr_out)) return rc;
+    int local_rows = 0;
+    if (int rc = check_mb(ctx, "rrt_capture_render_mb", n, cap->w, cap->h, &cap->band, &local_rows)) return rc;
+    if (local_rows == 0) return RRT_OK;
+
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DevGuard g(ctx->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t plane = (size_t)cap->w * cap->h;   // full-frame, like the capture's own planes
+    float* stack = nullptr;
+    if (int rc = scratch_alloc(ctx, "rrt_capture_render_mb: no memory for the sub-frame stack", 16 * n * plane, st, &stack)) return rc;
+    // the capture's state is in use from the first sub-frame to the last: wait for its previous render once, record once
+    int rc = RRT_OK;
+    if (cudaError_t e = cudaStreamWaitEvent(st, cap->done, 0)) {
+        rc = fail(ctx, RRT_ERR_CUDA, "rrt_capture_render_mb: cudaStreamWaitEvent", e);
+    } else {
+        for (int i = 0; i < n && rc == RRT_OK; ++i)
+            rc = capture_enqueue(cap, prm->exposure, fx, sky_texture, times[i], nullptr, RRT_OUT_FRAME, stack + 4 * plane * i, st);
+        // recorded even when a sub-frame failed: whatever was enqueued stays ordered before the capture's next render
+        const cudaError_t er = cudaEventRecord(cap->done, st);
+        if (rc == RRT_OK && er != cudaSuccess) rc = fail(ctx, RRT_ERR_CUDA, "rrt_capture_render_mb: cudaEventRecord", er);
+    }
+    if (rc == RRT_OK)
+        rc = launch_resolve(ctx, prm, fx, 1, n, cap->w, cap->h, &cap->band, local_rows, stack, plane, d_out, out_layout, hdr_out, st);
+    const cudaError_t e = cudaFreeAsync(stack, st);   // stream-ordered: the block goes back to the pool once the resolve has read it
+    if (rc == RRT_OK && e != cudaSuccess) return fail(ctx, RRT_ERR_CUDA, "rrt_capture_render_mb: cudaFreeAsync", e);
+    return rc;
 }
 
 int rrt_capture_info(const rrt_capture* cap, uint64_t out[8]) {

@@ -132,6 +132,17 @@ float rrt_path_clock(int frame, float fps) {
     return t;
 }
 
+int rrt_shutter_times(float t, float shutter, float fps, int n, float* out) {
+    if (!out || !(shutter >= 0.0f && shutter <= 1.0f) || !(fps > 0.0f) || n < 1 || n > 64) return RRT_ERR_BAD_ARG;
+    // a shutter open for `shutter` of the frame interval, centred on t; every operation one binary32 op (no contraction)
+    const float d = shutter / fps;
+    for (int i = 0; i < n; ++i) {
+        const float u = ((float)i + 0.5f) / (float)n - 0.5f;
+        out[i] = t + d * u;
+    }
+    return RRT_OK;
+}
+
 // ---- frame sink: the step immediately after the hot path --------------------------------------------------
 // The reference's ScreenRecorder (src/main.cpp:29-124) reads the window back with glReadPixels -- which, for the
 // 1:1 textured quad it draws (src/main.cpp:404-409, 471-479), returns exactly the bytes launch_raymarch wrote,

@@ -1,5 +1,5 @@
 // rrt_kernel.cuh -- the render kernel (one 8x4-pixel tile per persistent warp), its per-ray helpers, the re-shading
-// kernel (rrt_shade), the supersample resolve kernel (rrt_resolve) and the function-level probe kernels.  Compiled
+// kernel (rrt_shade), the resolve kernel (rrt_resolve, rrt_resolve_time) and the function-level probe kernels.  Compiled
 // TWICE, once per rounding contract (include/rrt_device.cuh):
 //   rrt_b200.cu   RRT_FMAD = 0, nvcc -fmad=false   -> rrt_kernels_strict()
 //   rrt_fmad.cu   RRT_FMAD = 1, nvcc -fmad=true    -> rrt_kernels_fmad()
@@ -47,7 +47,8 @@ struct KernelSet {
     void (*disk_density)(Consts, int, const float*, float, float*);
     void (*dust_density)(Consts, int, const float*, float, float*);
     void (*shade)(const FrameArgs, const rrt_planes);  // rrt_shade: the step after the ray loop, from traced planes
-    void (*resolve)(const FrameArgs, const float4*, int);  // rrt_resolve: box filter of an ss x ss hdr plane + post step
+    // rrt_resolve / rrt_resolve_time: mean of ss x ss blocks of n hdr planes + post step
+    void (*resolve)(const FrameArgs, const float4*, int, int, size_t);
 };
 const KernelSet* rrt_kernels_strict();
 const KernelSet* rrt_kernels_fmad();
@@ -558,16 +559,21 @@ __global__ void __launch_bounds__(kShadeBlock) shade_kernel(const __grid_constan
     finish_ray_inl(A, x, y, ly, uvx, uvy, I.x, I.y, I.z, hdr.w, mk(0.f, 0.f, 0.f), mk(v.x, v.y, v.z), 0, end);
 }
 
-// ---- supersample resolve (rrt_resolve, rrt_render_ss) -----------------------------------------------
-// Box filter of an ss*w x ss*h hdr plane `hi` ([Y * ss*w + X]) into the w x h frame of A: output pixel (x, y) is the mean
-// of sub-samples (ss*x + i, ss*y + j), summed from (0, 0) in row-major order (j outer, i inner) and divided by ss*ss, with
-// the explicit round-to-nearest intrinsics so that both contracts give the same bits (and numpy reproduces them).  The
-// mean (.w = mean T) goes to A.planes.hdr, then the render's own post step (bloom, vignette at the output pixel's
-// pixel_uv, tonemap, store) runs on it.  One thread per output pixel of the band, rows mapped like shade_kernel's;
-// neighbouring threads read neighbouring ss*16-byte runs of each sub-row.
+// ---- resolve: supersample and shutter mean (rrt_resolve, rrt_render_ss, rrt_resolve_time, rrt_render_mb) ------------
+// Box filter of n planes of ss*w x ss*h hdr values into the w x h frame of A.  Plane q starts at hi + q*plane_stride (in
+// float4) and is indexed [Y * ss*w + X].  Output pixel (x, y) is the mean of sub-samples (ss*x + i, ss*y + j) of every
+// plane, summed plane by plane (outer), then j, then i from (plane 0, 0, 0) and divided by n*ss*ss, with the explicit
+// round-to-nearest intrinsics so that both contracts give the same bits (and numpy reproduces them).  rrt_resolve is
+// n = 1, rrt_resolve_time is ss = 1.  The mean (.w = mean T) goes to A.planes.hdr, then the render's own post step
+// (bloom, vignette at the output pixel's pixel_uv, tonemap, store) runs on it.  One thread per output pixel of the band,
+// rows mapped like shade_kernel's; neighbouring threads read neighbouring ss*16-byte runs of each sub-row.
 constexpr int kResolveBlock = 256;
-__global__ void __launch_bounds__(kResolveBlock) resolve_kernel(const __grid_constant__ FrameArgs A, const float4* __restrict__ hi, int ss) {
-    const int i = blockIdx.x * kResolveBlock + threadIdx.x;   // w * local_rows <= 2^30 (rrt_resolve)
+__device__ __forceinline__ void add4_rn(float4& s, const float4 v) {
+    s.x = __fadd_rn(s.x, v.x); s.y = __fadd_rn(s.y, v.y); s.z = __fadd_rn(s.z, v.z); s.w = __fadd_rn(s.w, v.w);
+}
+__global__ void __launch_bounds__(kResolveBlock) resolve_kernel(const __grid_constant__ FrameArgs A, const float4* __restrict__ hi, int ss,
+                                                                int n, size_t plane_stride) {
+    const int i = blockIdx.x * kResolveBlock + threadIdx.x;   // w * local_rows <= 2^30 (rrt_resolve, rrt_resolve_time)
     if (i >= A.w * A.local_rows) return;
     const int ly = i / A.w, x = i - ly * A.w;
     const int grp = ly / A.band_group;
@@ -576,13 +582,16 @@ __global__ void __launch_bounds__(kResolveBlock) resolve_kernel(const __grid_con
     const size_t W = (size_t)ss * A.w;
     const float4* p = hi + (size_t)ss * y * W + (size_t)ss * x;
     float4 s = p[0];
-    for (int j = 0; j < ss; ++j)
-        for (int k = j == 0 ? 1 : 0; k < ss; ++k) {
-            const float4 v = p[j * W + k];
-            s.x = __fadd_rn(s.x, v.x); s.y = __fadd_rn(s.y, v.y); s.z = __fadd_rn(s.z, v.z); s.w = __fadd_rn(s.w, v.w);
-        }
-    const float n = (float)(ss * ss);
-    s = make_float4(__fdiv_rn(s.x, n), __fdiv_rn(s.y, n), __fdiv_rn(s.z, n), __fdiv_rn(s.w, n));
+    if (ss == 1) {   // one float4 per plane: unrolled so that the loads of several planes are in flight together
+#pragma unroll 4
+        for (int q = 1; q < n; ++q) add4_rn(s, p[q * plane_stride]);
+    } else {
+        for (int q = 0; q < n; ++q)
+            for (int j = 0; j < ss; ++j)
+                for (int k = q == 0 && j == 0 ? 1 : 0; k < ss; ++k) add4_rn(s, p[q * plane_stride + j * W + k]);
+    }
+    const float d = (float)(n * ss * ss);
+    s = make_float4(__fdiv_rn(s.x, d), __fdiv_rn(s.y, d), __fdiv_rn(s.z, d), __fdiv_rn(s.w, d));
     if (A.planes.hdr) reinterpret_cast<float4*>(A.planes.hdr)[(size_t)y * A.w + x] = s;
     if (!A.out) return;
     float uvx, uvy;

@@ -303,14 +303,25 @@ class PathSequence:
     C-ABI host functions (``rrt_path_state`` / ``rrt_path_clock``), so frame k is the same pure function of k
     on every rank count.  ``ss`` > 1 renders every frame anti-aliased with ss x ss rays per pixel (``Renderer.render_ss``
     into the slot's device frame, then the same pinned copy), which keeps the photon ring, the disk's inner edge and the
-    stars from crawling between frames."""
+    stars from crawling between frames.  ``samples`` > 1 renders every frame motion-blurred (``Renderer.render_mb``): a
+    shutter open for ``shutter`` (0..1) of the frame interval, centred on the frame's clock, with ``samples`` sub-frames at
+    ``shutter_times(path_clock(k, fps), shutter, fps, samples)``, each with the path's camera at its own time, so that the
+    disk's rotation and the camera's motion smear instead of strobing.  ``samples`` > 1 does not combine with ``ss`` > 1
+    here; the C ABI composes the two (rrt_resolve_time, then rrt_resolve)."""
 
-    def __init__(self, renderer, w: int, h: int, depth: int = 2, ss: int = 1):
+    def __init__(self, renderer, w: int, h: int, depth: int = 2, ss: int = 1, shutter: float = 0.0, samples: int = 1):
         if not 1 <= depth <= HOST_SLOTS:
             raise ValueError(f"depth must be 1..{HOST_SLOTS}")
         if not 1 <= ss <= 8:
             raise ValueError("ss must be 1..8")
+        if not 1 <= samples <= 64:
+            raise ValueError("samples must be 1..64")
+        if not 0.0 <= shutter <= 1.0:
+            raise ValueError("shutter must be in [0, 1]")
+        if ss > 1 and samples > 1:
+            raise ValueError("ss > 1 together with samples > 1 is not supported by PathSequence")
         self.r, self.w, self.h, self.depth, self.ss = renderer, w, h, depth, ss
+        self.shutter, self.samples = float(shutter), samples
         self.world = dist.get_world_size() if dist.is_initialized() else 1
         self.rank = dist.get_rank() if dist.is_initialized() else 0
         dev = renderer.device
@@ -318,14 +329,14 @@ class PathSequence:
         self.events = [torch.cuda.Event() for _ in range(depth)]
         root = self.rank == 0
         self.local = ([torch.zeros((h, w, 4), dtype=torch.uint8, device=dev) for _ in range(depth)]
-                      if self.world > 1 or ss > 1 else None)
+                      if self.world > 1 or ss > 1 or samples > 1 else None)
         self.gathered = ([torch.zeros((self.world, h, w, 4), dtype=torch.uint8, device=dev) for _ in range(depth)]
                          if root and self.world > 1 else None)
         self.host = [torch.zeros((self.world, h, w, 4), dtype=torch.uint8).pin_memory() for _ in range(depth)] if root else None
 
     def render(self, path_index: int, n_frames: int, prm, fx, sky, fps: float = 24.0, sink=None, first_frame: int = 1):
         """Render frames first_frame .. first_frame+n_frames-1 of the path.  Returns (frames_done, launches)."""
-        from .renderer import path_clock, path_state
+        from .renderer import path_clock, path_state, shutter_times
         cur = torch.cuda.current_stream(self.r.device)
         for s in self.streams:
             s.wait_stream(cur)
@@ -354,7 +365,7 @@ class PathSequence:
             mine = frames[self.rank]
             s = self.streams[k]
             with torch.cuda.stream(s):
-                if self.world == 1 and self.ss == 1:
+                if self.world == 1 and self.ss == 1 and self.samples == 1:
                     t = path_clock(mine, fps)
                     cam, _ = path_state(path_index, t)
                     self.r.render_host_async(prm, cam, fx, sky, t, self.w, self.h, self.host[k][0], slot=k, stream=s)
@@ -362,7 +373,11 @@ class PathSequence:
                     if mine is not None:
                         t = path_clock(mine, fps)
                         cam, _ = path_state(path_index, t)
-                        if self.ss == 1:
+                        if self.samples > 1:
+                            times = shutter_times(t, self.shutter, fps, self.samples)
+                            cams = [path_state(path_index, ti)[0] for ti in times]
+                            self.r.render_mb(prm, cams, fx, sky, times, self.w, self.h, out=self.local[k], stream=s)
+                        elif self.ss == 1:
                             self.r.render(prm, cam, fx, sky, t, self.w, self.h, out=self.local[k], stream=s)
                         else:
                             self.r.render_ss(prm, cam, fx, sky, t, self.w, self.h, self.ss, out=self.local[k], stream=s)

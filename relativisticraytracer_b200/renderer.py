@@ -54,6 +54,21 @@ def path_duration(path_index: int) -> float:
     return float(_capi.load().rrt_path_duration(int(path_index)))
 
 
+def shutter_times(t: float, shutter: float, fps: float, n: int) -> list:
+    """rrt_shutter_times: the n sub-frame times of a shutter open for ``shutter`` (0..1) of the frame interval 1/fps,
+    centred on t: t + (shutter/fps) * ((i + 0.5)/n - 0.5), each operation in float32.  n = 1 gives [t].  Host only."""
+    out = (C.c_float * max(int(n), 1))()
+    rc = _capi.load().rrt_shutter_times(float(t), float(shutter), float(fps), int(n), out)
+    if rc != 0:
+        raise RrtError(rc, f"rrt_shutter_times({t}, {shutter}, {fps}, {n}): shutter must be in [0, 1], fps > 0, n in 1..64")
+    return [float(v) for v in out]
+
+
+def _f32_array(values) -> C.Array:
+    values = [float(v) for v in values]
+    return (C.c_float * len(values))(*values)
+
+
 class Sky:
     """A skybox texture object (rrt_sky) -- the device half of the reference's loadSkybox."""
 
@@ -108,6 +123,21 @@ class Capture:
         st = stream if stream is not None else torch.cuda.current_stream(r.device)
         r._check(r._lib.rrt_capture_render(self._h, C.byref(prm), C.byref(fx), C.c_uint64(tex), float(time), C.c_void_p(out_ptr),
                                            int(layout), C.c_void_p(hdr_ptr), C.c_void_p(st.cuda_stream)))
+        return out
+
+    def render_mb(self, prm: Params, fx: Effects, sky: "Sky | int", times, *, out=None, layout: int = OUT_FRAME,
+                  hdr_out: Optional[torch.Tensor] = None, stream: Optional[torch.cuda.Stream] = None) -> torch.Tensor:
+        """rrt_capture_render_mb: the captured frame motion-blurred over ``times`` (1..64 sub-frames), without a new trace;
+        asynchronous.  Gives the bytes of ``Renderer.render_mb`` with the capture's camera for every sub-frame, under the
+        rules of ``render``.  ``out``, ``layout`` and ``hdr_out`` (the mean) as in ``render``; returns the frame."""
+        r = self._r
+        tex = sky.texture if isinstance(sky, Sky) else int(sky)
+        ts = _f32_array(times)
+        out, out_ptr = r._frame_out(out, layout, self.band, self.w, self.h)
+        hdr_ptr = r._plane_ptr("hdr", hdr_out, self.w, self.h) if hdr_out is not None else None
+        st = stream if stream is not None else torch.cuda.current_stream(r.device)
+        r._check(r._lib.rrt_capture_render_mb(self._h, C.byref(prm), C.byref(fx), C.c_uint64(tex), ts, len(ts), C.c_void_p(out_ptr),
+                                              int(layout), C.c_void_p(hdr_ptr), C.c_void_p(st.cuda_stream)))
         return out
 
     def info(self) -> dict:
@@ -277,6 +307,46 @@ class Renderer:
         self._check(self._lib.rrt_resolve(self._ctx, C.byref(prm), C.byref(fx), int(ss), int(w), int(h),
                                           C.byref(band) if band is not None else None, C.c_void_p(hi_ptr),
                                           C.c_void_p(out_ptr), int(layout), C.c_void_p(hdr_ptr), C.c_void_p(st.cuda_stream)))
+        return out
+
+    def resolve_time(self, prm: Params, fx: Effects, hdr_stack: torch.Tensor, w: int, h: int, *, band: Optional[Band] = None,
+                     out=None, layout: int = OUT_FRAME, hdr_out: Optional[torch.Tensor] = None,
+                     stream: Optional[torch.cuda.Stream] = None) -> torch.Tensor:
+        """rrt_resolve_time: the mean of the n planes of ``hdr_stack`` ((n, h, w, 4) float32, 1 <= n <= 64, e.g. the hdr
+        planes of n renders), summed from plane 0 in float32 and divided by n, then the post step (bloom, vignette, exposure
+        tonemap, store) on it; asynchronous.  ``hdr_out`` ((h, w, 4) float32, not overlapping ``hdr_stack``) receives the
+        mean.  ``band``, ``out`` and ``layout`` as in ``render``; returns the frame."""
+        out, out_ptr = self._frame_out(out, layout, band, w, h)
+        assert hdr_stack.dim() == 4 and tuple(hdr_stack.shape[1:]) == (h, w, 4), "hdr_stack must be (n, h, w, 4)"
+        n = int(hdr_stack.shape[0])
+        stack_ptr = self._plane_ptr("hdr", hdr_stack, w, n * h)
+        hdr_ptr = self._plane_ptr("hdr", hdr_out, w, h) if hdr_out is not None else None
+        st = stream if stream is not None else torch.cuda.current_stream(self.device)
+        self._check(self._lib.rrt_resolve_time(self._ctx, C.byref(prm), C.byref(fx), n, int(w), int(h),
+                                               C.byref(band) if band is not None else None, C.c_void_p(stack_ptr),
+                                               C.c_void_p(out_ptr), int(layout), C.c_void_p(hdr_ptr), C.c_void_p(st.cuda_stream)))
+        return out
+
+    def render_mb(self, prm: Params, cam, fx: Effects, sky: Sky | int, times, w: int, h: int, *, band: Optional[Band] = None,
+                  out=None, layout: int = OUT_FRAME, hdr_out: Optional[torch.Tensor] = None,
+                  stream: Optional[torch.cuda.Stream] = None) -> torch.Tensor:
+        """rrt_render_mb: one motion-blurred frame (or band), the mean of n = len(times) renders (1 <= n <= 64) with the
+        render's own bloom / vignette / tonemap on it; asynchronous.  Sub-frame i is ``render`` at ``times[i]`` with camera
+        ``cam`` (one Camera for every sub-frame) or ``cam[i]`` (a sequence of n); n = 1 is ``render``.  ``hdr_out``
+        (h, w, 4) float32 receives the mean (.w = mean T).  ``band``, ``out`` (a tensor or a PeerFrame) and ``layout`` as
+        in ``render``."""
+        tex = sky.texture if isinstance(sky, Sky) else int(sky)
+        ts = _f32_array(times)
+        cams = [cam] * len(ts) if isinstance(cam, Camera) else list(cam)
+        if len(cams) != len(ts):
+            raise ValueError(f"render_mb: {len(cams)} cameras for {len(ts)} times")
+        cam_arr = (Camera * max(len(cams), 1))(*cams)
+        out, out_ptr = self._frame_out(out, layout, band, w, h)
+        hdr_ptr = self._plane_ptr("hdr", hdr_out, w, h) if hdr_out is not None else None
+        st = stream if stream is not None else torch.cuda.current_stream(self.device)
+        self._check(self._lib.rrt_render_mb(self._ctx, C.byref(prm), cam_arr, C.byref(fx), C.c_uint64(tex), ts, len(ts),
+                                            int(w), int(h), C.byref(band) if band is not None else None,
+                                            C.c_void_p(out_ptr), int(layout), C.c_void_p(hdr_ptr), C.c_void_p(st.cuda_stream)))
         return out
 
     def capture(self, prm: Params, cam: Camera, fx: Effects, sky: Sky | int, w: int, h: int, *, band: Optional[Band] = None,
