@@ -215,6 +215,25 @@ int rrt_render_ss(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam
                   uint64_t sky_texture, float time, int w, int h, int ss, const rrt_band* band,
                   void* d_out, int out_layout, float* hdr_out, void* stream);
 
+/* ---- depth of field: each sub-sample of a supersampled pixel from its own camera --------------------------------------
+ * rrt_render_ss with a HOST table cams[ss*ss] in place of cam.  Sub-sample (i, j) of output pixel (x, y) is pixel
+ * (ss*x + i, ss*y + j) of rrt_render(P, cams[j*ss + i], F, S, time, ss*w, ss*h, band {r, N, ss*g}): its ray, step count,
+ * media and sky are that render's bit for bit.  The pixel's hdr value (and T, in .w) is the mean of its ss*ss sub-samples,
+ * summed and divided exactly as rrt_resolve does; bloom, vignette, tonemap and store then run exactly as in rrt_render.
+ * So with every camera equal to cam it is rrt_render_ss(cam) (same bytes, same hdr values), and with ss = 1 it is
+ * rrt_render(cams[0]); the (ss-1)/(2*ss)-pixel shift of rrt_render_ss applies unchanged.  With rrt_lens_cameras' table the
+ * frame has the depth of field of a thin lens at the cost of rrt_render_ss: one trace of ss*ss rays per pixel.
+ * Caveats of that lens: it is a flat-space thin lens at the camera; "in focus" is the plane at distance `focus` along
+ * forward in the camera's local frame, before any bending of the rays; every pixel uses the same ss*ss lens points, so a
+ * strongly defocused highlight (a star, the photon ring) shows as ss*ss discrete copies -- ss is the quality knob.
+ * Bands, RRT_OUT_PACKED and a peer-frame d_out work as in rrt_render_ss; scratch, RRT_ERR_NOMEM and counters are
+ * rrt_render_ss's (the camera table, 48*ss*ss bytes, rides in the same scratch block, copied on `stream`; the caller may
+ * reuse its table as soon as the call returns); launches: the large trace's + 1.  RRT_ERR_BAD_ARG for a NULL table, a
+ * non-finite camera field and everything rrt_render_ss refuses. */
+int rrt_render_dof(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cams, const rrt_effects* fx,
+                   uint64_t sky_texture, float time, int w, int h, int ss, const rrt_band* band,
+                   void* d_out, int out_layout, float* hdr_out, void* stream);
+
 /* ---- captures: one trace, renders at many times -------------------------------------------------------------------
  * With the camera fixed only the time moves, and the time enters only the disk and dust densities: trajectories, step
  * counts, classes and the positions of the media samples are the same at every time (a ray ends only at the horizon, on
@@ -333,8 +352,8 @@ int rrt_set_sample_pool(rrt_context* ctx, size_t max_bytes_per_stream, int max_p
  * the launch, [5] pool size in Ki slots of 32 bytes; all 0 when no frame went through the split pipeline. */
 int rrt_split_stats(rrt_context* ctx, uint32_t out[8]);
 /* Kernels this context has launched so far for rrt_render*, rrt_shade, rrt_resolve*, rrt_capture_* and rrt_assemble_bands
- * (1 per fused frame; 3 per pass + 1 per split frame; 1 per rrt_shade, rrt_resolve or rrt_resolve_time; rrt_render_ss: its
- * ss*w x ss*h render's + 1; rrt_render_mb: its n renders' + 1; 1 per rrt_capture_create, 3 or 4 per rrt_capture_render,
+ * (1 per fused frame; 3 per pass + 1 per split frame; 1 per rrt_shade, rrt_resolve or rrt_resolve_time; rrt_render_ss and
+ * rrt_render_dof: their ss*w x ss*h render's + 1; rrt_render_mb: its n renders' + 1; 1 per rrt_capture_create, 3 or 4 per rrt_capture_render,
  * n * (3 or 4) + 1 per rrt_capture_render_mb):
  * what a benchmark reports as its launch count. */
 uint64_t rrt_kernel_launches(rrt_context* ctx);
@@ -407,6 +426,18 @@ float rrt_path_clock(int frame, float fps);
  * contraction).  n = 1 gives t and shutter = 0 gives t n times (a t of -0 may come back as +0).  RRT_ERR_BAD_ARG for shutter outside
  * [0, 1], fps <= 0, n outside 1..64 or out NULL. */
 int rrt_shutter_times(float t, float shutter, float fps, int n, float* out);
+/* The ss*ss cameras of a thin lens of radius `aperture` at cam->pos, focused on the plane at distance `focus` along
+ * cam->forward (rrt_render_dof's table).  Lens sample k = j*ss + i is the centre of stratified cell (i, j),
+ * (a, b) = (2(i+0.5)/ss - 1, 2(j+0.5)/ss - 1), mapped to the unit disk by Shirley & Chiu's concentric map ((0, 0) -> (0, 0))
+ * and scaled by aperture: (ox, oy), the map evaluated in double precision and rounded to float32 once.  Camera k then is,
+ * per component c and every operation rounded to float32 on its own (no contraction):
+ *   o = right[c] * ox + up[c] * oy      (both products first, then the sum)
+ *   pos[c] = cam->pos[c] + o,   forward[c] = cam->forward[c] - o / focus,   right and up unchanged.
+ * Its ray for image-plane coordinate (u, v) passes through cam->pos + focus * (forward + right*u + up*v) for every lens
+ * point, so that plane is sharp.  aperture == 0, ss == 1 and the centre cell of an odd ss give exact copies of *cam.
+ * RRT_ERR_BAD_ARG for aperture < 0 or non-finite, focus <= 0 or non-finite, ss outside 1..8, or a NULL pointer.
+ * out holds ss*ss cameras. */
+int rrt_lens_cameras(const rrt_camera* cam, float aperture, float focus, int ss, rrt_camera* out);
 
 /* ---- frame sink: the step after the hot path ----------------------------------------------------------
  * Pure host code.  Replaces, for headless use, the reference's ScreenRecorder (src/main.cpp:29-124): frames

@@ -9,6 +9,7 @@
 //                            resolve_kernel, probe kernels
 //   csrc/rrt_packed.cuh      render_kernel_p (two rays per thread, no medium), FMAD contract only
 //   csrc/rrt_split.cuh       the split pipeline of launches with a medium: trace / media / fold kernels
+//                            (every kernel that creates rays also has a LENS variant: rrt_render_dof's per-sub-sample cameras)
 //   this file                band assembly, self-test / roofline probes, rrt_context, every extern "C" entry point
 //
 // Launch organisation (B200: 148 SMs, no tensor-core work on this path -- it is FP32 FMA-pipe bound):
@@ -24,12 +25,14 @@
 #include <algorithm>
 #include <climits>
 #include <cstddef>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <mutex>
 #include <new>
 #include <string>
+#include <vector>
 
 #include "../../include/rrt.h"
 #include "../../include/rrt_device.cuh"
@@ -535,7 +538,7 @@ static rrtk::SplitArgs split_args(uint4* slots, size_t cap_slots, rrtk::TileDesc
 // The split pipeline's tracer for a launch, as rrt_render picks it, and its persistent grid.
 struct TracePlan {
     bool packed;                                          // two rays per thread in packed f32x2 registers (FMAD contract)
-    void (*kernel)(const FrameArgs, const rrtk::SplitArgs);
+    void (*kernel)(const FrameArgs, const rrtk::SplitArgs, const rrtk::LensArgs);
     long long grid;                                       // already divided by the frames in flight
     unsigned ntiles;                                      // tickets of the launch: 16x4 tiles (packed) or 8x4 tiles
     unsigned ngroups;                                     // groups of 32 rays a pass can queue
@@ -543,13 +546,14 @@ struct TracePlan {
 };
 // Whether a launch with these parameters can go through the split pipeline: a tile's rows must fit a TileDesc.
 static bool split_fits(const rrt_params* prm) { return prm->max_steps + 2 <= 128 * (rrtk::kDescChunks - 2); }
-static TracePlan plan_trace(rrt_context* ctx, const rrt_params* prm, int w, int local_rows) {
+// lens: the LENS variant (every ray from its own camera of LensArgs::cams, rrt_render_dof).
+static TracePlan plan_trace(rrt_context* ctx, const rrt_params* prm, int w, int local_rows, bool lens = false) {
     const bool spin = prm->spin_a != 0.0f, fmad = (prm->flags & RRT_FLAG_FMAD) != 0;
     const rrtk::SplitKernels* sk = fmad ? rrtk::rrt_split_kernels_fmad() : rrtk::rrt_split_kernels_strict();
     TracePlan t;
     // the tracer: two rays per thread in packed f32x2 registers where that kernel exists (FMAD contract), else one per thread
     t.packed = sk->trace_packed[0] != nullptr && ctx->trace_choice != 1 && 2ll * (prm->max_steps + 1) + 2 <= 128ll * (rrtk::kDescChunks - 2);
-    t.kernel = t.packed ? sk->trace_packed[spin ? 1 : 0] : sk->trace[spin ? 1 : 0];
+    t.kernel = t.packed ? (lens ? sk->trace_packed_lens : sk->trace_packed)[spin ? 1 : 0] : (lens ? sk->trace_lens : sk->trace)[spin ? 1 : 0];
     const int per_sm_trace = resident_per_sm(ctx, (const void*)t.kernel, kRenderBlock, true);
     const unsigned ntiles8 = (unsigned)(((w + kRTileW - 1) / kRTileW) * ((local_rows + kRTileH - 1) / kRTileH));
     const unsigned ntiles16 = (unsigned)(((w + kTile16W - 1) / kTile16W) * ((local_rows + kTile16H - 1) / kTile16H));
@@ -584,12 +588,14 @@ static FrameArgs frame_args(const rrt_params& prm, const rrt_camera& cam, const 
 }
 
 // One frame through trace / media / fold passes and the closing sweep.  `grid_trace` = the persistent grid of the
-// tracing kernels for this launch (already divided by the frames in flight).
-static int render_split(rrt_context* ctx, const FrameArgs& A, bool spin, bool fmad, bool packed_trace, long long grid_trace, cudaStream_t st,
-                        rrt_context::SamplePool* pl) {
+// tracing kernels for this launch (already divided by the frames in flight).  A camera table in L (rrt_render_dof) selects
+// the LENS tracers: the passes, the redo list and the sweep re-create every ray from its own camera.
+static int render_split(rrt_context* ctx, const FrameArgs& A, const rrtk::LensArgs& L, bool spin, bool fmad, bool packed_trace,
+                        long long grid_trace, cudaStream_t st, rrt_context::SamplePool* pl) {
     const rrtk::SplitKernels* sk = fmad ? rrtk::rrt_split_kernels_fmad() : rrtk::rrt_split_kernels_strict();
-    auto k_trace = packed_trace ? sk->trace_packed[spin ? 1 : 0] : sk->trace[spin ? 1 : 0];
-    auto k_sweep = sk->sweep[spin ? 1 : 0];
+    const bool lens = L.cams != nullptr;
+    auto k_trace = packed_trace ? (lens ? sk->trace_packed_lens : sk->trace_packed)[spin ? 1 : 0] : (lens ? sk->trace_lens : sk->trace)[spin ? 1 : 0];
+    auto k_sweep = (lens ? sk->sweep_lens : sk->sweep)[spin ? 1 : 0];
     const unsigned ntiles = packed_trace ? (unsigned)(((A.w + kTile16W - 1) / kTile16W) * ((A.local_rows + kTile16H - 1) / kTile16H))
                                          : (unsigned)(((A.w + kRTileW - 1) / kRTileW) * ((A.local_rows + kRTileH - 1) / kRTileH));
 
@@ -619,7 +625,7 @@ static int render_split(rrt_context* ctx, const FrameArgs& A, bool spin, bool fm
         S.pc_prev = p ? pcs + (p - 1) : nullptr;
         S.redo_in = p ? redo + (size_t)(p - 1) * kRedoCap : nullptr;
         S.redo_out = redo + (size_t)p * kRedoCap;
-        k_trace<<<(unsigned)grid_trace, kRenderBlock, 0, st>>>(A, S);
+        k_trace<<<(unsigned)grid_trace, kRenderBlock, 0, st>>>(A, S, L);
         sk->media<<<(unsigned)(ctx->sm_count * per_sm_media), kMediaBlock, 0, st>>>(A, S);
         sk->fold<<<(unsigned)(ctx->sm_count * per_sm_fold), 128, 0, st>>>(A, S);
     }
@@ -630,7 +636,7 @@ static int render_split(rrt_context* ctx, const FrameArgs& A, bool spin, bool fm
     S.redo_out = redo + (size_t)passes * kRedoCap;
     long long grid_sweep = ((long long)ctx->sm_count * per_sm_sweep + ctx->frames_in_flight - 1) / ctx->frames_in_flight;
     if (grid_sweep > (long long)ntiles) grid_sweep = ntiles;
-    k_sweep<<<(unsigned)grid_sweep, kRenderBlock, 0, st>>>(A, S);
+    k_sweep<<<(unsigned)grid_sweep, kRenderBlock, 0, st>>>(A, S, L);
     RRT_CU(ctx, cudaGetLastError());
     ctx->launches += 3ull * (unsigned)passes + 1ull;
     RRT_CU(ctx, cudaMemcpyAsync(pl->h_stats, S.stats, 8 * sizeof(unsigned), cudaMemcpyDeviceToHost, st));
@@ -638,9 +644,15 @@ static int render_split(rrt_context* ctx, const FrameArgs& A, bool spin, bool fm
     return RRT_OK;
 }
 
-int rrt_render(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, const rrt_effects* fx, uint64_t sky_texture,
-               float time, int w, int h, const rrt_band* band, void* d_out, int out_layout, const rrt_planes* planes,
-               void* stream) {
+}  // extern "C"
+
+// rrt_render's body.  d_cams: null, or a DEVICE table of cam_ss * cam_ss cameras (rrt_render_dof) -- then the LENS variant
+// of the chosen tracer starts pixel (x, y)'s ray from d_cams[(y % cam_ss) * cam_ss + x % cam_ss] and `cam` is not read by
+// any kernel; cams_near: every camera of the table is in the branch-free domain (LensArgs::near).  Launch choice,
+// pipeline, counters and launch count are rrt_render's either way.
+static int render_frame(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, const rrt_effects* fx, uint64_t sky_texture,
+                        float time, int w, int h, const rrt_band* band, void* d_out, int out_layout, const rrt_planes* planes,
+                        void* stream, const rrt_camera* d_cams, int cam_ss, bool cams_near) {
     if (!ctx) return RRT_ERR_BAD_ARG;
     if (!prm || !cam || !fx || w <= 0 || h <= 0 || sky_texture == 0 || prm->max_steps < 0 ||
         (out_layout != RRT_OUT_FRAME && out_layout != RRT_OUT_PACKED) || (!d_out && !planes))
@@ -660,16 +672,18 @@ int rrt_render(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, c
     A.tile_log = ctx->tile_log;
     A.tile_log_cap = ctx->tile_log_cap;
     A.ticket = ctx->d_tickets + (ctx->ticket_next++ % kTicketRing);
+    rrtk::LensArgs L = {d_cams, d_cams ? cam_ss : 0, d_cams && cams_near ? 1 : 0};
     RRT_CU(ctx, cudaMemsetAsync(A.ticket, 0, sizeof(unsigned), st));
 
     const bool spin = prm->spin_a != 0.0f;
     const bool media = (prm->flags & (RRT_FLAG_DISK | RRT_FLAG_DUST)) != 0;
     const bool fmad = (prm->flags & RRT_FLAG_FMAD) != 0;
+    const bool lens = d_cams != nullptr;
     const rrtk::KernelSet* ks = fmad ? rrtk::rrt_kernels_fmad() : rrtk::rrt_kernels_strict();
-    void (*kern)(const FrameArgs) = ks->render[spin ? 1 : 0][media ? 1 : 0];
+    void (*kern)(const FrameArgs, const rrtk::LensArgs) = (lens ? ks->render_lens : ks->render)[spin ? 1 : 0][media ? 1 : 0];
     long long rays_per_block = kRenderBlock;
     if (fmad && !media && !ctx->scalar_kernel) {
-        kern = ks->render_packed[spin ? 1 : 0];
+        kern = (lens ? ks->render_packed_lens : ks->render_packed)[spin ? 1 : 0];
         rays_per_block = 64;
     }
     if ((long long)w * local_rows > (1ll << 30)) return fail(ctx, RRT_ERR_BAD_ARG, "rrt_render: band larger than 2^30 pixels");
@@ -696,15 +710,23 @@ int rrt_render(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, c
     // A launch with a medium goes through the split pipeline (csrc/rrt_split.cuh) unless the caller pinned the fused
     // kernel, the tile log is selected, or the pool cannot be allocated.
     if (media && ctx->pipeline != RRT_PIPELINE_FUSED && (!ctx->tile_log || ctx->pipeline == RRT_PIPELINE_SPLIT) && split_fits(prm)) {
-        const TracePlan tp = plan_trace(ctx, prm, w, local_rows);
+        const TracePlan tp = plan_trace(ctx, prm, w, local_rows, lens);
         if (rrt_context::SamplePool* pl = acquire_pool(ctx, st, (long long)w * local_rows, tp.ngroups, tp.grid, tp.rows_per_tile))
-            return render_split(ctx, A, spin, fmad, tp.packed, tp.grid, st, pl);
+            return render_split(ctx, A, L, spin, fmad, tp.packed, tp.grid, st, pl);
         if (ctx->pipeline == RRT_PIPELINE_SPLIT) return fail(ctx, RRT_ERR_NOMEM, "rrt_render: no memory for the sample pool of the split pipeline");
     }
-    kern<<<(unsigned)grid, kRenderBlock, 0, st>>>(A);
+    kern<<<(unsigned)grid, kRenderBlock, 0, st>>>(A, L);
     RRT_CU(ctx, cudaGetLastError());
     ctx->launches += 1;
     return RRT_OK;
+}
+
+extern "C" {
+
+int rrt_render(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, const rrt_effects* fx, uint64_t sky_texture,
+               float time, int w, int h, const rrt_band* band, void* d_out, int out_layout, const rrt_planes* planes,
+               void* stream) {
+    return render_frame(ctx, prm, cam, fx, sky_texture, time, w, h, band, d_out, out_layout, planes, stream, nullptr, 0, false);
 }
 
 int rrt_shade(rrt_context* ctx, const rrt_params* prm, const rrt_effects* fx, uint64_t sky_texture, int w, int h,
@@ -830,15 +852,26 @@ static int scratch_alloc(rrt_context* ctx, const char* nomem_msg, size_t bytes, 
     return RRT_OK;
 }
 
-int rrt_render_ss(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, const rrt_effects* fx, uint64_t sky_texture,
-                  float time, int w, int h, int ss, const rrt_band* band, void* d_out, int out_layout, float* hdr_out,
-                  void* stream) {
+// rrt_render_ss's body: the ss*w x ss*h trace into a scratch plane, then rrt_resolve.  cams: null (every sub-sample from
+// `cam`), or a HOST table of ss*ss cameras (rrt_render_dof), copied into the same scratch block behind the plane.
+static int render_ss_frame(rrt_context* ctx, const char* what, const rrt_params* prm, const rrt_camera* cam, const rrt_camera* cams,
+                           const rrt_effects* fx, uint64_t sky_texture, float time, int w, int h, int ss, const rrt_band* band,
+                           void* d_out, int out_layout, float* hdr_out, void* stream) {
+    const std::string m = what;
     if (!ctx) return RRT_ERR_BAD_ARG;
     if (!prm || !cam || !fx || sky_texture == 0 || prm->max_steps < 0 || (out_layout != RRT_OUT_FRAME && out_layout != RRT_OUT_PACKED) ||
         (!d_out && !hdr_out))
-        return fail(ctx, RRT_ERR_BAD_ARG, "rrt_render_ss: bad argument");
+        return fail(ctx, RRT_ERR_BAD_ARG, (m + ": bad argument").c_str());
     int local_rows = 0;
-    if (int rc = check_ss(ctx, "rrt_render_ss", ss, w, h, band, &local_rows)) return rc;
+    if (int rc = check_ss(ctx, what, ss, w, h, band, &local_rows)) return rc;
+    bool cams_near = true;   // trace_ray's fast_ok for every camera of the table: |pos|^2 < 1e8
+    if (cams)
+        for (int k = 0; k < ss * ss; ++k) {
+            const float* f = cams[k].pos;   // pos, forward, right, up: 12 consecutive floats
+            for (int c = 0; c < 12; ++c)
+                if (!std::isfinite(f[c])) return fail(ctx, RRT_ERR_BAD_ARG, (m + ": non-finite camera field").c_str());
+            cams_near = cams_near && (double)f[0] * f[0] + (double)f[1] * f[1] + (double)f[2] * f[2] < 1.0e8;
+        }
     if (local_rows == 0) return RRT_OK;
     // output group y / g is trace group (ss*y + j) / (ss*g): the band traces exactly the sub-rows of its own rows
     rrt_band tb = {0, 1, ss};
@@ -846,21 +879,50 @@ int rrt_render_ss(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam
     cudaStream_t st = (cudaStream_t)stream;
     float* hi = nullptr;   // full-frame indexed like every plane of this ABI, so full-frame sized even for a band
     const unsigned long long n_hi = (unsigned long long)ss * ss * w * h;
-    if (n_hi > SIZE_MAX / 16) return fail(ctx, RRT_ERR_NOMEM, "rrt_render_ss: supersampled hdr plane larger than the address space");
+    const size_t cam_bytes = cams ? sizeof(rrt_camera) * ss * ss : 0;
+    if (n_hi > (SIZE_MAX - cam_bytes) / 16) return fail(ctx, RRT_ERR_NOMEM, (m + ": supersampled hdr plane larger than the address space").c_str());
     {
         std::lock_guard<std::mutex> lk(ctx->mu);
-        if (int rc = scratch_alloc(ctx, "rrt_render_ss: no memory for the supersampled hdr plane", (size_t)16 * n_hi, st, &hi))
+        if (int rc = scratch_alloc(ctx, (m + ": no memory for the supersampled hdr plane").c_str(), (size_t)16 * n_hi + cam_bytes, st, &hi))
             return rc;
+    }
+    rrt_camera* d_cams = nullptr;
+    int rc = RRT_OK;
+    if (cams) {
+        // The table goes behind the plane (16-byte aligned).  The copy reads a pageable copy of the caller's table, which the
+        // runtime stages before cudaMemcpyAsync returns: the caller may reuse its table at once, also when it is pinned.
+        d_cams = (rrt_camera*)(hi + 4 * n_hi);
+        const std::vector<rrt_camera> staged(cams, cams + ss * ss);
+        DevGuard g(ctx->device);
+        const cudaError_t e = cudaMemcpyAsync(d_cams, staged.data(), cam_bytes, cudaMemcpyHostToDevice, st);
+        if (e != cudaSuccess) rc = fail(ctx, RRT_ERR_CUDA, (m + ": copy of the camera table").c_str(), e);
     }
     rrt_planes pl;
     std::memset(&pl, 0, sizeof(pl));
     pl.hdr = hi;
-    int rc = rrt_render(ctx, prm, cam, fx, sky_texture, time, ss * w, ss * h, &tb, nullptr, RRT_OUT_FRAME, &pl, stream);
+    if (rc == RRT_OK)
+        rc = render_frame(ctx, prm, cam, fx, sky_texture, time, ss * w, ss * h, &tb, nullptr, RRT_OUT_FRAME, &pl, stream, d_cams, ss, cams_near);
     if (rc == RRT_OK) rc = rrt_resolve(ctx, prm, fx, ss, w, h, band, hi, d_out, out_layout, hdr_out, stream);
     DevGuard g(ctx->device);
     const cudaError_t e = cudaFreeAsync(hi, st);   // stream-ordered: the block goes back to the pool once the resolve has read it
-    if (rc == RRT_OK && e != cudaSuccess) return fail(ctx, RRT_ERR_CUDA, "rrt_render_ss: cudaFreeAsync", e);
+    if (rc == RRT_OK && e != cudaSuccess) return fail(ctx, RRT_ERR_CUDA, (m + ": cudaFreeAsync").c_str(), e);
     return rc;
+}
+
+int rrt_render_ss(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, const rrt_effects* fx, uint64_t sky_texture,
+                  float time, int w, int h, int ss, const rrt_band* band, void* d_out, int out_layout, float* hdr_out,
+                  void* stream) {
+    return render_ss_frame(ctx, "rrt_render_ss", prm, cam, nullptr, fx, sky_texture, time, w, h, ss, band, d_out, out_layout, hdr_out,
+                           stream);
+}
+
+int rrt_render_dof(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cams, const rrt_effects* fx, uint64_t sky_texture,
+                   float time, int w, int h, int ss, const rrt_band* band, void* d_out, int out_layout, float* hdr_out,
+                   void* stream) {
+    if (!ctx) return RRT_ERR_BAD_ARG;
+    if (!cams) return fail(ctx, RRT_ERR_BAD_ARG, "rrt_render_dof: bad argument");
+    return render_ss_frame(ctx, "rrt_render_dof", prm, cams, cams, fx, sky_texture, time, w, h, ss, band, d_out, out_layout, hdr_out,
+                           stream);
 }
 
 // What rrt_resolve_time, rrt_render_mb and rrt_capture_render_mb check: n, the frame, the band (at most 2^30 pixels, like
@@ -1050,7 +1112,7 @@ int rrt_capture_create(rrt_context* ctx, const rrt_params* prm, const rrt_camera
     S.pc = pcs;
     S.redo_out = (unsigned*)(c->d_ctrl + kCapRedo);
     S.stats = (unsigned*)(c->d_ctrl + kCapStats);
-    tp.kernel<<<(unsigned)tp.grid, kRenderBlock, 0, st>>>(A, S);
+    tp.kernel<<<(unsigned)tp.grid, kRenderBlock, 0, st>>>(A, S, rrtk::LensArgs{});
     CAP_CU(cudaGetLastError());
     ctx->launches += 1;
     CAP_CU(cudaMemcpyAsync(c->d_ctrl + kCapTicket + sizeof(unsigned), c->d_ctrl + kCapTicket, sizeof(unsigned), cudaMemcpyDeviceToDevice, st));
@@ -1163,7 +1225,7 @@ static int capture_enqueue(rrt_capture* cap, float exposure, const rrt_effects* 
         S.pc_prev = pcs;
         long long grid_sweep = ((long long)ctx->sm_count * per_sm_sweep + ctx->frames_in_flight - 1) / ctx->frames_in_flight;
         if (grid_sweep > (long long)cap->ntiles) grid_sweep = cap->ntiles;
-        k_sweep<<<(unsigned)grid_sweep, kRenderBlock, 0, st>>>(A, S);
+        k_sweep<<<(unsigned)grid_sweep, kRenderBlock, 0, st>>>(A, S, rrtk::LensArgs{});
         ++launches;
     }
     RRT_CU(ctx, cudaGetLastError());

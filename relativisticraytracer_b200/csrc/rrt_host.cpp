@@ -143,6 +143,41 @@ int rrt_shutter_times(float t, float shutter, float fps, int n, float* out) {
     return RRT_OK;
 }
 
+int rrt_lens_cameras(const rrt_camera* cam, float aperture, float focus, int ss, rrt_camera* out) {
+    if (!cam || !out || !(aperture >= 0.0f) || !std::isfinite(aperture) || !(focus > 0.0f) || !std::isfinite(focus) || ss < 1 || ss > 8)
+        return RRT_ERR_BAD_ARG;
+    for (int j = 0; j < ss; ++j)
+        for (int i = 0; i < ss; ++i) {
+            rrt_camera& c = out[j * ss + i];
+            c = *cam;
+            // cell centre (a, b) = (na, nb) / ss in [-1, 1]^2; its image on the unit disk under Shirley & Chiu's concentric
+            // map, in double and rounded to float once: the larger coordinate is the radius, the ratio of the two the angle
+            const int na = 2 * i + 1 - ss, nb = 2 * j + 1 - ss;
+            if (aperture == 0.0f || (na == 0 && nb == 0)) continue;   // the pinhole itself: an exact copy (keeps -0 fields)
+            const double kPi4 = 0.78539816339744830962, a = (double)na / ss, b = (double)nb / ss;
+            double x, y;
+            if (std::abs(na) > std::abs(nb)) {
+                const double t = kPi4 * ((double)nb / na);
+                x = a * std::cos(t);
+                y = a * std::sin(t);
+            } else {   // phi = pi/2 - pi/4 * (a / b): cos(phi) = sin(pi/4 * a / b), sin(phi) = cos(pi/4 * a / b)
+                const double t = kPi4 * ((double)na / nb);
+                x = b * std::sin(t);
+                y = b * std::cos(t);
+            }
+            const float ox = (float)((double)aperture * x), oy = (float)((double)aperture * y);
+            // one binary32 operation each, in this order (no contraction): o = right * ox + up * oy, pos + o, forward - o / focus
+            for (int k = 0; k < 3; ++k) {
+                const float rx = cam->right[k] * ox, uy = cam->up[k] * oy;
+                const float o = rx + uy;
+                c.pos[k] = cam->pos[k] + o;
+                const float tilt = o / focus;
+                c.forward[k] = cam->forward[k] - tilt;
+            }
+        }
+    return RRT_OK;
+}
+
 // ---- frame sink: the step immediately after the hot path --------------------------------------------------
 // The reference's ScreenRecorder (src/main.cpp:29-124) reads the window back with glReadPixels -- which, for the
 // 1:1 textured quad it draws (src/main.cpp:404-409, 471-479), returns exactly the bytes launch_raymarch wrote,

@@ -32,10 +32,21 @@ struct FrameArgs {
     unsigned int tile_log_cap;     // entries the log can hold
 };
 
+// The camera table of rrt_render_dof, the last parameter of every kernel that creates rays; read by their LENS variants
+// only (zero for every other launch).  A separate parameter rather than more FrameArgs fields: appended at the end of the
+// parameter block it moves no parameter of the existing kernels.  Pixel (x, y) of the traced frame starts its ray from
+// cams[(y % ss) * ss + x % ss] instead of FrameArgs::cam.  near: every camera of the table lies in the branch-free domain
+// (trace_ray's fast_ok), decided once on the host so that the gate stays a launch constant as it is with one camera.
+struct LensArgs {
+    const rrt_camera* cams;
+    int ss;
+    int near;
+};
+
 // kernels of one rounding contract
 struct KernelSet {
-    void (*render[2][2])(const FrameArgs);  // [spin != 0][media]
-    void (*render_packed[2])(const FrameArgs);  // [spin != 0]; two rays per thread in f32x2 registers, no medium (rrt_packed.cuh); FMAD contract only
+    void (*render[2][2])(const FrameArgs, const LensArgs);  // [spin != 0][media]
+    void (*render_packed[2])(const FrameArgs, const LensArgs);  // [spin != 0]; two rays per thread in f32x2 registers, no medium (rrt_packed.cuh); FMAD contract only
     void (*acc)(Consts, int, const float*, const float*, float*);
     void (*rk4)(Consts, int, float*, float*, const float*);
     void (*euler)(Consts, int, float*, float*, const float*);
@@ -49,6 +60,9 @@ struct KernelSet {
     void (*shade)(const FrameArgs, const rrt_planes);  // rrt_shade: the step after the ray loop, from traced planes
     // rrt_resolve / rrt_resolve_time: mean of ss x ss blocks of n hdr planes + post step
     void (*resolve)(const FrameArgs, const float4*, int, int, size_t);
+    // the LENS variants of render / render_packed (rrt_render_dof): every ray from its own camera of LensArgs::cams
+    void (*render_lens[2][2])(const FrameArgs, const LensArgs);
+    void (*render_packed_lens[2])(const FrameArgs, const LensArgs);
 };
 const KernelSet* rrt_kernels_strict();
 const KernelSet* rrt_kernels_fmad();
@@ -58,6 +72,7 @@ using rrt::Consts;
 using rrt::V3;
 using rrt::mk;
 using rrtk::FrameArgs;
+using rrtk::LensArgs;
 
 namespace {
 
@@ -74,6 +89,9 @@ constexpr int kBurst = 8;
 // that better than the four the unconstrained 109-register build gets (4K C0 78.5 -> 76.2 ms, C3 147.6 -> 135.4;
 // 7 and 8 CTAs are no better).  The geodesic-only variant needs ~72 registers anyway.
 constexpr int kMinBlocks = 1, kMinBlocksMedia = 24;
+// The LENS variants (rrt_render_dof) of the media kernels -- render_kernel<SPIN, true, true> and sweep_kernel<SPIN, true>, the
+// fused fallbacks of a depth-of-field frame -- are asked for 18 warps per SM (<= 112 registers), where none of them spills.
+constexpr int kMinBlocksMediaLens = 18;
 
 struct RayResult {
     float hdr[3], T, I[3];
@@ -155,22 +173,31 @@ __device__ __forceinline__ void pixel_uv(const FrameArgs& A, int x, int y, float
     }
 }
 
+// The camera a pixel's ray starts from: the frame's, or with LENS (rrt_render_dof) its entry of the camera table.
+template <bool LENS>
+__device__ __forceinline__ const rrt_camera& ray_camera(const FrameArgs& A, const LensArgs& L, int x, int y) {
+    if (!LENS) return A.cam;
+    return L.cams[(y % L.ss) * L.ss + x % L.ss];
+}
+
+__device__ __forceinline__ V3 cam_pos(const rrt_camera& c) { return mk(c.pos[0], c.pos[1], c.pos[2]); }
+
 // initial ray of a pixel given its (distorted) image-plane coordinate (reference :27-34)
-__device__ __forceinline__ V3 ray_dir_uv(const FrameArgs& A, float uvx, float uvy) {
+__device__ __forceinline__ V3 ray_dir_uv(const FrameArgs& A, const rrt_camera& cam, float uvx, float uvy) {
     using namespace rrt;
     float uc = mad(uvx, 2.0f, -1.0f);  // :27
     const float vc = mad(uvy, 2.0f, -1.0f);  // :28
     const float aspect = (float)A.w / (float)A.h;
     uc = mul(uc, aspect);  // :30
     // forward + (right*u + up*v)
-    return unit3(mk(add(mad(A.cam.right[0], uc, mul(A.cam.up[0], vc)), A.cam.forward[0]),
-                    add(mad(A.cam.right[1], uc, mul(A.cam.up[1], vc)), A.cam.forward[1]),
-                    add(mad(A.cam.right[2], uc, mul(A.cam.up[2], vc)), A.cam.forward[2])));  // :33-34
+    return unit3(mk(add(mad(cam.right[0], uc, mul(cam.up[0], vc)), cam.forward[0]),
+                    add(mad(cam.right[1], uc, mul(cam.up[1], vc)), cam.forward[1]),
+                    add(mad(cam.right[2], uc, mul(cam.up[2], vc)), cam.forward[2])));  // :33-34
 }
-__device__ __forceinline__ V3 ray_dir(const FrameArgs& A, int x, int y) {
+__device__ __forceinline__ V3 ray_dir(const FrameArgs& A, const rrt_camera& cam, int x, int y) {
     float uvx, uvy;
     pixel_uv(A, x, y, uvx, uvy);
-    return ray_dir_uv(A, uvx, uvy);
+    return ray_dir_uv(A, cam, uvx, uvy);
 }
 
 constexpr unsigned kEndCaptured = 1u, kEndTouched = 2u, kEndExhausted = 4u;
@@ -264,14 +291,15 @@ struct NoEmit {
     __device__ __forceinline__ void emit(V3, V3, float, int, unsigned) {}
 };
 
-// One ray: reference raymarch_kernel lines 20-150.
-template <bool SPIN, int MEDIA, class EM>
-__device__ __forceinline__ void trace_ray(const FrameArgs& A, int x, int y, RayResult& R, EM& em) {
+// One ray: reference raymarch_kernel lines 20-150.  LENS: from the pixel's own camera (ray_camera).
+template <bool SPIN, int MEDIA, bool LENS, class EM>
+__device__ __forceinline__ void trace_ray(const FrameArgs& A, const LensArgs& L, int x, int y, RayResult& R, EM& em) {
     const Consts& C = A.C;
+    const rrt_camera& cam = ray_camera<LENS>(A, L, x, y);
     float uvx, uvy;
     pixel_uv(A, x, y, uvx, uvy);                                       // :20-25
-    V3 p = mk(A.cam.pos[0], A.cam.pos[1], A.cam.pos[2]);
-    V3 v = ray_dir_uv(A, uvx, uvy);                                    // :27-34
+    V3 p = mk(cam.pos[0], cam.pos[1], cam.pos[2]);
+    V3 v = ray_dir_uv(A, cam, uvx, uvy);                               // :27-34
 
     float Ir = 0.f, Ig = 0.f, Ib = 0.f, T = 1.0f;
     bool captured = false, touched = false, escaped = false;
@@ -280,8 +308,10 @@ __device__ __forceinline__ void trace_ray(const FrameArgs& A, int x, int y, RayR
     const int max_steps = C.max_steps;
     const bool want_disk = (C.flags & RRT_FLAG_DISK) != 0, want_dust = (C.flags & RRT_FLAG_DUST) != 0;
     // Domain of the branch-free div/sqrt (rrt_device.cuh): a ray that starts absurdly far out takes the
-    // general path for its whole life.  Uniform per launch in practice (depends on the camera only).
-    const bool fast_ok = rrt::dot3(p, p) < 1.0e8f && C.acc_rmin < C.horizon_r && C.horizon_r >= 1e-3f;
+    // general path for its whole life.  Uniform per launch in practice (depends on the camera only); with LENS decided
+    // for the whole camera table (LensArgs::near), which keeps it a launch constant.  Both paths give the same bits where
+    // the fast one is valid, so the gate decides only the speed.
+    const bool fast_ok = (LENS ? L.near != 0 : rrt::dot3(p, p) < 1.0e8f) && C.acc_rmin < C.horizon_r && C.horizon_r >= 1e-3f;
     const float zone_rmax = fmaxf(18.0f, fmaxf(C.disk_zone_r, C.dust_zone_r));
     // one compare per step for "redo with the general code": smallest stage radius below acc_rmin (or NaN), or
     // the whole ray outside the fast domain (+inf: every step is redone)
@@ -452,8 +482,9 @@ __device__ __forceinline__ void trace_ray(const FrameArgs& A, int x, int y, RayR
     R.uvx = uvx; R.uvy = uvy;
 }
 
-template <bool SPIN, bool MEDIA>
-__global__ void __launch_bounds__(kRenderBlock, MEDIA ? kMinBlocksMedia : kMinBlocks) render_kernel(const __grid_constant__ FrameArgs A) {
+template <bool SPIN, bool MEDIA, bool LENS>
+__global__ void __launch_bounds__(kRenderBlock, MEDIA ? (LENS ? kMinBlocksMediaLens : kMinBlocksMedia) : kMinBlocks)
+    render_kernel(const __grid_constant__ FrameArgs A, const __grid_constant__ LensArgs L) {
     const int lane = threadIdx.x & 31;
     const int ntx = (A.w + kRTileW - 1) / kRTileW;
     const int nty = (A.local_rows + kRTileH - 1) / kRTileH;
@@ -486,7 +517,7 @@ __global__ void __launch_bounds__(kRenderBlock, MEDIA ? kMinBlocksMedia : kMinBl
 #endif
         RayResult R;
         NoEmit no_emit;
-        trace_ray<SPIN, MEDIA ? kMediaInline : kMediaNone>(A, x, y, R, no_emit);
+        trace_ray<SPIN, MEDIA ? kMediaInline : kMediaNone, LENS>(A, L, x, y, R, no_emit);
 
         finish_ray_inl(A, x, y, ly, R.uvx, R.uvy, R.I[0], R.I[1], R.I[2], R.T, R.p, R.v, R.steps,
                        (R.captured ? kEndCaptured : 0u) | (R.touched ? kEndTouched : 0u) | (R.exhausted ? kEndExhausted : 0u));
@@ -667,14 +698,20 @@ __global__ void k_sky(cudaTextureObject_t sky, int n, const float* tx, const flo
 #include "rrt_split.cuh"   // trace / media / fold kernels of the split pipeline (both contracts)
 namespace {
 const rrtk::KernelSet kKernelSet = {
-    {{render_kernel<false, false>, render_kernel<false, true>}, {render_kernel<true, false>, render_kernel<true, true>}},
+    {{render_kernel<false, false, false>, render_kernel<false, true, false>}, {render_kernel<true, false, false>, render_kernel<true, true, false>}},
 #if RRT_FMAD
-    {render_kernel_p<false>, render_kernel_p<true>},
+    {render_kernel_p<false, false>, render_kernel_p<true, false>},
 #else
     {nullptr, nullptr},
 #endif
     k_acc, k_rk4, k_euler, k_redshift, k_hash31, k_noise3d, k_fbm, k_disk_temp, k_disk_density, k_dust_density,
     shade_kernel, resolve_kernel,
+    {{render_kernel<false, false, true>, render_kernel<false, true, true>}, {render_kernel<true, false, true>, render_kernel<true, true, true>}},
+#if RRT_FMAD
+    {render_kernel_p<false, true>, render_kernel_p<true, true>},
+#else
+    {nullptr, nullptr},
+#endif
 };
 }  // namespace
 

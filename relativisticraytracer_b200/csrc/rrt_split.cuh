@@ -88,13 +88,18 @@ struct SplitArgs {
     uint4* results;           // media_kernel<true> / fold_kernel<true>: {e.rgb, s} per slot, indexed like `slots` (rrt_capture)
 };
 struct SplitKernels {
-    void (*trace[2])(const FrameArgs, const SplitArgs);   // [spin != 0]
-    void (*trace_packed[2])(const FrameArgs, const SplitArgs);   // two rays per thread (FMAD contract only, else null)
+    void (*trace[2])(const FrameArgs, const SplitArgs, const LensArgs);   // [spin != 0]
+    void (*trace_packed[2])(const FrameArgs, const SplitArgs, const LensArgs);   // two rays per thread (FMAD contract only, else null)
     void (*media)(const FrameArgs, const SplitArgs);
     void (*fold)(const FrameArgs, const SplitArgs);
-    void (*sweep[2])(const FrameArgs, const SplitArgs);
+    void (*sweep[2])(const FrameArgs, const SplitArgs, const LensArgs);
     void (*media_results)(const FrameArgs, const SplitArgs);   // media_kernel<true>: the samples stay, results go to S.results
     void (*fold_results)(const FrameArgs, const SplitArgs);    // fold_kernel<true>: reads them from there
+    // the LENS variants of the tracers (rrt_render_dof): every ray from its own camera of LensArgs::cams; media and fold
+    // read only samples and planes and serve both
+    void (*trace_lens[2])(const FrameArgs, const SplitArgs, const LensArgs);
+    void (*trace_packed_lens[2])(const FrameArgs, const SplitArgs, const LensArgs);
+    void (*sweep_lens[2])(const FrameArgs, const SplitArgs, const LensArgs);
 };
 const SplitKernels* rrt_split_kernels_strict();
 const SplitKernels* rrt_split_kernels_fmad();
@@ -326,9 +331,10 @@ __device__ __forceinline__ void redo_later(const SplitArgs& S, unsigned tile, in
 }
 
 // ---- pass kernel 1: trajectories ------------------------------------------------------------------------------------
-template <bool SPIN>
+template <bool SPIN, bool LENS>
 __global__ void __launch_bounds__(kRenderBlock, kMinBlocks) trace_kernel(const __grid_constant__ FrameArgs A,
-                                                                              const __grid_constant__ SplitArgs S) {
+                                                                              const __grid_constant__ SplitArgs S,
+                                                                              const __grid_constant__ LensArgs L) {
     __shared__ unsigned chunk_tab[kRenderBlock / 32][kDescChunks];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     unsigned* tab = chunk_tab[warp];
@@ -363,7 +369,7 @@ __global__ void __launch_bounds__(kRenderBlock, kMinBlocks) trace_kernel(const _
         unsigned long long t_begin = 0;
         if (A.tile_log) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_begin));
 #endif
-        if (px.valid) trace_ray<SPIN, kMediaEmit>(A, px.x, px.y, R, em);
+        if (px.valid) trace_ray<SPIN, kMediaEmit, LENS>(A, L, px.x, px.y, R, em);
         __syncwarp();
 #ifdef RRT_WITH_TILE_LOG   // profiling build only (rrt_debug_tile_log): when did this warp trace which tile
         if (A.tile_log) {
@@ -436,8 +442,9 @@ struct Emitter2 {
     }
 };
 
-template <bool SPIN>
-__global__ void __launch_bounds__(32, kPackedMinBlocks) trace_kernel_p(const __grid_constant__ FrameArgs A, const __grid_constant__ SplitArgs S) {
+template <bool SPIN, bool LENS>
+__global__ void __launch_bounds__(32, kPackedMinBlocks) trace_kernel_p(const __grid_constant__ FrameArgs A, const __grid_constant__ SplitArgs S,
+                                                                          const __grid_constant__ LensArgs L) {
     using rrtp::F2;
     using rrtp::V3x2;
     __shared__ unsigned chunk_tab[kDescChunks];
@@ -451,7 +458,7 @@ __global__ void __launch_bounds__(32, kPackedMinBlocks) trace_kernel_p(const __g
     const bool want_disk = (C.flags & RRT_FLAG_DISK) != 0, want_dust = (C.flags & RRT_FLAG_DUST) != 0;
     const float zone_rmax = fmaxf(18.0f, fmaxf(C.disk_zone_r, C.dust_zone_r));
     const V3 cam_p = mk(A.cam.pos[0], A.cam.pos[1], A.cam.pos[2]);
-    const bool fast_ok = rrt::dot3(cam_p, cam_p) < 1.0e8f && C.acc_rmin < C.horizon_r && C.horizon_r >= 1e-3f;
+    const bool fast_ok = (LENS ? L.near != 0 : rrt::dot3(cam_p, cam_p) < 1.0e8f) && C.acc_rmin < C.horizon_r && C.horizon_r >= 1e-3f;
     const float redo_below = fast_ok ? C.acc_rmin : __int_as_float(0x7f800000);
     const V3 park_p = mk(0.0f, 100.0f, 0.0f), park_v = mk(0.0f, 0.0f, 0.0f);   // inert state of a finished half, see render_kernel_p
     const float burst_min = fmaxf(zone_rmax, fmaxf(C.horizon_r, redo_below));
@@ -500,8 +507,10 @@ __global__ void __launch_bounds__(32, kPackedMinBlocks) trace_kernel_p(const __g
         if (alive[0] || alive[1]) {
             V3x2 P, V;
             {
-                const V3 vA = alive[0] ? ray_dir(A, x0, y) : park_v, vB = alive[1] ? ray_dir(A, x0 + 1, y) : park_v;
-                const V3 pA = alive[0] ? cam_p : park_p, pB = alive[1] ? cam_p : park_p;
+                // the two halves are neighbouring pixels: with LENS each starts from its own camera
+                const rrt_camera &camA = ray_camera<LENS>(A, L, x0, y), &camB = ray_camera<LENS>(A, L, x0 + 1, y);
+                const V3 vA = alive[0] ? ray_dir(A, camA, x0, y) : park_v, vB = alive[1] ? ray_dir(A, camB, x0 + 1, y) : park_v;
+                const V3 pA = alive[0] ? (LENS ? cam_pos(camA) : cam_p) : park_p, pB = alive[1] ? (LENS ? cam_pos(camB) : cam_p) : park_p;
                 P.x = rrtp::pk(pA.x, pB.x); P.y = rrtp::pk(pA.y, pB.y); P.z = rrtp::pk(pA.z, pB.z);
                 V.x = rrtp::pk(vA.x, vB.x); V.y = rrtp::pk(vA.y, vB.y); V.z = rrtp::pk(vA.z, vB.z);
             }
@@ -930,9 +939,9 @@ __global__ void __launch_bounds__(128) fold_kernel(const __grid_constant__ Frame
 }
 
 // ---- after the last pass: whatever the split passes left, with the fused code ------------------------------------------
-template <bool SPIN>
-__global__ void __launch_bounds__(kRenderBlock, kMinBlocksMedia) sweep_kernel(const __grid_constant__ FrameArgs A,
-                                                                                    const __grid_constant__ SplitArgs S) {
+template <bool SPIN, bool LENS>
+__global__ void __launch_bounds__(kRenderBlock, LENS ? kMinBlocksMediaLens : kMinBlocksMedia)
+    sweep_kernel(const __grid_constant__ FrameArgs A, const __grid_constant__ SplitArgs S, const __grid_constant__ LensArgs L) {
     const int lane = threadIdx.x & 31;
     const unsigned ntiles = num_tiles(A);
     TileCounters cnt;
@@ -953,7 +962,7 @@ __global__ void __launch_bounds__(kRenderBlock, kMinBlocksMedia) sweep_kernel(co
             if (!px.valid) continue;
             RayResult R;
             NoEmit no_emit;
-            trace_ray<SPIN, kMediaInline>(A, px.x, px.y, R, no_emit);
+            trace_ray<SPIN, kMediaInline, LENS>(A, L, px.x, px.y, R, no_emit);
             finish_ray_inl(A, px.x, px.y, px.ly, R.uvx, R.uvy, R.I[0], R.I[1], R.I[2], R.T, R.p, R.v, R.steps,
                            (R.captured ? kEndCaptured : 0u) | (R.touched ? kEndTouched : 0u) | (R.exhausted ? kEndExhausted : 0u));
             cnt.steps += (unsigned)R.steps;
@@ -967,14 +976,21 @@ __global__ void __launch_bounds__(kRenderBlock, kMinBlocksMedia) sweep_kernel(co
 }
 
 const rrtk::SplitKernels kSplitKernels = {
-    {trace_kernel<false>, trace_kernel<true>},
+    {trace_kernel<false, false>, trace_kernel<true, false>},
 #if RRT_FMAD
-    {trace_kernel_p<false>, trace_kernel_p<true>},
+    {trace_kernel_p<false, false>, trace_kernel_p<true, false>},
 #else
     {nullptr, nullptr},
 #endif
-    media_kernel<false>, fold_kernel<false>, {sweep_kernel<false>, sweep_kernel<true>},
+    media_kernel<false>, fold_kernel<false>, {sweep_kernel<false, false>, sweep_kernel<true, false>},
     media_kernel<true>, fold_kernel<true>,
+    {trace_kernel<false, true>, trace_kernel<true, true>},
+#if RRT_FMAD
+    {trace_kernel_p<false, true>, trace_kernel_p<true, true>},
+#else
+    {nullptr, nullptr},
+#endif
+    {sweep_kernel<false, true>, sweep_kernel<true, true>},
 };
 }  // namespace
 

@@ -307,9 +307,13 @@ class PathSequence:
     shutter open for ``shutter`` (0..1) of the frame interval, centred on the frame's clock, with ``samples`` sub-frames at
     ``shutter_times(path_clock(k, fps), shutter, fps, samples)``, each with the path's camera at its own time, so that the
     disk's rotation and the camera's motion smear instead of strobing.  ``samples`` > 1 does not combine with ``ss`` > 1
-    here; the C ABI composes the two (rrt_resolve_time, then rrt_resolve)."""
+    here; the C ABI composes the two (rrt_resolve_time, then rrt_resolve).  ``aperture`` > 0 gives every frame depth of
+    field (``Renderer.render_dof`` with ``lens_cameras(path camera, aperture, focus, ss)``): a thin lens of that radius
+    focused at distance ``focus`` along the path camera's forward, its ss x ss lens points shared out among each pixel's
+    sub-samples; ``aperture`` = 0 keeps the pinhole.  Depth of field does not combine with motion blur here."""
 
-    def __init__(self, renderer, w: int, h: int, depth: int = 2, ss: int = 1, shutter: float = 0.0, samples: int = 1):
+    def __init__(self, renderer, w: int, h: int, depth: int = 2, ss: int = 1, shutter: float = 0.0, samples: int = 1,
+                 aperture: float = 0.0, focus: Optional[float] = None):
         if not 1 <= depth <= HOST_SLOTS:
             raise ValueError(f"depth must be 1..{HOST_SLOTS}")
         if not 1 <= ss <= 8:
@@ -320,6 +324,13 @@ class PathSequence:
             raise ValueError("shutter must be in [0, 1]")
         if ss > 1 and samples > 1:
             raise ValueError("ss > 1 together with samples > 1 is not supported by PathSequence")
+        if not (0.0 <= aperture < float("inf")):
+            raise ValueError("aperture must be finite and >= 0")
+        if aperture > 0.0 and not (focus is not None and 0.0 < focus < float("inf")):
+            raise ValueError("aperture > 0 needs a focus distance, finite and > 0")
+        if aperture > 0.0 and samples > 1:
+            raise ValueError("aperture > 0 (depth of field) together with samples > 1 (motion blur) is not supported by PathSequence")
+        self.aperture, self.focus = float(aperture), focus
         self.r, self.w, self.h, self.depth, self.ss = renderer, w, h, depth, ss
         self.shutter, self.samples = float(shutter), samples
         self.world = dist.get_world_size() if dist.is_initialized() else 1
@@ -329,14 +340,14 @@ class PathSequence:
         self.events = [torch.cuda.Event() for _ in range(depth)]
         root = self.rank == 0
         self.local = ([torch.zeros((h, w, 4), dtype=torch.uint8, device=dev) for _ in range(depth)]
-                      if self.world > 1 or ss > 1 or samples > 1 else None)
+                      if self.world > 1 or ss > 1 or samples > 1 or self.aperture > 0.0 else None)
         self.gathered = ([torch.zeros((self.world, h, w, 4), dtype=torch.uint8, device=dev) for _ in range(depth)]
                          if root and self.world > 1 else None)
         self.host = [torch.zeros((self.world, h, w, 4), dtype=torch.uint8).pin_memory() for _ in range(depth)] if root else None
 
     def render(self, path_index: int, n_frames: int, prm, fx, sky, fps: float = 24.0, sink=None, first_frame: int = 1):
         """Render frames first_frame .. first_frame+n_frames-1 of the path.  Returns (frames_done, launches)."""
-        from .renderer import path_clock, path_state, shutter_times
+        from .renderer import lens_cameras, path_clock, path_state, shutter_times
         cur = torch.cuda.current_stream(self.r.device)
         for s in self.streams:
             s.wait_stream(cur)
@@ -365,7 +376,7 @@ class PathSequence:
             mine = frames[self.rank]
             s = self.streams[k]
             with torch.cuda.stream(s):
-                if self.world == 1 and self.ss == 1 and self.samples == 1:
+                if self.world == 1 and self.ss == 1 and self.samples == 1 and self.aperture == 0.0:
                     t = path_clock(mine, fps)
                     cam, _ = path_state(path_index, t)
                     self.r.render_host_async(prm, cam, fx, sky, t, self.w, self.h, self.host[k][0], slot=k, stream=s)
@@ -377,6 +388,9 @@ class PathSequence:
                             times = shutter_times(t, self.shutter, fps, self.samples)
                             cams = [path_state(path_index, ti)[0] for ti in times]
                             self.r.render_mb(prm, cams, fx, sky, times, self.w, self.h, out=self.local[k], stream=s)
+                        elif self.aperture > 0.0:
+                            lens = lens_cameras(cam, self.aperture, self.focus, self.ss)
+                            self.r.render_dof(prm, lens, fx, sky, t, self.w, self.h, self.ss, out=self.local[k], stream=s)
                         elif self.ss == 1:
                             self.r.render(prm, cam, fx, sky, t, self.w, self.h, out=self.local[k], stream=s)
                         else:

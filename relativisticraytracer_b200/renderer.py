@@ -64,6 +64,21 @@ def shutter_times(t: float, shutter: float, fps: float, n: int) -> list:
     return [float(v) for v in out]
 
 
+def lens_cameras(cam: Camera, aperture: float, focus: float, ss: int) -> list:
+    """rrt_lens_cameras: the ss*ss cameras of a thin lens of radius ``aperture`` at ``cam``'s position, focused on the plane
+    at distance ``focus`` along ``cam.forward`` -- the table ``Renderer.render_dof`` takes.  Camera j*ss + i looks through
+    the centre of stratified lens cell (i, j) (Shirley & Chiu's concentric map), shifted in the right / up plane and tilted
+    so that its ray through every image-plane point meets the other cameras' on the focal plane.  ``aperture = 0`` and
+    ``ss = 1`` give copies of ``cam``.  Host only."""
+    ss = int(ss)
+    out = (Camera * max(ss * ss, 1))()
+    rc = _capi.load().rrt_lens_cameras(C.byref(cam), float(aperture), float(focus), ss, out)
+    if rc != 0:
+        raise RrtError(rc, f"rrt_lens_cameras(aperture={aperture}, focus={focus}, ss={ss}): aperture must be finite and >= 0, "
+                           "focus finite and > 0, ss in 1..8")
+    return list(out)
+
+
 def _f32_array(values) -> C.Array:
     values = [float(v) for v in values]
     return (C.c_float * len(values))(*values)
@@ -290,6 +305,26 @@ class Renderer:
         self._check(self._lib.rrt_render_ss(self._ctx, C.byref(prm), C.byref(cam), C.byref(fx), C.c_uint64(tex), float(time),
                                             int(w), int(h), int(ss), C.byref(band) if band is not None else None,
                                             C.c_void_p(out_ptr), int(layout), C.c_void_p(hdr_ptr), C.c_void_p(st.cuda_stream)))
+        return out
+
+    def render_dof(self, prm: Params, cams, fx: Effects, sky: Sky | int, time: float, w: int, h: int, ss: int, *,
+                   band: Optional[Band] = None, out=None, layout: int = OUT_FRAME, hdr_out: Optional[torch.Tensor] = None,
+                   stream: Optional[torch.cuda.Stream] = None) -> torch.Tensor:
+        """rrt_render_dof: ``render_ss`` with its own camera per sub-sample -- depth of field at the cost of ``render_ss``;
+        asynchronous.  ``cams`` is a sequence of ss*ss cameras (``lens_cameras`` gives a thin lens): sub-sample (i, j) of
+        pixel (x, y) is pixel (ss*x + i, ss*y + j) of the ss*w x ss*h ``render`` with ``cams[j*ss + i]``.  All cameras equal
+        is ``render_ss``; ss = 1 is ``render(cams[0])``.  ``hdr_out``, ``band``, ``out`` and ``layout`` as in ``render_ss``."""
+        tex = sky.texture if isinstance(sky, Sky) else int(sky)
+        cams = list(cams)
+        if len(cams) != int(ss) * int(ss):
+            raise ValueError(f"render_dof: {len(cams)} cameras for ss = {ss} (ss*ss needed)")
+        cam_arr = (Camera * max(len(cams), 1))(*cams)
+        out, out_ptr = self._frame_out(out, layout, band, w, h)
+        hdr_ptr = self._plane_ptr("hdr", hdr_out, w, h) if hdr_out is not None else None
+        st = stream if stream is not None else torch.cuda.current_stream(self.device)
+        self._check(self._lib.rrt_render_dof(self._ctx, C.byref(prm), cam_arr, C.byref(fx), C.c_uint64(tex), float(time),
+                                             int(w), int(h), int(ss), C.byref(band) if band is not None else None,
+                                             C.c_void_p(out_ptr), int(layout), C.c_void_p(hdr_ptr), C.c_void_p(st.cuda_stream)))
         return out
 
     def resolve(self, prm: Params, fx: Effects, hdr_hi: torch.Tensor, ss: int, w: int, h: int, *, band: Optional[Band] = None,
