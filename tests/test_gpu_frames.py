@@ -7,17 +7,26 @@ from parity import CAMERAS, DIR_TOL_RAD, RGB_TOL_REL, census
 pytestmark = pytest.mark.gpu
 
 
-def render_pair(gpu, ora, sky_np, cam_key, spin, flags, w, h, time=1.0, fx="off", **over):
+def render_pair(gpu, ora, sky_np, cam_key, spin, flags, w, h, time=1.0, fx="off", cam=None, **over):
+    """The frame with all its planes and counters from the GPU and from the oracle port.  cam_key names a survey camera;
+    `cam` (a Camera, e.g. of a path or a lens table) replaces it.  fx is "off", "default" or an Effects."""
     import relativisticraytracer_b200 as rrt
     import torch
-    pos, yaw, pitch = CAMERAS[cam_key]
+    from oracle import Camera as OraCamera, Effects as OraEffects
     pg = rrt.default_params(spin_a=spin, flags=flags, **over)
     po = ora.default_params(spin_a=spin, flags=flags, **over)
-    cg = rrt.camera_state_from(pos, yaw, pitch)
-    co = ora.camera_from(pos, yaw, pitch)
+    if cam is None:
+        pos, yaw, pitch = CAMERAS[cam_key]
+        cg = rrt.camera_state_from(pos, yaw, pitch)
+        co = ora.camera_from(pos, yaw, pitch)
+    else:
+        cg, co = cam, OraCamera.from_buffer_copy(bytes(cam))
     assert bytes(cg) == bytes(co)
-    fg = rrt.effects_off() if fx == "off" else rrt.default_effects()
-    fo = ora.effects_off() if fx == "off" else ora.default_effects()
+    if isinstance(fx, str):
+        fg = rrt.effects_off() if fx == "off" else rrt.default_effects()
+        fo = ora.effects_off() if fx == "off" else ora.default_effects()
+    else:
+        fg, fo = fx, OraEffects.from_buffer_copy(bytes(fx))
     sky = gpu.create_sky(sky_np)
     planes = gpu.alloc_planes(w, h)
     gpu.read_counters(reset=True)
