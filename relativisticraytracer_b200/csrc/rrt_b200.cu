@@ -32,6 +32,7 @@
 #include <mutex>
 #include <new>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "../../include/rrt.h"
@@ -136,10 +137,8 @@ struct rrt_context {
     // fused FMAD launches without a medium use the packed f32x2 kernel (two rays per thread; measured,
     // profiles/r2_history.md) unless RRT_KERNEL=scalar pins the scalar one.  RRT_KERNEL=auto|scalar.
     bool scalar_kernel = false;
-    // launch configuration of every render kernel seen so far (resident CTAs per SM, carve-out applied): queried once
-    struct LaunchCfg { const void* kern; int per_sm; };
-    LaunchCfg launch_cfg[16] = {};
-    int n_launch_cfg = 0;
+    // resident CTAs per SM of every kernel launched so far (carve-out applied): asked for once (resident_per_sm)
+    std::vector<std::pair<const void*, int>> resident;
     void* d_frame[RRT_HOST_SLOTS] = {};  // device frames behind the host-destination calls, one per slot
     size_t d_frame_bytes[RRT_HOST_SLOTS] = {};
     unsigned long long* tile_log = nullptr;   // rrt_debug_tile_log: caller-owned device buffer, or null
@@ -191,7 +190,7 @@ constexpr size_t kCtrlBytes = kCtrlHead + sizeof(unsigned) * kRedoCap * (kMaxPas
 constexpr unsigned kTicketRing = 1024;
 thread_local std::string g_create_err;
 
-int fail(rrt_context* ctx, int code, const char* what, cudaError_t e = cudaSuccess) {
+int fail(rrt_context* ctx, int code, const std::string& what, cudaError_t e = cudaSuccess) {
     std::string m = what;
     if (e != cudaSuccess) { m += ": "; m += cudaGetErrorString(e); }
     if (ctx) ctx->err = m; else g_create_err = m;
@@ -433,19 +432,36 @@ int rrt_band_rows(const rrt_band* band, int h) {
     return rows;
 }
 
+}  // extern "C"
 
-// ---- split pipeline: host side (csrc/rrt_split.cuh) ---------------------------------------------------------------
-// Resident CTAs per SM of a kernel, asked for once per context (see rrt_render).
+// ---- launch geometry -----------------------------------------------------------------------------------------------
+// Resident CTAs per SM of a kernel: a property of (kernel, device), asked for once per context, not per frame.
+// max_shared: the carve-out stays at the shared-memory end although the persistent kernels declare no shared memory:
+// every resident CTA still reserves 1 KB of it, and with one-warp CTAs (24-32 per SM) a small carve-out caps residency
+// -- measured with cudaSharedmemCarveoutMaxL1: 4K C0 73.3 -> 80.7 ms, C3 133 -> 164 ms.  Negative: the error code.
+// ctx->mu held, ctx->device current.
 static int resident_per_sm(rrt_context* ctx, const void* kern, int block, bool max_shared) {
-    for (int i = 0; i < ctx->n_launch_cfg; ++i)
-        if (ctx->launch_cfg[i].kern == kern) return ctx->launch_cfg[i].per_sm;
+    for (const auto& k : ctx->resident)
+        if (k.first == kern) return k.second;
+    if (max_shared) RRT_CU(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     int per_sm = 0;
-    if (max_shared) cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, block, 0) != cudaSuccess || per_sm < 1) per_sm = 1;
-    if (ctx->n_launch_cfg < 16) ctx->launch_cfg[ctx->n_launch_cfg++] = {kern, per_sm};
+    RRT_CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, block, 0));
+    per_sm = std::max(per_sm, 1);
+    ctx->resident.push_back({kern, per_sm});
     return per_sm;
 }
 
+// The grid of a persistent launch of `kern`, at most `cap` CTAs.  A persistent launch normally fills every resident-CTA
+// slot.  When the caller keeps n frames in flight, each launch takes 1/n of the slots so that the n kernels run side by
+// side from the start: a launch then lasts n times longer than its critical path (one tile of disk-plane rays, ~17 ms at
+// 4K) needs, instead of ending in a drain with most SMs idle (rrt_set_frames_in_flight).  Negative: the error code.
+static long long persistent_grid(rrt_context* ctx, const void* kern, int block, bool max_shared, long long cap) {
+    const int per_sm = resident_per_sm(ctx, kern, block, max_shared);
+    if (per_sm < 0) return per_sm;
+    return std::min(((long long)ctx->sm_count * per_sm + ctx->frames_in_flight - 1) / ctx->frames_in_flight, cap);
+}
+
+// ---- split pipeline: host side (csrc/rrt_split.cuh) ---------------------------------------------------------------
 // Slots of a sample pool for one frame, at most max_bytes: ~128 samples per pixel before a frame is cut into passes, plus
 // what the tracing warps hold in reserve: each takes the rows its tile could need in the worst case (max_steps + 1 rows of
 // 1 KiB per ray of a thread) before it traces it.
@@ -535,35 +551,34 @@ static rrtk::SplitArgs split_args(uint4* slots, size_t cap_slots, rrtk::TileDesc
     return S;
 }
 
-// The split pipeline's tracer for a launch, as rrt_render picks it, and its persistent grid.
+// The split pipeline's kernels for a launch, as rrt_render picks them, and the tracer's persistent grid.
 struct TracePlan {
+    const rrtk::SplitKernels* sk;                         // the kernels of the launch's rounding contract
     bool packed;                                          // two rays per thread in packed f32x2 registers (FMAD contract)
-    void (*kernel)(const FrameArgs, const rrtk::SplitArgs, const rrtk::LensArgs);
-    long long grid;                                       // already divided by the frames in flight
+    void (*trace)(const FrameArgs, const rrtk::SplitArgs, const rrtk::LensArgs);
+    void (*sweep)(const FrameArgs, const rrtk::SplitArgs, const rrtk::LensArgs);
+    long long grid;                                       // of the tracer, already divided by the frames in flight
     unsigned ntiles;                                      // tickets of the launch: 16x4 tiles (packed) or 8x4 tiles
     unsigned ngroups;                                     // groups of 32 rays a pass can queue
     int rows_per_tile;                                    // worst-case sample rows of one tile, exit states included
 };
 // Whether a launch with these parameters can go through the split pipeline: a tile's rows must fit a TileDesc.
 static bool split_fits(const rrt_params* prm) { return prm->max_steps + 2 <= 128 * (rrtk::kDescChunks - 2); }
-// lens: the LENS variant (every ray from its own camera of LensArgs::cams, rrt_render_dof).
-static TracePlan plan_trace(rrt_context* ctx, const rrt_params* prm, int w, int local_rows, bool lens = false) {
-    const bool spin = prm->spin_a != 0.0f, fmad = (prm->flags & RRT_FLAG_FMAD) != 0;
-    const rrtk::SplitKernels* sk = fmad ? rrtk::rrt_split_kernels_fmad() : rrtk::rrt_split_kernels_strict();
-    TracePlan t;
+// lens: the LENS variants (every ray from its own camera of LensArgs::cams, rrt_render_dof).
+static int plan_trace(rrt_context* ctx, const rrt_params& prm, int w, int local_rows, bool lens, TracePlan* t) {
+    const bool spin = prm.spin_a != 0.0f;
+    t->sk = (prm.flags & RRT_FLAG_FMAD) ? rrtk::rrt_split_kernels_fmad() : rrtk::rrt_split_kernels_strict();
     // the tracer: two rays per thread in packed f32x2 registers where that kernel exists (FMAD contract), else one per thread
-    t.packed = sk->trace_packed[0] != nullptr && ctx->trace_choice != 1 && 2ll * (prm->max_steps + 1) + 2 <= 128ll * (rrtk::kDescChunks - 2);
-    t.kernel = t.packed ? (lens ? sk->trace_packed_lens : sk->trace_packed)[spin ? 1 : 0] : (lens ? sk->trace_lens : sk->trace)[spin ? 1 : 0];
-    const int per_sm_trace = resident_per_sm(ctx, (const void*)t.kernel, kRenderBlock, true);
+    t->packed = t->sk->trace_packed[0][0] != nullptr && ctx->trace_choice != 1 && 2ll * (prm.max_steps + 1) + 2 <= 128ll * (rrtk::kDescChunks - 2);
+    t->trace = (t->packed ? t->sk->trace_packed : t->sk->trace)[lens][spin];
+    t->sweep = t->sk->sweep[lens][spin];
     const unsigned ntiles8 = (unsigned)(((w + kRTileW - 1) / kRTileW) * ((local_rows + kRTileH - 1) / kRTileH));
     const unsigned ntiles16 = (unsigned)(((w + kTile16W - 1) / kTile16W) * ((local_rows + kTile16H - 1) / kTile16H));
-    t.ntiles = t.packed ? ntiles16 : ntiles8;
-    t.ngroups = t.packed ? 2 * ntiles16 : ntiles8;
-    t.grid = ((long long)ctx->sm_count * per_sm_trace + ctx->frames_in_flight - 1) / ctx->frames_in_flight;
-    if (t.grid > (long long)t.ntiles) t.grid = t.ntiles;
-    if (t.grid > (long long)kRedoCap) t.grid = kRedoCap;
-    t.rows_per_tile = (t.packed ? 2 : 1) * (prm->max_steps + 1) + 1;
-    return t;
+    t->ntiles = t->packed ? ntiles16 : ntiles8;
+    t->ngroups = t->packed ? 2 * ntiles16 : ntiles8;
+    t->grid = persistent_grid(ctx, (const void*)t->trace, kRenderBlock, true, std::min<long long>(t->ntiles, kRedoCap));
+    t->rows_per_tile = (t->packed ? 2 : 1) * (prm.max_steps + 1) + 1;
+    return t->grid < 0 ? (int)t->grid : RRT_OK;
 }
 
 // Everything a render kernel reads about the frame except the planes, counters, ticket and tile log.
@@ -587,18 +602,19 @@ static FrameArgs frame_args(const rrt_params& prm, const rrt_camera& cam, const 
     return A;
 }
 
-// One frame through trace / media / fold passes and the closing sweep.  `grid_trace` = the persistent grid of the
-// tracing kernels for this launch (already divided by the frames in flight).  A camera table in L (rrt_render_dof) selects
-// the LENS tracers: the passes, the redo list and the sweep re-create every ray from its own camera.
-static int render_split(rrt_context* ctx, const FrameArgs& A, const rrtk::LensArgs& L, bool spin, bool fmad, bool packed_trace,
-                        long long grid_trace, cudaStream_t st, rrt_context::SamplePool* pl) {
-    const rrtk::SplitKernels* sk = fmad ? rrtk::rrt_split_kernels_fmad() : rrtk::rrt_split_kernels_strict();
-    const bool lens = L.cams != nullptr;
-    auto k_trace = packed_trace ? (lens ? sk->trace_packed_lens : sk->trace_packed)[spin ? 1 : 0] : (lens ? sk->trace_lens : sk->trace)[spin ? 1 : 0];
-    auto k_sweep = (lens ? sk->sweep_lens : sk->sweep)[spin ? 1 : 0];
-    const unsigned ntiles = packed_trace ? (unsigned)(((A.w + kTile16W - 1) / kTile16W) * ((A.local_rows + kTile16H - 1) / kTile16H))
-                                         : (unsigned)(((A.w + kRTileW - 1) / kRTileW) * ((A.local_rows + kRTileH - 1) / kRTileH));
+// The closing sweep of a split frame: the fused code over the tiles its passes left.  The caller checks the launch.
+static int launch_sweep(rrt_context* ctx, const TracePlan& tp, const FrameArgs& A, const rrtk::SplitArgs& S, const rrtk::LensArgs& L,
+                        cudaStream_t st) {
+    const long long grid = persistent_grid(ctx, (const void*)tp.sweep, kRenderBlock, true, tp.ntiles);
+    if (grid < 0) return (int)grid;
+    tp.sweep<<<(unsigned)grid, kRenderBlock, 0, st>>>(A, S, L);
+    return RRT_OK;
+}
 
+// One frame through trace / media / fold passes and the closing sweep.  A camera table in L (rrt_render_dof) selects the
+// LENS tracers of the plan: the passes, the redo list and the sweep re-create every ray from its own camera.
+static int render_split(rrt_context* ctx, const FrameArgs& A, const rrtk::LensArgs& L, const TracePlan& tp, cudaStream_t st,
+                        rrt_context::SamplePool* pl) {
     // passes to enqueue: what the last completed frame on this pool needed (the sweep renders whatever a wrong guess leaves)
     const unsigned* hs = pl->h_stats;   // [0] passes that took tiles [1] tiles swept [2] tiles taken by passes [3] passes enqueued [4] ntiles
     int passes = ctx->passes_hint;
@@ -610,33 +626,32 @@ static int render_split(rrt_context* ctx, const FrameArgs& A, const rrtk::LensAr
     if (passes < 1) passes = 1;
     if (passes > ctx->max_passes) passes = ctx->max_passes;
 
-    rrtk::SplitArgs S = split_args(pl->d_slots, pl->cap_slots, pl->d_desc, pl->d_work, pl->work_cap, packed_trace, A.C.max_steps, grid_trace);
+    rrtk::SplitArgs S = split_args(pl->d_slots, pl->cap_slots, pl->d_desc, pl->d_work, pl->work_cap, tp.packed, A.C.max_steps, tp.grid);
     rrtk::PassCtrl* pcs = (rrtk::PassCtrl*)pl->d_ctrl;
     S.stats = (unsigned*)(pl->d_ctrl + sizeof(rrtk::PassCtrl) * (kMaxPasses + 1));
     unsigned* redo = (unsigned*)(pl->d_ctrl + kCtrlHead);
 
     RRT_CU(ctx, cudaMemsetAsync(pl->d_ctrl, 0, kCtrlHead, st));
-    const int per_sm_media = resident_per_sm(ctx, (const void*)sk->media, kMediaBlock, true);
-    const int per_sm_fold = resident_per_sm(ctx, (const void*)sk->fold, 128, false);
-    const int per_sm_sweep = resident_per_sm(ctx, (const void*)k_sweep, kRenderBlock, true);
+    const int per_sm_media = resident_per_sm(ctx, (const void*)tp.sk->media, kMediaBlock, true);
+    if (per_sm_media < 0) return per_sm_media;
+    const int per_sm_fold = resident_per_sm(ctx, (const void*)tp.sk->fold, 128, false);
+    if (per_sm_fold < 0) return per_sm_fold;
     for (int p = 0; p < passes; ++p) {
         S.pass = (unsigned)p;
         S.pc = pcs + p;
         S.pc_prev = p ? pcs + (p - 1) : nullptr;
         S.redo_in = p ? redo + (size_t)(p - 1) * kRedoCap : nullptr;
         S.redo_out = redo + (size_t)p * kRedoCap;
-        k_trace<<<(unsigned)grid_trace, kRenderBlock, 0, st>>>(A, S, L);
-        sk->media<<<(unsigned)(ctx->sm_count * per_sm_media), kMediaBlock, 0, st>>>(A, S);
-        sk->fold<<<(unsigned)(ctx->sm_count * per_sm_fold), 128, 0, st>>>(A, S);
+        tp.trace<<<(unsigned)tp.grid, kRenderBlock, 0, st>>>(A, S, L);
+        tp.sk->media<<<(unsigned)(ctx->sm_count * per_sm_media), kMediaBlock, 0, st>>>(A, S);
+        tp.sk->fold<<<(unsigned)(ctx->sm_count * per_sm_fold), 128, 0, st>>>(A, S);
     }
     S.pass = (unsigned)passes;
     S.pc = pcs + passes;
     S.pc_prev = pcs + (passes - 1);
     S.redo_in = redo + (size_t)(passes - 1) * kRedoCap;
     S.redo_out = redo + (size_t)passes * kRedoCap;
-    long long grid_sweep = ((long long)ctx->sm_count * per_sm_sweep + ctx->frames_in_flight - 1) / ctx->frames_in_flight;
-    if (grid_sweep > (long long)ntiles) grid_sweep = ntiles;
-    k_sweep<<<(unsigned)grid_sweep, kRenderBlock, 0, st>>>(A, S, L);
+    if (int rc = launch_sweep(ctx, tp, A, S, L, st)) return rc;
     RRT_CU(ctx, cudaGetLastError());
     ctx->launches += 3ull * (unsigned)passes + 1ull;
     RRT_CU(ctx, cudaMemcpyAsync(pl->h_stats, S.stats, 8 * sizeof(unsigned), cudaMemcpyDeviceToHost, st));
@@ -644,137 +659,37 @@ static int render_split(rrt_context* ctx, const FrameArgs& A, const rrtk::LensAr
     return RRT_OK;
 }
 
-}  // extern "C"
-
-// rrt_render's body.  d_cams: null, or a DEVICE table of cam_ss * cam_ss cameras (rrt_render_dof) -- then the LENS variant
-// of the chosen tracer starts pixel (x, y)'s ray from d_cams[(y % cam_ss) * cam_ss + x % cam_ss] and `cam` is not read by
-// any kernel; cams_near: every camera of the table is in the branch-free domain (LensArgs::near).  Launch choice,
-// pipeline, counters and launch count are rrt_render's either way.
-static int render_frame(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, const rrt_effects* fx, uint64_t sky_texture,
-                        float time, int w, int h, const rrt_band* band, void* d_out, int out_layout, const rrt_planes* planes,
-                        void* stream, const rrt_camera* d_cams, int cam_ss, bool cams_near) {
-    if (!ctx) return RRT_ERR_BAD_ARG;
-    if (!prm || !cam || !fx || w <= 0 || h <= 0 || sky_texture == 0 || prm->max_steps < 0 ||
-        (out_layout != RRT_OUT_FRAME && out_layout != RRT_OUT_PACKED) || (!d_out && !planes))
-        return fail(ctx, RRT_ERR_BAD_ARG, "rrt_render: bad argument");
-    rrt_band b = {0, 1, 1};
-    if (band) b = *band;
-    const int local_rows = rrt_band_rows(&b, h);
-    if (local_rows < 0) return fail(ctx, RRT_ERR_BAD_ARG, "rrt_render: bad band");
-    if (local_rows == 0) return RRT_OK;
-
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    DevGuard g(ctx->device);
-    cudaStream_t st = (cudaStream_t)stream;
-    FrameArgs A = frame_args(*prm, *cam, *fx, sky_texture, time, w, h, b, local_rows, out_layout, d_out);
-    if (planes) A.planes = *planes;
-    A.counters = ctx->d_counters;
-    A.tile_log = ctx->tile_log;
-    A.tile_log_cap = ctx->tile_log_cap;
-    A.ticket = ctx->d_tickets + (ctx->ticket_next++ % kTicketRing);
-    rrtk::LensArgs L = {d_cams, d_cams ? cam_ss : 0, d_cams && cams_near ? 1 : 0};
-    RRT_CU(ctx, cudaMemsetAsync(A.ticket, 0, sizeof(unsigned), st));
-
-    const bool spin = prm->spin_a != 0.0f;
-    const bool media = (prm->flags & (RRT_FLAG_DISK | RRT_FLAG_DUST)) != 0;
-    const bool fmad = (prm->flags & RRT_FLAG_FMAD) != 0;
-    const bool lens = d_cams != nullptr;
-    const rrtk::KernelSet* ks = fmad ? rrtk::rrt_kernels_fmad() : rrtk::rrt_kernels_strict();
-    void (*kern)(const FrameArgs, const rrtk::LensArgs) = (lens ? ks->render_lens : ks->render)[spin ? 1 : 0][media ? 1 : 0];
-    long long rays_per_block = kRenderBlock;
-    if (fmad && !media && !ctx->scalar_kernel) {
-        kern = (lens ? ks->render_packed_lens : ks->render_packed)[spin ? 1 : 0];
-        rays_per_block = 64;
-    }
-    if ((long long)w * local_rows > (1ll << 30)) return fail(ctx, RRT_ERR_BAD_ARG, "rrt_render: band larger than 2^30 pixels");
-    // Resident CTAs per SM and the shared-memory carve-out are properties of (kernel, device): asked for once per
-    // context, not per frame.  The carve-out stays at the shared-memory end although render_kernel declares no shared
-    // memory: every resident CTA still reserves 1 KB of it, and with one-warp CTAs (24-32 per SM) a small carve-out
-    // caps residency -- measured with cudaSharedmemCarveoutMaxL1: 4K C0 73.3 -> 80.7 ms, C3 133 -> 164 ms.
-    int per_sm = 0;
-    for (int i = 0; i < ctx->n_launch_cfg; ++i)
-        if (ctx->launch_cfg[i].kern == (const void*)kern) per_sm = ctx->launch_cfg[i].per_sm;
-    if (per_sm == 0) {
-        RRT_CU(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        RRT_CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kRenderBlock, 0));
-        if (per_sm < 1) per_sm = 1;
-        if (ctx->n_launch_cfg < 16) ctx->launch_cfg[ctx->n_launch_cfg++] = {(const void*)kern, per_sm};
-    }
-    // A persistent launch normally fills every resident-CTA slot.  When the caller keeps n frames in flight, each
-    // launch takes 1/n of the slots so that the n kernels run side by side from the start: a launch then lasts
-    // n times longer than its critical path (one tile of disk-plane rays, ~17 ms at 4K) needs, instead of ending
-    // in a drain with most SMs idle (rrt_set_frames_in_flight).
-    long long grid = ((long long)ctx->sm_count * per_sm + ctx->frames_in_flight - 1) / ctx->frames_in_flight;
-    const long long need = ((long long)w * local_rows + rays_per_block - 1) / rays_per_block;
-    if (grid > need) grid = need;
-    // A launch with a medium goes through the split pipeline (csrc/rrt_split.cuh) unless the caller pinned the fused
-    // kernel, the tile log is selected, or the pool cannot be allocated.
-    if (media && ctx->pipeline != RRT_PIPELINE_FUSED && (!ctx->tile_log || ctx->pipeline == RRT_PIPELINE_SPLIT) && split_fits(prm)) {
-        const TracePlan tp = plan_trace(ctx, prm, w, local_rows, lens);
-        if (rrt_context::SamplePool* pl = acquire_pool(ctx, st, (long long)w * local_rows, tp.ngroups, tp.grid, tp.rows_per_tile))
-            return render_split(ctx, A, L, spin, fmad, tp.packed, tp.grid, st, pl);
-        if (ctx->pipeline == RRT_PIPELINE_SPLIT) return fail(ctx, RRT_ERR_NOMEM, "rrt_render: no memory for the sample pool of the split pipeline");
-    }
-    kern<<<(unsigned)grid, kRenderBlock, 0, st>>>(A, L);
-    RRT_CU(ctx, cudaGetLastError());
-    ctx->launches += 1;
-    return RRT_OK;
+// ---- argument checks: every entry point runs them before it takes ctx->mu or enqueues anything ---------------------
+// A destination: a known layout and at least one of the uchar4 frame and the hdr plane (or planes).
+static bool outputs_ok(int out_layout, const void* d_out, const void* hdr) {
+    return (out_layout == RRT_OUT_FRAME || out_layout == RRT_OUT_PACKED) && (d_out || hdr);
 }
 
-extern "C" {
-
-int rrt_render(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, const rrt_effects* fx, uint64_t sky_texture,
-               float time, int w, int h, const rrt_band* band, void* d_out, int out_layout, const rrt_planes* planes,
-               void* stream) {
-    return render_frame(ctx, prm, cam, fx, sky_texture, time, w, h, band, d_out, out_layout, planes, stream, nullptr, 0, false);
-}
-
-int rrt_shade(rrt_context* ctx, const rrt_params* prm, const rrt_effects* fx, uint64_t sky_texture, int w, int h,
-              const rrt_band* band, const rrt_planes* traced, void* d_out, int out_layout, float* hdr_out, void* stream) {
-    if (!ctx) return RRT_ERR_BAD_ARG;
-    if (!prm || !fx || w <= 0 || h <= 0 || sky_texture == 0 || (out_layout != RRT_OUT_FRAME && out_layout != RRT_OUT_PACKED) ||
-        !traced || !traced->vel || !traced->emis || !traced->hdr || !traced->cls || (!d_out && !hdr_out))
-        return fail(ctx, RRT_ERR_BAD_ARG, "rrt_shade: bad argument");
-    rrt_band b = {0, 1, 1};
-    if (band) b = *band;
-    const int local_rows = rrt_band_rows(&b, h);
-    if (local_rows < 0) return fail(ctx, RRT_ERR_BAD_ARG, "rrt_shade: bad band");
-    if (local_rows == 0) return RRT_OK;
-    if ((long long)w * local_rows > (1ll << 30)) return fail(ctx, RRT_ERR_BAD_ARG, "rrt_shade: band larger than 2^30 pixels");
-
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    DevGuard g(ctx->device);
-    FrameArgs A;
-    std::memset(&A, 0, sizeof(A));   // no camera, counters, ticket or tile log: nothing is traced
-    A.C = make_consts(*prm);         // finish_ray_inl reads exposure only
-    A.fx = *fx;
-    A.w = w;
-    A.h = h;
-    A.band_rank = b.rank;
-    A.band_nranks = b.nranks;
-    A.band_group = b.group;
-    A.local_rows = local_rows;
-    A.out_layout = out_layout;
-    A.out = (uchar4*)d_out;
-    A.planes.hdr = hdr_out;
-    A.sky = (cudaTextureObject_t)sky_texture;
-    const long long n = (long long)w * local_rows;
-    kset(prm)->shade<<<(unsigned)((n + kShadeBlock - 1) / kShadeBlock), kShadeBlock, 0, (cudaStream_t)stream>>>(A, *traced);
-    RRT_CU(ctx, cudaGetLastError());
-    ctx->launches += 1;
-    return RRT_OK;
-}
-
-// What rrt_resolve and rrt_render_ss both check: ss, the ss*w x ss*h frame and the band, whose traced form {rank, nranks,
-// ss*group} must stay within rrt_render's 2^30 rays.  Sets *local_rows, the band's rows of the w x h frame.
-static int check_ss(rrt_context* ctx, const char* what, int ss, int w, int h, const rrt_band* band, int* local_rows) {
-    std::string m = what;
-    if (ss < 1 || ss > 8 || w <= 0 || h <= 0 || (long long)ss * w > INT_MAX || (long long)ss * h > INT_MAX)
-        return fail(ctx, RRT_ERR_BAD_ARG, (m + ": bad argument").c_str());
-    const int rows = rrt_band_rows(band, h);
-    if (rows < 0 || (band && (long long)ss * band->group > INT_MAX)) return fail(ctx, RRT_ERR_BAD_ARG, (m + ": bad band").c_str());
-    if ((long long)ss * ss * w * rows > (1ll << 30)) return fail(ctx, RRT_ERR_BAD_ARG, (m + ": band larger than 2^30 sub-samples").c_str());
+// The band of a call on a w x h frame: `band`, or the whole frame {0, 1, 1}, into *b and its rows into *local_rows.
+// Traced with ss x ss rays per pixel it is the band {rank, nranks, ss*group} of the ss*w x ss*h frame, which must stay
+// within rrt_render's 2^30 rays.
+static int band_of(rrt_context* ctx, const std::string& what, const rrt_band* band, int w, int h, int ss, rrt_band* b, int* local_rows) {
+    *b = band ? *band : rrt_band{0, 1, 1};
+    const int rows = rrt_band_rows(b, h);
+    if (rows < 0 || (long long)ss * b->group > INT_MAX) return fail(ctx, RRT_ERR_BAD_ARG, what + ": bad band");
+    if ((long long)ss * ss * w * rows > (1ll << 30))
+        return fail(ctx, RRT_ERR_BAD_ARG, what + (ss == 1 ? ": band larger than 2^30 pixels" : ": band larger than 2^30 sub-samples"));
     *local_rows = rows;
+    return RRT_OK;
+}
+
+// A supersampling factor and the w x h frame it resolves to, whose ss*w x ss*h trace must have int sizes.
+static bool ss_ok(int ss, int w, int h) {
+    return ss >= 1 && ss <= 8 && w > 0 && h > 0 && (long long)ss * w <= INT_MAX && (long long)ss * h <= INT_MAX;
+}
+
+// What rrt_resolve_time, rrt_render_mb and rrt_capture_render_mb check: n, the frame, the band and a stack of n
+// full-frame planes that fits the address space.
+static int check_mb(rrt_context* ctx, const std::string& what, int n, int w, int h, const rrt_band* band, rrt_band* b, int* local_rows) {
+    if (n < 1 || n > 64 || w <= 0 || h <= 0) return fail(ctx, RRT_ERR_BAD_ARG, what + ": bad argument");
+    if (int rc = band_of(ctx, what, band, w, h, 1, b, local_rows)) return rc;
+    if ((unsigned long long)w * h > SIZE_MAX / 16 / (unsigned)n)
+        return fail(ctx, RRT_ERR_BAD_ARG, what + ": sub-frame stack larger than the address space");
     return RRT_OK;
 }
 
@@ -784,57 +699,70 @@ static bool f4_overlap(const void* src, unsigned long long src_n, const void* ds
     return b >= a ? (b - a) / 16 < src_n : (a - b) / 16 < dst_n;
 }
 
-// The launch of rrt_resolve and rrt_resolve_time: resolve_kernel over the band's rows of the w x h frame, n planes of
-// ss*w x ss*h from `src`, one plane_stride (float4) apart.  Arguments checked; ctx->mu held.
-static int launch_resolve(rrt_context* ctx, const rrt_params* prm, const rrt_effects* fx, int ss, int n, int w, int h,
-                          const rrt_band* band, int local_rows, const float* src, size_t plane_stride, void* d_out,
-                          int out_layout, float* hdr_out, cudaStream_t st) {
-    DevGuard g(ctx->device);
-    FrameArgs A;
-    std::memset(&A, 0, sizeof(A));   // no camera, sky, counters, ticket or tile log: nothing is traced or sampled
-    A.C = make_consts(*prm);         // the post step reads exposure only
-    A.fx = *fx;
-    A.w = w;
-    A.h = h;
-    if (band) {
-        A.band_rank = band->rank;
-        A.band_nranks = band->nranks;
-        A.band_group = band->group;
-    } else {
-        A.band_nranks = A.band_group = 1;
+// ---- bodies: arguments checked, ctx->mu held, ctx->device current ---------------------------------------------------
+// rrt_render's body.  L.cams: null, or a DEVICE table of L.ss * L.ss cameras (rrt_render_dof) -- then the LENS variant of
+// the chosen kernel starts pixel (x, y)'s ray from L.cams[(y % L.ss) * L.ss + x % L.ss] and `cam` is not read by any
+// kernel.  Launch choice, pipeline, counters and launch count are rrt_render's either way.
+static int render_frame(rrt_context* ctx, const rrt_params& prm, const rrt_camera& cam, const rrt_effects& fx, uint64_t sky_texture,
+                        float time, int w, int h, const rrt_band& b, int local_rows, void* d_out, int out_layout, const rrt_planes* planes,
+                        cudaStream_t st, const rrtk::LensArgs& L) {
+    FrameArgs A = frame_args(prm, cam, fx, sky_texture, time, w, h, b, local_rows, out_layout, d_out);
+    if (planes) A.planes = *planes;
+    A.counters = ctx->d_counters;
+    A.tile_log = ctx->tile_log;
+    A.tile_log_cap = ctx->tile_log_cap;
+    A.ticket = ctx->d_tickets + (ctx->ticket_next++ % kTicketRing);
+    RRT_CU(ctx, cudaMemsetAsync(A.ticket, 0, sizeof(unsigned), st));
+
+    const bool spin = prm.spin_a != 0.0f;
+    const bool media = (prm.flags & (RRT_FLAG_DISK | RRT_FLAG_DUST)) != 0;
+    const bool fmad = (prm.flags & RRT_FLAG_FMAD) != 0;
+    const bool lens = L.cams != nullptr;
+    // A launch with a medium goes through the split pipeline (csrc/rrt_split.cuh) unless the caller pinned the fused
+    // kernel, the tile log is selected, or the pool cannot be allocated.
+    if (media && ctx->pipeline != RRT_PIPELINE_FUSED && (!ctx->tile_log || ctx->pipeline == RRT_PIPELINE_SPLIT) && split_fits(&prm)) {
+        TracePlan tp;
+        if (int rc = plan_trace(ctx, prm, w, local_rows, lens, &tp)) return rc;
+        if (rrt_context::SamplePool* pl = acquire_pool(ctx, st, (long long)w * local_rows, tp.ngroups, tp.grid, tp.rows_per_tile))
+            return render_split(ctx, A, L, tp, st, pl);
+        if (ctx->pipeline == RRT_PIPELINE_SPLIT) return fail(ctx, RRT_ERR_NOMEM, "rrt_render: no memory for the sample pool of the split pipeline");
     }
-    A.local_rows = local_rows;
-    A.out_layout = out_layout;
-    A.out = (uchar4*)d_out;
+    const rrtk::KernelSet* ks = kset(&prm);
+    void (*kern)(const FrameArgs, const rrtk::LensArgs) = ks->render[lens][spin][media];
+    long long rays_per_block = kRenderBlock;
+    if (fmad && !media && !ctx->scalar_kernel) {
+        kern = ks->render_packed[lens][spin];
+        rays_per_block = 64;
+    }
+    const long long grid = persistent_grid(ctx, (const void*)kern, kRenderBlock, true, ((long long)w * local_rows + rays_per_block - 1) / rays_per_block);
+    if (grid < 0) return (int)grid;
+    kern<<<(unsigned)grid, kRenderBlock, 0, st>>>(A, L);
+    RRT_CU(ctx, cudaGetLastError());
+    ctx->launches += 1;
+    return RRT_OK;
+}
+
+// The launch of rrt_resolve and rrt_resolve_time: resolve_kernel over the band's rows of the w x h frame, n planes of
+// ss*w x ss*h from `src`, one plane_stride (float4) apart.
+static int launch_resolve(rrt_context* ctx, const rrt_params& prm, const rrt_effects& fx, int ss, int n, int w, int h, const rrt_band& b,
+                          int local_rows, const float* src, size_t plane_stride, void* d_out, int out_layout, float* hdr_out, cudaStream_t st) {
+    // no camera, sky, counters, ticket or tile log: nothing is traced or sampled; the post step reads exposure only
+    FrameArgs A = frame_args(prm, rrt_camera{}, fx, 0, 0.0f, w, h, b, local_rows, out_layout, d_out);
     A.planes.hdr = hdr_out;
     const long long npix = (long long)w * local_rows;
-    kset(prm)->resolve<<<(unsigned)((npix + kResolveBlock - 1) / kResolveBlock), kResolveBlock, 0, st>>>(
+    kset(&prm)->resolve<<<(unsigned)((npix + kResolveBlock - 1) / kResolveBlock), kResolveBlock, 0, st>>>(
         A, (const float4*)src, ss, n, plane_stride);
     RRT_CU(ctx, cudaGetLastError());
     ctx->launches += 1;
     return RRT_OK;
 }
 
-int rrt_resolve(rrt_context* ctx, const rrt_params* prm, const rrt_effects* fx, int ss, int w, int h, const rrt_band* band,
-                const float* hdr_hi, void* d_out, int out_layout, float* hdr_out, void* stream) {
-    if (!ctx) return RRT_ERR_BAD_ARG;
-    if (!prm || !fx || !hdr_hi || (out_layout != RRT_OUT_FRAME && out_layout != RRT_OUT_PACKED) || (!d_out && !hdr_out))
-        return fail(ctx, RRT_ERR_BAD_ARG, "rrt_resolve: bad argument");
-    int local_rows = 0;
-    if (int rc = check_ss(ctx, "rrt_resolve", ss, w, h, band, &local_rows)) return rc;
-    // the kernel reads hdr_hi while it writes hdr_out: the two must not share a byte
-    if (hdr_out && f4_overlap(hdr_hi, (unsigned long long)ss * ss * w * h, hdr_out, (unsigned long long)w * h))
-        return fail(ctx, RRT_ERR_BAD_ARG, "rrt_resolve: hdr_out overlaps hdr_hi");
-    if (local_rows == 0) return RRT_OK;
-
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    return launch_resolve(ctx, prm, fx, ss, 1, w, h, band, local_rows, hdr_hi, 0, d_out, out_layout, hdr_out, (cudaStream_t)stream);
-}
-
-// A stream-ordered block of `bytes` from the context's scratch pool (created on first use), for rrt_render_ss's
-// supersampled plane and the sub-frame stacks of rrt_render_mb / rrt_capture_render_mb.  ctx->mu held.
-static int scratch_alloc(rrt_context* ctx, const char* nomem_msg, size_t bytes, cudaStream_t st, float** out) {
-    DevGuard g(ctx->device);
+// body(block) with a stream-ordered block of `bytes` from the context's scratch pool (created on first use), which keeps
+// freed blocks for the next frame instead of returning them to the device: rrt_render_ss's supersampled plane, the
+// sub-frame stacks of rrt_render_mb / rrt_capture_render_mb.  The block goes back to the pool behind whatever body
+// enqueued; the first error wins.
+template <typename Body>
+static int with_scratch(rrt_context* ctx, const std::string& what, const char* block_name, size_t bytes, cudaStream_t st, Body body) {
     if (!ctx->ss_pool) {
         cudaMemPoolProps props;
         std::memset(&props, 0, sizeof(props));
@@ -845,73 +773,131 @@ static int scratch_alloc(rrt_context* ctx, const char* nomem_msg, size_t bytes, 
         uint64_t keep = UINT64_MAX;   // hold freed blocks: the next frame of a sequence reuses them without a new allocation
         RRT_CU(ctx, cudaMemPoolSetAttribute(ctx->ss_pool, cudaMemPoolAttrReleaseThreshold, &keep));
     }
-    if (cudaMallocFromPoolAsync((void**)out, bytes, ctx->ss_pool, st) != cudaSuccess) {
+    float* block = nullptr;
+    if (cudaMallocFromPoolAsync((void**)&block, bytes, ctx->ss_pool, st) != cudaSuccess) {
         cudaGetLastError();
-        return fail(ctx, RRT_ERR_NOMEM, nomem_msg);
+        return fail(ctx, RRT_ERR_NOMEM, what + ": no memory for the " + block_name);
     }
+    const int rc = body(block);
+    const cudaError_t e = cudaFreeAsync(block, st);   // stream-ordered: the block goes back once the last kernel has read it
+    if (rc == RRT_OK && e != cudaSuccess) return fail(ctx, RRT_ERR_CUDA, what + ": cudaFreeAsync", e);
+    return rc;
+}
+
+extern "C" {
+
+int rrt_render(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, const rrt_effects* fx, uint64_t sky_texture,
+               float time, int w, int h, const rrt_band* band, void* d_out, int out_layout, const rrt_planes* planes,
+               void* stream) {
+    if (!ctx) return RRT_ERR_BAD_ARG;
+    if (!prm || !cam || !fx || w <= 0 || h <= 0 || sky_texture == 0 || prm->max_steps < 0 || !outputs_ok(out_layout, d_out, planes))
+        return fail(ctx, RRT_ERR_BAD_ARG, "rrt_render: bad argument");
+    rrt_band b;
+    int local_rows = 0;
+    if (int rc = band_of(ctx, "rrt_render", band, w, h, 1, &b, &local_rows)) return rc;
+    if (local_rows == 0) return RRT_OK;
+
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DevGuard g(ctx->device);
+    return render_frame(ctx, *prm, *cam, *fx, sky_texture, time, w, h, b, local_rows, d_out, out_layout, planes, (cudaStream_t)stream,
+                        rrtk::LensArgs{});
+}
+
+int rrt_shade(rrt_context* ctx, const rrt_params* prm, const rrt_effects* fx, uint64_t sky_texture, int w, int h,
+              const rrt_band* band, const rrt_planes* traced, void* d_out, int out_layout, float* hdr_out, void* stream) {
+    if (!ctx) return RRT_ERR_BAD_ARG;
+    if (!prm || !fx || w <= 0 || h <= 0 || sky_texture == 0 || !traced || !traced->vel || !traced->emis || !traced->hdr || !traced->cls ||
+        !outputs_ok(out_layout, d_out, hdr_out))
+        return fail(ctx, RRT_ERR_BAD_ARG, "rrt_shade: bad argument");
+    rrt_band b;
+    int local_rows = 0;
+    if (int rc = band_of(ctx, "rrt_shade", band, w, h, 1, &b, &local_rows)) return rc;
+    if (local_rows == 0) return RRT_OK;
+
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DevGuard g(ctx->device);
+    // no camera, counters, ticket or tile log: nothing is traced; finish_ray_inl reads exposure only
+    FrameArgs A = frame_args(*prm, rrt_camera{}, *fx, sky_texture, 0.0f, w, h, b, local_rows, out_layout, d_out);
+    A.planes.hdr = hdr_out;
+    const long long n = (long long)w * local_rows;
+    kset(prm)->shade<<<(unsigned)((n + kShadeBlock - 1) / kShadeBlock), kShadeBlock, 0, (cudaStream_t)stream>>>(A, *traced);
+    RRT_CU(ctx, cudaGetLastError());
+    ctx->launches += 1;
     return RRT_OK;
 }
 
-// rrt_render_ss's body: the ss*w x ss*h trace into a scratch plane, then rrt_resolve.  cams: null (every sub-sample from
-// `cam`), or a HOST table of ss*ss cameras (rrt_render_dof), copied into the same scratch block behind the plane.
+int rrt_resolve(rrt_context* ctx, const rrt_params* prm, const rrt_effects* fx, int ss, int w, int h, const rrt_band* band,
+                const float* hdr_hi, void* d_out, int out_layout, float* hdr_out, void* stream) {
+    if (!ctx) return RRT_ERR_BAD_ARG;
+    if (!prm || !fx || !hdr_hi || !ss_ok(ss, w, h) || !outputs_ok(out_layout, d_out, hdr_out))
+        return fail(ctx, RRT_ERR_BAD_ARG, "rrt_resolve: bad argument");
+    rrt_band b;
+    int local_rows = 0;
+    if (int rc = band_of(ctx, "rrt_resolve", band, w, h, ss, &b, &local_rows)) return rc;
+    // the kernel reads hdr_hi while it writes hdr_out: the two must not share a byte
+    if (hdr_out && f4_overlap(hdr_hi, (unsigned long long)ss * ss * w * h, hdr_out, (unsigned long long)w * h))
+        return fail(ctx, RRT_ERR_BAD_ARG, "rrt_resolve: hdr_out overlaps hdr_hi");
+    if (local_rows == 0) return RRT_OK;
+
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DevGuard g(ctx->device);
+    return launch_resolve(ctx, *prm, *fx, ss, 1, w, h, b, local_rows, hdr_hi, 0, d_out, out_layout, hdr_out, (cudaStream_t)stream);
+}
+
+// rrt_render_ss and rrt_render_dof: the ss*w x ss*h trace into a scratch plane, then rrt_resolve's launch.  cams: null
+// (every sub-sample from `cam`), or a HOST table of ss*ss cameras (rrt_render_dof), copied into the same scratch block
+// behind the plane.
 static int render_ss_frame(rrt_context* ctx, const char* what, const rrt_params* prm, const rrt_camera* cam, const rrt_camera* cams,
                            const rrt_effects* fx, uint64_t sky_texture, float time, int w, int h, int ss, const rrt_band* band,
                            void* d_out, int out_layout, float* hdr_out, void* stream) {
     const std::string m = what;
-    if (!ctx) return RRT_ERR_BAD_ARG;
-    if (!prm || !cam || !fx || sky_texture == 0 || prm->max_steps < 0 || (out_layout != RRT_OUT_FRAME && out_layout != RRT_OUT_PACKED) ||
-        (!d_out && !hdr_out))
-        return fail(ctx, RRT_ERR_BAD_ARG, (m + ": bad argument").c_str());
+    if (!prm || !cam || !fx || sky_texture == 0 || prm->max_steps < 0 || !ss_ok(ss, w, h) || !outputs_ok(out_layout, d_out, hdr_out))
+        return fail(ctx, RRT_ERR_BAD_ARG, m + ": bad argument");
+    rrt_band b;
     int local_rows = 0;
-    if (int rc = check_ss(ctx, what, ss, w, h, band, &local_rows)) return rc;
+    if (int rc = band_of(ctx, m, band, w, h, ss, &b, &local_rows)) return rc;
     bool cams_near = true;   // trace_ray's fast_ok for every camera of the table: |pos|^2 < 1e8
     if (cams)
         for (int k = 0; k < ss * ss; ++k) {
             const float* f = cams[k].pos;   // pos, forward, right, up: 12 consecutive floats
             for (int c = 0; c < 12; ++c)
-                if (!std::isfinite(f[c])) return fail(ctx, RRT_ERR_BAD_ARG, (m + ": non-finite camera field").c_str());
+                if (!std::isfinite(f[c])) return fail(ctx, RRT_ERR_BAD_ARG, m + ": non-finite camera field");
             cams_near = cams_near && (double)f[0] * f[0] + (double)f[1] * f[1] + (double)f[2] * f[2] < 1.0e8;
         }
     if (local_rows == 0) return RRT_OK;
-    // output group y / g is trace group (ss*y + j) / (ss*g): the band traces exactly the sub-rows of its own rows
-    rrt_band tb = {0, 1, ss};
-    if (band) tb = {band->rank, band->nranks, ss * band->group};
-    cudaStream_t st = (cudaStream_t)stream;
-    float* hi = nullptr;   // full-frame indexed like every plane of this ABI, so full-frame sized even for a band
-    const unsigned long long n_hi = (unsigned long long)ss * ss * w * h;
+    const unsigned long long n_hi = (unsigned long long)ss * ss * w * h;   // full-frame indexed like every plane of this ABI
     const size_t cam_bytes = cams ? sizeof(rrt_camera) * ss * ss : 0;
-    if (n_hi > (SIZE_MAX - cam_bytes) / 16) return fail(ctx, RRT_ERR_NOMEM, (m + ": supersampled hdr plane larger than the address space").c_str());
-    {
-        std::lock_guard<std::mutex> lk(ctx->mu);
-        if (int rc = scratch_alloc(ctx, (m + ": no memory for the supersampled hdr plane").c_str(), (size_t)16 * n_hi + cam_bytes, st, &hi))
-            return rc;
-    }
-    rrt_camera* d_cams = nullptr;
-    int rc = RRT_OK;
-    if (cams) {
-        // The table goes behind the plane (16-byte aligned).  The copy reads a pageable copy of the caller's table, which the
-        // runtime stages before cudaMemcpyAsync returns: the caller may reuse its table at once, also when it is pinned.
-        d_cams = (rrt_camera*)(hi + 4 * n_hi);
-        const std::vector<rrt_camera> staged(cams, cams + ss * ss);
-        DevGuard g(ctx->device);
-        const cudaError_t e = cudaMemcpyAsync(d_cams, staged.data(), cam_bytes, cudaMemcpyHostToDevice, st);
-        if (e != cudaSuccess) rc = fail(ctx, RRT_ERR_CUDA, (m + ": copy of the camera table").c_str(), e);
-    }
-    rrt_planes pl;
-    std::memset(&pl, 0, sizeof(pl));
-    pl.hdr = hi;
-    if (rc == RRT_OK)
-        rc = render_frame(ctx, prm, cam, fx, sky_texture, time, ss * w, ss * h, &tb, nullptr, RRT_OUT_FRAME, &pl, stream, d_cams, ss, cams_near);
-    if (rc == RRT_OK) rc = rrt_resolve(ctx, prm, fx, ss, w, h, band, hi, d_out, out_layout, hdr_out, stream);
+    if (n_hi > (SIZE_MAX - cam_bytes) / 16) return fail(ctx, RRT_ERR_NOMEM, m + ": supersampled hdr plane larger than the address space");
+
+    std::lock_guard<std::mutex> lk(ctx->mu);
     DevGuard g(ctx->device);
-    const cudaError_t e = cudaFreeAsync(hi, st);   // stream-ordered: the block goes back to the pool once the resolve has read it
-    if (rc == RRT_OK && e != cudaSuccess) return fail(ctx, RRT_ERR_CUDA, (m + ": cudaFreeAsync").c_str(), e);
-    return rc;
+    const cudaStream_t st = (cudaStream_t)stream;
+    return with_scratch(ctx, m, "supersampled hdr plane", (size_t)16 * n_hi + cam_bytes, st, [&](float* hi) {
+        rrtk::LensArgs L = {};
+        if (cams) {
+            // The table goes behind the plane (16-byte aligned).  The copy reads a pageable copy of the caller's table, which
+            // the runtime stages before cudaMemcpyAsync returns: the caller may reuse its table at once, also when it is pinned.
+            rrt_camera* d_cams = (rrt_camera*)(hi + 4 * n_hi);
+            const std::vector<rrt_camera> staged(cams, cams + ss * ss);
+            const cudaError_t e = cudaMemcpyAsync(d_cams, staged.data(), cam_bytes, cudaMemcpyHostToDevice, st);
+            if (e != cudaSuccess) return fail(ctx, RRT_ERR_CUDA, m + ": copy of the camera table", e);
+            L = {d_cams, ss, cams_near ? 1 : 0};
+        }
+        rrt_planes pl;
+        std::memset(&pl, 0, sizeof(pl));
+        pl.hdr = hi;
+        // output group y / g is trace group (ss*y + j) / (ss*g): the band traces exactly the ss sub-rows of each of its rows
+        const rrt_band tb = {b.rank, b.nranks, ss * b.group};
+        if (int rc = render_frame(ctx, *prm, *cam, *fx, sky_texture, time, ss * w, ss * h, tb, ss * local_rows, nullptr, RRT_OUT_FRAME, &pl, st, L))
+            return rc;
+        return launch_resolve(ctx, *prm, *fx, ss, 1, w, h, b, local_rows, hi, 0, d_out, out_layout, hdr_out, st);
+    });
 }
 
 int rrt_render_ss(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, const rrt_effects* fx, uint64_t sky_texture,
                   float time, int w, int h, int ss, const rrt_band* band, void* d_out, int out_layout, float* hdr_out,
                   void* stream) {
+    if (!ctx) return RRT_ERR_BAD_ARG;
     return render_ss_frame(ctx, "rrt_render_ss", prm, cam, nullptr, fx, sky_texture, time, w, h, ss, band, d_out, out_layout, hdr_out,
                            stream);
 }
@@ -925,34 +911,22 @@ int rrt_render_dof(rrt_context* ctx, const rrt_params* prm, const rrt_camera* ca
                            stream);
 }
 
-// What rrt_resolve_time, rrt_render_mb and rrt_capture_render_mb check: n, the frame, the band (at most 2^30 pixels, like
-// rrt_render) and a stack of n full-frame planes that fits the address space.  Sets *local_rows, the band's rows.
-static int check_mb(rrt_context* ctx, const char* what, int n, int w, int h, const rrt_band* band, int* local_rows) {
-    std::string m = what;
-    if (n < 1 || n > 64 || w <= 0 || h <= 0) return fail(ctx, RRT_ERR_BAD_ARG, (m + ": bad argument").c_str());
-    const int rows = rrt_band_rows(band, h);
-    if (rows < 0) return fail(ctx, RRT_ERR_BAD_ARG, (m + ": bad band").c_str());
-    if ((long long)w * rows > (1ll << 30)) return fail(ctx, RRT_ERR_BAD_ARG, (m + ": band larger than 2^30 pixels").c_str());
-    if ((unsigned long long)w * h > SIZE_MAX / 16 / (unsigned)n)
-        return fail(ctx, RRT_ERR_BAD_ARG, (m + ": sub-frame stack larger than the address space").c_str());
-    *local_rows = rows;
-    return RRT_OK;
-}
-
 int rrt_resolve_time(rrt_context* ctx, const rrt_params* prm, const rrt_effects* fx, int n, int w, int h, const rrt_band* band,
                      const float* hdr_stack, void* d_out, int out_layout, float* hdr_out, void* stream) {
     if (!ctx) return RRT_ERR_BAD_ARG;
-    if (!prm || !fx || !hdr_stack || (out_layout != RRT_OUT_FRAME && out_layout != RRT_OUT_PACKED) || (!d_out && !hdr_out))
+    if (!prm || !fx || !hdr_stack || !outputs_ok(out_layout, d_out, hdr_out))
         return fail(ctx, RRT_ERR_BAD_ARG, "rrt_resolve_time: bad argument");
+    rrt_band b;
     int local_rows = 0;
-    if (int rc = check_mb(ctx, "rrt_resolve_time", n, w, h, band, &local_rows)) return rc;
+    if (int rc = check_mb(ctx, "rrt_resolve_time", n, w, h, band, &b, &local_rows)) return rc;
     const unsigned long long plane = (unsigned long long)w * h;
     if (hdr_out && f4_overlap(hdr_stack, (unsigned long long)n * plane, hdr_out, plane))
         return fail(ctx, RRT_ERR_BAD_ARG, "rrt_resolve_time: hdr_out overlaps hdr_stack");
     if (local_rows == 0) return RRT_OK;
 
     std::lock_guard<std::mutex> lk(ctx->mu);
-    return launch_resolve(ctx, prm, fx, 1, n, w, h, band, local_rows, hdr_stack, (size_t)plane, d_out, out_layout, hdr_out,
+    DevGuard g(ctx->device);
+    return launch_resolve(ctx, *prm, *fx, 1, n, w, h, b, local_rows, hdr_stack, (size_t)plane, d_out, out_layout, hdr_out,
                           (cudaStream_t)stream);
 }
 
@@ -960,31 +934,28 @@ int rrt_render_mb(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam
                   const float* times, int n, int w, int h, const rrt_band* band, void* d_out, int out_layout, float* hdr_out,
                   void* stream) {
     if (!ctx) return RRT_ERR_BAD_ARG;
-    if (!prm || !cams || !fx || !times || sky_texture == 0 || prm->max_steps < 0 ||
-        (out_layout != RRT_OUT_FRAME && out_layout != RRT_OUT_PACKED) || (!d_out && !hdr_out))
+    if (!prm || !cams || !fx || !times || sky_texture == 0 || prm->max_steps < 0 || !outputs_ok(out_layout, d_out, hdr_out))
         return fail(ctx, RRT_ERR_BAD_ARG, "rrt_render_mb: bad argument");
+    rrt_band b;
     int local_rows = 0;
-    if (int rc = check_mb(ctx, "rrt_render_mb", n, w, h, band, &local_rows)) return rc;
+    if (int rc = check_mb(ctx, "rrt_render_mb", n, w, h, band, &b, &local_rows)) return rc;
     if (local_rows == 0) return RRT_OK;
-    cudaStream_t st = (cudaStream_t)stream;
-    const size_t plane = (size_t)w * h;   // full-frame indexed like every plane of this ABI, so full-frame sized even for a band
-    float* stack = nullptr;
-    {
-        std::lock_guard<std::mutex> lk(ctx->mu);
-        if (int rc = scratch_alloc(ctx, "rrt_render_mb: no memory for the sub-frame stack", 16 * n * plane, st, &stack)) return rc;
-    }
-    rrt_planes pl;
-    std::memset(&pl, 0, sizeof(pl));
-    int rc = RRT_OK;
-    for (int i = 0; i < n && rc == RRT_OK; ++i) {
-        pl.hdr = stack + 4 * plane * i;
-        rc = rrt_render(ctx, prm, &cams[i], fx, sky_texture, times[i], w, h, band, nullptr, RRT_OUT_FRAME, &pl, stream);
-    }
-    if (rc == RRT_OK) rc = rrt_resolve_time(ctx, prm, fx, n, w, h, band, stack, d_out, out_layout, hdr_out, stream);
+
+    std::lock_guard<std::mutex> lk(ctx->mu);
     DevGuard g(ctx->device);
-    const cudaError_t e = cudaFreeAsync(stack, st);   // stream-ordered: the block goes back to the pool once the resolve has read it
-    if (rc == RRT_OK && e != cudaSuccess) return fail(ctx, RRT_ERR_CUDA, "rrt_render_mb: cudaFreeAsync", e);
-    return rc;
+    const cudaStream_t st = (cudaStream_t)stream;
+    const size_t plane = (size_t)w * h;   // full-frame indexed like every plane of this ABI, so full-frame sized even for a band
+    return with_scratch(ctx, "rrt_render_mb", "sub-frame stack", 16 * n * plane, st, [&](float* stack) {
+        rrt_planes pl;
+        std::memset(&pl, 0, sizeof(pl));
+        for (int i = 0; i < n; ++i) {
+            pl.hdr = stack + 4 * plane * i;
+            if (int rc = render_frame(ctx, *prm, cams[i], *fx, sky_texture, times[i], w, h, b, local_rows, nullptr, RRT_OUT_FRAME, &pl, st,
+                                      rrtk::LensArgs{}))
+                return rc;
+        }
+        return launch_resolve(ctx, *prm, *fx, 1, n, w, h, b, local_rows, stack, plane, d_out, out_layout, hdr_out, st);
+    });
 }
 
 }  // extern "C"
@@ -1001,7 +972,7 @@ struct rrt_capture {
     rrt_effects fx;
     rrt_band band = {0, 1, 1};
     int w = 0, h = 0, local_rows = 0;
-    unsigned ntiles = 0;              // tickets of the frame: 16x4 tiles (packed tracer) or 8x4 tiles
+    TracePlan plan;                   // the pass's kernels and tickets: 16x4 tiles (packed tracer) or 8x4 tiles
     unsigned tiles_left = 0;          // tickets the pass did not trace: its redo list + the tickets it never took
     rrtk::SplitArgs S;                // media / fold over what the capture holds; the sweep's pass derives from it
     char* d_ctrl = nullptr;           // PassCtrl[2] (the pass, the sweep) | stats[8] | ticket | ticket after the pass | redo list
@@ -1053,11 +1024,9 @@ int rrt_capture_create(rrt_context* ctx, const rrt_params* prm, const rrt_camera
     if (!(prm->flags & (RRT_FLAG_DISK | RRT_FLAG_DUST)))
         return fail(ctx, RRT_ERR_BAD_ARG, "rrt_capture_create: no medium (RRT_FLAG_DISK / RRT_FLAG_DUST): nothing depends on the time, re-shade with rrt_shade");
     if (!split_fits(prm)) return fail(ctx, RRT_ERR_BAD_ARG, "rrt_capture_create: max_steps too large for the split pipeline");
-    rrt_band b = {0, 1, 1};
-    if (band) b = *band;
-    const int local_rows = rrt_band_rows(&b, h);
-    if (local_rows < 0) return fail(ctx, RRT_ERR_BAD_ARG, "rrt_capture_create: bad band");
-    if ((long long)w * local_rows > (1ll << 30)) return fail(ctx, RRT_ERR_BAD_ARG, "rrt_capture_create: band larger than 2^30 pixels");
+    rrt_band b;
+    int local_rows = 0;
+    if (int rc = band_of(ctx, "rrt_capture_create", band, w, h, 1, &b, &local_rows)) return rc;
 
     std::lock_guard<std::mutex> lk(ctx->mu);
     DevGuard g(ctx->device);
@@ -1093,8 +1062,11 @@ int rrt_capture_create(rrt_context* ctx, const rrt_params* prm, const rrt_camera
     }
 
     // the pass: rrt_render's tracer and grid, into a pool of this capture's own
-    const TracePlan tp = plan_trace(ctx, prm, w, local_rows);
-    c->ntiles = tp.ntiles;
+    const TracePlan& tp = c->plan;
+    if (int rc = plan_trace(ctx, *prm, w, local_rows, false, &c->plan)) {
+        free_capture(c);
+        return rc;
+    }
     size_t cap_slots = pool_slots(ctx->pool_bytes_max, (long long)npix, tp.grid, tp.rows_per_tile);
     if (max_bytes) cap_slots = std::min<size_t>(std::max<size_t>(max_bytes / kSlotBytes, 1024), 0xfff00000ull);
     const size_t work_cap = cap_slots / kMediaBatch + tp.ngroups + 64;   // as acquire_pool sizes it
@@ -1112,7 +1084,7 @@ int rrt_capture_create(rrt_context* ctx, const rrt_params* prm, const rrt_camera
     S.pc = pcs;
     S.redo_out = (unsigned*)(c->d_ctrl + kCapRedo);
     S.stats = (unsigned*)(c->d_ctrl + kCapStats);
-    tp.kernel<<<(unsigned)tp.grid, kRenderBlock, 0, st>>>(A, S, rrtk::LensArgs{});
+    tp.trace<<<(unsigned)tp.grid, kRenderBlock, 0, st>>>(A, S, rrtk::LensArgs{});
     CAP_CU(cudaGetLastError());
     ctx->launches += 1;
     CAP_CU(cudaMemcpyAsync(c->d_ctrl + kCapTicket + sizeof(unsigned), c->d_ctrl + kCapTicket, sizeof(unsigned), cudaMemcpyDeviceToDevice, st));
@@ -1179,30 +1151,31 @@ int rrt_capture_create(rrt_context* ctx, const rrt_params* prm, const rrt_camera
 static int check_capture_render(rrt_capture* cap, const char* what, const rrt_params* prm, const rrt_effects* fx, uint64_t sky_texture,
                                 void* d_out, int out_layout, float* hdr_out) {
     const std::string m = what;
-    if (!prm || !fx || sky_texture == 0 || (out_layout != RRT_OUT_FRAME && out_layout != RRT_OUT_PACKED) || (!d_out && !hdr_out))
-        return fail(cap->ctx, RRT_ERR_BAD_ARG, (m + ": bad argument").c_str());
+    if (!prm || !fx || sky_texture == 0 || !outputs_ok(out_layout, d_out, hdr_out))
+        return fail(cap->ctx, RRT_ERR_BAD_ARG, m + ": bad argument");
     if (((prm->flags ^ cap->prm.flags) & RRT_FLAG_FMAD) || fx->use_lens != cap->fx.use_lens ||
         std::memcmp(&fx->distortion_amount, &cap->fx.distortion_amount, sizeof(float)) != 0)
-        return fail(cap->ctx, RRT_ERR_BAD_ARG, (m + ": the RRT_FLAG_FMAD bit, use_lens and distortion_amount must be the capture's").c_str());
+        return fail(cap->ctx, RRT_ERR_BAD_ARG, m + ": the RRT_FLAG_FMAD bit, use_lens and distortion_amount must be the capture's");
     return RRT_OK;
 }
 
 // The kernels of one render of a capture at `time`, enqueued on `st`: shade, media, fold and, when the pass left tiles,
-// the sweep.  Arguments checked, ctx->mu held, `st` ordered after the capture's previous render.
+// the sweep.  Arguments checked, ctx->mu held, ctx->device current, `st` ordered after the capture's previous render.
 static int capture_enqueue(rrt_capture* cap, float exposure, const rrt_effects* fx, uint64_t sky_texture, float time, void* d_out,
                            int out_layout, float* hdr_out, cudaStream_t st) {
     rrt_context* ctx = cap->ctx;
     rrt_params P = cap->prm;
     P.exposure = exposure;
-    const bool fmad = (P.flags & RRT_FLAG_FMAD) != 0;
-    const rrtk::SplitKernels* sk = fmad ? rrtk::rrt_split_kernels_fmad() : rrtk::rrt_split_kernels_strict();
+    const rrtk::SplitKernels* sk = cap->plan.sk;
     FrameArgs A = frame_args(P, cap->cam, *fx, sky_texture, time, cap->w, cap->h, cap->band, cap->local_rows, out_layout, d_out);
     A.planes.hdr = hdr_out;
     A.counters = ctx->d_counters;
     A.ticket = (unsigned*)(cap->d_ctrl + kCapTicket);
     rrtk::PassCtrl* pcs = (rrtk::PassCtrl*)cap->d_ctrl;
     const int per_sm_media = resident_per_sm(ctx, (const void*)sk->media_results, kMediaBlock, true);
+    if (per_sm_media < 0) return per_sm_media;
     const int per_sm_fold = resident_per_sm(ctx, (const void*)sk->fold_results, 128, false);
+    if (per_sm_fold < 0) return per_sm_fold;
     // 1. every pixel from the planes; right for the rays the trace finished, overwritten below for the others
     const long long n = (long long)cap->w * cap->local_rows;
     kset(&P)->shade<<<(unsigned)((n + kShadeBlock - 1) / kShadeBlock), kShadeBlock, 0, st>>>(A, cap->planes);
@@ -1214,18 +1187,13 @@ static int capture_enqueue(rrt_capture* cap, float exposure, const rrt_effects* 
     int launches = 3;
     // 5. the tiles the pass could not hold, with the fused code: its redo list first, then the tickets it never took
     if (cap->tiles_left) {
-        const bool spin = P.spin_a != 0.0f;
-        auto k_sweep = sk->sweep[spin ? 1 : 0];
-        const int per_sm_sweep = resident_per_sm(ctx, (const void*)k_sweep, kRenderBlock, true);
         RRT_CU(ctx, cudaMemcpyAsync(A.ticket, A.ticket + 1, sizeof(unsigned), cudaMemcpyDeviceToDevice, st));
         RRT_CU(ctx, cudaMemsetAsync(&pcs[1], 0, sizeof(rrtk::PassCtrl), st));
         rrtk::SplitArgs S = cap->S;
         S.pass = 1;
         S.pc = pcs + 1;
         S.pc_prev = pcs;
-        long long grid_sweep = ((long long)ctx->sm_count * per_sm_sweep + ctx->frames_in_flight - 1) / ctx->frames_in_flight;
-        if (grid_sweep > (long long)cap->ntiles) grid_sweep = cap->ntiles;
-        k_sweep<<<(unsigned)grid_sweep, kRenderBlock, 0, st>>>(A, S, rrtk::LensArgs{});
+        if (int rc = launch_sweep(ctx, cap->plan, A, S, rrtk::LensArgs{}, st)) return rc;
         ++launches;
     }
     RRT_CU(ctx, cudaGetLastError());
@@ -1260,32 +1228,27 @@ int rrt_capture_render_mb(rrt_capture* cap, const rrt_params* prm, const rrt_eff
     rrt_context* ctx = cap->ctx;
     if (!times) return fail(ctx, RRT_ERR_BAD_ARG, "rrt_capture_render_mb: bad argument");
     if (int rc = check_capture_render(cap, "rrt_capture_render_mb", prm, fx, sky_texture, d_out, out_layout, hdr_out)) return rc;
+    rrt_band b;
     int local_rows = 0;
-    if (int rc = check_mb(ctx, "rrt_capture_render_mb", n, cap->w, cap->h, &cap->band, &local_rows)) return rc;
+    if (int rc = check_mb(ctx, "rrt_capture_render_mb", n, cap->w, cap->h, &cap->band, &b, &local_rows)) return rc;
     if (local_rows == 0) return RRT_OK;
 
     std::lock_guard<std::mutex> lk(ctx->mu);
     DevGuard g(ctx->device);
-    cudaStream_t st = (cudaStream_t)stream;
+    const cudaStream_t st = (cudaStream_t)stream;
     const size_t plane = (size_t)cap->w * cap->h;   // full-frame, like the capture's own planes
-    float* stack = nullptr;
-    if (int rc = scratch_alloc(ctx, "rrt_capture_render_mb: no memory for the sub-frame stack", 16 * n * plane, st, &stack)) return rc;
-    // the capture's state is in use from the first sub-frame to the last: wait for its previous render once, record once
-    int rc = RRT_OK;
-    if (cudaError_t e = cudaStreamWaitEvent(st, cap->done, 0)) {
-        rc = fail(ctx, RRT_ERR_CUDA, "rrt_capture_render_mb: cudaStreamWaitEvent", e);
-    } else {
+    return with_scratch(ctx, "rrt_capture_render_mb", "sub-frame stack", 16 * n * plane, st, [&](float* stack) {
+        // the capture's state is in use from the first sub-frame to the last: wait for its previous render once, record once
+        if (cudaError_t e = cudaStreamWaitEvent(st, cap->done, 0)) return fail(ctx, RRT_ERR_CUDA, "rrt_capture_render_mb: cudaStreamWaitEvent", e);
+        int rc = RRT_OK;
         for (int i = 0; i < n && rc == RRT_OK; ++i)
             rc = capture_enqueue(cap, prm->exposure, fx, sky_texture, times[i], nullptr, RRT_OUT_FRAME, stack + 4 * plane * i, st);
         // recorded even when a sub-frame failed: whatever was enqueued stays ordered before the capture's next render
-        const cudaError_t er = cudaEventRecord(cap->done, st);
-        if (rc == RRT_OK && er != cudaSuccess) rc = fail(ctx, RRT_ERR_CUDA, "rrt_capture_render_mb: cudaEventRecord", er);
-    }
-    if (rc == RRT_OK)
-        rc = launch_resolve(ctx, prm, fx, 1, n, cap->w, cap->h, &cap->band, local_rows, stack, plane, d_out, out_layout, hdr_out, st);
-    const cudaError_t e = cudaFreeAsync(stack, st);   // stream-ordered: the block goes back to the pool once the resolve has read it
-    if (rc == RRT_OK && e != cudaSuccess) return fail(ctx, RRT_ERR_CUDA, "rrt_capture_render_mb: cudaFreeAsync", e);
-    return rc;
+        const cudaError_t e = cudaEventRecord(cap->done, st);
+        if (rc != RRT_OK) return rc;
+        if (e != cudaSuccess) return fail(ctx, RRT_ERR_CUDA, "rrt_capture_render_mb: cudaEventRecord", e);
+        return launch_resolve(ctx, *prm, *fx, 1, n, cap->w, cap->h, b, local_rows, stack, plane, d_out, out_layout, hdr_out, st);
+    });
 }
 
 int rrt_capture_info(const rrt_capture* cap, uint64_t out[8]) {

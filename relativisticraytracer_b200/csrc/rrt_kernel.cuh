@@ -45,8 +45,9 @@ struct LensArgs {
 
 // kernels of one rounding contract
 struct KernelSet {
-    void (*render[2][2])(const FrameArgs, const LensArgs);  // [spin != 0][media]
-    void (*render_packed[2])(const FrameArgs, const LensArgs);  // [spin != 0]; two rays per thread in f32x2 registers, no medium (rrt_packed.cuh); FMAD contract only
+    // [lens][spin != 0][media]; lens: the LENS variant (rrt_render_dof), every ray from its own camera of LensArgs::cams
+    void (*render[2][2][2])(const FrameArgs, const LensArgs);
+    void (*render_packed[2][2])(const FrameArgs, const LensArgs);  // [lens][spin != 0]; two rays per thread in f32x2 registers, no medium (rrt_packed.cuh); FMAD contract only
     void (*acc)(Consts, int, const float*, const float*, float*);
     void (*rk4)(Consts, int, float*, float*, const float*);
     void (*euler)(Consts, int, float*, float*, const float*);
@@ -60,9 +61,6 @@ struct KernelSet {
     void (*shade)(const FrameArgs, const rrt_planes);  // rrt_shade: the step after the ray loop, from traced planes
     // rrt_resolve / rrt_resolve_time: mean of ss x ss blocks of n hdr planes + post step
     void (*resolve)(const FrameArgs, const float4*, int, int, size_t);
-    // the LENS variants of render / render_packed (rrt_render_dof): every ray from its own camera of LensArgs::cams
-    void (*render_lens[2][2])(const FrameArgs, const LensArgs);
-    void (*render_packed_lens[2])(const FrameArgs, const LensArgs);
 };
 const KernelSet* rrt_kernels_strict();
 const KernelSet* rrt_kernels_fmad();
@@ -157,6 +155,18 @@ __device__ __forceinline__ MediaOut media_sample(const Consts& C, V3 q, V3 v, fl
     const float dd = (zones & 1u) ? rrt::disk_density(C, q, time) : 0.0f;                 // :68
     const float dc = (zones & 2u) ? rrt::dust_density(C, q, time) : 0.0f;                 // :69
     return media_final(C, q, v, r, h, dd, dc);
+}
+
+// Image row of row ly of the band (groups of band_group rows dealt round-robin to the band's ranks).
+__device__ __forceinline__ int band_row(const FrameArgs& A, int ly) {
+    const int grp = ly / A.band_group;
+    return (grp * A.band_nranks + A.band_rank) * A.band_group + (ly - grp * A.band_group);
+}
+// Tile row of the k-th of nty tile rows, handed out from the image centre outwards.
+__device__ __forceinline__ int centre_out_row(int k, int nty) {
+    const int c = nty >> 1, m = min(c, nty - 1 - c);
+    if (k <= 2 * m) return (k & 1) ? c + ((k + 1) >> 1) : c - (k >> 1);
+    return (c > nty - 1 - c) ? (c - m - 1) - (k - (2 * m + 1)) : (c + m + 1) + (k - (2 * m + 1));
 }
 
 // image-plane coordinate of a pixel after the optional lens distortion (reference :20-25)
@@ -500,15 +510,11 @@ __global__ void __launch_bounds__(kRenderBlock, MEDIA ? (LENS ? kMinBlocksMediaL
         // Tile rows are handed out from the image centre outwards: the rows that cross the hole and the
         // disk are the expensive ones, so they start first and the cheap sky rows fill the tail of the launch.
         const int tx = (int)(tile % (unsigned)ntx), k = (int)(tile / (unsigned)ntx);
-        const int c = nty >> 1, m = min(c, nty - 1 - c);
-        int ty;
-        if (k <= 2 * m) ty = (k & 1) ? c + ((k + 1) >> 1) : c - (k >> 1);
-        else ty = (c > nty - 1 - c) ? (c - m - 1) - (k - (2 * m + 1)) : (c + m + 1) + (k - (2 * m + 1));
+        const int ty = centre_out_row(k, nty);
         const int x = tx * kRTileW + (lane & (kRTileW - 1));
         const int ly = ty * kRTileH + lane / kRTileW;
         if (x >= A.w || ly >= A.local_rows) continue;
-        const int grp = ly / A.band_group;
-        const int y = (grp * A.band_nranks + A.band_rank) * A.band_group + (ly - grp * A.band_group);
+        const int y = band_row(A, ly);
         if (y >= A.h) continue;
 
 #ifdef RRT_WITH_TILE_LOG
@@ -575,8 +581,7 @@ __global__ void __launch_bounds__(kShadeBlock) shade_kernel(const __grid_constan
     const int i = blockIdx.x * kShadeBlock + threadIdx.x;   // w * local_rows <= 2^30 (rrt_shade)
     if (i >= A.w * A.local_rows) return;
     const int ly = i / A.w, x = i - ly * A.w;
-    const int grp = ly / A.band_group;
-    const int y = (grp * A.band_nranks + A.band_rank) * A.band_group + (ly - grp * A.band_group);
+    const int y = band_row(A, ly);
     if (y >= A.h) return;
     const size_t pix = (size_t)y * A.w + x;
     const float4 v = reinterpret_cast<const float4*>(traced.vel)[pix];
@@ -607,8 +612,7 @@ __global__ void __launch_bounds__(kResolveBlock) resolve_kernel(const __grid_con
     const int i = blockIdx.x * kResolveBlock + threadIdx.x;   // w * local_rows <= 2^30 (rrt_resolve, rrt_resolve_time)
     if (i >= A.w * A.local_rows) return;
     const int ly = i / A.w, x = i - ly * A.w;
-    const int grp = ly / A.band_group;
-    const int y = (grp * A.band_nranks + A.band_rank) * A.band_group + (ly - grp * A.band_group);
+    const int y = band_row(A, ly);
     if (y >= A.h) return;
     const size_t W = (size_t)ss * A.w;
     const float4* p = hi + (size_t)ss * y * W + (size_t)ss * x;
@@ -698,20 +702,15 @@ __global__ void k_sky(cudaTextureObject_t sky, int n, const float* tx, const flo
 #include "rrt_split.cuh"   // trace / media / fold kernels of the split pipeline (both contracts)
 namespace {
 const rrtk::KernelSet kKernelSet = {
-    {{render_kernel<false, false, false>, render_kernel<false, true, false>}, {render_kernel<true, false, false>, render_kernel<true, true, false>}},
+    {{{render_kernel<false, false, false>, render_kernel<false, true, false>}, {render_kernel<true, false, false>, render_kernel<true, true, false>}},
+     {{render_kernel<false, false, true>, render_kernel<false, true, true>}, {render_kernel<true, false, true>, render_kernel<true, true, true>}}},
 #if RRT_FMAD
-    {render_kernel_p<false, false>, render_kernel_p<true, false>},
+    {{render_kernel_p<false, false>, render_kernel_p<true, false>}, {render_kernel_p<false, true>, render_kernel_p<true, true>}},
 #else
-    {nullptr, nullptr},
+    {{nullptr, nullptr}, {nullptr, nullptr}},
 #endif
     k_acc, k_rk4, k_euler, k_redshift, k_hash31, k_noise3d, k_fbm, k_disk_temp, k_disk_density, k_dust_density,
     shade_kernel, resolve_kernel,
-    {{render_kernel<false, false, true>, render_kernel<false, true, true>}, {render_kernel<true, false, true>, render_kernel<true, true, true>}},
-#if RRT_FMAD
-    {render_kernel_p<false, true>, render_kernel_p<true, true>},
-#else
-    {nullptr, nullptr},
-#endif
 };
 }  // namespace
 

@@ -87,19 +87,16 @@ struct SplitArgs {
     unsigned tile16;          // tickets and redo lists count 16x4 tiles (the packed tracer) instead of 8x4 tiles
     uint4* results;           // media_kernel<true> / fold_kernel<true>: {e.rgb, s} per slot, indexed like `slots` (rrt_capture)
 };
+// The tracers are indexed [lens][spin != 0]; lens: the LENS variant (rrt_render_dof), every ray from its own camera of
+// LensArgs::cams.  Media and fold read only samples and planes and serve both.
 struct SplitKernels {
-    void (*trace[2])(const FrameArgs, const SplitArgs, const LensArgs);   // [spin != 0]
-    void (*trace_packed[2])(const FrameArgs, const SplitArgs, const LensArgs);   // two rays per thread (FMAD contract only, else null)
+    void (*trace[2][2])(const FrameArgs, const SplitArgs, const LensArgs);
+    void (*trace_packed[2][2])(const FrameArgs, const SplitArgs, const LensArgs);   // two rays per thread (FMAD contract only, else null)
     void (*media)(const FrameArgs, const SplitArgs);
     void (*fold)(const FrameArgs, const SplitArgs);
-    void (*sweep[2])(const FrameArgs, const SplitArgs, const LensArgs);
+    void (*sweep[2][2])(const FrameArgs, const SplitArgs, const LensArgs);
     void (*media_results)(const FrameArgs, const SplitArgs);   // media_kernel<true>: the samples stay, results go to S.results
     void (*fold_results)(const FrameArgs, const SplitArgs);    // fold_kernel<true>: reads them from there
-    // the LENS variants of the tracers (rrt_render_dof): every ray from its own camera of LensArgs::cams; media and fold
-    // read only samples and planes and serve both
-    void (*trace_lens[2])(const FrameArgs, const SplitArgs, const LensArgs);
-    void (*trace_packed_lens[2])(const FrameArgs, const SplitArgs, const LensArgs);
-    void (*sweep_lens[2])(const FrameArgs, const SplitArgs, const LensArgs);
 };
 const SplitKernels* rrt_split_kernels_strict();
 const SplitKernels* rrt_split_kernels_fmad();
@@ -126,15 +123,11 @@ __device__ __forceinline__ TilePix tile_pixel(const FrameArgs& A, unsigned tile,
     const int ntx = (A.w + kRTileW - 1) / kRTileW;
     const int nty = (A.local_rows + kRTileH - 1) / kRTileH;
     const int tx = (int)(tile % (unsigned)ntx), k = (int)(tile / (unsigned)ntx);
-    const int c = nty >> 1, m = min(c, nty - 1 - c);
-    int ty;
-    if (k <= 2 * m) ty = (k & 1) ? c + ((k + 1) >> 1) : c - (k >> 1);
-    else ty = (c > nty - 1 - c) ? (c - m - 1) - (k - (2 * m + 1)) : (c + m + 1) + (k - (2 * m + 1));
+    const int ty = centre_out_row(k, nty);
     TilePix t;
     t.x = tx * kRTileW + (lane & (kRTileW - 1));
     t.ly = ty * kRTileH + lane / kRTileW;
-    const int grp = t.ly / A.band_group;
-    t.y = (grp * A.band_nranks + A.band_rank) * A.band_group + (t.ly - grp * A.band_group);
+    t.y = band_row(A, t.ly);
     t.valid = t.x < A.w && t.ly < A.local_rows && t.y < A.h;
     return t;
 }
@@ -148,15 +141,11 @@ __device__ __forceinline__ TilePix tile_pixel16(const FrameArgs& A, unsigned til
     const int ntx = (A.w + kTile16W - 1) / kTile16W;
     const int nty = (A.local_rows + kTile16H - 1) / kTile16H;
     const int tx = (int)(tile % (unsigned)ntx), k = (int)(tile / (unsigned)ntx);
-    const int c = nty >> 1, m = min(c, nty - 1 - c);
-    int ty;
-    if (k <= 2 * m) ty = (k & 1) ? c + ((k + 1) >> 1) : c - (k >> 1);
-    else ty = (c > nty - 1 - c) ? (c - m - 1) - (k - (2 * m + 1)) : (c + m + 1) + (k - (2 * m + 1));
+    const int ty = centre_out_row(k, nty);
     TilePix t;
     t.x = tx * kTile16W + 2 * (lane & 7) + hf;
     t.ly = ty * kTile16H + (lane >> 3);
-    const int grp = t.ly / A.band_group;
-    t.y = (grp * A.band_nranks + A.band_rank) * A.band_group + (t.ly - grp * A.band_group);
+    t.y = band_row(A, t.ly);
     t.valid = t.x < A.w && t.ly < A.local_rows && t.y < A.h;
     return t;
 }
@@ -976,21 +965,15 @@ __global__ void __launch_bounds__(kRenderBlock, LENS ? kMinBlocksMediaLens : kMi
 }
 
 const rrtk::SplitKernels kSplitKernels = {
-    {trace_kernel<false, false>, trace_kernel<true, false>},
+    {{trace_kernel<false, false>, trace_kernel<true, false>}, {trace_kernel<false, true>, trace_kernel<true, true>}},
 #if RRT_FMAD
-    {trace_kernel_p<false, false>, trace_kernel_p<true, false>},
+    {{trace_kernel_p<false, false>, trace_kernel_p<true, false>}, {trace_kernel_p<false, true>, trace_kernel_p<true, true>}},
 #else
-    {nullptr, nullptr},
+    {{nullptr, nullptr}, {nullptr, nullptr}},
 #endif
-    media_kernel<false>, fold_kernel<false>, {sweep_kernel<false, false>, sweep_kernel<true, false>},
+    media_kernel<false>, fold_kernel<false>,
+    {{sweep_kernel<false, false>, sweep_kernel<true, false>}, {sweep_kernel<false, true>, sweep_kernel<true, true>}},
     media_kernel<true>, fold_kernel<true>,
-    {trace_kernel<false, true>, trace_kernel<true, true>},
-#if RRT_FMAD
-    {trace_kernel_p<false, true>, trace_kernel_p<true, true>},
-#else
-    {nullptr, nullptr},
-#endif
-    {sweep_kernel<false, true>, sweep_kernel<true, true>},
 };
 }  // namespace
 

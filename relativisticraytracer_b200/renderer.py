@@ -84,6 +84,16 @@ def _f32_array(values) -> C.Array:
     return (C.c_float * len(values))(*values)
 
 
+def _tex(sky: "Sky | int") -> C.c_uint64:
+    """The cudaTextureObject_t of a Sky, or a raw texture object as it is."""
+    return C.c_uint64(sky.texture if isinstance(sky, Sky) else int(sky))
+
+
+def _band_ref(band: Optional[Band]):
+    """The rrt_band* of an optional band: NULL renders the whole frame."""
+    return C.byref(band) if band is not None else None
+
+
 class Sky:
     """A skybox texture object (rrt_sky) -- the device half of the reference's loadSkybox."""
 
@@ -119,25 +129,20 @@ class Capture:
 
     def __init__(self, renderer: "Renderer", prm: Params, cam: Camera, fx: Effects, sky: "Sky | int", w: int, h: int, *,
                  band: Optional[Band] = None, max_bytes: int = 0, stream: Optional[torch.cuda.Stream] = None):
-        tex = sky.texture if isinstance(sky, Sky) else int(sky)
         self._r, self.w, self.h, self.band = renderer, int(w), int(h), band
         self._h = C.c_void_p()
-        st = stream if stream is not None else torch.cuda.current_stream(renderer.device)
-        renderer._check(renderer._lib.rrt_capture_create(renderer._ctx, C.byref(prm), C.byref(cam), C.byref(fx), C.c_uint64(tex),
-                                                         self.w, self.h, C.byref(band) if band is not None else None,
-                                                         C.c_size_t(int(max_bytes)), C.c_void_p(st.cuda_stream), C.byref(self._h)))
+        renderer._check(renderer._lib.rrt_capture_create(renderer._ctx, C.byref(prm), C.byref(cam), C.byref(fx), _tex(sky),
+                                                         self.w, self.h, _band_ref(band), C.c_size_t(int(max_bytes)),
+                                                         renderer._stream(stream), C.byref(self._h)))
 
     def render(self, prm: Params, fx: Effects, sky: "Sky | int", time: float, *, out=None, layout: int = OUT_FRAME,
                hdr_out: Optional[torch.Tensor] = None, stream: Optional[torch.cuda.Stream] = None) -> torch.Tensor:
         """rrt_capture_render: the captured frame (or band) at ``time``; asynchronous.  ``out`` (a tensor or a PeerFrame),
         ``layout`` and ``hdr_out`` ((h, w, 4) float32) as in ``Renderer.render`` / ``Renderer.shade``; returns the frame."""
         r = self._r
-        tex = sky.texture if isinstance(sky, Sky) else int(sky)
         out, out_ptr = r._frame_out(out, layout, self.band, self.w, self.h)
-        hdr_ptr = r._plane_ptr("hdr", hdr_out, self.w, self.h) if hdr_out is not None else None
-        st = stream if stream is not None else torch.cuda.current_stream(r.device)
-        r._check(r._lib.rrt_capture_render(self._h, C.byref(prm), C.byref(fx), C.c_uint64(tex), float(time), C.c_void_p(out_ptr),
-                                           int(layout), C.c_void_p(hdr_ptr), C.c_void_p(st.cuda_stream)))
+        r._check(r._lib.rrt_capture_render(self._h, C.byref(prm), C.byref(fx), _tex(sky), float(time), C.c_void_p(out_ptr),
+                                           int(layout), r._hdr_ptr(hdr_out, self.w, self.h), r._stream(stream)))
         return out
 
     def render_mb(self, prm: Params, fx: Effects, sky: "Sky | int", times, *, out=None, layout: int = OUT_FRAME,
@@ -146,13 +151,10 @@ class Capture:
         asynchronous.  Gives the bytes of ``Renderer.render_mb`` with the capture's camera for every sub-frame, under the
         rules of ``render``.  ``out``, ``layout`` and ``hdr_out`` (the mean) as in ``render``; returns the frame."""
         r = self._r
-        tex = sky.texture if isinstance(sky, Sky) else int(sky)
         ts = _f32_array(times)
         out, out_ptr = r._frame_out(out, layout, self.band, self.w, self.h)
-        hdr_ptr = r._plane_ptr("hdr", hdr_out, self.w, self.h) if hdr_out is not None else None
-        st = stream if stream is not None else torch.cuda.current_stream(r.device)
-        r._check(r._lib.rrt_capture_render_mb(self._h, C.byref(prm), C.byref(fx), C.c_uint64(tex), ts, len(ts), C.c_void_p(out_ptr),
-                                              int(layout), C.c_void_p(hdr_ptr), C.c_void_p(st.cuda_stream)))
+        r._check(r._lib.rrt_capture_render_mb(self._h, C.byref(prm), C.byref(fx), _tex(sky), ts, len(ts), C.c_void_p(out_ptr),
+                                              int(layout), r._hdr_ptr(hdr_out, self.w, self.h), r._stream(stream)))
         return out
 
     def info(self) -> dict:
@@ -203,9 +205,8 @@ class PeerFrame:
     def read_into(self, dst: torch.Tensor, stream: Optional[torch.cuda.Stream] = None) -> None:
         """Stream-ordered copy of the frame into `dst` (pinned host or device uint8 tensor of the frame's size)."""
         assert dst.dtype == torch.uint8 and dst.is_contiguous() and dst.numel() == self.nbytes
-        st = stream if stream is not None else torch.cuda.current_stream(self.r.device)
         self.r._check(self.r._lib.rrt_peer_frame_read(self.r._ctx, C.c_void_p(self.ptr), C.c_size_t(self.nbytes),
-                                                      C.c_void_p(dst.data_ptr()), C.c_void_p(st.cuda_stream)))
+                                                      C.c_void_p(dst.data_ptr()), self.r._stream(stream)))
 
     def close(self):
         if self.ptr:
@@ -232,6 +233,10 @@ class Renderer:
         if rc != 0:
             raise RrtError(rc, (self._lib.rrt_last_error(self._ctx) or b"").decode())
 
+    def _stream(self, stream: Optional[torch.cuda.Stream]) -> C.c_void_p:
+        """The cudaStream_t of `stream`, by default the current stream of this renderer's device."""
+        return C.c_void_p((stream if stream is not None else torch.cuda.current_stream(self.device)).cuda_stream)
+
     def close(self):
         if self._ctx:
             self._lib.rrt_context_destroy(self._ctx)
@@ -248,7 +253,7 @@ class Renderer:
 
     @staticmethod
     def band_rows(band: Optional[Band], h: int) -> int:
-        return int(_capi.load().rrt_band_rows(C.byref(band) if band is not None else None, int(h)))
+        return int(_capi.load().rrt_band_rows(_band_ref(band), int(h)))
 
     def alloc_planes(self, w: int, h: int, names=("hdr", "dir", "emis", "pos", "vel", "cls", "steps")):
         out = {}
@@ -263,14 +268,11 @@ class Renderer:
                band: Optional[Band] = None, out: Optional[torch.Tensor] = None, layout: int = OUT_FRAME,
                planes: Optional[dict] = None, stream: Optional[torch.cuda.Stream] = None) -> torch.Tensor:
         """rrt_render: one frame (or one band of it) into a device uchar4 tensor; asynchronous."""
-        tex = sky.texture if isinstance(sky, Sky) else int(sky)
         out, out_ptr = self._frame_out(out, layout, band, w, h)
         pl = self._planes(planes, w, h) if planes else None
-        st = stream if stream is not None else torch.cuda.current_stream(self.device)
-        self._check(self._lib.rrt_render(self._ctx, C.byref(prm), C.byref(cam), C.byref(fx), C.c_uint64(tex),
-                                         float(time), int(w), int(h), C.byref(band) if band is not None else None,
-                                         C.c_void_p(out_ptr), int(layout),
-                                         C.byref(pl) if pl is not None else None, C.c_void_p(st.cuda_stream)))
+        self._check(self._lib.rrt_render(self._ctx, C.byref(prm), C.byref(cam), C.byref(fx), _tex(sky),
+                                         float(time), int(w), int(h), _band_ref(band), C.c_void_p(out_ptr), int(layout),
+                                         C.byref(pl) if pl is not None else None, self._stream(stream)))
         return out
 
     def shade(self, prm: Params, fx: Effects, sky: Sky | int, traced: dict, w: int, h: int, *, band: Optional[Band] = None,
@@ -281,14 +283,11 @@ class Renderer:
         asynchronous.  Gives the bytes (and ``hdr_out`` values) of a fresh render with this sky, exposure and bloom /
         vignette / CA settings; ``prm`` must keep the trace's FLAG_FMAD bit and ``fx`` its lens fields.  ``band``,
         ``out`` (a tensor or a PeerFrame) and ``layout`` as in ``render``; returns the frame."""
-        tex = sky.texture if isinstance(sky, Sky) else int(sky)
         out, out_ptr = self._frame_out(out, layout, band, w, h)
         pl = self._planes(traced, w, h)
-        hdr_ptr = self._plane_ptr("hdr", hdr_out, w, h) if hdr_out is not None else None
-        st = stream if stream is not None else torch.cuda.current_stream(self.device)
-        self._check(self._lib.rrt_shade(self._ctx, C.byref(prm), C.byref(fx), C.c_uint64(tex), int(w), int(h),
-                                        C.byref(band) if band is not None else None, C.byref(pl), C.c_void_p(out_ptr),
-                                        int(layout), C.c_void_p(hdr_ptr), C.c_void_p(st.cuda_stream)))
+        self._check(self._lib.rrt_shade(self._ctx, C.byref(prm), C.byref(fx), _tex(sky), int(w), int(h), _band_ref(band),
+                                        C.byref(pl), C.c_void_p(out_ptr), int(layout), self._hdr_ptr(hdr_out, w, h),
+                                        self._stream(stream)))
         return out
 
     def render_ss(self, prm: Params, cam: Camera, fx: Effects, sky: Sky | int, time: float, w: int, h: int, ss: int, *,
@@ -298,13 +297,10 @@ class Renderer:
         Pixel (x, y) is the box-filtered mean of pixels (ss*x + i, ss*y + j) of the ss*w x ss*h render, then the render's
         own bloom / vignette / tonemap; ss = 1 is ``render``.  ``hdr_out`` (h, w, 4) float32 receives the averaged linear
         value (.w = mean T).  ``band``, ``out`` (a tensor or a PeerFrame) and ``layout`` as in ``render``."""
-        tex = sky.texture if isinstance(sky, Sky) else int(sky)
         out, out_ptr = self._frame_out(out, layout, band, w, h)
-        hdr_ptr = self._plane_ptr("hdr", hdr_out, w, h) if hdr_out is not None else None
-        st = stream if stream is not None else torch.cuda.current_stream(self.device)
-        self._check(self._lib.rrt_render_ss(self._ctx, C.byref(prm), C.byref(cam), C.byref(fx), C.c_uint64(tex), float(time),
-                                            int(w), int(h), int(ss), C.byref(band) if band is not None else None,
-                                            C.c_void_p(out_ptr), int(layout), C.c_void_p(hdr_ptr), C.c_void_p(st.cuda_stream)))
+        self._check(self._lib.rrt_render_ss(self._ctx, C.byref(prm), C.byref(cam), C.byref(fx), _tex(sky), float(time),
+                                            int(w), int(h), int(ss), _band_ref(band), C.c_void_p(out_ptr), int(layout),
+                                            self._hdr_ptr(hdr_out, w, h), self._stream(stream)))
         return out
 
     def render_dof(self, prm: Params, cams, fx: Effects, sky: Sky | int, time: float, w: int, h: int, ss: int, *,
@@ -314,17 +310,14 @@ class Renderer:
         asynchronous.  ``cams`` is a sequence of ss*ss cameras (``lens_cameras`` gives a thin lens): sub-sample (i, j) of
         pixel (x, y) is pixel (ss*x + i, ss*y + j) of the ss*w x ss*h ``render`` with ``cams[j*ss + i]``.  All cameras equal
         is ``render_ss``; ss = 1 is ``render(cams[0])``.  ``hdr_out``, ``band``, ``out`` and ``layout`` as in ``render_ss``."""
-        tex = sky.texture if isinstance(sky, Sky) else int(sky)
         cams = list(cams)
         if len(cams) != int(ss) * int(ss):
             raise ValueError(f"render_dof: {len(cams)} cameras for ss = {ss} (ss*ss needed)")
         cam_arr = (Camera * max(len(cams), 1))(*cams)
         out, out_ptr = self._frame_out(out, layout, band, w, h)
-        hdr_ptr = self._plane_ptr("hdr", hdr_out, w, h) if hdr_out is not None else None
-        st = stream if stream is not None else torch.cuda.current_stream(self.device)
-        self._check(self._lib.rrt_render_dof(self._ctx, C.byref(prm), cam_arr, C.byref(fx), C.c_uint64(tex), float(time),
-                                             int(w), int(h), int(ss), C.byref(band) if band is not None else None,
-                                             C.c_void_p(out_ptr), int(layout), C.c_void_p(hdr_ptr), C.c_void_p(st.cuda_stream)))
+        self._check(self._lib.rrt_render_dof(self._ctx, C.byref(prm), cam_arr, C.byref(fx), _tex(sky), float(time),
+                                             int(w), int(h), int(ss), _band_ref(band), C.c_void_p(out_ptr), int(layout),
+                                             self._hdr_ptr(hdr_out, w, h), self._stream(stream)))
         return out
 
     def resolve(self, prm: Params, fx: Effects, hdr_hi: torch.Tensor, ss: int, w: int, h: int, *, band: Optional[Band] = None,
@@ -337,11 +330,9 @@ class Renderer:
         out, out_ptr = self._frame_out(out, layout, band, w, h)
         assert tuple(hdr_hi.shape) == (ss * h, ss * w, 4), "hdr_hi must be (ss*h, ss*w, 4)"
         hi_ptr = self._plane_ptr("hdr", hdr_hi, ss * w, ss * h)
-        hdr_ptr = self._plane_ptr("hdr", hdr_out, w, h) if hdr_out is not None else None
-        st = stream if stream is not None else torch.cuda.current_stream(self.device)
-        self._check(self._lib.rrt_resolve(self._ctx, C.byref(prm), C.byref(fx), int(ss), int(w), int(h),
-                                          C.byref(band) if band is not None else None, C.c_void_p(hi_ptr),
-                                          C.c_void_p(out_ptr), int(layout), C.c_void_p(hdr_ptr), C.c_void_p(st.cuda_stream)))
+        self._check(self._lib.rrt_resolve(self._ctx, C.byref(prm), C.byref(fx), int(ss), int(w), int(h), _band_ref(band),
+                                          C.c_void_p(hi_ptr), C.c_void_p(out_ptr), int(layout), self._hdr_ptr(hdr_out, w, h),
+                                          self._stream(stream)))
         return out
 
     def resolve_time(self, prm: Params, fx: Effects, hdr_stack: torch.Tensor, w: int, h: int, *, band: Optional[Band] = None,
@@ -355,11 +346,9 @@ class Renderer:
         assert hdr_stack.dim() == 4 and tuple(hdr_stack.shape[1:]) == (h, w, 4), "hdr_stack must be (n, h, w, 4)"
         n = int(hdr_stack.shape[0])
         stack_ptr = self._plane_ptr("hdr", hdr_stack, w, n * h)
-        hdr_ptr = self._plane_ptr("hdr", hdr_out, w, h) if hdr_out is not None else None
-        st = stream if stream is not None else torch.cuda.current_stream(self.device)
-        self._check(self._lib.rrt_resolve_time(self._ctx, C.byref(prm), C.byref(fx), n, int(w), int(h),
-                                               C.byref(band) if band is not None else None, C.c_void_p(stack_ptr),
-                                               C.c_void_p(out_ptr), int(layout), C.c_void_p(hdr_ptr), C.c_void_p(st.cuda_stream)))
+        self._check(self._lib.rrt_resolve_time(self._ctx, C.byref(prm), C.byref(fx), n, int(w), int(h), _band_ref(band),
+                                               C.c_void_p(stack_ptr), C.c_void_p(out_ptr), int(layout),
+                                               self._hdr_ptr(hdr_out, w, h), self._stream(stream)))
         return out
 
     def render_mb(self, prm: Params, cam, fx: Effects, sky: Sky | int, times, w: int, h: int, *, band: Optional[Band] = None,
@@ -370,18 +359,15 @@ class Renderer:
         ``cam`` (one Camera for every sub-frame) or ``cam[i]`` (a sequence of n); n = 1 is ``render``.  ``hdr_out``
         (h, w, 4) float32 receives the mean (.w = mean T).  ``band``, ``out`` (a tensor or a PeerFrame) and ``layout`` as
         in ``render``."""
-        tex = sky.texture if isinstance(sky, Sky) else int(sky)
         ts = _f32_array(times)
         cams = [cam] * len(ts) if isinstance(cam, Camera) else list(cam)
         if len(cams) != len(ts):
             raise ValueError(f"render_mb: {len(cams)} cameras for {len(ts)} times")
         cam_arr = (Camera * max(len(cams), 1))(*cams)
         out, out_ptr = self._frame_out(out, layout, band, w, h)
-        hdr_ptr = self._plane_ptr("hdr", hdr_out, w, h) if hdr_out is not None else None
-        st = stream if stream is not None else torch.cuda.current_stream(self.device)
-        self._check(self._lib.rrt_render_mb(self._ctx, C.byref(prm), cam_arr, C.byref(fx), C.c_uint64(tex), ts, len(ts),
-                                            int(w), int(h), C.byref(band) if band is not None else None,
-                                            C.c_void_p(out_ptr), int(layout), C.c_void_p(hdr_ptr), C.c_void_p(st.cuda_stream)))
+        self._check(self._lib.rrt_render_mb(self._ctx, C.byref(prm), cam_arr, C.byref(fx), _tex(sky), ts, len(ts),
+                                            int(w), int(h), _band_ref(band), C.c_void_p(out_ptr), int(layout),
+                                            self._hdr_ptr(hdr_out, w, h), self._stream(stream)))
         return out
 
     def capture(self, prm: Params, cam: Camera, fx: Effects, sky: Sky | int, w: int, h: int, *, band: Optional[Band] = None,
@@ -409,6 +395,11 @@ class Renderer:
         return t.data_ptr()
 
     @classmethod
+    def _hdr_ptr(cls, hdr_out: Optional[torch.Tensor], w: int, h: int) -> C.c_void_p:
+        """The float* of an optional (h, w, 4) float32 hdr destination (NULL: none)."""
+        return C.c_void_p(cls._plane_ptr("hdr", hdr_out, w, h) if hdr_out is not None else None)
+
+    @classmethod
     def _planes(cls, planes: dict, w: int, h: int) -> Planes:
         pl = Planes()
         for n, t in planes.items():
@@ -418,36 +409,32 @@ class Renderer:
     def render_host(self, prm: Params, cam: Camera, fx: Effects, sky: Sky | int, time: float, w: int, h: int,
                     host_out) -> None:
         """rrt_render_host: end-to-end call, HOST destination (numpy array or pinned torch tensor)."""
-        tex = sky.texture if isinstance(sky, Sky) else int(sky)
         if isinstance(host_out, torch.Tensor):
             assert not host_out.is_cuda and host_out.is_contiguous() and host_out.numel() * host_out.element_size() >= w * h * 4
             ptr = host_out.data_ptr()
         else:
             assert host_out.flags["C_CONTIGUOUS"] and host_out.nbytes >= w * h * 4
             ptr = host_out.ctypes.data
-        self._check(self._lib.rrt_render_host(self._ctx, C.byref(prm), C.byref(cam), C.byref(fx), C.c_uint64(tex),
+        self._check(self._lib.rrt_render_host(self._ctx, C.byref(prm), C.byref(cam), C.byref(fx), _tex(sky),
                                               float(time), int(w), int(h), C.c_void_p(ptr)))
 
     def render_host_async(self, prm: Params, cam: Camera, fx: Effects, sky: Sky | int, time: float, w: int, h: int,
                           host_out: torch.Tensor, slot: int = 0, stream: Optional[torch.cuda.Stream] = None) -> None:
         """rrt_render_host_async: trace + device->host copy enqueued on `stream`, no synchronisation.
         ``host_out`` must be a pinned CPU tensor; ``slot`` < HOST_SLOTS selects the context's device frame."""
-        tex = sky.texture if isinstance(sky, Sky) else int(sky)
         assert (not host_out.is_cuda) and host_out.is_pinned() and host_out.is_contiguous()
         assert host_out.numel() * host_out.element_size() >= w * h * 4
-        st = stream if stream is not None else torch.cuda.current_stream(self.device)
-        self._check(self._lib.rrt_render_host_async(self._ctx, C.byref(prm), C.byref(cam), C.byref(fx), C.c_uint64(tex),
+        self._check(self._lib.rrt_render_host_async(self._ctx, C.byref(prm), C.byref(cam), C.byref(fx), _tex(sky),
                                                     float(time), int(w), int(h), C.c_void_p(host_out.data_ptr()),
-                                                    int(slot), C.c_void_p(st.cuda_stream)))
+                                                    int(slot), self._stream(stream)))
 
     def assemble_bands(self, packed: torch.Tensor, rows_per_rank: int, w: int, h: int, nranks: int, group: int,
                        frame: Optional[torch.Tensor] = None, stream: Optional[torch.cuda.Stream] = None) -> torch.Tensor:
         if frame is None:
             frame = torch.empty((h, w, 4), dtype=torch.uint8, device=self.device)
-        st = stream if stream is not None else torch.cuda.current_stream(self.device)
         self._check(self._lib.rrt_assemble_bands(self._ctx, C.c_void_p(packed.data_ptr()), int(rows_per_rank), int(w),
                                                  int(h), int(nranks), int(group), C.c_void_p(frame.data_ptr()),
-                                                 C.c_void_p(st.cuda_stream)))
+                                                 self._stream(stream)))
         return frame
 
     def read_counters(self, reset: bool = True) -> dict:
@@ -580,10 +567,9 @@ class Renderer:
         return out
 
     def sky_sample(self, sky: Sky | int, tx, ty):
-        tex = sky.texture if isinstance(sky, Sky) else int(sky)
         tx, ty = self._f32(tx), self._f32(ty)
         out = np.empty((len(tx), 4), np.float32)
-        self._check(self._lib.rrt_sky_sample_batch(self._ctx, C.c_uint64(tex), len(tx), self._p(tx), self._p(ty), self._p(out)))
+        self._check(self._lib.rrt_sky_sample_batch(self._ctx, _tex(sky), len(tx), self._p(tx), self._p(ty), self._p(out)))
         return out
 
 
