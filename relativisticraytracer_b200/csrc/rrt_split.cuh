@@ -458,12 +458,17 @@ __global__ void __launch_bounds__(32, kPackedMinBlocks) trace_kernel_p(const __g
     // the warp sits well inside SOME zone (each its own: vacuum counts), kBurst steps are taken with each ray's zone step
     // and none of the per-step zone logic; each step still stores its media sample (the zone flags of a sample do not
     // influence the trajectory).  Afterwards the burst is validated -- every pre-step state of a ray must have been in the
-    // zone its step came from, above the horizon, short of the escape sphere and in the branch-free domain -- and rolled
-    // back otherwise (the samples it stored are overwritten).
+    // zone its step came from, at or above the horizon radius (:47), and every pre-step and stage radius at or above
+    // redo_below (the branch-free domain); in the disk zone also at most 250 (the escape test, :120, which the near-hole
+    // zone's r < 18 already rules out) -- and rolled back otherwise (the samples it stored are overwritten).  None of these
+    // thresholds is ordered against 18 or 250 in general (a hole with event_horizon > 17.8 puts the horizon inside the disk
+    // zone, disk_out > 245 puts the escape sphere inside it, and without fast_ok redo_below is infinite), so each zone's
+    // window and validation take all of them.
     const float zb_floor = fmaxf(C.horizon_r, redo_below);
+    const float disk_floor = fmaxf(18.0f, zb_floor);
     const float zb_m1 = 1.25f * (float)kBurst * C.h[1], zb_m2 = 1.25f * (float)kBurst * C.h[2];
     const float near_lo = zb_floor + zb_m1, near_hi = 18.0f - zb_m1;
-    const float disk_lo = 18.0f + zb_m2, disk_hi = C.disk_zone_r - zb_m2, disk_y = C.disk_zone_y - zb_m2;
+    const float disk_lo = disk_floor + zb_m2, disk_hi = fminf(C.disk_zone_r, 250.0f) - zb_m2, disk_y = C.disk_zone_y - zb_m2;
     const float kInf = __int_as_float(0x7f800000);
     auto zone_for_burst = [&](float r, float ay) -> int {
         if (r >= burst_lo && r <= burst_hi) return 0;
@@ -474,7 +479,7 @@ __global__ void __launch_bounds__(32, kPackedMinBlocks) trace_kernel_p(const __g
     auto burst_was_valid = [&](int m, float mn, float mx, float my) -> bool {
         if (m == 0) return mn >= burst_min && mx <= 250.0f;                      // no zone, no medium, no escape test to miss
         if (m == 1) return mn >= zb_floor && mx < 18.0f;                         // :56
-        return mn >= 18.0f && mx < C.disk_zone_r && my < C.disk_zone_y;          // :57 and not :56
+        return mn >= disk_floor && mx < C.disk_zone_r && mx <= 250.0f && my < C.disk_zone_y;   // :57 and not :56
     };
     TileCounters cnt;
     Emitter2 em(S, tab, C);

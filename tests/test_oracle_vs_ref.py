@@ -18,10 +18,17 @@ def test_defaults_match_reference_macros(ora, ref):
     assert bytes(ora.default_effects()) == bytes(ref.default_effects())    # camera_settings.h
 
 
-@pytest.mark.parametrize("spin", [0.0, 0.3, 0.99])
-def test_functions(ora, ref, spin):
+# the hole and disk of tests/test_gpu_params.py's big-hole and disk-past-escape regimes
+BIG_HOLE = dict(event_horizon=20.0, isco_radius=22.0, disk_out=60.0, cloud_out=60.0)
+DISK_PAST_ESCAPE = dict(disk_out=300.0)
+
+
+@pytest.mark.parametrize("kw", [pytest.param(dict(spin_a=a), id=str(a)) for a in (0.0, 0.3, 0.99)] +
+                         [pytest.param(dict(spin_a=0.99, **BIG_HOLE), id="big-hole"),
+                          pytest.param(dict(spin_a=0.99, **DISK_PAST_ESCAPE), id="disk-past-escape")])
+def test_functions(ora, ref, kw):
     q, v = phase_space(seed=7, n=4096)
-    po, pr = ora.default_params(spin_a=spin), ref.default_params(spin_a=spin)
+    po, pr = ora.default_params(**kw), ref.default_params(**kw)
     assert same(ora.geodesic_acc(po, q, v), ref.geodesic_acc(pr, q, v))
     h = np.random.Generator(np.random.PCG64(3)).choice(np.float32([0.3, 0.03, 0.09, 0.15]), size=len(q))
     a, b = ora.rk4_step(po, q, v, h), ref.rk4_step(pr, q, v, h)
@@ -60,7 +67,8 @@ def test_camera_and_paths(ora, ref):
 
 @pytest.mark.parametrize("cam", ["C0", "C3"])
 @pytest.mark.parametrize("kw", [dict(spin_a=0.99, flags=3), dict(spin_a=0.0, flags=1),
-                                dict(spin_a=0.6, flags=3, max_steps=600, step_size=0.25, cloud_h=3.0, event_horizon=1.5)])
+                                dict(spin_a=0.6, flags=3, max_steps=600, step_size=0.25, cloud_h=3.0, event_horizon=1.5),
+                                dict(spin_a=0.99, flags=3, **BIG_HOLE), dict(spin_a=0.99, flags=3, **DISK_PAST_ESCAPE)])
 def test_frames(ora, ref, sky_small, cam, kw):
     for fxo, fxr in ((ora.default_effects(use_ca=1), ref.default_effects(use_ca=1)), (ora.effects_off(), ref.effects_off())):
         a = ora.render(ora.default_params(**kw), ora.camera_from(*CAMERAS[cam]), fxo, sky_small, 2.5, 80, 45)
