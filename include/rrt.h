@@ -234,6 +234,28 @@ int rrt_render_dof(rrt_context* ctx, const rrt_params* prm, const rrt_camera* ca
                    uint64_t sky_texture, float time, int w, int h, int ss, const rrt_band* band,
                    void* d_out, int out_layout, float* hdr_out, void* stream);
 
+/* ---- panoramas: a 360 x 180 degree equirectangular frame -------------------------------------------------------------
+ * Every direction around cam->pos in one w x h frame: column x is longitude lam = 2 pi ((x + 0.5) / w - 0.5) about up,
+ * row y latitude phi = pi ((y + 0.5) / h - 0.5), and pixel (x, y) starts at cam->pos in the direction unit3(d), d being
+ * rrt_pano_directions' vector of that pixel (forward at the centre, right at lam = pi/2, up at the top).  The contract:
+ * pixel (x, y) of rrt_render_pano(P, cam, F, S, t, w, h, ss = 1) equals pixel (1, 1) of
+ * rrt_render(P, {cam->pos, d, cam->right, cam->up}, F, S, t, 2, 2) -- whose ray is that same unit3(d) -- in cls, steps,
+ * pos, vel, dir, emis and hdr, and in its byte when the vignette is off (the post step runs at pixel_uv (x/w, y/h): the
+ * vignette darkens the panorama's edges as it does a pinhole frame's).  With the row-flipped RRT_OUT_FRAME store the
+ * zenith is the first buffer row, the layout 360-degree players and environment maps expect.
+ * ss = 1: rrt_render's pipeline choice, counters, launch count, bands, RRT_OUT_PACKED, peer-frame d_out and all seven planes.
+ * ss = 2..8: the ss*w x ss*h panorama traced into scratch and resolved as rrt_render_ss does (band {r, N, ss*g}); only
+ * planes->hdr, the w x h mean, is offered.  The result is bit for bit rrt_resolve(ss) of the hdr plane of
+ * rrt_render_pano(ss*w, ss*h, ss = 1): the sub-samples are the cell centres of the large panorama, so unlike
+ * rrt_render_ss there is no half-pixel shift.  Counters and launches: the large trace's, + 1 launch for the resolve.
+ * The w + h (ss*w + ss*h) direction factors are computed on the host per call and copied on `stream` into a block of the
+ * scratch pool (behind the supersampled plane when ss > 1); the caller's data is not involved.  Lens distortion has no
+ * meaning here: RRT_ERR_BAD_ARG, before anything is enqueued, for fx->use_lens != 0, ss outside 1..8, a plane other than
+ * hdr when ss > 1 and everything rrt_render / rrt_render_ss refuse; RRT_ERR_NOMEM when the scratch block cannot be had. */
+int rrt_render_pano(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, const rrt_effects* fx,
+                    uint64_t sky_texture, float time, int w, int h, int ss, const rrt_band* band,
+                    void* d_out, int out_layout, const rrt_planes* planes, void* stream);
+
 /* ---- captures: one trace, renders at many times -------------------------------------------------------------------
  * With the camera fixed only the time moves, and the time enters only the disk and dust densities: trajectories, step
  * counts, classes and the positions of the media samples are the same at every time (a ray ends only at the horizon, on
@@ -353,7 +375,8 @@ int rrt_set_sample_pool(rrt_context* ctx, size_t max_bytes_per_stream, int max_p
 int rrt_split_stats(rrt_context* ctx, uint32_t out[8]);
 /* Kernels this context has launched so far for rrt_render*, rrt_shade, rrt_resolve*, rrt_capture_* and rrt_assemble_bands
  * (1 per fused frame; 3 per pass + 1 per split frame; 1 per rrt_shade, rrt_resolve or rrt_resolve_time; rrt_render_ss and
- * rrt_render_dof: their ss*w x ss*h render's + 1; rrt_render_mb: its n renders' + 1; 1 per rrt_capture_create, 3 or 4 per rrt_capture_render,
+ * rrt_render_dof: their ss*w x ss*h render's + 1; rrt_render_pano: rrt_render's at ss = 1, its ss*w x ss*h render's + 1 at
+ * ss > 1; rrt_render_mb: its n renders' + 1; 1 per rrt_capture_create, 3 or 4 per rrt_capture_render,
  * n * (3 or 4) + 1 per rrt_capture_render_mb):
  * what a benchmark reports as its launch count. */
 uint64_t rrt_kernel_launches(rrt_context* ctx);
@@ -438,6 +461,15 @@ int rrt_shutter_times(float t, float shutter, float fps, int n, float* out);
  * RRT_ERR_BAD_ARG for aperture < 0 or non-finite, focus <= 0 or non-finite, ss outside 1..8, or a NULL pointer.
  * out holds ss*ss cameras. */
 int rrt_lens_cameras(const rrt_camera* cam, float aperture, float focus, int ss, rrt_camera* out);
+
+/* The un-normalised direction of every pixel of a w x h rrt_render_pano frame: out[(y*w + x)*3 + c] = d[c].  With
+ * lam = 2 pi ((x + 0.5) / w - 0.5) and phi = pi ((y + 0.5) / h - 0.5) evaluated in double (as pi (2x + 1 - w) / w and
+ * pi/2 (2y + 1 - h) / h, so that mirrored columns and rows get exactly opposite angles) and (cos, sin) of each rounded to
+ * float32 once, per component c and every operation rounded to float32 on its own (no contraction) in this order:
+ *   a = cos phi * cos lam,   b = cos phi * sin lam,   d[c] = (a * forward[c] + b * right[c]) + sin phi * up[c].
+ * The panorama's ray of that pixel is unit3(d) from cam->pos.  No orthonormality of the camera is assumed.
+ * RRT_ERR_BAD_ARG for a NULL pointer, w or h <= 0, or w*h*3 floats beyond the address space. */
+int rrt_pano_directions(const rrt_camera* cam, int w, int h, float* out);
 
 /* ---- frame sink: the step after the hot path ----------------------------------------------------------
  * Pure host code.  Replaces, for headless use, the reference's ScreenRecorder (src/main.cpp:29-124): frames

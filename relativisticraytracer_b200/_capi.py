@@ -70,8 +70,8 @@ class Counters(C.Structure):
 SYMBOLS = [
     "rrt_abi_version", "rrt_build_info", "rrt_context_create", "rrt_context_destroy", "rrt_last_error",
     "rrt_default_params", "rrt_default_effects", "rrt_sky_create", "rrt_sky_texture", "rrt_sky_destroy",
-    "rrt_render", "rrt_shade", "rrt_resolve", "rrt_render_ss", "rrt_render_dof", "rrt_capture_create", "rrt_capture_render", "rrt_capture_info",
-    "rrt_capture_destroy", "rrt_resolve_time", "rrt_render_mb", "rrt_capture_render_mb", "rrt_shutter_times", "rrt_lens_cameras", "rrt_render_host", "rrt_render_host_async", "rrt_band_rows", "rrt_assemble_bands", "rrt_read_counters",
+    "rrt_render", "rrt_shade", "rrt_resolve", "rrt_render_ss", "rrt_render_dof", "rrt_render_pano", "rrt_capture_create", "rrt_capture_render", "rrt_capture_info",
+    "rrt_capture_destroy", "rrt_resolve_time", "rrt_render_mb", "rrt_capture_render_mb", "rrt_shutter_times", "rrt_lens_cameras", "rrt_pano_directions", "rrt_render_host", "rrt_render_host_async", "rrt_band_rows", "rrt_assemble_bands", "rrt_read_counters",
     "rrt_geodesic_acc_batch", "rrt_rk4_step_batch", "rrt_euler_step_batch", "rrt_redshift_batch",
     "rrt_hash31_batch", "rrt_noise3d_batch", "rrt_fbm_batch", "rrt_disk_temperature_batch",
     "rrt_disk_density_batch", "rrt_dust_density_batch", "rrt_sky_sample_batch", "rrt_fp32_peak_probe",
@@ -120,6 +120,8 @@ def load() -> C.CDLL:
                                   vp]
     lib.rrt_render_dof.argtypes = [vp, P(Params), P(Camera), P(Effects), C.c_uint64, cf, ci, ci, ci, P(Band), vp, ci, vp,
                                    vp]
+    lib.rrt_render_pano.argtypes = [vp, P(Params), P(Camera), P(Effects), C.c_uint64, cf, ci, ci, ci, P(Band), vp, ci,
+                                    P(Planes), vp]
     lib.rrt_capture_create.argtypes = [vp, P(Params), P(Camera), P(Effects), C.c_uint64, ci, ci, P(Band), C.c_size_t, vp, P(vp)]
     lib.rrt_capture_render.argtypes = [vp, P(Params), P(Effects), C.c_uint64, cf, vp, ci, vp, vp]
     lib.rrt_capture_info.argtypes = [vp, P(C.c_uint64)]
@@ -130,6 +132,7 @@ def load() -> C.CDLL:
     lib.rrt_capture_render_mb.argtypes = [vp, P(Params), P(Effects), C.c_uint64, P(cf), ci, vp, ci, vp, vp]
     lib.rrt_shutter_times.argtypes = [cf, cf, cf, ci, P(cf)]
     lib.rrt_lens_cameras.argtypes = [P(Camera), cf, cf, ci, P(Camera)]
+    lib.rrt_pano_directions.argtypes = [P(Camera), ci, ci, vp]
     lib.rrt_render_host.argtypes = [vp, P(Params), P(Camera), P(Effects), C.c_uint64, cf, ci, ci, vp]
     lib.rrt_render_host_async.argtypes = [vp, P(Params), P(Camera), P(Effects), C.c_uint64, cf, ci, ci, vp, ci, vp]
     lib.rrt_band_rows.argtypes = [P(Band), ci]

@@ -9,7 +9,8 @@
 //                            resolve_kernel, probe kernels
 //   csrc/rrt_packed.cuh      render_kernel_p (two rays per thread, no medium), FMAD contract only
 //   csrc/rrt_split.cuh       the split pipeline of launches with a medium: trace / media / fold kernels
-//                            (every kernel that creates rays also has a LENS variant: rrt_render_dof's per-sub-sample cameras)
+//                            (every kernel that creates rays also has LENS variants: rrt_render_dof's per-sub-sample cameras
+//                            and rrt_render_pano's equirectangular directions)
 //   this file                band assembly, self-test / roofline probes, rrt_context, every extern "C" entry point
 //
 // Launch organisation (B200: 148 SMs, no tensor-core work on this path -- it is FP32 FMA-pipe bound):
@@ -564,8 +565,8 @@ struct TracePlan {
 };
 // Whether a launch with these parameters can go through the split pipeline: a tile's rows must fit a TileDesc.
 static bool split_fits(const rrt_params* prm) { return prm->max_steps + 2 <= 128 * (rrtk::kDescChunks - 2); }
-// lens: the LENS variants (every ray from its own camera of LensArgs::cams, rrt_render_dof).
-static int plan_trace(rrt_context* ctx, const rrt_params& prm, int w, int local_rows, bool lens, TracePlan* t) {
+// lens: the ray source of the LENS variants (rrt_render: kRaysPinhole, rrt_render_dof: kRaysLens, rrt_render_pano: kRaysPano).
+static int plan_trace(rrt_context* ctx, const rrt_params& prm, int w, int local_rows, int lens, TracePlan* t) {
     const bool spin = prm.spin_a != 0.0f;
     t->sk = (prm.flags & RRT_FLAG_FMAD) ? rrtk::rrt_split_kernels_fmad() : rrtk::rrt_split_kernels_strict();
     // the tracer: two rays per thread in packed f32x2 registers where that kernel exists (FMAD contract), else one per thread
@@ -611,8 +612,9 @@ static int launch_sweep(rrt_context* ctx, const TracePlan& tp, const FrameArgs& 
     return RRT_OK;
 }
 
-// One frame through trace / media / fold passes and the closing sweep.  A camera table in L (rrt_render_dof) selects the
-// LENS tracers of the plan: the passes, the redo list and the sweep re-create every ray from its own camera.
+// One frame through trace / media / fold passes and the closing sweep.  A camera table (rrt_render_dof) or panorama table
+// (rrt_render_pano) in L goes with the LENS tracers of the plan: the passes, the redo list and the sweep re-create every ray
+// from it.
 static int render_split(rrt_context* ctx, const FrameArgs& A, const rrtk::LensArgs& L, const TracePlan& tp, cudaStream_t st,
                         rrt_context::SamplePool* pl) {
     // passes to enqueue: what the last completed frame on this pool needed (the sweep renders whatever a wrong guess leaves)
@@ -700,9 +702,11 @@ static bool f4_overlap(const void* src, unsigned long long src_n, const void* ds
 }
 
 // ---- bodies: arguments checked, ctx->mu held, ctx->device current ---------------------------------------------------
-// rrt_render's body.  L.cams: null, or a DEVICE table of L.ss * L.ss cameras (rrt_render_dof) -- then the LENS variant of
-// the chosen kernel starts pixel (x, y)'s ray from L.cams[(y % L.ss) * L.ss + x % L.ss] and `cam` is not read by any
-// kernel.  Launch choice, pipeline, counters and launch count are rrt_render's either way.
+// rrt_render's body.  L.cams: null, or a DEVICE table of L.ss * L.ss cameras (rrt_render_dof) -- then the kRaysLens variant
+// of the chosen kernel starts pixel (x, y)'s ray from L.cams[(y % L.ss) * L.ss + x % L.ss] and `cam` is not read by any
+// kernel.  L.pano: null, or the DEVICE table of a w x h panorama (rrt_render_pano) -- then the kRaysPano variant starts
+// every ray at cam.pos in the direction of pano_dir.  Launch choice, pipeline, counters and launch count are rrt_render's
+// in every case.
 static int render_frame(rrt_context* ctx, const rrt_params& prm, const rrt_camera& cam, const rrt_effects& fx, uint64_t sky_texture,
                         float time, int w, int h, const rrt_band& b, int local_rows, void* d_out, int out_layout, const rrt_planes* planes,
                         cudaStream_t st, const rrtk::LensArgs& L) {
@@ -717,7 +721,7 @@ static int render_frame(rrt_context* ctx, const rrt_params& prm, const rrt_camer
     const bool spin = prm.spin_a != 0.0f;
     const bool media = (prm.flags & (RRT_FLAG_DISK | RRT_FLAG_DUST)) != 0;
     const bool fmad = (prm.flags & RRT_FLAG_FMAD) != 0;
-    const bool lens = L.cams != nullptr;
+    const int lens = L.pano ? kRaysPano : (L.cams ? kRaysLens : kRaysPinhole);
     // A launch with a medium goes through the split pipeline (csrc/rrt_split.cuh) unless the caller pinned the fused
     // kernel, the tile log is selected, or the pool cannot be allocated.
     if (media && ctx->pipeline != RRT_PIPELINE_FUSED && (!ctx->tile_log || ctx->pipeline == RRT_PIPELINE_SPLIT) && split_fits(&prm)) {
@@ -909,6 +913,49 @@ int rrt_render_dof(rrt_context* ctx, const rrt_params* prm, const rrt_camera* ca
     if (!cams) return fail(ctx, RRT_ERR_BAD_ARG, "rrt_render_dof: bad argument");
     return render_ss_frame(ctx, "rrt_render_dof", prm, cams, cams, fx, sky_texture, time, w, h, ss, band, d_out, out_layout, hdr_out,
                            stream);
+}
+
+int rrt_render_pano(rrt_context* ctx, const rrt_params* prm, const rrt_camera* cam, const rrt_effects* fx, uint64_t sky_texture,
+                    float time, int w, int h, int ss, const rrt_band* band, void* d_out, int out_layout, const rrt_planes* planes,
+                    void* stream) {
+    if (!ctx) return RRT_ERR_BAD_ARG;
+    const std::string m = "rrt_render_pano";
+    // ss > 1 offers the averaged hdr plane only, like rrt_render_ss
+    const bool hdr_only = !planes || (!planes->dir && !planes->emis && !planes->pos && !planes->vel && !planes->cls && !planes->steps);
+    if (!prm || !cam || !fx || sky_texture == 0 || prm->max_steps < 0 || !ss_ok(ss, w, h) || fx->use_lens != 0 ||
+        !outputs_ok(out_layout, d_out, ss == 1 ? (const void*)planes : (const void*)(planes ? planes->hdr : nullptr)) ||
+        (ss > 1 && !hdr_only))
+        return fail(ctx, RRT_ERR_BAD_ARG, m + ": bad argument");
+    rrt_band b;
+    int local_rows = 0;
+    if (int rc = band_of(ctx, m, band, w, h, ss, &b, &local_rows)) return rc;
+    if (local_rows == 0) return RRT_OK;
+    const int W = ss * w, H = ss * h;   // the traced panorama
+    const unsigned long long n_hi = ss == 1 ? 0ull : (unsigned long long)W * H;   // the supersampled plane, full-frame indexed
+    const size_t tab_bytes = sizeof(float2) * ((size_t)W + H);
+    if (n_hi > (SIZE_MAX - tab_bytes) / 16) return fail(ctx, RRT_ERR_NOMEM, m + ": supersampled hdr plane larger than the address space");
+    std::vector<float2> tab((size_t)W + H);   // pageable: staged by cudaMemcpyAsync before it returns
+    rrtk::pano_table(W, H, (float*)tab.data());
+
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DevGuard g(ctx->device);
+    const cudaStream_t st = (cudaStream_t)stream;
+    return with_scratch(ctx, m, ss == 1 ? "panorama table" : "supersampled hdr plane", (size_t)16 * n_hi + tab_bytes, st, [&](float* blk) {
+        float2* d_tab = (float2*)(blk + 4 * n_hi);   // behind the plane when there is one
+        const cudaError_t e = cudaMemcpyAsync(d_tab, tab.data(), tab_bytes, cudaMemcpyHostToDevice, st);
+        if (e != cudaSuccess) return fail(ctx, RRT_ERR_CUDA, m + ": copy of the panorama table", e);
+        rrtk::LensArgs L = {};
+        L.pano = d_tab;
+        if (ss == 1)
+            return render_frame(ctx, *prm, *cam, *fx, sky_texture, time, w, h, b, local_rows, d_out, out_layout, planes, st, L);
+        rrt_planes pl;
+        std::memset(&pl, 0, sizeof(pl));
+        pl.hdr = blk;
+        const rrt_band tb = {b.rank, b.nranks, ss * b.group};   // as in render_ss_frame: the ss sub-rows of each of the band's rows
+        if (int rc = render_frame(ctx, *prm, *cam, *fx, sky_texture, time, W, H, tb, ss * local_rows, nullptr, RRT_OUT_FRAME, &pl, st, L))
+            return rc;
+        return launch_resolve(ctx, *prm, *fx, ss, 1, w, h, b, local_rows, blk, 0, d_out, out_layout, planes ? planes->hdr : nullptr, st);
+    });
 }
 
 int rrt_resolve_time(rrt_context* ctx, const rrt_params* prm, const rrt_effects* fx, int n, int w, int h, const rrt_band* band,

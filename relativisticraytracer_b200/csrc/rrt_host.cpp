@@ -7,6 +7,7 @@
 // tables of src/camera_paths.cpp.  Built with -ffp-contract=off: every operation is one binary32 op in
 // the reference's order, so the basis vectors are bit-identical to the reference's on the same libm.
 #include <cmath>
+#include <cstdint>
 #include <cstdio>
 #include <cstring>
 #include <new>
@@ -82,6 +83,26 @@ void basis_from(Vec pos, float yaw, float pitch, rrt_camera* out) {
 }
 
 }  // namespace
+
+namespace rrtk {
+// rrt_render_pano's device table and rrt_pano_directions' factors: w entries (cos, sin) of each column's longitude
+// lam = 2 pi ((x + 0.5) / w - 0.5), then h entries (cos, sin) of each row's latitude phi = pi ((y + 0.5) / h - 0.5), in
+// double and rounded to float once.  The angle is taken as pi * (2x + 1 - w) / w (the same value): the integer numerator
+// is exact, so mirrored columns and rows get exactly opposite angles, equal cosines and opposite sines.
+void pano_table(int w, int h, float* out) {
+    const double kPi = 3.14159265358979323846;
+    for (int x = 0; x < w; ++x) {
+        const double lam = kPi * ((double)(2ll * x + 1 - w) / w);
+        out[2 * x] = (float)std::cos(lam);
+        out[2 * x + 1] = (float)std::sin(lam);
+    }
+    for (int y = 0; y < h; ++y) {
+        const double phi = 0.5 * kPi * ((double)(2ll * y + 1 - h) / h);
+        out[2 * ((size_t)w + y)] = (float)std::cos(phi);
+        out[2 * ((size_t)w + y) + 1] = (float)std::sin(phi);
+    }
+}
+}  // namespace rrtk
 
 extern "C" {
 
@@ -173,6 +194,25 @@ int rrt_lens_cameras(const rrt_camera* cam, float aperture, float focus, int ss,
                 c.pos[k] = cam->pos[k] + o;
                 const float tilt = o / focus;
                 c.forward[k] = cam->forward[k] - tilt;
+            }
+        }
+    return RRT_OK;
+}
+
+int rrt_pano_directions(const rrt_camera* cam, int w, int h, float* out) {
+    if (!cam || !out || w <= 0 || h <= 0 || (unsigned long long)w * h > SIZE_MAX / (3 * sizeof(float))) return RRT_ERR_BAD_ARG;
+    std::vector<float> t(2 * ((size_t)w + h));
+    rrtk::pano_table(w, h, t.data());
+    const float* lat = t.data() + 2 * (size_t)w;
+    for (int y = 0; y < h; ++y)
+        for (int x = 0; x < w; ++x) {
+            // one binary32 operation each, in this order (no contraction), as pano_dir does on the device
+            const float a = lat[2 * y] * t[2 * x], b = lat[2 * y] * t[2 * x + 1];
+            float* d = out + ((size_t)y * w + x) * 3;
+            for (int c = 0; c < 3; ++c) {
+                const float af = a * cam->forward[c], br = b * cam->right[c], su = lat[2 * y + 1] * cam->up[c];
+                const float s = af + br;
+                d[c] = s + su;
             }
         }
     return RRT_OK;

@@ -32,22 +32,34 @@ struct FrameArgs {
     unsigned int tile_log_cap;     // entries the log can hold
 };
 
-// The camera table of rrt_render_dof, the last parameter of every kernel that creates rays; read by their LENS variants
-// only (zero for every other launch).  A separate parameter rather than more FrameArgs fields: appended at the end of the
-// parameter block it moves no parameter of the existing kernels.  Pixel (x, y) of the traced frame starts its ray from
-// cams[(y % ss) * ss + x % ss] instead of FrameArgs::cam.  near: every camera of the table lies in the branch-free domain
-// (trace_ray's fast_ok), decided once on the host so that the gate stays a launch constant as it is with one camera.
+// The ray source of a kernel that creates rays, its LENS template argument:
+//   kRaysPinhole  the frame's camera, FrameArgs::cam (rrt_render)
+//   kRaysLens     each pixel's camera of the table LensArgs::cams (rrt_render_dof)
+//   kRaysPano     FrameArgs::cam's position, the equirectangular direction of the pixel from LensArgs::pano (rrt_render_pano)
+enum : int { kRaysPinhole = 0, kRaysLens = 1, kRaysPano = 2, kRaySources = 3 };
+
+// The tables of the other ray sources, the last parameter of every kernel that creates rays; read by their kRaysLens and kRaysPano
+// variants only (zero for every other launch).  A separate parameter rather than more FrameArgs fields: appended at the
+// end of the parameter block it moves no parameter of the existing kernels, and each member appended to it moves none of
+// the members before it.
+//   cams, ss, near: pixel (x, y) of the traced frame starts its ray from cams[(y % ss) * ss + x % ss] instead of
+//     FrameArgs::cam.  near: every camera of the table lies in the branch-free domain (trace_ray's fast_ok), decided once
+//     on the host so that the gate stays a launch constant as it is with one camera.
+//   pano: w column entries (cos, sin) of the longitude, then h row entries (cos, sin) of the latitude (rrt_pano_directions).
 struct LensArgs {
     const rrt_camera* cams;
     int ss;
     int near;
+    const float2* pano;
 };
+// The w + h entries of LensArgs::pano for a w x h panorama, as 2 * (w + h) floats (host code, rrt_host.cpp).
+void pano_table(int w, int h, float* out);
 
 // kernels of one rounding contract
 struct KernelSet {
-    // [lens][spin != 0][media]; lens: the LENS variant (rrt_render_dof), every ray from its own camera of LensArgs::cams
-    void (*render[2][2][2])(const FrameArgs, const LensArgs);
-    void (*render_packed[2][2])(const FrameArgs, const LensArgs);  // [lens][spin != 0]; two rays per thread in f32x2 registers, no medium (rrt_packed.cuh); FMAD contract only
+    // [lens][spin != 0][media]; lens: the ray source (kRaysPinhole, kRaysLens, kRaysPano) of the LENS template argument
+    void (*render[kRaySources][2][2])(const FrameArgs, const LensArgs);
+    void (*render_packed[kRaySources][2])(const FrameArgs, const LensArgs);  // [lens][spin != 0]; two rays per thread in f32x2 registers, no medium (rrt_packed.cuh); FMAD contract only
     void (*acc)(Consts, int, const float*, const float*, float*);
     void (*rk4)(Consts, int, float*, float*, const float*);
     void (*euler)(Consts, int, float*, float*, const float*);
@@ -71,6 +83,9 @@ using rrt::V3;
 using rrt::mk;
 using rrtk::FrameArgs;
 using rrtk::LensArgs;
+using rrtk::kRaysPinhole;
+using rrtk::kRaysLens;
+using rrtk::kRaysPano;
 
 namespace {
 
@@ -87,8 +102,9 @@ constexpr int kBurst = 8;
 // that better than the four the unconstrained 109-register build gets (4K C0 78.5 -> 76.2 ms, C3 147.6 -> 135.4;
 // 7 and 8 CTAs are no better).  The geodesic-only variant needs ~72 registers anyway.
 constexpr int kMinBlocks = 1, kMinBlocksMedia = 24;
-// The LENS variants (rrt_render_dof) of the media kernels -- render_kernel<SPIN, true, true> and sweep_kernel<SPIN, true>, the
-// fused fallbacks of a depth-of-field frame -- are asked for 18 warps per SM (<= 112 registers), where none of them spills.
+// The kRaysLens and kRaysPano variants (rrt_render_dof, rrt_render_pano) of the media kernels -- render_kernel<SPIN, true, LENS>
+// and sweep_kernel<SPIN, LENS>, the fused fallbacks of such a frame -- are asked for 18 warps per SM (<= 112 registers), where
+// none of them spills.
 constexpr int kMinBlocksMediaLens = 18;
 
 struct RayResult {
@@ -183,10 +199,10 @@ __device__ __forceinline__ void pixel_uv(const FrameArgs& A, int x, int y, float
     }
 }
 
-// The camera a pixel's ray starts from: the frame's, or with LENS (rrt_render_dof) its entry of the camera table.
-template <bool LENS>
+// The camera a pixel's ray starts from: the frame's, or with kRaysLens (rrt_render_dof) its entry of the camera table.
+template <int LENS>
 __device__ __forceinline__ const rrt_camera& ray_camera(const FrameArgs& A, const LensArgs& L, int x, int y) {
-    if (!LENS) return A.cam;
+    if (LENS != kRaysLens) return A.cam;
     return L.cams[(y % L.ss) * L.ss + x % L.ss];
 }
 
@@ -208,6 +224,25 @@ __device__ __forceinline__ V3 ray_dir(const FrameArgs& A, const rrt_camera& cam,
     float uvx, uvy;
     pixel_uv(A, x, y, uvx, uvy);
     return ray_dir_uv(A, cam, uvx, uvy);
+}
+// initial ray of pixel (x, y) of an equirectangular panorama (kRaysPano, rrt_render_pano): with (cl, sl) = pano[x] and
+// (cp, sp) = pano[w + y], d = (cp*cl * forward + cp*sl * right) + sp * up, every operation rounded on its own in that
+// order -- rrt_pano_directions' vector bit for bit -- then unit3 like the pinhole ray.  The pinhole ray of pixel (1, 1) of
+// a 2 x 2 frame with forward = d is that same unit3(d).
+__device__ __forceinline__ V3 pano_dir(const FrameArgs& A, const LensArgs& L, int x, int y) {
+    using namespace rrt;
+    const float2 lon = L.pano[x], lat = L.pano[A.w + y];
+    const float a = mul(lat.x, lon.x), b = mul(lat.x, lon.y);
+    const rrt_camera& c = A.cam;
+    return unit3(mk(add(add(mul(a, c.forward[0]), mul(b, c.right[0])), mul(lat.y, c.up[0])),
+                    add(add(mul(a, c.forward[1]), mul(b, c.right[1])), mul(lat.y, c.up[1])),
+                    add(add(mul(a, c.forward[2]), mul(b, c.right[2])), mul(lat.y, c.up[2]))));
+}
+// the initial direction of pixel (x, y) from camera `cam` (ray_camera<LENS>), whatever the ray source
+template <int LENS>
+__device__ __forceinline__ V3 ray_dir_src(const FrameArgs& A, const LensArgs& L, const rrt_camera& cam, int x, int y) {
+    if (LENS == kRaysPano) return pano_dir(A, L, x, y);
+    return ray_dir(A, cam, x, y);
 }
 
 constexpr unsigned kEndCaptured = 1u, kEndTouched = 2u, kEndExhausted = 4u;
@@ -301,15 +336,15 @@ struct NoEmit {
     __device__ __forceinline__ void emit(V3, V3, float, int, unsigned) {}
 };
 
-// One ray: reference raymarch_kernel lines 20-150.  LENS: from the pixel's own camera (ray_camera).
-template <bool SPIN, int MEDIA, bool LENS, class EM>
+// One ray: reference raymarch_kernel lines 20-150.  LENS: the ray source (ray_camera, pano_dir).
+template <bool SPIN, int MEDIA, int LENS, class EM>
 __device__ __forceinline__ void trace_ray(const FrameArgs& A, const LensArgs& L, int x, int y, RayResult& R, EM& em) {
     const Consts& C = A.C;
     const rrt_camera& cam = ray_camera<LENS>(A, L, x, y);
     float uvx, uvy;
     pixel_uv(A, x, y, uvx, uvy);                                       // :20-25
     V3 p = mk(cam.pos[0], cam.pos[1], cam.pos[2]);
-    V3 v = ray_dir_uv(A, cam, uvx, uvy);                               // :27-34
+    V3 v = LENS == kRaysPano ? pano_dir(A, L, x, y) : ray_dir_uv(A, cam, uvx, uvy);   // :27-34
 
     float Ir = 0.f, Ig = 0.f, Ib = 0.f, T = 1.0f;
     bool captured = false, touched = false, escaped = false;
@@ -318,10 +353,10 @@ __device__ __forceinline__ void trace_ray(const FrameArgs& A, const LensArgs& L,
     const int max_steps = C.max_steps;
     const bool want_disk = (C.flags & RRT_FLAG_DISK) != 0, want_dust = (C.flags & RRT_FLAG_DUST) != 0;
     // Domain of the branch-free div/sqrt (rrt_device.cuh): a ray that starts absurdly far out takes the
-    // general path for its whole life.  Uniform per launch in practice (depends on the camera only); with LENS decided
+    // general path for its whole life.  Uniform per launch in practice (depends on the camera only); with kRaysLens decided
     // for the whole camera table (LensArgs::near), which keeps it a launch constant.  Both paths give the same bits where
     // the fast one is valid, so the gate decides only the speed.
-    const bool fast_ok = (LENS ? L.near != 0 : rrt::dot3(p, p) < 1.0e8f) && C.acc_rmin < C.horizon_r && C.horizon_r >= 1e-3f;
+    const bool fast_ok = (LENS == kRaysLens ? L.near != 0 : rrt::dot3(p, p) < 1.0e8f) && C.acc_rmin < C.horizon_r && C.horizon_r >= 1e-3f;
     const float zone_rmax = fmaxf(18.0f, fmaxf(C.disk_zone_r, C.dust_zone_r));
     // one compare per step for "redo with the general code": smallest stage radius below acc_rmin (or NaN), or
     // the whole ray outside the fast domain (+inf: every step is redone)
@@ -492,8 +527,8 @@ __device__ __forceinline__ void trace_ray(const FrameArgs& A, const LensArgs& L,
     R.uvx = uvx; R.uvy = uvy;
 }
 
-template <bool SPIN, bool MEDIA, bool LENS>
-__global__ void __launch_bounds__(kRenderBlock, MEDIA ? (LENS ? kMinBlocksMediaLens : kMinBlocksMedia) : kMinBlocks)
+template <bool SPIN, bool MEDIA, int LENS>
+__global__ void __launch_bounds__(kRenderBlock, MEDIA ? (LENS != kRaysPinhole ? kMinBlocksMediaLens : kMinBlocksMedia) : kMinBlocks)
     render_kernel(const __grid_constant__ FrameArgs A, const __grid_constant__ LensArgs L) {
     const int lane = threadIdx.x & 31;
     const int ntx = (A.w + kRTileW - 1) / kRTileW;
@@ -702,12 +737,14 @@ __global__ void k_sky(cudaTextureObject_t sky, int n, const float* tx, const flo
 #include "rrt_split.cuh"   // trace / media / fold kernels of the split pipeline (both contracts)
 namespace {
 const rrtk::KernelSet kKernelSet = {
-    {{{render_kernel<false, false, false>, render_kernel<false, true, false>}, {render_kernel<true, false, false>, render_kernel<true, true, false>}},
-     {{render_kernel<false, false, true>, render_kernel<false, true, true>}, {render_kernel<true, false, true>, render_kernel<true, true, true>}}},
+    {{{render_kernel<false, false, 0>, render_kernel<false, true, 0>}, {render_kernel<true, false, 0>, render_kernel<true, true, 0>}},
+     {{render_kernel<false, false, 1>, render_kernel<false, true, 1>}, {render_kernel<true, false, 1>, render_kernel<true, true, 1>}},
+     {{render_kernel<false, false, 2>, render_kernel<false, true, 2>}, {render_kernel<true, false, 2>, render_kernel<true, true, 2>}}},
 #if RRT_FMAD
-    {{render_kernel_p<false, false>, render_kernel_p<true, false>}, {render_kernel_p<false, true>, render_kernel_p<true, true>}},
+    {{render_kernel_p<false, 0>, render_kernel_p<true, 0>}, {render_kernel_p<false, 1>, render_kernel_p<true, 1>},
+     {render_kernel_p<false, 2>, render_kernel_p<true, 2>}},
 #else
-    {{nullptr, nullptr}, {nullptr, nullptr}},
+    {{nullptr, nullptr}, {nullptr, nullptr}, {nullptr, nullptr}},
 #endif
     k_acc, k_rk4, k_euler, k_redshift, k_hash31, k_noise3d, k_fbm, k_disk_temp, k_disk_density, k_dust_density,
     shade_kernel, resolve_kernel,

@@ -87,14 +87,14 @@ struct SplitArgs {
     unsigned tile16;          // tickets and redo lists count 16x4 tiles (the packed tracer) instead of 8x4 tiles
     uint4* results;           // media_kernel<true> / fold_kernel<true>: {e.rgb, s} per slot, indexed like `slots` (rrt_capture)
 };
-// The tracers are indexed [lens][spin != 0]; lens: the LENS variant (rrt_render_dof), every ray from its own camera of
-// LensArgs::cams.  Media and fold read only samples and planes and serve both.
+// The tracers are indexed [lens][spin != 0]; lens: the ray source of the LENS template argument (kRaysPinhole, kRaysLens,
+// kRaysPano).  Media and fold read only samples and planes and serve every source.
 struct SplitKernels {
-    void (*trace[2][2])(const FrameArgs, const SplitArgs, const LensArgs);
-    void (*trace_packed[2][2])(const FrameArgs, const SplitArgs, const LensArgs);   // two rays per thread (FMAD contract only, else null)
+    void (*trace[kRaySources][2])(const FrameArgs, const SplitArgs, const LensArgs);
+    void (*trace_packed[kRaySources][2])(const FrameArgs, const SplitArgs, const LensArgs);   // two rays per thread (FMAD contract only, else null)
     void (*media)(const FrameArgs, const SplitArgs);
     void (*fold)(const FrameArgs, const SplitArgs);
-    void (*sweep[2][2])(const FrameArgs, const SplitArgs, const LensArgs);
+    void (*sweep[kRaySources][2])(const FrameArgs, const SplitArgs, const LensArgs);
     void (*media_results)(const FrameArgs, const SplitArgs);   // media_kernel<true>: the samples stay, results go to S.results
     void (*fold_results)(const FrameArgs, const SplitArgs);    // fold_kernel<true>: reads them from there
 };
@@ -320,7 +320,7 @@ __device__ __forceinline__ void redo_later(const SplitArgs& S, unsigned tile, in
 }
 
 // ---- pass kernel 1: trajectories ------------------------------------------------------------------------------------
-template <bool SPIN, bool LENS>
+template <bool SPIN, int LENS>
 __global__ void __launch_bounds__(kRenderBlock, kMinBlocks) trace_kernel(const __grid_constant__ FrameArgs A,
                                                                               const __grid_constant__ SplitArgs S,
                                                                               const __grid_constant__ LensArgs L) {
@@ -431,7 +431,7 @@ struct Emitter2 {
     }
 };
 
-template <bool SPIN, bool LENS>
+template <bool SPIN, int LENS>
 __global__ void __launch_bounds__(32, kPackedMinBlocks) trace_kernel_p(const __grid_constant__ FrameArgs A, const __grid_constant__ SplitArgs S,
                                                                           const __grid_constant__ LensArgs L) {
     using rrtp::F2;
@@ -447,7 +447,7 @@ __global__ void __launch_bounds__(32, kPackedMinBlocks) trace_kernel_p(const __g
     const bool want_disk = (C.flags & RRT_FLAG_DISK) != 0, want_dust = (C.flags & RRT_FLAG_DUST) != 0;
     const float zone_rmax = fmaxf(18.0f, fmaxf(C.disk_zone_r, C.dust_zone_r));
     const V3 cam_p = mk(A.cam.pos[0], A.cam.pos[1], A.cam.pos[2]);
-    const bool fast_ok = (LENS ? L.near != 0 : rrt::dot3(cam_p, cam_p) < 1.0e8f) && C.acc_rmin < C.horizon_r && C.horizon_r >= 1e-3f;
+    const bool fast_ok = (LENS == kRaysLens ? L.near != 0 : rrt::dot3(cam_p, cam_p) < 1.0e8f) && C.acc_rmin < C.horizon_r && C.horizon_r >= 1e-3f;
     const float redo_below = fast_ok ? C.acc_rmin : __int_as_float(0x7f800000);
     const V3 park_p = mk(0.0f, 100.0f, 0.0f), park_v = mk(0.0f, 0.0f, 0.0f);   // inert state of a finished half, see render_kernel_p
     const float burst_min = fmaxf(zone_rmax, fmaxf(C.horizon_r, redo_below));
@@ -501,10 +501,11 @@ __global__ void __launch_bounds__(32, kPackedMinBlocks) trace_kernel_p(const __g
         if (alive[0] || alive[1]) {
             V3x2 P, V;
             {
-                // the two halves are neighbouring pixels: with LENS each starts from its own camera
+                // the two halves are neighbouring pixels: with kRaysLens each starts from its own camera, with kRaysPano
+                // each takes its own column
                 const rrt_camera &camA = ray_camera<LENS>(A, L, x0, y), &camB = ray_camera<LENS>(A, L, x0 + 1, y);
-                const V3 vA = alive[0] ? ray_dir(A, camA, x0, y) : park_v, vB = alive[1] ? ray_dir(A, camB, x0 + 1, y) : park_v;
-                const V3 pA = alive[0] ? (LENS ? cam_pos(camA) : cam_p) : park_p, pB = alive[1] ? (LENS ? cam_pos(camB) : cam_p) : park_p;
+                const V3 vA = alive[0] ? ray_dir_src<LENS>(A, L, camA, x0, y) : park_v, vB = alive[1] ? ray_dir_src<LENS>(A, L, camB, x0 + 1, y) : park_v;
+                const V3 pA = alive[0] ? (LENS == kRaysLens ? cam_pos(camA) : cam_p) : park_p, pB = alive[1] ? (LENS == kRaysLens ? cam_pos(camB) : cam_p) : park_p;
                 P.x = rrtp::pk(pA.x, pB.x); P.y = rrtp::pk(pA.y, pB.y); P.z = rrtp::pk(pA.z, pB.z);
                 V.x = rrtp::pk(vA.x, vB.x); V.y = rrtp::pk(vA.y, vB.y); V.z = rrtp::pk(vA.z, vB.z);
             }
@@ -933,8 +934,8 @@ __global__ void __launch_bounds__(128) fold_kernel(const __grid_constant__ Frame
 }
 
 // ---- after the last pass: whatever the split passes left, with the fused code ------------------------------------------
-template <bool SPIN, bool LENS>
-__global__ void __launch_bounds__(kRenderBlock, LENS ? kMinBlocksMediaLens : kMinBlocksMedia)
+template <bool SPIN, int LENS>
+__global__ void __launch_bounds__(kRenderBlock, LENS != kRaysPinhole ? kMinBlocksMediaLens : kMinBlocksMedia)
     sweep_kernel(const __grid_constant__ FrameArgs A, const __grid_constant__ SplitArgs S, const __grid_constant__ LensArgs L) {
     const int lane = threadIdx.x & 31;
     const unsigned ntiles = num_tiles(A);
@@ -970,14 +971,15 @@ __global__ void __launch_bounds__(kRenderBlock, LENS ? kMinBlocksMediaLens : kMi
 }
 
 const rrtk::SplitKernels kSplitKernels = {
-    {{trace_kernel<false, false>, trace_kernel<true, false>}, {trace_kernel<false, true>, trace_kernel<true, true>}},
+    {{trace_kernel<false, 0>, trace_kernel<true, 0>}, {trace_kernel<false, 1>, trace_kernel<true, 1>}, {trace_kernel<false, 2>, trace_kernel<true, 2>}},
 #if RRT_FMAD
-    {{trace_kernel_p<false, false>, trace_kernel_p<true, false>}, {trace_kernel_p<false, true>, trace_kernel_p<true, true>}},
+    {{trace_kernel_p<false, 0>, trace_kernel_p<true, 0>}, {trace_kernel_p<false, 1>, trace_kernel_p<true, 1>},
+     {trace_kernel_p<false, 2>, trace_kernel_p<true, 2>}},
 #else
-    {{nullptr, nullptr}, {nullptr, nullptr}},
+    {{nullptr, nullptr}, {nullptr, nullptr}, {nullptr, nullptr}},
 #endif
     media_kernel<false>, fold_kernel<false>,
-    {{sweep_kernel<false, false>, sweep_kernel<true, false>}, {sweep_kernel<false, true>, sweep_kernel<true, true>}},
+    {{sweep_kernel<false, 0>, sweep_kernel<true, 0>}, {sweep_kernel<false, 1>, sweep_kernel<true, 1>}, {sweep_kernel<false, 2>, sweep_kernel<true, 2>}},
     media_kernel<true>, fold_kernel<true>,
 };
 }  // namespace

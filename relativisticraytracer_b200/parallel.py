@@ -310,10 +310,13 @@ class PathSequence:
     here; the C ABI composes the two (rrt_resolve_time, then rrt_resolve).  ``aperture`` > 0 gives every frame depth of
     field (``Renderer.render_dof`` with ``lens_cameras(path camera, aperture, focus, ss)``): a thin lens of that radius
     focused at distance ``focus`` along the path camera's forward, its ss x ss lens points shared out among each pixel's
-    sub-samples; ``aperture`` = 0 keeps the pinhole.  Depth of field does not combine with motion blur here."""
+    sub-samples; ``aperture`` = 0 keeps the pinhole.  Depth of field does not combine with motion blur here.
+    ``projection="equirect"`` renders every frame as a 360-degree equirectangular panorama around the path camera
+    (``Renderer.render_pano``, with ``ss`` as its supersampling factor), the layout 360-degree video players take; it does
+    not combine with depth of field or motion blur.  The default ``"pinhole"`` is the path camera's own view."""
 
     def __init__(self, renderer, w: int, h: int, depth: int = 2, ss: int = 1, shutter: float = 0.0, samples: int = 1,
-                 aperture: float = 0.0, focus: Optional[float] = None):
+                 aperture: float = 0.0, focus: Optional[float] = None, projection: str = "pinhole"):
         if not 1 <= depth <= HOST_SLOTS:
             raise ValueError(f"depth must be 1..{HOST_SLOTS}")
         if not 1 <= ss <= 8:
@@ -330,6 +333,11 @@ class PathSequence:
             raise ValueError("aperture > 0 needs a focus distance, finite and > 0")
         if aperture > 0.0 and samples > 1:
             raise ValueError("aperture > 0 (depth of field) together with samples > 1 (motion blur) is not supported by PathSequence")
+        if projection not in ("pinhole", "equirect"):
+            raise ValueError(f"projection must be 'pinhole' or 'equirect', not {projection!r}")
+        if projection == "equirect" and (aperture > 0.0 or samples > 1):
+            raise ValueError("projection='equirect' does not combine with aperture > 0 or samples > 1")
+        self.projection = projection
         self.aperture, self.focus = float(aperture), focus
         self.r, self.w, self.h, self.depth, self.ss = renderer, w, h, depth, ss
         self.shutter, self.samples = float(shutter), samples
@@ -340,7 +348,7 @@ class PathSequence:
         self.events = [torch.cuda.Event() for _ in range(depth)]
         root = self.rank == 0
         self.local = ([torch.zeros((h, w, 4), dtype=torch.uint8, device=dev) for _ in range(depth)]
-                      if self.world > 1 or ss > 1 or samples > 1 or self.aperture > 0.0 else None)
+                      if self.world > 1 or ss > 1 or samples > 1 or self.aperture > 0.0 or projection != "pinhole" else None)
         self.gathered = ([torch.zeros((self.world, h, w, 4), dtype=torch.uint8, device=dev) for _ in range(depth)]
                          if root and self.world > 1 else None)
         self.host = [torch.zeros((self.world, h, w, 4), dtype=torch.uint8).pin_memory() for _ in range(depth)] if root else None
@@ -376,7 +384,7 @@ class PathSequence:
             mine = frames[self.rank]
             s = self.streams[k]
             with torch.cuda.stream(s):
-                if self.world == 1 and self.ss == 1 and self.samples == 1 and self.aperture == 0.0:
+                if self.world == 1 and self.ss == 1 and self.samples == 1 and self.aperture == 0.0 and self.projection == "pinhole":
                     t = path_clock(mine, fps)
                     cam, _ = path_state(path_index, t)
                     self.r.render_host_async(prm, cam, fx, sky, t, self.w, self.h, self.host[k][0], slot=k, stream=s)
@@ -384,7 +392,9 @@ class PathSequence:
                     if mine is not None:
                         t = path_clock(mine, fps)
                         cam, _ = path_state(path_index, t)
-                        if self.samples > 1:
+                        if self.projection == "equirect":
+                            self.r.render_pano(prm, cam, fx, sky, t, self.w, self.h, ss=self.ss, out=self.local[k], stream=s)
+                        elif self.samples > 1:
                             times = shutter_times(t, self.shutter, fps, self.samples)
                             cams = [path_state(path_index, ti)[0] for ti in times]
                             self.r.render_mb(prm, cams, fx, sky, times, self.w, self.h, out=self.local[k], stream=s)

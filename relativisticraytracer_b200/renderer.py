@@ -79,6 +79,19 @@ def lens_cameras(cam: Camera, aperture: float, focus: float, ss: int) -> list:
     return list(out)
 
 
+def pano_directions(cam: Camera, w: int, h: int) -> np.ndarray:
+    """rrt_pano_directions: the (h, w, 3) float32 un-normalised direction of every pixel of a w x h ``render_pano`` frame:
+    with lam = 2 pi ((x + 0.5)/w - 0.5) and phi = pi ((y + 0.5)/h - 0.5), d = (cos phi cos lam * forward + cos phi sin lam
+    * right) + sin phi * up, each operation in float32 in that order (``include/rrt.h`` gives the exact rule).  Pixel
+    (x, y) of the panorama traces the ray ``render`` traces at pixel (1, 1) of a 2 x 2 frame with forward = d[y, x].
+    Host only."""
+    out = np.empty((max(int(h), 0), max(int(w), 0), 3), np.float32)
+    rc = _capi.load().rrt_pano_directions(C.byref(cam), int(w), int(h), out.ctypes.data_as(C.c_void_p))
+    if rc != 0:
+        raise RrtError(rc, f"rrt_pano_directions({w}, {h}): w and h must be > 0")
+    return out
+
+
 def _f32_array(values) -> C.Array:
     values = [float(v) for v in values]
     return (C.c_float * len(values))(*values)
@@ -318,6 +331,24 @@ class Renderer:
         self._check(self._lib.rrt_render_dof(self._ctx, C.byref(prm), cam_arr, C.byref(fx), _tex(sky), float(time),
                                              int(w), int(h), int(ss), _band_ref(band), C.c_void_p(out_ptr), int(layout),
                                              self._hdr_ptr(hdr_out, w, h), self._stream(stream)))
+        return out
+
+    def render_pano(self, prm: Params, cam: Camera, fx: Effects, sky: Sky | int, time: float, w: int, h: int, *, ss: int = 1,
+                    band: Optional[Band] = None, out=None, layout: int = OUT_FRAME, planes: Optional[dict] = None,
+                    stream: Optional[torch.cuda.Stream] = None) -> torch.Tensor:
+        """rrt_render_pano: a 360 x 180 degree equirectangular frame (or band) of everything around ``cam.pos``;
+        asynchronous.  Column x looks at longitude 2 pi ((x + 0.5)/w - 0.5) from ``cam.forward`` towards ``cam.right``,
+        row y at latitude pi ((y + 0.5)/h - 0.5) towards ``cam.up``, so the frame's first row (``layout`` OUT_FRAME) is the
+        zenith.  Pixel (x, y) traces the ray of ``render`` at pixel (1, 1) of a 2 x 2 frame with forward =
+        ``pano_directions(cam, w, h)[y, x]``.  ss = 1: ``planes`` (any of the seven), ``band``, ``out`` and ``layout`` as in
+        ``render``.  ss = 2..8: the ss*w x ss*h panorama box-filtered like ``render_ss`` (no sub-pixel shift: sub-samples
+        sit at the large panorama's pixel centres); ``planes`` may hold only "hdr" (h, w, 4), the mean.  ``fx`` must have
+        the lens distortion off."""
+        out, out_ptr = self._frame_out(out, layout, band, w, h)
+        pl = self._planes(planes, w, h) if planes else None
+        self._check(self._lib.rrt_render_pano(self._ctx, C.byref(prm), C.byref(cam), C.byref(fx), _tex(sky), float(time),
+                                              int(w), int(h), int(ss), _band_ref(band), C.c_void_p(out_ptr), int(layout),
+                                              C.byref(pl) if pl is not None else None, self._stream(stream)))
         return out
 
     def resolve(self, prm: Params, fx: Effects, hdr_hi: torch.Tensor, ss: int, w: int, h: int, *, band: Optional[Band] = None,
